@@ -19,6 +19,9 @@ the same two measurements for the split-bf16 mode ("bf16x3": the tensor-core num
 random-init weights, 3x the MMAs), the other BASELINE configs as extra keys -- "c2_rules" (2^20 playouts), "c4_stress"
 (4096 trees x 800 simulations, throughput mode) -- and "cycle": BASELINE config 5's self-play stage (4096 games per GPU,
 weight broadcast + packed history gather to rank 0 over NCCL when N > 1).  `--numerics bf16x3` makes bf16x3 the line itself.
+
+`--dump-outputs DIR` writes the history of rank 0's last timed step (see dump_outputs) so that two builds can be compared
+output for output: the model, the seeds and the game indices depend on the arguments only.
 """
 import argparse
 import json
@@ -28,6 +31,8 @@ import sys
 import threading
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "ultimate-tictactoe-alphazero_b200")
 for p in (PKG, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
@@ -36,6 +41,7 @@ for p in (PKG, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
 
 TRUNK_FLOP_PER_POSITION = 32 * 2 * 81 * 128 * 1152          # SURVEY 8(d): 764,411,904 (dense 3x3 convs)
 NET_FLOP_PER_POSITION = 765102212
+DUMP_LIMIT_BYTES = 60 << 20                          # --dump-outputs: below 64 MB with the .npy headers
 
 
 def measured_peaks():
@@ -109,7 +115,6 @@ def run_reference(args, rank):
     torch.set_num_threads(cores)
     torch.manual_seed(0)
     from dual_network import DualNetwork
-    import numpy as np
     try:
         ref = cpu_selfplay.load_reference_module()
         kind = "reference"
@@ -150,6 +155,29 @@ class Ctx:
     pass
 
 
+def dump_outputs(out_dir, hist, stats):
+    """Write a History of self-play games and the run's stats [plies, sims, evals, rounds] as out_dir/<name>.npy: integers
+    below 2^24 as float32, packed states (uint32 words) and stats as float64.  Plies past a game's length hold whatever
+    earlier runs left in the engine's buffers and are written as zeros.  Above DUMP_LIMIT_BYTES a fixed seeded sample of
+    the games is written; `game` holds their indices within the step."""
+    n = hist.n_games
+    per_game = 81 * 8 * 8 + 81 * 81 * 4 + 81 * 4 + 3 * 8
+    games = np.arange(n)
+    if n * per_game > DUMP_LIMIT_BYTES:
+        games = np.sort(np.random.RandomState(0).choice(n, DUMP_LIMIT_BYTES // per_game, replace=False))
+    live = np.arange(81)[None, :] < hist.lens[games, None]
+    arrays = {"game": games.astype(np.float64), "lens": hist.lens[games].astype(np.float32),
+              "final": hist.final[games].astype(np.float32),
+              "actions": np.where(live, hist.actions[games], 0).astype(np.float32),
+              "counts": np.where(live[:, :, None], hist.counts[games], 0).astype(np.float32),
+              "states": np.where(live[:, :, None], hist.states[games], 0).astype(np.float64),
+              "stats": np.asarray(stats, dtype=np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return arrays
+
+
 def timed_selfplay(c, eng, ev_kind, steps, warmup, games, seed0):
     """device-resident leg: CUDA events on the launching stream around every cycle -> dict of rank-local sums"""
     import torch
@@ -173,6 +201,7 @@ def timed_selfplay(c, eng, ev_kind, steps, warmup, games, seed0):
         e1.record(c.stream)
         e1.synchronize()
         out["dev_ms"] += e0.elapsed_time(e1)
+        out["last_stats"] = st
         out["plies"] += int(st[0]); out["sims"] += int(st[1]); out["evals"] += int(st[2]); out["rounds"] += int(st[3])
         prof = eng.last_run_profile()
         tt = prof["trunk_timed"]
@@ -334,7 +363,13 @@ def main():
                     help="also time one cycle of this many concurrent games per GPU (0 = skip)")
     ap.add_argument("--cycle-games", type=int, default=4096, help="games per GPU of the config-5 cycle leg (0 = skip)")
     ap.add_argument("--no-extras", action="store_true", help="skip the bf16x3 / c2 / c4 / cycle legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the history of rank 0's last timed step as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the B200 engine's history; the reference arm has none")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -344,7 +379,6 @@ def main():
         run_reference(args, rank)
         return
 
-    import numpy as np  # noqa: F401
     import torch
     import torch.distributed as dist
     import engine
@@ -392,6 +426,8 @@ def main():
     leg = timed_selfplay(c, eng, ev_kind, args.steps, 0, args.games, 0)
     wall_s = time.perf_counter() - t_wall0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng.selfplay_fetch(args.games), leg["last_stats"])
     dev_ms, plies, evals, rounds = leg["dev_ms"], leg["plies"], leg["evals"], leg["rounds"]
     trunk_ms, trunk_launches, trunk_evals = leg["trunk_ms"], leg["trunk_launches"], leg["trunk_evals"]
     # diagnostic, outside the timed region: one more cycle with every kernel bracketed by events (level 2 costs ~1.5 %
@@ -413,7 +449,7 @@ def main():
     # ---------------- the same two measurements with split-bf16 numerics (the mode that meets the 1e-2 parity bar)
     x3 = None
     if args.numerics == "bf16" and not args.no_extras:
-        k3 = max(2, min(args.steps, 3))
+        k3 = args.steps
         leg3 = timed_selfplay(c, eng, engine.EVAL_NET_BF16X3, k3, 3, args.games, 50)
         p3, s3 = timed_e2e(c, eng, engine.EVAL_NET_BF16X3, k3, args.games, hist)
         (d3, es3), (pl3, _, ev3, ep3, _) = reduce_leg(c, leg3, p3, s3)

@@ -7,8 +7,16 @@ Every array below is an output of the reference's own UTTT::State / UTTT::pv_mct
 (cpp/uttt_game.cpp, cpp/uttt_mcts.cpp) driven through oracle/ref_harness.cpp with
 deterministic inputs (Philox playouts, integer-hash evaluator).  The vectors pin
 oracle/uttt_oracle.c (CPU tests) and the CUDA library (GPU tests).
+
+Two generators read the reference's Python files instead, from the directory given on the command line, and record that
+directory's name as `source`:
+    python oracle/gen_golden.py --trainer DIR               -> trainer.npz: DIR/train_network.py on the inputs of
+                                                               tests/test_train_cpu.py
+    python oracle/gen_golden.py --train-cycle-imports DIR   -> train_cycle_imports.json: the import block of DIR/train_cycle.py
 """
+import ast
 import ctypes as C
+import json
 import os
 import sys
 
@@ -259,7 +267,44 @@ def gen_pymcts():
     print("pymcts.npz:", len(states), "states,", len(cases), "cases (numpy %s)" % np.__version__)
 
 
+def gen_trainer(ref_dir):
+    """weights and epoch lines of DIR/train_network.py on tests/test_train_cpu.py's inputs (2 epochs of 200 synthetic
+    samples from a seed-0 best.pth, torch seed 123, 4 threads, on the CPU): a SHA-256 per state_dict tensor, plus the
+    values at 8 seeded positions of each tensor so that a mismatch shows its size"""
+    import tempfile
+    import torch
+    import test_train_cpu as T
+    with tempfile.TemporaryDirectory() as d:
+        sd, lines = T.run_recorded_case(d, os.path.abspath(ref_dir))
+    rng = np.random.RandomState(0)
+    idx = np.stack([rng.randint(0, v.numel(), 8) for v in sd.values()])
+    vals = np.stack([v.reshape(-1)[torch.from_numpy(i)].double().numpy() for v, i in zip(sd.values(), idx)])
+    np.savez_compressed(os.path.join(OUT, "trainer.npz"), names=np.array(list(sd.keys())), sha256=np.array(T.digests(sd)),
+                        sample_idx=idx, sample_val=vals, epoch_lines=np.array(lines), torch_version=np.array(torch.__version__),
+                        source=np.array("train_network.py of " + os.path.basename(os.path.abspath(ref_dir))))
+    print("trainer.npz:", lines)
+
+
+def gen_train_cycle_imports(ref_dir):
+    """(module, name) of every import in DIR/train_cycle.py (name None for `import module`)"""
+    wanted = []
+    for node in ast.walk(ast.parse(open(os.path.join(ref_dir, "train_cycle.py"), encoding="utf-8-sig").read())):
+        if isinstance(node, ast.ImportFrom):
+            wanted += [[node.module, a.name] for a in node.names]
+        elif isinstance(node, ast.Import):
+            wanted += [[a.name, None] for a in node.names]
+    with open(os.path.join(OUT, "train_cycle_imports.json"), "w") as f:
+        json.dump({"source": "train_cycle.py of " + os.path.basename(os.path.abspath(ref_dir)), "imports": wanted}, f, indent=1)
+    print("train_cycle_imports.json:", wanted)
+
+
 if __name__ == "__main__":
+    if "--trainer" in sys.argv:
+        gen_trainer(sys.argv[sys.argv.index("--trainer") + 1])
+        sys.exit(0)
+    if "--train-cycle-imports" in sys.argv:
+        gen_train_cycle_imports(sys.argv[sys.argv.index("--train-cycle-imports") + 1])
+        sys.exit(0)
     if not O.ref_available():
         sys.exit("oracle/_ref is not built: run `make -C oracle ref` where /root/reference exists")
     os.makedirs(OUT, exist_ok=True)
