@@ -311,9 +311,9 @@ def test_fp32_trunk_vs_reference_golden_outputs(setup, golden_dir):
     assert (pb.argmax(1) == g["policy"].argmax(1)).mean() >= 0.9
 
 
-def test_trunk_variant_boundaries_give_identical_rows(setup, monkeypatch):
+def test_trunk_variant_boundaries_give_identical_rows(setup):
     """The trunk kernel is chosen on the device from the batch size and the group sizes from ceil(n / pairs): every
-    boundary of that dispatch must produce the same rows.  Default (UTTT_TRUNK=4, one launch that branches on the device,
+    boundary of that dispatch must produce the same rows.  One launch that branches on the device (trunk_auto_kernel,
     net_auto.cu): one group per CTA pair up to 370 positions (net_tc2: cta_group::2 MMAs with per-CTA weight halves up to 148
     positions = one tile per CTA, cta_group::1 MMAs above), two groups in flight above (net_pp, cta_group::2).  All of them accumulate a row in the
     same order: bit-identical rows -- including the one-tile group of the 6/7-positions-per-pair case (371..518
@@ -354,16 +354,6 @@ def test_trunk_variant_boundaries_give_identical_rows(setup, monkeypatch):
                     assert (p == ref_n[n][0]).all() and (v == ref_n[n][1]).all(), (rows, n)
         finally:
             ef.close()
-    # UTTT_TRUNK=3: the same two kernels as separate launches (each exits if the batch is not in its range)
-    monkeypatch.setenv("UTTT_TRUNK", "3")
-    ev = engine.Engine(n_slots=800, max_sims=50, max_batch=8, max_games=8)
-    try:
-        ev.upload_model(model)
-        for n in same_n:
-            p, v = _forward(ev, big[:n], engine.EVAL_NET_BF16)
-            assert (p == ref_n[n][0]).all() and (v == ref_n[n][1]).all(), n
-    finally:
-        ev.close()
 
 
 def test_state_dict_upload_paths_give_identical_networks(setup):

@@ -1,5 +1,4 @@
-"""Device time of the 500-game cycle (BASELINE config 3) at a given per-kernel event level: python tools/cycle_time.py [level] [steps] [numerics]
-(environment knobs such as UTTT_PDL are read by the library at its first launch: one process per setting)"""
+"""Device time of the 500-game cycle (BASELINE config 3) at a given per-kernel event level: python tools/cycle_time.py [level] [steps] [numerics]"""
 import os
 import sys
 
@@ -30,6 +29,6 @@ for i in range(steps):
     ms.append(e0.elapsed_time(e1))
     plies += int(st[0])
 prof = e.last_run_profile()
-print("UTTT_PDL=%s level=%d games=%d: %.2f ms/cycle (min %.2f), %.0f moves/s, rounds %d, trunk %.2f ms" % (
-    os.environ.get("UTTT_PDL", "default"), level, games, sum(ms) / len(ms), min(ms), plies / (sum(ms) / 1e3), int(st[3]), prof["trunk"][0]))
+print("level=%d games=%d: %.2f ms/cycle (min %.2f), %.0f moves/s, rounds %d, trunk %.2f ms" % (
+    level, games, sum(ms) / len(ms), min(ms), plies / (sum(ms) / 1e3), int(st[3]), prof["trunk"][0]))
 e.close()

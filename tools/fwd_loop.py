@@ -21,5 +21,5 @@ for _ in range(reps):
     e.net_forward(d, MODE)
 t1.record(); torch.cuda.synchronize()
 us = 1e3 * t0.elapsed_time(t1) / reps
-print("n=%d  %s  %.1f us per forward = %.0f TFLOP/s useful (gather + trunk + heads + 2 copies; UTTT_TRUNK=%s)" % (
-    n, numerics, us, n * 764411904 / us / 1e6, os.environ.get("UTTT_TRUNK", "")))
+print("n=%d  %s  %.1f us per forward = %.0f TFLOP/s useful (gather + trunk + heads + 2 copies)" % (
+    n, numerics, us, n * 764411904 / us / 1e6))

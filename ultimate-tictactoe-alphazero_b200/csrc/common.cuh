@@ -35,8 +35,7 @@ static inline int ceil_div(int64_t a, int64_t b) { return (int)((a + b - 1) / b)
 // one's output from its first instruction, but its blocks can be scheduled and resident while the previous kernel drains,
 // which hides the launch latency of the boundary).  A kernel launched through launch_pdl may start before its predecessor
 // in the stream has finished: it must execute pdl_wait() before touching anything the predecessor writes, and may call
-// pdl_trigger() to let its own successor be scheduled early.  UTTT_PDL=0 turns the attribute off (plain stream order).
-bool pdl_enabled();
+// pdl_trigger() to let its own successor be scheduled early.
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
@@ -47,7 +46,7 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 #endif
@@ -190,26 +189,20 @@ cudaError_t launch_heads_fc(const NetWeights& w, const float* headfeat, const in
 cudaError_t launch_heads(const NetWeights& w, const float* act_f32, const __nv_bfloat16* act_bf16,
                          const int32_t* count, int max_rows, float* policy, float* value, int row_stride,
                          cudaStream_t s);
-// cluster-of-2 variant (net_tc2.cu): one group of positions per CTA pair; skip: [n_sm][16][256] fp16x8
+// split-bf16 numerics (UTTT_EVAL_NET_BF16X3, net_tc2.cu): any batch size in one launch; skip: [n_sm][16][256] fp32x8
 cudaError_t trunk_tc2_init();
-// split-bf16 numerics (UTTT_EVAL_NET_BF16X3): any batch size in one launch; skip: [n_sm][16][256] fp32x8
 cudaError_t launch_trunk_x3(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count,
                             int max_rows, float* skip, int n_sm, cudaStream_t s, long long* dbg);
-// batches up to trunk_tc2_small_capacity (one group of <= 5 positions per CTA pair); larger ones go to launch_trunk_pp
-cudaError_t launch_trunk_tc2_small(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count,
-                                   int max_rows, float* skip, int n_sm, cudaStream_t s, long long* dbg);
-int trunk_tc2_small_capacity(int n_sm);
-// two groups of positions per CTA pair in flight (net_pp.cu): batches of more than min_count positions
+// cta_group::2 weight halves (net_pp.cu)
 // (subs = 16-byte-unit blocks per K-block: 1, or 2 for the split-bf16 arrays whose blocks are a hi and a lo part)
 cudaError_t launch_split_weights_2sm(const __nv_bfloat16* src, __nv_bfloat16* dst, int n_blocks, int blocks_per_stage, cudaStream_t s,
                                      int subs = 1);
-cudaError_t launch_trunk_pp(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count, int max_rows,
-                            float* skip, int n_sm, cudaStream_t s, long long* dbg, int min_count);
+// two groups of positions per CTA pair in flight (net_pp.cu): batches of more than trunk_pp_cap1 positions
 cudaError_t trunk_pp_init();
-int trunk_pp_cap1(int n_sm);         // largest batch of the 7-positions-per-pair instantiation
+int trunk_pp_cap1(int n_sm);         // largest batch of trunk_auto_kernel (7 positions per CTA pair)
 cudaError_t launch_trunk_pp_large(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count,
                                   int max_rows, float* skip, int n_sm, cudaStream_t s, long long* dbg);
-// one launch for every batch up to trunk_pp_cap1: device-side choice between trunk_tc2_kernel<2> and trunk_pp_kernel<1>
+// one launch for every batch up to trunk_pp_cap1: device-side choice between the bodies of net_tc2_kernel.cuh and net_pp_kernel.cuh
 // (policy / value non-null: the heads' FC layers run in the kernel's tail; requires max_rows <= trunk_pp_cap1)
 cudaError_t launch_trunk_auto(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count, int max_rows,
                               float* skip, int n_sm, cudaStream_t s, long long* dbg, float* policy, float* value,

@@ -95,9 +95,6 @@ struct uttt_engine {
     int prof_sample;        // level 1: the trunk is bracketed in every prof_sample-th window of rounds only (see uttt_set_profile_level)
     int64_t prof_sampled_launches, prof_sampled_evals;      // trunk launches with events in the last run, positions they evaluated
     int lane_threshold;     // slots from which self-play splits into two overlapped lanes
-    int trunk_variant;      // 4 (default): CTA pair per group (net_tc2) up to 370 positions, two groups in flight per pair with
-                            // cta_group::2 MMAs (net_pp) above, chosen on the device inside ONE launch (net_auto.cu); 3 (kept
-                            // for comparison): the same two bodies as separate launches
     NetWeights w;
     float* raw_res;         // staging for the raw residual conv weights / bn of an upload
     float* raw_res_bn;
@@ -189,28 +186,17 @@ int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_
         // conv_input runs inside the trunk kernels (tensor pipe, "layer -1").  The queue length is only known on the
         // device: small batches (one wave of CTA pairs) are latency-bound -> one group per pair with the next layer
         // overlapping the epilogue, larger ones are throughput-bound -> two groups in flight with cta_group::2 MMAs.
-        // Variant 4 makes that choice inside one launch; the older variants enqueue one kernel per range and the ones
-        // that do not match exit at once.  Counted as ONE trunk launch per round.
+        // trunk_auto_kernel makes that choice inside one launch (net_auto.cu).  Counted as ONE trunk launch per round.
         if (ev3) cudaEventRecord(ev3[0], s);
-        if (e->trunk_variant == 4) {
-            // one launch: the kernel branches on the queue length (net_auto.cu); batches above 7 positions per CTA pair
-            // (only possible when max_rows allows them) are left to the 10-positions-per-pair instantiation
-            // (if no batch can exceed one group per pair, the heads' FC layers run in the tail of the same kernel)
-            heads_fused = max_rows <= trunk_pp_cap1(e->n_sm);
-            UTTT_CHECK(heads_fused || !b.slot_flags, "slot mode needs the fused heads");
-            UTTT_CUDA_OK(launch_trunk_auto(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg,
-                                           heads_fused ? b.policy : nullptr, heads_fused ? b.value : nullptr, b.slot_flags,
-                                           b.n_slots));
-            if (!heads_fused)
-                UTTT_CUDA_OK(launch_trunk_pp_large(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg));
-        } else {
-            // UTTT_TRUNK=3 (comparison): up to one wave of 5-position groups: cluster kernel whose next layer overlaps the epilogue; above: the
-            // two-groups-in-flight kernel (net_pp.cu)
-            const int cap = trunk_tc2_small_capacity(e->n_sm);
-            UTTT_CUDA_OK(launch_trunk_tc2_small(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg));
-            if (max_rows > cap)
-                UTTT_CUDA_OK(launch_trunk_pp(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg, cap));
-        }
+        // batches above 7 positions per CTA pair (only possible when max_rows allows them) are left to the
+        // 10-positions-per-pair kernel; if no batch can exceed that, the heads' FC layers run in the tail of trunk_auto_kernel
+        heads_fused = max_rows <= trunk_pp_cap1(e->n_sm);
+        UTTT_CHECK(heads_fused || !b.slot_flags, "slot mode needs the fused heads");
+        UTTT_CUDA_OK(launch_trunk_auto(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg,
+                                       heads_fused ? b.policy : nullptr, heads_fused ? b.value : nullptr, b.slot_flags,
+                                       b.n_slots));
+        if (!heads_fused)
+            UTTT_CUDA_OK(launch_trunk_pp_large(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg));
         e->prof_launches[1] += 1;
     } else {
         UTTT_CHECK(false, "evaluator %d cannot run on the device", evaluator);
@@ -275,9 +261,7 @@ int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const in
 // Slot mode (net_auto.cu: reproducible runs with the split-K group of the large-batch trunk): the reference-exact search
 // with the tensor-core evaluator, when one trunk_auto_kernel launch with fused heads covers every possible batch.
 bool slot_mode_applies(uttt_engine* e, int evaluator, bool throughput, int rows) {
-    static const bool enabled = !(getenv("UTTT_SLOT_MODE") && atoi(getenv("UTTT_SLOT_MODE")) == 0);
-    return enabled && evaluator == UTTT_EVAL_NET_BF16 && !throughput && e->trunk_variant == 4 && rows <= trunk_pp_cap1(e->n_sm) &&
-           rows <= 544;
+    return evaluator == UTTT_EVAL_NET_BF16 && !throughput && rows <= trunk_pp_cap1(e->n_sm) && rows <= 544;
 }
 
 int check_search_args(uttt_engine* e, int n_roots, int sims, int batch) {
@@ -307,7 +291,6 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     e->trace_on = false;
     e->progress_cb = nullptr;
     e->progress_user = nullptr;
-    e->trunk_variant = getenv("UTTT_TRUNK") ? atoi(getenv("UTTT_TRUNK")) : 4;
     e->prof_level = getenv("UTTT_PROFILE") ? atoi(getenv("UTTT_PROFILE")) : 1;
     e->prof_sample = getenv("UTTT_PROFILE_SAMPLE") ? atoi(getenv("UTTT_PROFILE_SAMPLE")) : 4;
     if (e->prof_sample < 1) e->prof_sample = 1;

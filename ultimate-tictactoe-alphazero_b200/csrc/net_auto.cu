@@ -1,21 +1,21 @@
-// net_auto.cu -- trunk_auto_kernel: ONE launch per evaluator round.  The queue length is only known on the device, so
-// the engine used to enqueue both trunk kernels every round and the one whose range did not contain the batch size
-// exited at once; an exit still costs a full kernel boundary (3.4 us under ncu, ~6 us between dependent launches).
-// Here the bodies sit behind one device-side branch on *count: batches of up to one wave of 5-position groups run
-// tc2::trunk_tc2_body<2> (next layer overlaps the epilogue) -- with cta_group::2 MMAs while a CTA owns a single accumulator
-// tile (up to 2 positions per pair: 128 -> 147 us per forward, the tile's cta_group::1 MMAs saturate shared memory and the
+// net_auto.cu -- trunk_auto_kernel: ONE launch per evaluator round.  The queue length is only known on the device, and a
+// kernel that exits at once still costs a full kernel boundary (3.4 us under ncu, ~6 us between dependent launches), so
+// the bodies sit behind one device-side branch on the batch size: batches of up to one wave of 5-position groups run
+// tc2::trunk_tc2_body (next layer overlaps the epilogue) -- with cta_group::2 MMAs while a CTA owns a single accumulator
+// tile (up to 2 positions per pair: 147 -> 128 us per forward, the tile's cta_group::1 MMAs saturate shared memory and the
 // weight stream slows them down; with two tiles per CTA the pair form measures the same as cta_group::1, which stays) --,
 // larger ones pp::trunk_pp_body<1> (two groups in flight, cta_group::2 MMAs).  All use 19 warps, clusters of two CTAs and
-// the same grid; shared memory is the largest footprint.  Batches above 7 positions per pair still get a second launch (pp<2>).
+// the same grid; shared memory is the largest footprint.  Batches above 7 positions per pair are left to a second launch,
+// trunk_pp_large_kernel (net_pp.cu).
 #include "heads_fc.cuh"
 #include "net_pp_kernel.cuh"
 #include "net_tc2_kernel.cuh"
 
 namespace uttt {
 
-static_assert(tc2::Cfg<2>::THREADS == pp::THREADS, "one block size for both bodies");
+static_assert(tc2::Cfg<>::THREADS == pp::THREADS, "one block size for both bodies");
 constexpr int max3(int a, int b, int c) { return a > b ? (a > c ? a : c) : (b > c ? b : c); }
-constexpr int AUTO_SMEM = max3(tc2::Cfg<2>::SMEM_BYTES, tc2::Cfg<2, false, true>::SMEM_BYTES, pp::Cfg<1>::SMEM_BYTES);
+constexpr int AUTO_SMEM = max3(tc2::Cfg<>::SMEM_BYTES, tc2::Cfg<false, true>::SMEM_BYTES, pp::Cfg<1>::SMEM_BYTES);
 static_assert(HEADS_SMEM_BYTES <= AUTO_SMEM, "the fused heads reuse the trunk's shared memory");
 
 // Slot mode.  With an atomic counter the leaves of a round land in the evaluator queue in arrival order, which differs
@@ -41,7 +41,7 @@ __device__ __forceinline__ void scan_slots(const uint8_t* __restrict__ flags, in
         bal[j] = __ballot_sync(0xFFFFFFFFu, (mine >> j) & 1u);
         n_pos += __popc(bal[j]);
     }
-    const int P = n_pos <= small_cap ? tc2::group_positions<2>(n_pos, n_pairs) : pp::pair_positions<1>(n_pos, n_pairs);
+    const int P = n_pos <= small_cap ? tc2::group_positions(n_pos, n_pairs) : pp::pair_positions<1>(n_pos, n_pairs);
     const int first = pair * P, last = min(n_pos, first + P);
     int run = 0;
 #pragma unroll
@@ -63,7 +63,7 @@ trunk_auto_kernel(const __nv_bfloat16* __restrict__ wq, const __nv_bfloat16* __r
                   const __nv_bfloat16* __restrict__ wq2, const __nv_bfloat16* __restrict__ wq2_in,
                   const __nv_bfloat16* __restrict__ wq2_bias,                     // per-CTA halves, 18-block stages (net_pp<1>)
                   const __nv_bfloat16* __restrict__ planes, const float* __restrict__ headw, float* headfeat, uint4* skip,
-                  const int32_t* __restrict__ count, int small_cap, int max_count, long long* dbg,
+                  const int32_t* __restrict__ count, int small_cap, int cap1, long long* dbg,
                   HeadsFC fc, float* policy, float* value /* null: the heads' FC layers are a separate kernel */,
                   const uint8_t* __restrict__ slot_flags, int n_slots /* slot mode (needs the fused heads), else null */,
                   const __nv_bfloat16* __restrict__ wq8, const __nv_bfloat16* __restrict__ wq8_in /* per-CTA halves in 8-block
@@ -86,19 +86,23 @@ trunk_auto_kernel(const __nv_bfloat16* __restrict__ wq, const __nv_bfloat16* __r
     }
     const int* src = slot_flags ? s_src : nullptr;
     const bool small = n_pos <= small_cap;
-    if (n_pos <= pair_cap)
-        tc2::trunk_tc2_body<2, false, true>(wq8, wq8_in, wq2_bias, planes, headw, headfeat, skip, count, 0, small_cap, dbg, n_pos, src);
-    else if (small)
-        tc2::trunk_tc2_body<2>(wq, wq_in, wq_bias, planes, headw, headfeat, skip, count, 0, small_cap, dbg, n_pos, src);
+    if (n_pos <= 0 || n_pos > cap1) return;        // (larger batches are trunk_pp_large_kernel's)
+    tcx::count_batch(dbg, n_pos);
+    // (with the statements above and the branches below in this order ptxas fits the kernel into 96 registers without
+    // spills; the other orders tried spill 32-64 bytes)
+    if (!small)
+        pp::trunk_pp_body<1>(wq2, wq2_in, wq2_bias, planes, headw, headfeat, skip, dbg, n_pos, src);
+    else if (n_pos > pair_cap)
+        tc2::trunk_tc2_body<false, false>(wq, wq_in, wq_bias, planes, headw, headfeat, skip, dbg, n_pos, src, 0, false);
     else
-        pp::trunk_pp_body<1>(wq2, wq2_in, wq2_bias, planes, headw, headfeat, skip, count, small_cap, max_count, dbg, n_pos, src);
+        tc2::trunk_tc2_body<false, true>(wq8, wq8_in, wq2_bias, planes, headw, headfeat, skip, dbg, n_pos, src, 0, false);
     if (stamp) dbg[201] = clock64();
-    if (policy == nullptr || n_pos > max_count) return;
+    if (policy == nullptr) return;
     // Fused heads (the host passes policy / value only if no batch can exceed one group per pair): the pair's head
     // features were written to global memory by both CTAs' last epilogues and ordered by the cluster barrier that ends
     // the body (release / acquire); they are read back with ld.global.cg.  The two CTAs take alternate positions of
     // the pair (at most 4 each); the body's shared memory is free now.
-    const int P = small ? tc2::group_positions<2>(n_pos, n_pairs) : pp::pair_positions<1>(n_pos, n_pairs);
+    const int P = small ? tc2::group_positions(n_pos, n_pairs) : pp::pair_positions<1>(n_pos, n_pairs);
     const int first = pair * P, last = min(n_pos, first + P);
     const int rank = (int)tcx::cluster_rank();
     const int row0 = first + rank;
@@ -122,15 +126,14 @@ cudaError_t launch_trunk_auto(const NetWeights& w, const __nv_bfloat16* planes, 
                               const uint8_t* slot_flags, int n_slots) {
     int pairs = n_sm / 2;
     if (max_rows < pairs) pairs = max_rows < 1 ? 1 : max_rows;
-    const int small_cap = (n_sm / 2) * tc2::Cfg<2>::MAX_P;
+    const int small_cap = (n_sm / 2) * tc2::Cfg<>::MAX_P;
     const int cap1 = (n_sm / 2) * (pp::Cfg<1>::MAX_PA + pp::Cfg<1>::MAX_PB);
-    static const bool one_tile_pair = !(getenv("UTTT_TC2_PAIR") && atoi(getenv("UTTT_TC2_PAIR")) == 0);   // (0: comparison runs)
     if (policy && max_rows > cap1) return cudaErrorInvalidValue;
     if (slot_flags && (!policy || n_slots > 32 * SLOT_CHUNKS || n_slots > max_rows)) return cudaErrorInvalidValue;
     return launch_pdl(trunk_auto_kernel, dim3(2 * pairs), dim3(pp::THREADS), AUTO_SMEM_TOTAL, s, w.res_w_bf16, w.conv_in_w_bf16,
                       w.bias_blk, w.res_w_2sm18, w.conv_in_w_2sm18, w.bias_blk_2sm, planes, w.head_w, headfeat,
                       reinterpret_cast<uint4*>(skip), count, small_cap, cap1, dbg, heads_fc_of(w), policy, value, slot_flags, n_slots,
-                      w.res_w_2sm, w.conv_in_w_2sm, one_tile_pair ? 2 * (n_sm / 2) : 0);
+                      w.res_w_2sm, w.conv_in_w_2sm, 2 * (n_sm / 2));
 }
 
 }  // namespace uttt

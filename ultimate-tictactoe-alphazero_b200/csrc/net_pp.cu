@@ -1,23 +1,25 @@
-// net_pp.cu -- __global__ wrappers and launchers of trunk_pp_kernel (body: net_pp_kernel.cuh), weight splitting for the
-// cta_group::2 B operand
+// net_pp.cu -- trunk_pp_large_kernel, the large-batch form of the two-groups-in-flight trunk (body: net_pp_kernel.cuh), and
+// the weight splitting for the cta_group::2 B operand
 #include "net_pp_kernel.cuh"
 
 namespace uttt {
 namespace pp {
 
-template <int LTB>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
-trunk_pp_kernel(const __nv_bfloat16* __restrict__ wq,
-                const __nv_bfloat16* __restrict__ wq_in,
-                const __nv_bfloat16* __restrict__ wq_bias,
-                const __nv_bfloat16* __restrict__ planes,
-                const float* __restrict__ headw,
-                float* headfeat,
-                uint4* skip,
-                const int32_t* __restrict__ count,
-                int min_count, int max_count,
-                long long* dbg) {
-    trunk_pp_body<LTB>(wq, wq_in, wq_bias, planes, headw, headfeat, skip, count, min_count, max_count, dbg);
+trunk_pp_large_kernel(const __nv_bfloat16* __restrict__ wq,
+                      const __nv_bfloat16* __restrict__ wq_in,
+                      const __nv_bfloat16* __restrict__ wq_bias,
+                      const __nv_bfloat16* __restrict__ planes,
+                      const float* __restrict__ headw,
+                      float* headfeat,
+                      uint4* skip,
+                      const int32_t* __restrict__ count,
+                      int cap1,                     // trunk_pp_cap1: smaller batches are trunk_auto_kernel's
+                      long long* dbg) {
+    const int n_pos = *count;
+    if (n_pos <= cap1) return;
+    count_batch(dbg, n_pos);
+    trunk_pp_body<2>(wq, wq_in, wq_bias, planes, headw, headfeat, skip, dbg, n_pos, nullptr);
 }
 
 }  // namespace pp
@@ -43,38 +45,17 @@ cudaError_t launch_split_weights_2sm(const __nv_bfloat16* src, __nv_bfloat16* ds
 }
 
 cudaError_t trunk_pp_init() {
-    cudaError_t e = cudaFuncSetAttribute(pp::trunk_pp_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, pp::Cfg<1>::SMEM_BYTES);
-    if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(pp::trunk_pp_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, pp::Cfg<2>::SMEM_BYTES);
+    return cudaFuncSetAttribute(pp::trunk_pp_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pp::Cfg<2>::SMEM_BYTES);
 }
 
-// Evaluator batches of more than min_count positions (smaller ones belong to launch_trunk_tc2_small).  Two instantiations
-// are enqueued, the queue length read on the device selects one: up to 7 positions per pair -> group B has one tile per
-// CTA and the weight ring six stages; more -> two tiles and four stages.
-cudaError_t launch_trunk_pp(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count, int max_rows,
-                            float* skip, int n_sm, cudaStream_t s, long long* dbg, int min_count) {
-    int pairs = n_sm / 2;
-    if (max_rows < pairs) pairs = max_rows < 1 ? 1 : max_rows;
-    const int cap1 = (n_sm / 2) * (pp::Cfg<1>::MAX_PA + pp::Cfg<1>::MAX_PB);
-    pp::trunk_pp_kernel<1><<<2 * pairs, pp::THREADS, pp::Cfg<1>::SMEM_BYTES, s>>>(
-        w.res_w_2sm18, w.conv_in_w_2sm18, w.bias_blk_2sm, planes, w.head_w, headfeat, reinterpret_cast<uint4*>(skip), count, min_count,
-        cap1, dbg);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess || max_rows <= cap1) return e;
-    pp::trunk_pp_kernel<2><<<2 * pairs, pp::THREADS, pp::Cfg<2>::SMEM_BYTES, s>>>(
-        w.res_w_2sm, w.conv_in_w_2sm, w.bias_blk_2sm, planes, w.head_w, headfeat, reinterpret_cast<uint4*>(skip), count, cap1,
-        0x7FFFFFFF, dbg);
-    return cudaGetLastError();
-}
-
-// only the 10-positions-per-pair instantiation: batches above trunk_pp_cap1 (what launch_trunk_auto leaves over)
+// batches above trunk_pp_cap1 (what launch_trunk_auto leaves over): super-groups of up to 10 positions per CTA pair
 cudaError_t launch_trunk_pp_large(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count,
                                   int max_rows, float* skip, int n_sm, cudaStream_t s, long long* dbg) {
     int pairs = n_sm / 2;
     if (max_rows < pairs) pairs = max_rows < 1 ? 1 : max_rows;
-    pp::trunk_pp_kernel<2><<<2 * pairs, pp::THREADS, pp::Cfg<2>::SMEM_BYTES, s>>>(
+    pp::trunk_pp_large_kernel<<<2 * pairs, pp::THREADS, pp::Cfg<2>::SMEM_BYTES, s>>>(
         w.res_w_2sm, w.conv_in_w_2sm, w.bias_blk_2sm, planes, w.head_w, headfeat, reinterpret_cast<uint4*>(skip), count,
-        trunk_pp_cap1(n_sm), 0x7FFFFFFF, dbg);
+        trunk_pp_cap1(n_sm), dbg);
     return cudaGetLastError();
 }
 

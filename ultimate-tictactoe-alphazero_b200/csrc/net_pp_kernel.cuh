@@ -1,6 +1,7 @@
-// net_pp_kernel.cuh -- trunk_pp_kernel: the residual trunk with two independent groups of positions in flight per CTA
-// pair and cta_group::2 MMAs.  The default for evaluator batches above one wave of 5-position groups (370 positions on
-// 148 SMs); smaller batches run trunk_tc2_kernel<2> (net_tc2_kernel.cuh).
+// net_pp_kernel.cuh -- trunk_pp_body: the residual trunk with two independent groups of positions in flight per CTA
+// pair and cta_group::2 MMAs.  It runs evaluator batches above one wave of 5-position groups (370 positions on 148 SMs):
+// up to 7 positions per pair inside trunk_auto_kernel (net_auto.cu), more in trunk_pp_large_kernel (net_pp.cu); smaller
+// batches run tc2::trunk_tc2_body (net_tc2_kernel.cuh).
 //
 // A thread-block cluster of two CTAs (as in net_tc2_kernel.cuh: positions padded to 100 GEMM rows, a group's rows split
 // between the two CTAs, 11 halo rows exchanged at the split) alternates between two groups layer by layer:
@@ -104,7 +105,8 @@ __host__ __device__ inline int pair_positions(int n_pos, int n_pairs) {
     return P < 1 ? 1 : (P > Cfg<LTB>::MAX_PA + Cfg<LTB>::MAX_PB ? Cfg<LTB>::MAX_PA + Cfg<LTB>::MAX_PB : P);
 }
 
-// the kernel body (see net_tc2_kernel.cuh); __global__ wrappers in net_pp.cu, device-side dispatch in net_auto.cu
+// the kernel body (see net_tc2_kernel.cuh): trunk_pp_large_kernel (net_pp.cu) runs LTB = 2, trunk_auto_kernel (net_auto.cu)
+// LTB = 1.  The caller has read the batch size and counted it (count_batch).
 template <int LTB>
 __device__ __forceinline__ void trunk_pp_body(const __nv_bfloat16* __restrict__ wq,        // [32 * STAGES_PER_LAYER stages][2 ranks][STAGE_BLOCKS K-blocks][2][64][8] bf16
                 const __nv_bfloat16* __restrict__ wq_in,     // conv_input: [IN_STAGES][2 ranks][STAGE_BLOCKS tap slots][2][64][8] bf16
@@ -113,11 +115,10 @@ __device__ __forceinline__ void trunk_pp_body(const __nv_bfloat16* __restrict__ 
                 const float* __restrict__ headw,             // [3][128] policy conv (2) + value conv; [384..386] shifts
                 float* headfeat,                             // out: [rows][243]
                 uint4* skip,                                 // [gridDim][NG][16 panels][256 rows] fp16x8 skip connection
-                const int32_t* __restrict__ count,
-                int min_count, int max_count,                // this launch handles min_count < batch <= max_count
                 long long* dbg,
-                int n_pos_known = -1,                        // >= 0: the batch size (slot mode, see net_auto.cu)
-                const int* src_rows = nullptr) {             // slot mode: position i of this pair reads planes row src_rows[i]
+                int n_pos,                                   // the batch size
+                const int* src_rows) {                       // slot mode (net_auto.cu): position i of this pair reads planes row
+                                                             // src_rows[i], else null
     using C = Cfg<LTB>;
     constexpr int STAGES = C::STAGES, BAR_OFF = C::BAR_OFF, HEAD_OFF = C::HEAD_OFF, CONST_OFF = C::CONST_OFF,
                   STAGE_BLOCKS = C::STAGE_BLOCKS, STAGE_BYTES = C::STAGE_BYTES, STAGES_PER_LAYER = C::STAGES_PER_LAYER,
@@ -128,10 +129,6 @@ __device__ __forceinline__ void trunk_pp_body(const __nv_bfloat16* __restrict__ 
     const uint32_t rank = cluster_rank();
     const uint32_t peer = rank ^ 1u;
     const int n_pairs = (int)gridDim.x >> 1, pair = (int)blockIdx.x >> 1;
-    const int n_pos = n_pos_known >= 0 ? n_pos_known : *count;
-    if (n_pos <= min_count || n_pos > max_count) return;
-    if (dbg && blockIdx.x == 0 && threadIdx.x == 0)          // diagnostics: histogram of evaluator batch sizes (16 per bucket)
-        atomicAdd(reinterpret_cast<unsigned long long*>(dbg) + 128 + min(n_pos >> 4, 63), 1ull);
     const int Ptot = pair_positions<LTB>(n_pos, n_pairs);     // positions per pair and super-group
     const int n_super = (n_pos + Ptot - 1) / Ptot;
     if (pair >= n_super) return;                              // both CTAs of the pair take the same branch

@@ -1,21 +1,23 @@
-// net_tc2_kernel.cuh -- trunk_tc2_kernel (wrappers + launchers: net_tc2.cu): the residual trunk as a tcgen05 implicit GEMM where a thread-block
-// CLUSTER of two CTAs (two SMs) shares one group of positions, split by GEMM rows.
+// net_tc2_kernel.cuh -- trunk_tc2_body: the residual trunk as a tcgen05 implicit GEMM where a thread-block CLUSTER of two
+// CTAs (two SMs) shares one group of up to 5 positions, split by GEMM rows.  It runs inside trunk_auto_kernel (net_auto.cu:
+// bf16 batches of up to one wave of groups) and trunk_x3_kernel (net_tc2.cu: split-bf16, any batch).
 //
-// Same math and layouts as trunk_tc_kernel (net_tc.cu: padded 100-row positions, no-swizzle K-major A panels
-// resident in shared memory, bulk-copied pre-packed weights, TMEM accumulators, in-place epilogue), but the
-// up-to-4 accumulator tiles of a group are divided between the two CTAs of a cluster (2+2, 2+1, 1+1 or 1+0).
-// Per CTA that halves the serial work of a forward pass -- the self-play rounds are latency-bound at the
-// reference's 500-game cycle (about 345 queued leaves per round = 69 groups of 5: one CTA per group would
-// use 69 of 148 SMs, a CTA pair per group uses 138) -- and frees shared memory for an 8-stage weight ring.
+// Positions are padded to 100 GEMM rows; the activations stay in shared memory as no-swizzle K-major A panels, the
+// pre-packed weights arrive by bulk copies, the accumulators live in TMEM and the epilogue writes the next layer's input
+// in place.  The up-to-4 accumulator tiles of a group are divided between the two CTAs of a cluster (2+2, 2+1, 1+1 or
+// 1+0).  Per CTA that halves the serial work of a forward pass -- the self-play rounds are latency-bound at the
+// reference's 500-game cycle (about 345 queued leaves per round = 69 groups of 5: one CTA per group would use 69 of 148
+// SMs, a CTA pair per group uses 138).
 //
-// The only coupling between the two CTAs is the 11-row halo of the 3x3 taps at the split:
-//   * the epilogue warp that owns the last 11 rows of rank 0 (first 11 rows of rank 1) also stores them into
-//     the peer's lead (tail) margin through distributed shared memory (st.shared::cluster), then arrives on the
-//     peer's act_ready barrier of its boundary tile (mbarrier.arrive.release.cluster on a mapa address);
-//   * before it overwrites the peer's margin it waits until the peer's boundary-tile MMAs of the current
-//     layer have retired: the peer's issuer signals that with a multicast tcgen05.commit onto the
-//     `bnd_accum` barrier of THIS CTA.
-// Everything else (weights, accumulators, skip connection, barriers) is CTA-private.
+// The CTAs exchange the 11-row halo of the 3x3 taps at the split:
+//   * the epilogue warp that owns the last 11 rows of rank 0 (first 11 rows of rank 1) pushes them into the peer's lead
+//     (tail) margin with bulk shared->shared copies whose bytes complete on the peer's act_ready barrier of its boundary
+//     tile (the peer's boundary warp announces them with expect_tx);
+//   * before it overwrites the peer's margin it waits until the peer's boundary-tile MMAs of the current layer have
+//     retired: the peer's issuer signals that with a multicast tcgen05.commit onto the `bnd_accum` barrier of THIS CTA
+//     (PAIR: the commits of the pair MMAs arrive on both CTAs' accumulator barriers).
+// Without PAIR everything else (weights, accumulators, skip connection, barriers) is CTA-private; with PAIR the leader
+// issues the MMAs of both CTAs (see Cfg).
 //
 // Warp roles (19 warps): 0-15 epilogue (2 tiles x 4 TMEM lane quarters x 2 column halves -- the epilogue is
 // instruction-latency bound, so it wants warps, not wider threads), 16 weight producer, 17-18 MMA issuers.
@@ -33,7 +35,7 @@ constexpr int LEAD = 11;
 constexpr int GROUP_LAYERS = NET_LAYERS + 1;     // conv_input runs as layer -1 through the same pipeline
 constexpr uint32_t IDESC = tcx::IDESC_M128_N128_BF16;
 
-// LT = accumulator tiles per CTA.  LT=2: up to 5 positions per CTA pair (2+2 tiles), 4 weight stages of 32 KiB.
+// Two accumulator tiles per CTA (LOC_TILES): up to 5 positions per CTA pair (2+2 tiles), 4 weight stages of 32 KiB.
 // X3 = split-bf16 numerics ("bf16x3", UTTT_EVAL_NET_BF16X3): activations and weights are kept as bf16 hi + lo pairs
 // (lo = bf16(x - hi)) and every K-block costs three MMAs, hi*hi + lo*hi + hi*lo, accumulated in fp32 in TMEM; the skip
 // connection is kept in fp32.  That is ~16 mantissa bits per operand: the mode that meets the reference's fp32 forward
@@ -46,12 +48,11 @@ constexpr uint32_t IDESC = tcx::IDESC_M128_N128_BF16;
 // all the shared-memory bandwidth of an SM, so the weight stream (one-tile groups of the split-bf16 mode: 590 KB per layer)
 // and the epilogue's stores slow the tensor pipe down (tools/micro/mma_shapes.cu, DESIGN.md section 9); a pair MMA reads
 // 4 + 2 KiB per CTA.  Rows are bit-identical to the cta_group::1 form (same K-block order into the same accumulators).
-template <int LT, bool X3 = false, bool PAIR = false>
+template <bool X3 = false, bool PAIR = false>
 struct Cfg {
-    static_assert(LT == 2, "one instantiation: 2 tiles per CTA");
-    static constexpr int LOC_TILES = LT;
-    static constexpr int MAX_P = (LT == 2) ? 5 : 7;
-    static constexpr int AROWS = (LEAD + 128 * LT + 11 + 7) / 8 * 8;
+    static constexpr int LOC_TILES = 2;
+    static constexpr int MAX_P = 5;
+    static constexpr int AROWS = (LEAD + 128 * LOC_TILES + 11 + 7) / 8 * 8;
     static constexpr int PANEL_BYTES = AROWS * 16;
     static constexpr int ACT_PANELS = X3 ? 32 : 16;        // channel panels [ci/8][row][8] bf16 (X3: panels 16.. hold the lo parts)
     static constexpr int A_BYTES = (ACT_PANELS + 2) * PANEL_BYTES;      // + the constant panel pair of the bias MMA
@@ -68,19 +69,17 @@ struct Cfg {
     static constexpr int STAGES_PER_LAYER = 72 / STAGE_BLOCKS;
     static constexpr int IN_STAGES = (9 + STAGE_BLOCKS - 1) / STAGE_BLOCKS;   // conv_input: 9 taps x (K=16: 3 real channels) in IN_STAGES * STAGE_BLOCKS tap slots
     static constexpr int GROUP_STAGES = (IN_STAGES + 1) + NET_LAYERS * (STAGES_PER_LAYER + 1);   // every layer starts with its bias block
-    // LT = 2 has TMEM for two accumulators per tile (4 x 128 = 512 columns): the layers alternate between them, and the
-    // epilogue publishes its output per 16-column chunk (NQ act_ready barriers per tile), so the MMAs of layer L+1
-    // run while the epilogue of layer L is still converting the other chunks.  (LT = 3 has one spare accumulator only;
-    // giving it to tile 0 was measured and does not help: tiles 1 and 2 still wait for their whole epilogue.)
-    static constexpr int NQ = (LT == 2) ? 4 : 1;
+    // TMEM holds two accumulators per tile (4 x 128 = 512 columns): the layers alternate between them, and the epilogue
+    // publishes its output per 16-column chunk (NQ act_ready barriers per tile), so the MMAs of layer L+1 run while the
+    // epilogue of layer L is still converting the other chunks.
+    static constexpr int NQ = 4;
     static constexpr uint32_t ALT_COLS = 256u;                         // column offset of a tile's second accumulator
-    static __host__ __device__ constexpr bool two_accumulators(int) { return LT == 2; }
     static constexpr int BAR_OFF = A_BYTES + STAGES * STAGE_BYTES;
-    static constexpr int HEAD_OFF = BAR_OFF + 256;                 // [128*LT rows][4] floats: head partial sums
-    static constexpr int SMEM_BYTES = HEAD_OFF + 128 * LT * 16;
-    static constexpr int EPI_WARPS = 8 * LT;         // (tile, lane quarter, column half)
-    static constexpr int THREADS = (EPI_WARPS + 1 + LT) * 32;
-    static constexpr int SKIP_ROWS = 128 * LT;
+    static constexpr int HEAD_OFF = BAR_OFF + 256;                 // [128*LOC_TILES rows][4] floats: head partial sums
+    static constexpr int SMEM_BYTES = HEAD_OFF + 128 * LOC_TILES * 16;
+    static constexpr int EPI_WARPS = 8 * LOC_TILES;  // (tile, lane quarter, column half)
+    static constexpr int THREADS = (EPI_WARPS + 1 + LOC_TILES) * 32;
+    static constexpr int SKIP_ROWS = 128 * LOC_TILES;
     static constexpr int SKIP_U4 = X3 ? 2 : 1;             // 16-byte units per (panel, row) of the skip buffer: 8 fp16 / 8 fp32
     static constexpr uint32_t TMEM_COLS = 512u;
     static_assert(SMEM_BYTES <= 232448, "shared memory");
@@ -89,19 +88,18 @@ struct Cfg {
 using namespace tcx;
 
 // positions per CTA pair (= per group) for a batch of n_pos positions on n_pairs pairs
-template <int LT>
 __host__ __device__ inline int group_positions(int n_pos, int n_pairs) {
     int P = (n_pos + n_pairs - 1) / n_pairs;
-    P = P < 1 ? 1 : (P > Cfg<LT>::MAX_P ? Cfg<LT>::MAX_P : P);
+    P = P < 1 ? 1 : (P > Cfg<>::MAX_P ? Cfg<>::MAX_P : P);
     if (P == 4) P = 5;                                // 4 positions need the same 4 tiles as 5
-    if (P == 6) P = 7;                                // 6 positions need 5 tiles = 3+2: same time as 3+3
     return P;
 }
 
-// the kernel body (a __device__ function so that net_auto.cu can put it behind a device-side dispatch together with
-// pp::trunk_pp_body); the __global__ wrappers are in net_tc2.cu
+// the kernel body (a __device__ function: trunk_auto_kernel, net_auto.cu, puts it behind a device-side dispatch together
+// with pp::trunk_pp_body; trunk_x3_kernel, net_tc2.cu, runs it once per group).  The caller has read the batch size and
+// counted it (count_batch).
 // (PAIR: the three weight arrays hold per-CTA halves, stage-major: [stage][2 ranks][STAGE_BLOCKS blocks]([hi, lo])[2][64][8])
-template <int LT, bool X3 = false, bool PAIR = false>
+template <bool X3, bool PAIR>
 __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__ wq,   // [32][72 K-blocks][2][128][8] bf16 (X3: [32][72][hi, lo][2][128][8])
                  const __nv_bfloat16* __restrict__ wq_in,// conv_input: [16 tap slots (9 used)][2][128][8] bf16 (X3: [9 taps][hi, lo][2][128][8])
                  const __nv_bfloat16* __restrict__ wq_bias,   // [33][2][128][8] bf16: per layer the BN shift as a K=16 B block
@@ -109,30 +107,23 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                  const float* __restrict__ headw,        // [3][128] policy conv (2) + value conv, BN scale folded; [384..386] shifts
                  float* headfeat,                        // out: [rows][243] = relu(policy conv)[2][81], relu(value conv)[81]
                  uint4* skip,                            // [gridDim][16 panels][256 rows] fp16x8 skip connection (X3: fp32x8)
-                 const int32_t* __restrict__ count,
-                 int min_count, int max_count,           // this launch handles min_count < batch <= max_count
                  long long* dbg,
-                 int n_pos_known = -1,                   // >= 0: the batch size (slot mode: counted from the slot flags, `count` unused)
-                 const int* src_rows = nullptr,          // slot mode: position i of this CTA pair reads planes row src_rows[i]
-                 int pos_base = 0, bool solo = false) {  // solo: this CTA pair alone evaluates the n_pos_known positions that
-                                                         // start at row pos_base of planes / headfeat (trunk_x3_kernel)
-    using C = Cfg<LT, X3, PAIR>;
-    constexpr int LOC_TILES = C::LOC_TILES, MAX_P = C::MAX_P, PANEL_BYTES = C::PANEL_BYTES, A_BYTES = C::A_BYTES,
+                 int n_pos,                              // the batch size
+                 const int* src_rows,                    // slot mode: position i of this CTA pair reads planes row src_rows[i], else null
+                 int pos_base, bool solo) {              // solo: this CTA pair alone evaluates the n_pos positions that start
+                                                         // at row pos_base of planes / headfeat (trunk_x3_kernel)
+    using C = Cfg<X3, PAIR>;
+    constexpr int LOC_TILES = C::LOC_TILES, PANEL_BYTES = C::PANEL_BYTES, A_BYTES = C::A_BYTES,
                   STAGES = C::STAGES, BAR_OFF = C::BAR_OFF, EPI_WARPS = C::EPI_WARPS, THREADS = C::THREADS,
                   SKIP_ROWS = C::SKIP_ROWS, NQ = C::NQ, STAGE_BLOCKS = C::STAGE_BLOCKS, STAGE_BYTES = C::STAGE_BYTES,
                   STAGES_PER_LAYER = C::STAGES_PER_LAYER, IN_STAGES = C::IN_STAGES, GROUP_STAGES = C::GROUP_STAGES,
                   ACT_PANELS = C::ACT_PANELS, SKIP_U4 = C::SKIP_U4, BLOCK_BYTES = C::BLOCK_BYTES;
-    (void)MAX_P;
     extern __shared__ __align__(1024) uint8_t smem[];
     const long long t_entry = clock64();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_rank();
     const int n_pairs = solo ? 1 : (int)gridDim.x >> 1, pair = solo ? 0 : (int)blockIdx.x >> 1;
-    const int n_pos = n_pos_known >= 0 ? n_pos_known : *count;
-    if (n_pos <= min_count || n_pos > max_count) return;
-    if (dbg && blockIdx.x == 0 && threadIdx.x == 0 && !solo) // diagnostics: histogram of evaluator batch sizes (16 per bucket)
-        atomicAdd(reinterpret_cast<unsigned long long*>(dbg) + 128 + min(n_pos >> 4, 63), 1ull);
-    const int P = group_positions<LT>(n_pos, n_pairs);
+    const int P = group_positions(n_pos, n_pairs);
     const int T = (P * POS_ROWS + 127) / 128;         // tiles of the pair: 1..4
     const int T0 = (T + 1) >> 1;                      // rank 0 takes the first ceil(T/2) tiles
     const int tiles = (rank == 0) ? T0 : T - T0;      // this CTA's tiles (0..2)
@@ -146,7 +137,7 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
     const uint32_t sA_u = smem_u32(sA);
     const uint32_t sB_u = sA_u + A_BYTES;
     const uint32_t bar_u = sA_u + BAR_OFF;
-    // barriers: full[STAGES], empty[STAGES], accum[LT], act[LT][NQ], bnd_accum; then the tmem base holder
+    // barriers: full[STAGES], empty[STAGES], accum[LOC_TILES], act[LOC_TILES][NQ], bnd_accum; then the tmem base holder
     const uint32_t bar_full = bar_u, bar_empty = bar_u + 8 * STAGES, bar_accum = bar_u + 16 * STAGES,
                    bar_act = bar_accum + 8 * LOC_TILES, bar_bnd = bar_act + 8 * LOC_TILES * NQ;
     static_assert(16 * STAGES + 8 * LOC_TILES * (1 + NQ) + 8 + 4 <= 256, "barrier block");
@@ -274,17 +265,14 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
             auto epilogue_layer = [&](auto last_tag) {
                 constexpr bool last = decltype(last_tag)::value;
                 const uint32_t lpar = (uint32_t)((iter * GROUP_LAYERS + layer + 1) & 1);
-                const uint32_t tsrc = taddr + (C::two_accumulators(lt) ? lpar * C::ALT_COLS : 0u);       // this layer's accumulator
+                const uint32_t tsrc = taddr + lpar * C::ALT_COLS;       // this layer's accumulator
                 const bool second = (layer >= 0) && (layer & 1) != 0;   // conv2 of a block: add the skip connection
                 const bool keep = second || (layer < 0);                // output is the input of the next block: keep it as skip
                 // the skip connection (8 x 16 B per thread) is fetched from L2 while the MMAs still run
-                // (LT = 3 runs 896 threads at 72 registers: only the first half is prefetched there, the second half is
-                // fetched two chunks ahead of its use)
                 // (X3: fp32, 4 x 16 B per 16-column chunk; the chunks 0 and 1 are prefetched, 2 and 3 follow as 0 and 1 are used)
-                constexpr int SKP = (LT == 2) ? 8 : 4;
-                uint4 sk[SKP];
+                uint4 sk[8];
 #pragma unroll
-                for (int j = 0; j < SKP; j++) {
+                for (int j = 0; j < 8; j++) {
                     if constexpr (X3) sk[j] = (second && valid) ? srow_skip[(size_t)(j >> 1) * SKIP_ROWS * 2 + (j & 1)] : zero4;
                     else sk[j] = (second && valid) ? srow_skip[(size_t)j * SKIP_ROWS] : zero4;
                 }
@@ -319,12 +307,8 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                                 sk[4 * (ch & 1) + j] = srow_skip[(size_t)(2 * (ch + 2) + (j >> 1)) * SKIP_ROWS * 2 + (j & 1)];
                         }
                     } else {
-                        f16x8_add2(sk[(2 * ch) % SKP], v);
-                        f16x8_add2(sk[(2 * ch + 1) % SKP], v + 8);
-                        if (SKP == 4 && ch < 2 && second && valid) {     // refill the two registers just consumed: panels +4
-                            sk[(2 * ch) % SKP] = srow_skip[(size_t)(2 * ch + 4) * SKIP_ROWS];
-                            sk[(2 * ch + 1) % SKP] = srow_skip[(size_t)(2 * ch + 5) * SKIP_ROWS];
-                        }
+                        f16x8_add2(sk[2 * ch], v);
+                        f16x8_add2(sk[2 * ch + 1], v + 8);
                     }
                     if constexpr (last) {
                         // the trunk output never leaves the SM: policy_conv / value_conv (1x1, dual_network.py:102,111)
@@ -362,28 +346,19 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                                 if (keep && valid) srow_skip[(size_t)(ch * 2 + j) * SKIP_ROWS] = relu_pack8_f16(v + 8 * j);
                             }
                         }
-                        if (NQ == 4 || ch == 3) {        // channels 16(4*chalf + ch) .. +15 of these rows are in place
-                            if (detail && ch == 0) dbg[162] = clock64();
-                            fence_async_smem();
-                            tc_fence_before();
-                            __syncwarp();
-                            if (detail && ch == 0) dbg[163] = clock64();
-                            if (lane == 0) {
-                                if (NQ == 4) {
-                                    publish(ch, (X3 ? 8 : 4) * HALO_BYTES);
-                                    if (bnd) {
-                                        push_halo(2 * ch, ch); push_halo(2 * ch + 1, ch);
-                                        if (X3) { push_halo(16 + 2 * ch, ch); push_halo(16 + 2 * ch + 1, ch); }
-                                    }
-                                    if (detail) dbg[164 + ch] = clock64();
-                                } else {
-                                    publish(0, 16 * HALO_BYTES);
-                                    if (bnd) {
-#pragma unroll
-                                        for (int pnl = 0; pnl < 8; pnl++) push_halo(pnl, 0);
-                                    }
-                                }
+                        // channels 16(4*chalf + ch) .. +15 of these rows are in place
+                        if (detail && ch == 0) dbg[162] = clock64();
+                        fence_async_smem();
+                        tc_fence_before();
+                        __syncwarp();
+                        if (detail && ch == 0) dbg[163] = clock64();
+                        if (lane == 0) {
+                            publish(ch, (X3 ? 8 : 4) * HALO_BYTES);
+                            if (bnd) {
+                                push_halo(2 * ch, ch); push_halo(2 * ch + 1, ch);
+                                if (X3) { push_halo(16 + 2 * ch, ch); push_halo(16 + 2 * ch + 1, ch); }
                             }
+                            if (detail) dbg[164 + ch] = clock64();
                         }
                     }
                 }
@@ -407,7 +382,6 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
         } else if (warp == EPI_WARPS) {
             // ================= weight producer =================
             if (PAIR ? (T0 == 0) : (tiles == 0)) continue;      // (PAIR: the peer's half of the B operand is needed whatever it owns)
-#pragma unroll 1
             int gn = iter * GROUP_STAGES;
 #pragma unroll 1
             for (int layer = -1; layer < NET_LAYERS; layer++) {
@@ -512,10 +486,10 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
 #pragma unroll 1
             for (int layer = -1; layer < NET_LAYERS; layer++) {
                 const uint32_t apar = (uint32_t)((iter * GROUP_LAYERS + layer + 1) & 1);
-                const uint32_t tmem_d = tmem_base + (uint32_t)(lt * 128) + (C::two_accumulators(lt) ? apar * C::ALT_COLS : 0u);
+                const uint32_t tmem_d = tmem_base + (uint32_t)(lt * 128) + apar * C::ALT_COLS;
                 // accumulator := BN shift (constant panel x bias block); starts the layer's accumulation.  With two
                 // accumulators per tile this needs no activation: it is issued while the previous epilogue still runs.
-                if (!C::two_accumulators(lt) || layer < 0) {
+                if (layer < 0) {
 #pragma unroll
                     for (int q = 0; q < NQ; q++) wait_act(q, apar);
                     if (dbg && blockIdx.x == 0 && iter == 0 && lt == 0 && leader && layer >= 0) dbg[layer * 4 + 0] = clock64();
@@ -559,7 +533,7 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
 #pragma unroll
                         for (int ks = 0; ks < STAGE_BLOCKS; ks++) {
                             const int m = STAGE_BLOCKS * s + ks, q = m / 18, r = m % 18, tap = r >> 1, unit = q + 4 * (r & 1);
-                            if (r == 0 && C::two_accumulators(lt)) {
+                            if (r == 0) {
                                 wait_act(q, apar);
                                 if (q == 0 && dbg && blockIdx.x == 0 && iter == 0 && lt == 0 && leader) dbg[layer * 4 + 0] = clock64();
                                 if (dbg && blockIdx.x == 0 && iter == 0 && lt == 0 && leader && layer == 21) dbg[168 + q] = clock64();

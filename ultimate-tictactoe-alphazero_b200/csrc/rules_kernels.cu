@@ -5,7 +5,6 @@
 // one thread per 32-byte state, two 128-bit loads / stores per state, fully coalesced
 // (a warp touches 1 KiB of contiguous states); grids are sized from n, no shared memory needed.
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <string>
@@ -15,11 +14,6 @@
 namespace uttt {
 
 static thread_local char g_err[512] = "";
-
-bool pdl_enabled() {
-    static const bool on = !(getenv("UTTT_PDL") && atoi(getenv("UTTT_PDL")) == 0);
-    return on;
-}
 
 void set_error(const char* fmt, ...) {
     va_list ap;

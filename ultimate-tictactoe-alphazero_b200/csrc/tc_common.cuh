@@ -1,4 +1,4 @@
-// tc_common.cuh -- PTX wrappers shared by the tensor-core trunk kernels (net_tc.cu, net_tc2.cu): UMMA shared-memory
+// tc_common.cuh -- PTX wrappers shared by the tensor-core trunk kernels (net_tc2.cu, net_pp.cu, net_auto.cu): UMMA shared-memory
 // descriptors, mbarriers, bulk async copies, tcgen05 MMA / commit / TMEM loads, cluster (DSMEM) helpers, and the
 // packed-math epilogue helpers.
 #pragma once
@@ -261,7 +261,12 @@ __device__ __forceinline__ void f16x8_add2(const uint4& q, float* v) {
 #pragma unroll
     for (int i = 0; i < 4; i++) v2[i] = __fadd2_rn(v2[i], __half22float2(h[i]));
 }
-
+// diagnostics (dbg non-null): histogram of evaluator batch sizes, 16 per bucket, read by uttt_debug_batch_histogram.
+// Every trunk kernel counts once per launch that evaluates a batch.
+__device__ __forceinline__ void count_batch(long long* dbg, int n_pos) {
+    if (dbg && blockIdx.x == 0 && threadIdx.x == 0)
+        atomicAdd(reinterpret_cast<unsigned long long*>(dbg) + 128 + min(n_pos >> 4, 63), 1ull);
+}
 
 }  // namespace tcx
 }  // namespace uttt
