@@ -367,6 +367,7 @@ def test_state_dict_upload_paths_give_identical_networks(setup):
     e.upload_state_dict(sd)
     p0, v0 = _forward(e, sts[:300], engine.EVAL_NET_BF16)
     q0, w0 = _forward(e, sts[:64], engine.EVAL_NET_FP32)
+    r0, x0 = _forward(e, sts[:300], engine.EVAL_NET_BF16X3)
     pinned = {k: v.pin_memory() for k, v in sd.items()}
     halves = {k: v.double() for k, v in sd.items()}                  # wrong dtype -> packed path (converted to fp32)
     on_gpu = {k: v.cuda() for k, v in sd.items()}                    # device tensors: read where they lie, too
@@ -378,7 +379,9 @@ def test_state_dict_upload_paths_give_identical_networks(setup):
         e.upload_state_dict(other)
         p, v = _forward(e, sts[:300], engine.EVAL_NET_BF16)
         q, w = _forward(e, sts[:64], engine.EVAL_NET_FP32)
+        r, x = _forward(e, sts[:300], engine.EVAL_NET_BF16X3)
         assert (p == p0).all() and (v == v0).all() and (q == q0).all() and (w == w0).all()
+        assert (r == r0).all() and (x == x0).all()
     bad = dict(sd)
     bad["residual_blocks.3.conv2.weight"] = torch.zeros(128, 64, 3, 3)
     with pytest.raises(ValueError):

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libuttt_b200.so")
-SOURCES = ["rules_kernels.cu", "tree_kernels.cu", "tree_tp_kernels.cu", "history_kernels.cu", "net_fp32.cu", "net_tc2.cu", "net_pp.cu", "net_auto.cu", "engine.cu"]
+SOURCES = ["rules_kernels.cu", "tree_kernels.cu", "tree_tp_kernels.cu", "history_kernels.cu", "net_fp32.cu", "net_tc2.cu", "net_pp.cu", "net_auto.cu", "weights.cu", "engine.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--ptxas-options=-v", "-cudart", "static"]
 

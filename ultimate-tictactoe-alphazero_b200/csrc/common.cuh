@@ -143,6 +143,7 @@ cudaError_t launch_unpack_samples(const void* samples, int64_t n, float* x, floa
 
 // ---------------------------------------------------------------- network
 struct NetWeights {
+    // every array is a region of `block`, one allocation per engine laid out and filled by weights.cu
     // fp32 path: folded BN (scale into the weights, shift separate); layout [layer][tap][cin][cout]
     float* conv_in_w;     // [9][3][128]
     float* conv_in_b;     // [128]
@@ -151,32 +152,47 @@ struct NetWeights {
     // bf16 tensor-core path: [layer][72 K-blocks, tcx::kblock_of][2 k-panels][cout 128][8]  (UMMA canonical K-major, no swizzle)
     __nv_bfloat16* res_w_bf16;
     __nv_bfloat16* conv_in_w_bf16;   // conv_input as a K=16-per-tap tensor-core layer: [16 tap slots (9 used)][2][128][8]
-    float* bias_all;                 // [33][128]: conv_input shift followed by the 32 trunk layers' shifts
-    __nv_bfloat16* bias_blk;         // [33][2][128][8] bf16: each layer's shift as a tensor-core B block (hi, lo in k = 0, 1)
-    // the same three arrays for cta_group::2 MMAs (net_pp.cu): the B operand is split by output channel between the two
-    // CTAs of a pair, and a CTA's share of a weight stage is contiguous: [stage][cta rank 2][blocks][2 k-panels][64 co][8]
+    __nv_bfloat16* bias_blk;         // [33][2][128][8] bf16: conv_input's and the 32 trunk layers' shifts as tensor-core B
+                                     // blocks (hi, lo in k = 0, 1)
+    // the same three arrays for cta_group::2 MMAs: the B operand is split by output channel between the two CTAs of a
+    // pair, and a CTA's share of a weight stage is contiguous: [stage][cta rank 2][blocks][2 k-panels][64 co][8]
     __nv_bfloat16* res_w_2sm;        // [32*9 stages][2][8 blocks]...
     __nv_bfloat16* conv_in_w_2sm;    // [2 stages][2][8 taps]... (16 tap slots, 9 used)
     __nv_bfloat16* bias_blk_2sm;     // [33][2][1 block]...
     // the 7-positions-per-pair instantiation (the 500-game cycle's batches) streams a quarter of a layer per stage
     __nv_bfloat16* res_w_2sm18;      // [32*4 stages][2][18 blocks]...
     __nv_bfloat16* conv_in_w_2sm18;  // [1 stage][2][18 tap slots (9 used)]...
-    // split-bf16 ("bf16x3") copies: every block is followed by its lo part, lo = bf16(w - hi) (staging for the split below)
-    __nv_bfloat16* res_w_x3;         // [32][72 K-blocks][hi, lo][2 k-panels][128][8]
-    __nv_bfloat16* conv_in_w_x3;     // [9 taps][hi, lo][2][128][8]
-    __nv_bfloat16* bias_blk_x3;      // [33][2][128][8]: shift as three bf16 terms in k = 0, 1, 2
-    // ... and their per-CTA halves, what trunk_x3_kernel (cta_group::2 MMAs) streams: stages of 6 K-blocks
+    // split-bf16 ("bf16x3"), what trunk_x3_kernel (cta_group::2 MMAs) streams: per-CTA halves in stages of 6 K-blocks,
+    // every block followed by its lo part, lo = bf16(w - hi)
     __nv_bfloat16* res_w_x3p;        // [32*12 stages][2 ranks][6 blocks][hi, lo][2 k-panels][64][8]
     __nv_bfloat16* conv_in_w_x3p;    // [2 stages][2 ranks][6 tap slots (9 of 12 used)][hi, lo][2][64][8]
-    __nv_bfloat16* bias_blk_x3p;     // [33][2 ranks][2][64][8]
-    float* head_w;                   // [3][128] policy conv (2 rows) + value conv, BN scale folded; [384..386] BN shifts
-    // heads (fp32): policy conv [2][128] + shift[2], fc [81][162] + b; value conv [128] + shift, fc1 [256][81]+b, fc2 [256]+b
-    float* pol_conv_w; float* pol_conv_b; float* pol_fc_w; float* pol_fc_b;
-    float* val_conv_w; float* val_conv_b; float* val_fc1_w; float* val_fc1_b; float* val_fc2_w; float* val_fc2_b;
+    __nv_bfloat16* bias_blk_x3p;     // [33][2 ranks][2][64][8]: shift as three bf16 terms in k = 0, 1, 2
+    // heads (fp32)
+    float* head_w;          // [3][128] policy conv (2 rows) + value conv, BN scale folded; [384..386] BN shifts
+    float* pol_fc_w;        // [162 in][81 out] + pol_fc_b [81]
+    float* pol_fc_b;
+    float* val_fc1_w;       // [81 in][256 out] + val_fc1_b [256]; val_fc2_w [256] + val_fc2_b [1]
+    float* val_fc1_b; float* val_fc2_w; float* val_fc2_b;
     float* heads_pack;      // policy_fc / value_fc1 weights in the chunk order of heads_fc.cuh (bulk-copied to shared memory)
+    float* raw_res;         // staging of an upload: the caller's residual convolutions and BN vectors as they are
+    float* raw_res_bn;
+    uint8_t* block;         // null before the first upload
     bool loaded;
 };
 
+// weights.cu: fold and pack a checkpoint into w on stream s (the device is set, nothing else uses w meanwhile; returns when
+// done).  res_tab / res_bn_tab (optional): the 32 residual convolutions and their 32 x 4 BatchNorm vectors as separate
+// tensors, each in host or device memory.  release_weights frees the allocation.
+int upload_weights(NetWeights& w, const uttt_weights* src, int on_device, const float* const* res_tab,
+                   const float* const (*res_bn_tab)[4], cudaStream_t s);
+void release_weights(NetWeights& w);
+
+// dynamic shared-memory limits of the network kernels, one function per file (net_fp32.cu, net_tc2.cu, net_pp.cu,
+// net_auto.cu); they act on the current device, so uttt_create calls them for every engine
+cudaError_t net_fp32_init();
+cudaError_t trunk_tc2_init();
+cudaError_t trunk_pp_init();
+cudaError_t trunk_auto_init();
 // trunk input: bf16 planes [rows][3][81]; output: final trunk activations [rows][81][128] (fp32 or bf16)
 cudaError_t launch_conv_input(const NetWeights& w, const __nv_bfloat16* planes, const int32_t* count, int max_rows,
                               float* out, cudaStream_t s);
@@ -190,15 +206,9 @@ cudaError_t launch_heads(const NetWeights& w, const float* act_f32, const __nv_b
                          const int32_t* count, int max_rows, float* policy, float* value, int row_stride,
                          cudaStream_t s);
 // split-bf16 numerics (UTTT_EVAL_NET_BF16X3, net_tc2.cu): any batch size in one launch; skip: [n_sm][16][256] fp32x8
-cudaError_t trunk_tc2_init();
 cudaError_t launch_trunk_x3(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count,
                             int max_rows, float* skip, int n_sm, cudaStream_t s, long long* dbg);
-// cta_group::2 weight halves (net_pp.cu)
-// (subs = 16-byte-unit blocks per K-block: 1, or 2 for the split-bf16 arrays whose blocks are a hi and a lo part)
-cudaError_t launch_split_weights_2sm(const __nv_bfloat16* src, __nv_bfloat16* dst, int n_blocks, int blocks_per_stage, cudaStream_t s,
-                                     int subs = 1);
 // two groups of positions per CTA pair in flight (net_pp.cu): batches of more than trunk_pp_cap1 positions
-cudaError_t trunk_pp_init();
 int trunk_pp_cap1(int n_sm);         // largest batch of trunk_auto_kernel (7 positions per CTA pair)
 cudaError_t launch_trunk_pp_large(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count,
                                   int max_rows, float* skip, int n_sm, cudaStream_t s, long long* dbg);
@@ -207,6 +217,5 @@ cudaError_t launch_trunk_pp_large(const NetWeights& w, const __nv_bfloat16* plan
 cudaError_t launch_trunk_auto(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count, int max_rows,
                               float* skip, int n_sm, cudaStream_t s, long long* dbg, float* policy, float* value,
                               const uint8_t* slot_flags = nullptr, int n_slots = 0);
-cudaError_t trunk_auto_init();
 
 }  // namespace uttt

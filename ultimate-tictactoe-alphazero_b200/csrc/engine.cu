@@ -17,8 +17,6 @@
 #include <vector>
 
 #include "common.cuh"
-#include "tc_common.cuh"
-#include "heads_fc.cuh"
 
 using namespace uttt;
 
@@ -31,35 +29,6 @@ constexpr int EV_POOL = N_WINDOWS * CHECK_EVERY * 4 * N_LANES;
 
 __global__ void set_int_kernel(int32_t* p, int32_t v) { *p = v; }
 __global__ void set_u64_kernel(unsigned long long* p, unsigned long long v) { *p = v; }
-
-// BatchNorm folding + repacking of the 32 residual 3x3 convolutions on the device:
-// raw (32)(co,ci,ky,kx) fp32 + bn (32)(4)(128) -> fp32 [l][tap][ci][co], bias [l][co], bf16 [l][tap][ci/8][co][ci%8]
-// and the split-bf16 copy [l][K-block][hi, lo][ci/8 % 2][co][ci%8] with lo = bf16(w - hi)
-__global__ void __launch_bounds__(256) pack_res_kernel(const float* __restrict__ raw, const float* __restrict__ bn,
-                                                       float* __restrict__ w32, float* __restrict__ b32,
-                                                       __nv_bfloat16* __restrict__ w16, __nv_bfloat16* __restrict__ w16x3) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;      // index into raw
-    if (i >= (size_t)32 * 128 * 128 * 9) return;
-    int tap = (int)(i % 9);
-    size_t r = i / 9;
-    int ci = (int)(r % 128);
-    r /= 128;
-    int co = (int)(r % 128);
-    int l = (int)(r / 128);
-    const float* b = bn + (size_t)l * 4 * 128;
-    float g = b[co], beta = b[128 + co], m = b[256 + co], v = b[384 + co];
-    float sc = __fdiv_rn(g, __fsqrt_rn(__fadd_rn(v, 1e-5f)));
-    float val = __fmul_rn(raw[i], sc);
-    w32[(((size_t)l * 9 + tap) * 128 + ci) * 128 + co] = val;
-    // tensor-core copy: 72 K-blocks per layer in the order of tcx::kblock_of, each [2 panels][128 co][8 ci]
-    int blk = tcx::kblock_of(tap, ci / 16);
-    const __nv_bfloat16 hi = __float2bfloat16(val);
-    w16[((((size_t)l * 72 + blk) * 2 + ((ci / 8) & 1)) * 128 + co) * 8 + (ci % 8)] = hi;
-    const size_t x3 = (((((size_t)l * 72 + blk) * 2) * 2 + ((ci / 8) & 1)) * 128 + co) * 8 + (ci % 8);
-    w16x3[x3] = hi;
-    w16x3[x3 + 2 * 128 * 8] = __float2bfloat16(__fsub_rn(val, __bfloat162float(hi)));
-    if (ci == 0 && tap == 0) b32[l * 128 + co] = __fsub_rn(beta, __fmul_rn(m, sc));
-}
 
 template <typename T>
 cudaError_t dmalloc(T** p, size_t n) { return cudaMalloc((void**)p, n * sizeof(T)); }
@@ -96,8 +65,6 @@ struct uttt_engine {
     int64_t prof_sampled_launches, prof_sampled_evals;      // trunk launches with events in the last run, positions they evaluated
     int lane_threshold;     // slots from which self-play splits into two overlapped lanes
     NetWeights w;
-    float* raw_res;         // staging for the raw residual conv weights / bn of an upload
-    float* raw_res_bn;
     unsigned long long* h_counters;   // pinned [8 * (1 + N_WINDOWS)]: [0..7] general use, then one copy per self-play window
     int32_t* h_count;                 // pinned [2]
     // step-wise search state
@@ -295,6 +262,10 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     e->prof_sample = getenv("UTTT_PROFILE_SAMPLE") ? atoi(getenv("UTTT_PROFILE_SAMPLE")) : 4;
     if (e->prof_sample < 1) e->prof_sample = 1;
     e->lane_threshold = getenv("UTTT_LANE_THRESHOLD") ? atoi(getenv("UTTT_LANE_THRESHOLD")) : 1024;
+    UTTT_CUDA_OK(net_fp32_init());
+    UTTT_CUDA_OK(trunk_tc2_init());
+    UTTT_CUDA_OK(trunk_pp_init());
+    UTTT_CUDA_OK(trunk_auto_init());
     cudaDeviceProp prop;
     UTTT_CUDA_OK(cudaGetDeviceProperties(&prop, cfg->device));
     e->n_sm = prop.multiProcessorCount;
@@ -356,12 +327,7 @@ int uttt_destroy(uttt_engine* e) {
     cudaSetDevice(e->cfg.device);
     cudaDeviceSynchronize();
     for (void* p : e->allocs) cudaFree(p);
-    float* wp[] = {(float*)e->w.res_w_x3p, (float*)e->w.conv_in_w_x3p, (float*)e->w.bias_blk_x3p, (float*)e->w.res_w_x3, (float*)e->w.conv_in_w_x3, (float*)e->w.bias_blk_x3, e->w.conv_in_w, e->w.conv_in_b, e->w.res_w, e->w.res_b, (float*)e->w.res_w_bf16, (float*)e->w.conv_in_w_bf16, e->w.bias_all, (float*)e->w.bias_blk, (float*)e->w.res_w_2sm, (float*)e->w.conv_in_w_2sm, (float*)e->w.bias_blk_2sm, (float*)e->w.res_w_2sm18, (float*)e->w.conv_in_w_2sm18, e->w.head_w, e->w.pol_conv_w,
-                   e->w.pol_conv_b, e->w.pol_fc_w, e->w.pol_fc_b, e->w.val_conv_w, e->w.val_conv_b, e->w.val_fc1_w,
-                   e->w.val_fc1_b, e->w.val_fc2_w, e->w.val_fc2_b, e->w.heads_pack};
-    for (float* p : wp) if (p) cudaFree(p);
-    if (e->raw_res) cudaFree(e->raw_res);
-    if (e->raw_res_bn) cudaFree(e->raw_res_bn);
+    release_weights(e->w);
     if (e->h_counters) cudaFreeHost(e->h_counters);
     if (e->h_count) cudaFreeHost(e->h_count);
     for (int i = 0; i < EV_POOL; i++) if (e->ev[i]) cudaEventDestroy(e->ev[i]);
@@ -379,25 +345,6 @@ int uttt_destroy(uttt_engine* e) {
 }
 
 // ---------------------------------------------------------------------------- weights
-// Eval-mode BatchNorm folding: y = gamma*(x-mean)/sqrt(var+eps) + beta = scale*x + shift.
-static void bn_fold(const float* bn, int C, std::vector<float>& scale, std::vector<float>& shift) {
-    scale.resize(C); shift.resize(C);
-    for (int c = 0; c < C; c++) {
-        float g = bn[c], b = bn[C + c], m = bn[2 * C + c], v = bn[3 * C + c];
-        float s = g / sqrtf(v + 1e-5f);
-        scale[c] = s;
-        shift[c] = b - m * s;
-    }
-}
-
-static int to_device(float** dst, const std::vector<float>& v) {
-    if (!*dst) UTTT_CUDA_OK(cudaMalloc((void**)dst, v.size() * sizeof(float)));
-    UTTT_CUDA_OK(cudaMemcpy(*dst, v.data(), v.size() * sizeof(float), cudaMemcpyHostToDevice));
-    return 0;
-}
-
-// res_tab / res_bn_tab (optional): the 32 residual convolutions and their 32 x 4 BatchNorm vectors as separate tensors
-// (state_dict entries copied straight from the caller's memory, no host-side concatenation)
 static int upload_impl(uttt_engine* e, const uttt_weights* w, int on_device, const float* const* res_tab,
                        const float* const (*res_bn_tab)[4]) {
     UTTT_CHECK(e && w, "null argument");
@@ -406,193 +353,7 @@ static int upload_impl(uttt_engine* e, const uttt_weights* w, int on_device, con
         UTTT_CUDA_OK(cudaEventSynchronize(e->ev_fwd));
         e->fwd_pending = false;
     }
-    auto fetch = [&](const float* p, size_t n, std::vector<float>& v) -> int {
-        v.resize(n);
-        UTTT_CHECK(p != nullptr, "null weight tensor");
-        if (on_device) UTTT_CUDA_OK(cudaMemcpy(v.data(), p, n * sizeof(float), cudaMemcpyDeviceToHost));
-        else memcpy(v.data(), p, n * sizeof(float));
-        return 0;
-    };
-    std::vector<float> ciw, bni, pcw, pbn, pfw, pfb, vcw, vbn, v1w, v1b, v2w, v2b;
-    if (fetch(w->conv_input_w, 128 * 27, ciw) || fetch(w->bn_input, 4 * 128, bni) ||
-        fetch(w->policy_conv_w, 2 * 128, pcw) || fetch(w->policy_bn, 8, pbn) || fetch(w->policy_fc_w, 81 * 162, pfw) ||
-        fetch(w->policy_fc_b, 81, pfb) || fetch(w->value_conv_w, 128, vcw) || fetch(w->value_bn, 4, vbn) ||
-        fetch(w->value_fc1_w, 256 * 81, v1w) || fetch(w->value_fc1_b, 256, v1b) || fetch(w->value_fc2_w, 256, v2w) ||
-        fetch(w->value_fc2_b, 1, v2b))
-        return 1;
-    UTTT_CHECK(res_tab || (w->res_conv_w && w->res_bn), "null weight tensor");
-
-    // the 32 residual convolutions (4.7 M weights) are folded and repacked by a kernel
-    const size_t n_res = (size_t)32 * 128 * 128 * 9, n_rbn = (size_t)32 * 4 * 128;
-    NetWeights& W = e->w;
-    if (!e->raw_res) {
-        UTTT_CUDA_OK(cudaMalloc((void**)&e->raw_res, n_res * sizeof(float)));
-        UTTT_CUDA_OK(cudaMalloc((void**)&e->raw_res_bn, n_rbn * sizeof(float)));
-        UTTT_CUDA_OK(cudaMalloc((void**)&W.res_w, n_res * sizeof(float)));
-        UTTT_CUDA_OK(cudaMalloc((void**)&W.res_b, 32 * 128 * sizeof(float)));
-        UTTT_CUDA_OK(cudaMalloc((void**)&W.res_w_bf16, n_res * sizeof(__nv_bfloat16)));
-        UTTT_CUDA_OK(cudaMalloc((void**)&W.res_w_x3, 2 * n_res * sizeof(__nv_bfloat16)));
-    }
-    cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    if (res_tab) {
-        const size_t per = (size_t)128 * 128 * 9;
-        for (int l = 0; l < 32; l++) {
-            UTTT_CHECK(res_tab[l] != nullptr, "null weight tensor");
-            // (cudaMemcpyDefault: each tensor may lie in host or device memory, whatever `on_device` says about `small`)
-            UTTT_CUDA_OK(cudaMemcpyAsync(e->raw_res + l * per, res_tab[l], per * sizeof(float), cudaMemcpyDefault, e->stream));
-            for (int j = 0; j < 4; j++) {
-                UTTT_CHECK(res_bn_tab[l][j] != nullptr, "null weight tensor");
-                UTTT_CUDA_OK(cudaMemcpyAsync(e->raw_res_bn + (l * 4 + j) * 128, res_bn_tab[l][j], 128 * sizeof(float), cudaMemcpyDefault,
-                                             e->stream));
-            }
-        }
-    } else {
-        UTTT_CUDA_OK(cudaMemcpyAsync(e->raw_res, w->res_conv_w, n_res * sizeof(float), kind, e->stream));
-        UTTT_CUDA_OK(cudaMemcpyAsync(e->raw_res_bn, w->res_bn, n_rbn * sizeof(float), kind, e->stream));
-    }
-    pack_res_kernel<<<ceil_div((int64_t)n_res, 256), 256, 0, e->stream>>>(e->raw_res, e->raw_res_bn, W.res_w, W.res_b,
-                                                                         W.res_w_bf16, W.res_w_x3);
-    UTTT_CUDA_OK(cudaGetLastError());
-
-    std::vector<float> sc, sh;
-    // conv_input: (128,3,3,3) [co][ci][ky][kx] -> [tap][ci][co]
-    bn_fold(bni.data(), 128, sc, sh);
-    std::vector<float> ci_w(9 * 3 * 128), ci_b(sh);
-    for (int co = 0; co < 128; co++)
-        for (int ci = 0; ci < 3; ci++)
-            for (int tap = 0; tap < 9; tap++)
-                ci_w[(tap * 3 + ci) * 128 + co] = ciw[(co * 3 + ci) * 9 + tap] * sc[co];
-    // heads
-    bn_fold(pbn.data(), 2, sc, sh);
-    std::vector<float> pc_w(256), pc_b(sh);
-    for (int j = 0; j < 2; j++)
-        for (int c = 0; c < 128; c++) pc_w[j * 128 + c] = pcw[j * 128 + c] * sc[j];
-    std::vector<float> pf_t(162 * 81);
-    for (int o = 0; o < 81; o++)
-        for (int i = 0; i < 162; i++) pf_t[i * 81 + o] = pfw[o * 162 + i];
-    bn_fold(vbn.data(), 1, sc, sh);
-    std::vector<float> vc_w(128), vc_b(sh);
-    for (int c = 0; c < 128; c++) vc_w[c] = vcw[c] * sc[0];
-    std::vector<float> v1_t(81 * 256);
-    for (int j = 0; j < 256; j++)
-        for (int i = 0; i < 81; i++) v1_t[i * 256 + j] = v1w[j * 81 + i];
-
-    // conv_input for the tensor pipe: [16 tap slots (9 used)][2 panels][128 co][8 ci]; channels 3..15 are zero
-    {
-        std::vector<__nv_bfloat16> ci_h((size_t)16 * 2 * 128 * 8, __float2bfloat16(0.0f));     // 16 tap slots, 9 used
-        for (int tap = 0; tap < 9; tap++)
-            for (int ci = 0; ci < 3; ci++)
-                for (int co = 0; co < 128; co++)
-                    ci_h[((size_t)(tap * 2) * 128 + co) * 8 + ci] = __float2bfloat16(ci_w[(tap * 3 + ci) * 128 + co]);
-        if (!W.conv_in_w_bf16) UTTT_CUDA_OK(cudaMalloc((void**)&W.conv_in_w_bf16, ci_h.size() * sizeof(__nv_bfloat16)));
-        UTTT_CUDA_OK(cudaMemcpy(W.conv_in_w_bf16, ci_h.data(), ci_h.size() * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice));
-        if (!W.bias_all) UTTT_CUDA_OK(cudaMalloc((void**)&W.bias_all, 33 * 128 * sizeof(float)));
-        UTTT_CUDA_OK(cudaMemcpy(W.bias_all, ci_b.data(), 128 * sizeof(float), cudaMemcpyHostToDevice));
-        UTTT_CUDA_OK(cudaMemcpyAsync(W.bias_all + 128, W.res_b, 32 * 128 * sizeof(float), cudaMemcpyDeviceToDevice, e->stream));
-        // bias blocks of the cluster trunk: shift = hi + lo (two bf16) against a constant (1,1,0,..) A row
-        std::vector<float> ball(33 * 128);
-        UTTT_CUDA_OK(cudaStreamSynchronize(e->stream));
-        UTTT_CUDA_OK(cudaMemcpy(ball.data(), W.bias_all, ball.size() * sizeof(float), cudaMemcpyDeviceToHost));
-        std::vector<__nv_bfloat16> bb((size_t)33 * 2 * 128 * 8, __float2bfloat16(0.0f));
-        for (int l = 0; l < 33; l++)
-            for (int co = 0; co < 128; co++) {
-                float b = ball[l * 128 + co];
-                __nv_bfloat16 hi = __float2bfloat16(b);
-                __nv_bfloat16 lo = __float2bfloat16(b - __bfloat162float(hi));
-                bb[((size_t)l * 2 * 128 + co) * 8 + 0] = hi;
-                bb[((size_t)l * 2 * 128 + co) * 8 + 1] = lo;
-            }
-        if (!W.bias_blk) UTTT_CUDA_OK(cudaMalloc((void**)&W.bias_blk, bb.size() * sizeof(__nv_bfloat16)));
-        UTTT_CUDA_OK(cudaMemcpy(W.bias_blk, bb.data(), bb.size() * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice));
-        // split-bf16 trunk: conv_input as [9 taps][hi, lo][2][128][8], the shifts as three bf16 terms (k = 0, 1, 2)
-        {
-            std::vector<__nv_bfloat16> cx((size_t)9 * 2 * 2 * 128 * 8, __float2bfloat16(0.0f));
-            for (int tap = 0; tap < 9; tap++)
-                for (int ci = 0; ci < 3; ci++)
-                    for (int co = 0; co < 128; co++) {
-                        float v = ci_w[(tap * 3 + ci) * 128 + co];
-                        __nv_bfloat16 hi = __float2bfloat16(v);
-                        cx[(((size_t)tap * 2 + 0) * 2 * 128 + co) * 8 + ci] = hi;
-                        cx[(((size_t)tap * 2 + 1) * 2 * 128 + co) * 8 + ci] = __float2bfloat16(v - __bfloat162float(hi));
-                    }
-            if (!W.conv_in_w_x3) UTTT_CUDA_OK(cudaMalloc((void**)&W.conv_in_w_x3, cx.size() * sizeof(__nv_bfloat16)));
-            UTTT_CUDA_OK(cudaMemcpy(W.conv_in_w_x3, cx.data(), cx.size() * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice));
-            std::vector<__nv_bfloat16> b3((size_t)33 * 2 * 128 * 8, __float2bfloat16(0.0f));
-            for (int l = 0; l < 33; l++)
-                for (int co = 0; co < 128; co++) {
-                    float b = ball[l * 128 + co];
-                    for (int k = 0; k < 3; k++) {
-                        __nv_bfloat16 t = __float2bfloat16(b);
-                        b3[((size_t)l * 2 * 128 + co) * 8 + k] = t;
-                        b -= __bfloat162float(t);
-                    }
-                }
-            if (!W.bias_blk_x3) UTTT_CUDA_OK(cudaMalloc((void**)&W.bias_blk_x3, b3.size() * sizeof(__nv_bfloat16)));
-            UTTT_CUDA_OK(cudaMemcpy(W.bias_blk_x3, b3.data(), b3.size() * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice));
-            // per-CTA halves for the cta_group::2 form (stages of 6 K-blocks; conv_input: 12 tap slots, 9 used)
-            const size_t blk3 = 2 * 2 * 128 * 8;
-            if (!W.res_w_x3p) UTTT_CUDA_OK(cudaMalloc((void**)&W.res_w_x3p, (size_t)32 * 72 * blk3 * sizeof(__nv_bfloat16)));
-            if (!W.conv_in_w_x3p) {
-                UTTT_CUDA_OK(cudaMalloc((void**)&W.conv_in_w_x3p, (size_t)12 * blk3 * sizeof(__nv_bfloat16)));
-                UTTT_CUDA_OK(cudaMemset(W.conv_in_w_x3p, 0, (size_t)12 * blk3 * sizeof(__nv_bfloat16)));
-            }
-            if (!W.bias_blk_x3p) UTTT_CUDA_OK(cudaMalloc((void**)&W.bias_blk_x3p, b3.size() * sizeof(__nv_bfloat16)));
-            UTTT_CUDA_OK(launch_split_weights_2sm(W.res_w_x3, W.res_w_x3p, 32 * 72, 6, e->stream, 2));
-            UTTT_CUDA_OK(launch_split_weights_2sm(W.conv_in_w_x3, W.conv_in_w_x3p, 9, 6, e->stream, 2));
-            UTTT_CUDA_OK(launch_split_weights_2sm(W.bias_blk_x3, W.bias_blk_x3p, 33, 1, e->stream));
-        }
-        // per-CTA halves of the three B-operand arrays for the cta_group::2 trunk
-        const size_t blk = 2 * 128 * 8;
-        if (!W.res_w_2sm) UTTT_CUDA_OK(cudaMalloc((void**)&W.res_w_2sm, (size_t)32 * 72 * blk * sizeof(__nv_bfloat16)));
-        if (!W.conv_in_w_2sm) {
-            UTTT_CUDA_OK(cudaMalloc((void**)&W.conv_in_w_2sm, (size_t)16 * blk * sizeof(__nv_bfloat16)));
-            UTTT_CUDA_OK(cudaMemset(W.conv_in_w_2sm, 0, (size_t)16 * blk * sizeof(__nv_bfloat16)));
-        }
-        if (!W.bias_blk_2sm) UTTT_CUDA_OK(cudaMalloc((void**)&W.bias_blk_2sm, (size_t)33 * blk * sizeof(__nv_bfloat16)));
-        UTTT_CUDA_OK(launch_split_weights_2sm(W.res_w_bf16, W.res_w_2sm, 32 * 72, 8, e->stream));
-        UTTT_CUDA_OK(launch_split_weights_2sm(W.conv_in_w_bf16, W.conv_in_w_2sm, 12, 8, e->stream));
-        UTTT_CUDA_OK(launch_split_weights_2sm(W.bias_blk, W.bias_blk_2sm, 33, 1, e->stream));
-        if (!W.res_w_2sm18) UTTT_CUDA_OK(cudaMalloc((void**)&W.res_w_2sm18, (size_t)32 * 72 * blk * sizeof(__nv_bfloat16)));
-        if (!W.conv_in_w_2sm18) {
-            UTTT_CUDA_OK(cudaMalloc((void**)&W.conv_in_w_2sm18, (size_t)18 * blk * sizeof(__nv_bfloat16)));
-            UTTT_CUDA_OK(cudaMemset(W.conv_in_w_2sm18, 0, (size_t)18 * blk * sizeof(__nv_bfloat16)));
-        }
-        UTTT_CUDA_OK(launch_split_weights_2sm(W.res_w_bf16, W.res_w_2sm18, 32 * 72, 18, e->stream));
-        UTTT_CUDA_OK(launch_split_weights_2sm(W.conv_in_w_bf16, W.conv_in_w_2sm18, 12, 18, e->stream));
-    }
-    {
-        std::vector<float> hw(387);
-        for (int i = 0; i < 256; i++) hw[i] = pc_w[i];
-        for (int i = 0; i < 128; i++) hw[256 + i] = vc_w[i];
-        hw[384] = pc_b[0]; hw[385] = pc_b[1]; hw[386] = vc_b[0];
-        if (to_device(&W.head_w, hw)) return 1;
-    }
-    {
-        // FC weights of the heads in the order heads_fc_block streams them: 3 chunks of 27 input rows
-        std::vector<float> pack(HEADS_PACK_FLOATS, 0.0f);
-        for (int c = 0; c < HEADS_CHUNKS; c++) {
-            float* dst = pack.data() + (size_t)c * HEADS_CHUNK_FLOATS;
-            for (int h = 0; h < 2; h++)
-                for (int i = 0; i < HEADS_CHUNK_ROWS; i++)
-                    for (int o = 0; o < 81; o++)
-                        dst[h * HEADS_POL_FLOATS + i * 81 + o] = pf_t[(size_t)(h * 81 + c * HEADS_CHUNK_ROWS + i) * 81 + o];
-            for (int i = 0; i < HEADS_CHUNK_ROWS; i++)
-                for (int j = 0; j < 256; j++)
-                    dst[2 * HEADS_POL_FLOATS + i * 256 + j] = v1_t[(size_t)(c * HEADS_CHUNK_ROWS + i) * 256 + j];
-        }
-        if (to_device(&W.heads_pack, pack)) return 1;
-    }
-    if (to_device(&W.conv_in_w, ci_w) || to_device(&W.conv_in_b, ci_b) || to_device(&W.pol_conv_w, pc_w) || to_device(&W.pol_conv_b, pc_b) ||
-        to_device(&W.pol_fc_w, pf_t) || to_device(&W.pol_fc_b, pfb) || to_device(&W.val_conv_w, vc_w) ||
-        to_device(&W.val_conv_b, vc_b) || to_device(&W.val_fc1_w, v1_t) || to_device(&W.val_fc1_b, v1b) ||
-        to_device(&W.val_fc2_w, v2w) || to_device(&W.val_fc2_b, v2b))
-        return 1;
-    UTTT_CUDA_OK(cudaStreamSynchronize(e->stream));
-    UTTT_CUDA_OK(trunk_tc2_init());
-    UTTT_CUDA_OK(trunk_pp_init());
-    UTTT_CUDA_OK(trunk_auto_init());
-    W.loaded = true;
-    return 0;
+    return upload_weights(e->w, w, on_device, res_tab, res_bn_tab, e->stream);
 }
 
 int uttt_upload_weights(uttt_engine* e, const uttt_weights* w, int on_device) {

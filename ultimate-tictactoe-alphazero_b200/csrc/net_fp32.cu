@@ -131,12 +131,13 @@ __global__ void __launch_bounds__(128) heads_kernel(NetWeights W, const float* _
     __shared__ float logit[81];
     int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 
+    // head_w: policy conv [2][128], value conv [128], their BN shifts [384..386]
     float wp0[4], wp1[4], wv[4];
 #pragma unroll
     for (int i = 0; i < 4; i++) {
-        wp0[i] = W.pol_conv_w[lane * 4 + i];
-        wp1[i] = W.pol_conv_w[128 + lane * 4 + i];
-        wv[i] = W.val_conv_w[lane * 4 + i];
+        wp0[i] = W.head_w[lane * 4 + i];
+        wp1[i] = W.head_w[128 + lane * 4 + i];
+        wv[i] = W.head_w[256 + lane * 4 + i];
     }
     for (int cell = warp; cell < 81; cell += 4) {
         float x[4];
@@ -159,9 +160,9 @@ __global__ void __launch_bounds__(128) heads_kernel(NetWeights W, const float* _
             s2 += __shfl_xor_sync(0xFFFFFFFFu, s2, off);
         }
         if (lane == 0) {
-            ph[cell] = fmaxf(s0 + W.pol_conv_b[0], 0.0f);
-            ph[81 + cell] = fmaxf(s1 + W.pol_conv_b[1], 0.0f);
-            vh[cell] = fmaxf(s2 + W.val_conv_b[0], 0.0f);
+            ph[cell] = fmaxf(s0 + W.head_w[384], 0.0f);
+            ph[81 + cell] = fmaxf(s1 + W.head_w[385], 0.0f);
+            vh[cell] = fmaxf(s2 + W.head_w[386], 0.0f);
         }
     }
     __syncthreads();
@@ -220,14 +221,14 @@ __global__ void __launch_bounds__(HEADS_THREADS) heads_fc_kernel(HeadsFC W, cons
     heads_fc_block(W, headfeat, row0, 1, min(HEADS_P, n - row0), policy, value, row_stride, heads_sm);
 }
 
+cudaError_t net_fp32_init() {
+    cudaError_t e = cudaFuncSetAttribute(heads_fc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, HEADS_SMEM_BYTES);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(conv3x3_fp32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, F32_SMEM);
+}
+
 cudaError_t launch_heads_fc(const NetWeights& w, const float* headfeat, const int32_t* count, int max_rows, float* policy,
                             float* value, int row_stride, cudaStream_t s) {
-    static bool attr = false;
-    if (!attr) {
-        cudaError_t e = cudaFuncSetAttribute(heads_fc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, HEADS_SMEM_BYTES);
-        if (e != cudaSuccess) return e;
-        attr = true;
-    }
     return launch_pdl(heads_fc_kernel, dim3((max_rows + HEADS_P - 1) / HEADS_P), dim3(HEADS_THREADS), HEADS_SMEM_BYTES, s, heads_fc_of(w),
                       headfeat, count, policy, value, row_stride);
 }
@@ -240,12 +241,6 @@ cudaError_t launch_conv_input(const NetWeights& w, const __nv_bfloat16* planes, 
 
 cudaError_t launch_trunk_fp32(const NetWeights& w, const __nv_bfloat16* planes, const int32_t* count, int max_rows,
                               float* act_a, float* act_b, cudaStream_t s) {
-    static bool attr = false;
-    if (!attr) {
-        cudaError_t e = cudaFuncSetAttribute(conv3x3_fp32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, F32_SMEM);
-        if (e != cudaSuccess) return e;
-        attr = true;
-    }
     cudaError_t e = launch_conv_input(w, planes, count, max_rows, act_a, s);
     if (e != cudaSuccess) return e;
     // residual block: a --conv1--> b --conv2(+a)--> a          dual_network.py:36-45

@@ -1,5 +1,4 @@
-// net_pp.cu -- trunk_pp_large_kernel, the large-batch form of the two-groups-in-flight trunk (body: net_pp_kernel.cuh), and
-// the weight splitting for the cta_group::2 B operand
+// net_pp.cu -- trunk_pp_large_kernel, the large-batch form of the two-groups-in-flight trunk (body: net_pp_kernel.cuh)
 #include "net_pp_kernel.cuh"
 
 namespace uttt {
@@ -24,25 +23,6 @@ trunk_pp_large_kernel(const __nv_bfloat16* __restrict__ wq,
 
 }  // namespace pp
 
-
-// [block][2 k-panels][128 co][8] -> [stage][cta rank][block of the stage][2 k-panels][64 co][8]: each CTA of a pair holds the
-// output channels 64*rank .. 64*rank+63 of the B operand, and its share of a weight stage is one contiguous bulk copy
-// (subs = 2: split-bf16 arrays, [block][hi, lo][2][128][8] -> [stage][rank][block][hi, lo][2][64][8])
-__global__ void split_weights_2sm_kernel(const uint4* __restrict__ src, uint4* __restrict__ dst, int n_blocks, int bps, int subs) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;               // one 16-byte (co, 8 ci) unit
-    if (i >= n_blocks * subs * 256) return;
-    int u = i >> 8, pnl = (i >> 7) & 1, co = i & 127;
-    int b = u / subs, sub = u - b * subs;
-    int stage = b / bps, j = b - stage * bps, r = co >> 6;
-    dst[(((((size_t)stage * 2 + r) * bps + j) * subs + sub) * 2 + pnl) * 64 + (co & 63)] = src[i];
-}
-cudaError_t launch_split_weights_2sm(const __nv_bfloat16* src, __nv_bfloat16* dst, int n_blocks, int blocks_per_stage, cudaStream_t s,
-                                     int subs) {
-    split_weights_2sm_kernel<<<(n_blocks * subs * 256 + 255) / 256, 256, 0, s>>>(reinterpret_cast<const uint4*>(src),
-                                                                                    reinterpret_cast<uint4*>(dst), n_blocks,
-                                                                                    blocks_per_stage, subs);
-    return cudaGetLastError();
-}
 
 cudaError_t trunk_pp_init() {
     return cudaFuncSetAttribute(pp::trunk_pp_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pp::Cfg<2>::SMEM_BYTES);

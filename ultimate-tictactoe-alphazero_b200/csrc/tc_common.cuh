@@ -18,7 +18,7 @@ constexpr uint32_t IDESC_M128_N128_BF16 = (1u << 4) | (1u << 7) | (1u << 10) | (
 // the 16 input channels of unit u = q + 4h (channels 16u .. 16u+15).  The order is channel-quarter-major: an epilogue
 // warp writes units 0..3 (column half 0) or 4..7 (column half 1) in that order, so the blocks of quarter q only need
 // the q-th 16-column chunk of every epilogue warp -- the next layer's MMAs start while the epilogue is still running.
-// The pre-packed weights (pack_res_kernel, engine.cu) are stored in the same order, 4 KiB per block.
+// The pre-packed weights (pack_res_kernel, weights.cu) are stored in the same order, 4 KiB per block.
 __host__ __device__ __forceinline__ int kblock_of(int tap, int unit) { return 18 * (unit & 3) + 2 * tap + (unit >> 2); }
 __device__ __forceinline__ void kblock_decode(int m, int& q, int& tap, int& unit) {
     q = m / 18;
