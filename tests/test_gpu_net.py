@@ -314,8 +314,8 @@ def test_fp32_trunk_vs_reference_golden_outputs(setup, golden_dir):
 def test_trunk_variant_boundaries_give_identical_rows(setup):
     """The trunk kernel is chosen on the device from the batch size and the group sizes from ceil(n / pairs): every
     boundary of that dispatch must produce the same rows.  One launch that branches on the device (trunk_auto_kernel,
-    net_auto.cu): one group per CTA pair up to 370 positions (net_tc2: cta_group::2 MMAs with per-CTA weight halves up to 148
-    positions = one tile per CTA, cta_group::1 MMAs above), two groups in flight above (net_pp, cta_group::2).  All of them accumulate a row in the
+    net_auto.cu): one group per CTA pair up to 370 positions (net_tc2), two groups in flight above (net_pp), both with
+    cta_group::2 MMAs on per-CTA weight halves.  All of them accumulate a row in the
     same order: bit-identical rows -- including the one-tile group of the 6/7-positions-per-pair case (371..518
     positions), whose weight stages are issued by two threads in turn into one accumulator."""
     import copy

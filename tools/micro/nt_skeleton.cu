@@ -12,6 +12,25 @@
 
 using namespace uttt::tcx;
 
+// cta_group::1 MMA and commits (the library's trunks issue cta_group::2 MMAs only)
+__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
+        : "memory");
+}
+__device__ __forceinline__ void umma_commit(uint32_t bar) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+}
+// arrive on the barrier at the same shared-memory offset in every CTA of `mask`
+__device__ __forceinline__ void umma_commit_mcast(uint32_t bar, uint16_t mask) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
+                 "h"(mask)
+                 : "memory");
+}
+
 constexpr int LEAD = 11;
 constexpr int BLOCK_BYTES = 4096, STAGE_BLOCKS = 4, STAGE_BYTES = STAGE_BLOCKS * BLOCK_BYTES, STAGES = 7;
 constexpr int SPL = 72 / STAGE_BLOCKS;                  // weight stages per layer (+ 1 bias stage)

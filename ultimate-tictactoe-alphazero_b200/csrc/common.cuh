@@ -149,12 +149,10 @@ struct NetWeights {
     float* conv_in_b;     // [128]
     float* res_w;         // [32][9][128][128]
     float* res_b;         // [32][128]
-    // bf16 tensor-core path: [layer][72 K-blocks, tcx::kblock_of][2 k-panels][cout 128][8]  (UMMA canonical K-major, no swizzle)
-    __nv_bfloat16* res_w_bf16;
-    __nv_bfloat16* conv_in_w_bf16;   // conv_input as a K=16-per-tap tensor-core layer: [16 tap slots (9 used)][2][128][8]
-    __nv_bfloat16* bias_blk;         // [33][2][128][8] bf16: conv_input's and the 32 trunk layers' shifts as tensor-core B
-                                     // blocks (hi, lo in k = 0, 1)
-    // the same three arrays for cta_group::2 MMAs: the B operand is split by output channel between the two CTAs of a
+    // bf16 tensor-core path: the B operand of one K=16 MMA is a block [2 k-panels][cout 128][8] (UMMA canonical K-major,
+    // no swizzle): 72 per residual layer in the order of tcx::kblock_of, conv_input as a K=16-per-tap layer (one block
+    // per tap, channels 3..15 zero), and per layer (conv_input's and the 32 trunk layers') the BN shift as one block
+    // (hi, lo in k = 0, 1).  The MMAs are cta_group::2: every block is split by output channel between the two CTAs of a
     // pair, and a CTA's share of a weight stage is contiguous: [stage][cta rank 2][blocks][2 k-panels][64 co][8]
     __nv_bfloat16* res_w_2sm;        // [32*9 stages][2][8 blocks]...
     __nv_bfloat16* conv_in_w_2sm;    // [2 stages][2][8 taps]... (16 tap slots, 9 used)

@@ -1,12 +1,10 @@
 // net_auto.cu -- trunk_auto_kernel: ONE launch per evaluator round.  The queue length is only known on the device, and a
 // kernel that exits at once still costs a full kernel boundary (3.4 us under ncu, ~6 us between dependent launches), so
 // the bodies sit behind one device-side branch on the batch size: batches of up to one wave of 5-position groups run
-// tc2::trunk_tc2_body (next layer overlaps the epilogue) -- with cta_group::2 MMAs while a CTA owns a single accumulator
-// tile (up to 2 positions per pair: 147 -> 128 us per forward, the tile's cta_group::1 MMAs saturate shared memory and the
-// weight stream slows them down; with two tiles per CTA the pair form measures the same as cta_group::1, which stays) --,
-// larger ones pp::trunk_pp_body<1> (two groups in flight, cta_group::2 MMAs).  All use 19 warps, clusters of two CTAs and
-// the same grid; shared memory is the largest footprint.  Batches above 7 positions per pair are left to a second launch,
-// trunk_pp_large_kernel (net_pp.cu).
+// tc2::trunk_tc2_body (next layer overlaps the epilogue), larger ones pp::trunk_pp_body<1> (two groups in flight).  Both
+// issue cta_group::2 MMAs on per-CTA weight halves and use 19 warps, clusters of two CTAs and the same grid; shared memory
+// is the larger footprint.  Batches above 7 positions per pair are left to a second launch, trunk_pp_large_kernel
+// (net_pp.cu).
 #include "heads_fc.cuh"
 #include "net_pp_kernel.cuh"
 #include "net_tc2_kernel.cuh"
@@ -14,8 +12,7 @@
 namespace uttt {
 
 static_assert(tc2::Cfg<>::THREADS == pp::THREADS, "one block size for both bodies");
-constexpr int max3(int a, int b, int c) { return a > b ? (a > c ? a : c) : (b > c ? b : c); }
-constexpr int AUTO_SMEM = max3(tc2::Cfg<>::SMEM_BYTES, tc2::Cfg<false, true>::SMEM_BYTES, pp::Cfg<1>::SMEM_BYTES);
+constexpr int AUTO_SMEM = tc2::Cfg<>::SMEM_BYTES > pp::Cfg<1>::SMEM_BYTES ? tc2::Cfg<>::SMEM_BYTES : pp::Cfg<1>::SMEM_BYTES;
 static_assert(HEADS_SMEM_BYTES <= AUTO_SMEM, "the fused heads reuse the trunk's shared memory");
 
 // Slot mode.  With an atomic counter the leaves of a round land in the evaluator queue in arrival order, which differs
@@ -58,16 +55,13 @@ __device__ __forceinline__ void scan_slots(const uint8_t* __restrict__ flags, in
 constexpr int AUTO_SMEM_TOTAL = AUTO_SMEM + 64;                 // + the slot table of the pair and the batch size
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(pp::THREADS, 1)
-trunk_auto_kernel(const __nv_bfloat16* __restrict__ wq, const __nv_bfloat16* __restrict__ wq_in,
-                  const __nv_bfloat16* __restrict__ wq_bias,                      // cta_group::1 packing (net_tc2)
-                  const __nv_bfloat16* __restrict__ wq2, const __nv_bfloat16* __restrict__ wq2_in,
-                  const __nv_bfloat16* __restrict__ wq2_bias,                     // per-CTA halves, 18-block stages (net_pp<1>)
+trunk_auto_kernel(const __nv_bfloat16* __restrict__ res_w8, const __nv_bfloat16* __restrict__ conv_in_w8,     // tc2: 8-block stages
+                  const __nv_bfloat16* __restrict__ res_w18, const __nv_bfloat16* __restrict__ conv_in_w18,   // pp<1>: 18-block stages
+                  const __nv_bfloat16* __restrict__ bias_2sm,     // the bias blocks of both (all per-CTA weight halves)
                   const __nv_bfloat16* __restrict__ planes, const float* __restrict__ headw, float* headfeat, uint4* skip,
                   const int32_t* __restrict__ count, int small_cap, int cap1, long long* dbg,
                   HeadsFC fc, float* policy, float* value /* null: the heads' FC layers are a separate kernel */,
-                  const uint8_t* __restrict__ slot_flags, int n_slots /* slot mode (needs the fused heads), else null */,
-                  const __nv_bfloat16* __restrict__ wq8, const __nv_bfloat16* __restrict__ wq8_in /* per-CTA halves in 8-block
-                  stages (with wq2_bias): */, int pair_cap /* batches of up to pair_cap positions run cta_group::2 MMAs */) {
+                  const uint8_t* __restrict__ slot_flags, int n_slots /* slot mode (needs the fused heads), else null */) {
     extern __shared__ __align__(1024) uint8_t smem[];
     pdl_trigger();          // the next round's tree kernel may be scheduled (it waits for this grid's policy / value rows)
     pdl_wait();             // this round's tree kernel has finished: slot flags / queue length and planes are visible
@@ -91,11 +85,9 @@ trunk_auto_kernel(const __nv_bfloat16* __restrict__ wq, const __nv_bfloat16* __r
     // (with the statements above and the branches below in this order ptxas fits the kernel into 96 registers without
     // spills; the other orders tried spill 32-64 bytes)
     if (!small)
-        pp::trunk_pp_body<1>(wq2, wq2_in, wq2_bias, planes, headw, headfeat, skip, dbg, n_pos, src);
-    else if (n_pos > pair_cap)
-        tc2::trunk_tc2_body<false, false>(wq, wq_in, wq_bias, planes, headw, headfeat, skip, dbg, n_pos, src, 0, false);
+        pp::trunk_pp_body<1>(res_w18, conv_in_w18, bias_2sm, planes, headw, headfeat, skip, dbg, n_pos, src);
     else
-        tc2::trunk_tc2_body<false, true>(wq8, wq8_in, wq2_bias, planes, headw, headfeat, skip, dbg, n_pos, src, 0, false);
+        tc2::trunk_tc2_body<false>(res_w8, conv_in_w8, bias_2sm, planes, headw, headfeat, skip, dbg, n_pos, src, 0, false);
     if (stamp) dbg[201] = clock64();
     if (policy == nullptr) return;
     // Fused heads (the host passes policy / value only if no batch can exceed one group per pair): the pair's head
@@ -130,10 +122,9 @@ cudaError_t launch_trunk_auto(const NetWeights& w, const __nv_bfloat16* planes, 
     const int cap1 = (n_sm / 2) * (pp::Cfg<1>::MAX_PA + pp::Cfg<1>::MAX_PB);
     if (policy && max_rows > cap1) return cudaErrorInvalidValue;
     if (slot_flags && (!policy || n_slots > 32 * SLOT_CHUNKS || n_slots > max_rows)) return cudaErrorInvalidValue;
-    return launch_pdl(trunk_auto_kernel, dim3(2 * pairs), dim3(pp::THREADS), AUTO_SMEM_TOTAL, s, w.res_w_bf16, w.conv_in_w_bf16,
-                      w.bias_blk, w.res_w_2sm18, w.conv_in_w_2sm18, w.bias_blk_2sm, planes, w.head_w, headfeat,
-                      reinterpret_cast<uint4*>(skip), count, small_cap, cap1, dbg, heads_fc_of(w), policy, value, slot_flags, n_slots,
-                      w.res_w_2sm, w.conv_in_w_2sm, 2 * (n_sm / 2));
+    return launch_pdl(trunk_auto_kernel, dim3(2 * pairs), dim3(pp::THREADS), AUTO_SMEM_TOTAL, s, w.res_w_2sm, w.conv_in_w_2sm,
+                      w.res_w_2sm18, w.conv_in_w_2sm18, w.bias_blk_2sm, planes, w.head_w, headfeat, reinterpret_cast<uint4*>(skip),
+                      count, small_cap, cap1, dbg, heads_fc_of(w), policy, value, slot_flags, n_slots);
 }
 
 }  // namespace uttt

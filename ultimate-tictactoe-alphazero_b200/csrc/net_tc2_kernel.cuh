@@ -9,15 +9,14 @@
 // reference's 500-game cycle (about 345 queued leaves per round = 69 groups of 5: one CTA per group would use 69 of 148
 // SMs, a CTA pair per group uses 138).
 //
-// The CTAs exchange the 11-row halo of the 3x3 taps at the split:
+// The MMAs are cta_group::2 pair MMAs issued by the leader CTA (rank 0) for both CTAs (see Cfg).  The CTAs exchange the
+// 11-row halo of the 3x3 taps at the split:
 //   * the epilogue warp that owns the last 11 rows of rank 0 (first 11 rows of rank 1) pushes them into the peer's lead
 //     (tail) margin with bulk shared->shared copies whose bytes complete on the peer's act_ready barrier of its boundary
 //     tile (the peer's boundary warp announces them with expect_tx);
 //   * before it overwrites the peer's margin it waits until the peer's boundary-tile MMAs of the current layer have
-//     retired: the peer's issuer signals that with a multicast tcgen05.commit onto the `bnd_accum` barrier of THIS CTA
-//     (PAIR: the commits of the pair MMAs arrive on both CTAs' accumulator barriers).
-// Without PAIR everything else (weights, accumulators, skip connection, barriers) is CTA-private; with PAIR the leader
-// issues the MMAs of both CTAs (see Cfg).
+//     retired: they are the other half of a pair MMA, whose commit arrives on the accumulator barriers of both CTAs.
+// Rank 1 issues no MMAs: its issuer warps forward its weight-stage and activation barriers to the leader.
 //
 // Warp roles (19 warps): 0-15 epilogue (2 tiles x 4 TMEM lane quarters x 2 column halves -- the epilogue is
 // instruction-latency bound, so it wants warps, not wider threads), 16 weight producer, 17-18 MMA issuers.
@@ -33,22 +32,22 @@ namespace tc2 {
 constexpr int POS_ROWS = 100;
 constexpr int LEAD = 11;
 constexpr int GROUP_LAYERS = NET_LAYERS + 1;     // conv_input runs as layer -1 through the same pipeline
-constexpr uint32_t IDESC = tcx::IDESC_M128_N128_BF16;
 
-// Two accumulator tiles per CTA (LOC_TILES): up to 5 positions per CTA pair (2+2 tiles), 4 weight stages of 32 KiB.
+// Two accumulator tiles per CTA (LOC_TILES): up to 5 positions per CTA pair (2+2 tiles), 8 weight stages of 16 KiB (this
+// CTA's halves of 8 K-blocks).
 // X3 = split-bf16 numerics ("bf16x3", UTTT_EVAL_NET_BF16X3): activations and weights are kept as bf16 hi + lo pairs
 // (lo = bf16(x - hi)) and every K-block costs three MMAs, hi*hi + lo*hi + hi*lo, accumulated in fp32 in TMEM; the skip
 // connection is kept in fp32.  That is ~16 mantissa bits per operand: the mode that meets the reference's fp32 forward
 // (dual_network.py:89-121) within 1e-2 on random-init weights (SURVEY.md H1), at a third of the MMA rate.
-// Shared memory then holds 32 activation panels (16 hi + 16 lo) and a ring of 3 stages of 3 K-blocks (hi + lo = 8 KiB each).
+// Shared memory then holds 32 activation panels (16 hi + 16 lo) and a ring of 3 stages of 6 K-blocks (hi + lo = 4 KiB each).
 //
-// PAIR = the MMAs are cta_group::2 pair MMAs (M = 256: local tile t of the leader CTA and local tile t of its peer, issued by
-// the leader only, as in net_pp_kernel.cuh) and the B operand is split by output channel: each CTA streams and stores HALF
-// of every weight block.  Why: a cta_group::1 MMA of M = N = 128 reads 4 KiB of A and 4 KiB of B per 64 cycles = 128 B/clk,
+// The MMAs are cta_group::2 pair MMAs (M = 256: local tile t of the leader CTA and local tile t of its peer, issued by the
+// leader only, as in net_pp_kernel.cuh) and the B operand is split by output channel: each CTA streams and stores HALF of
+// every weight block.  Why: a cta_group::1 MMA of M = N = 128 reads 4 KiB of A and 4 KiB of B per 64 cycles = 128 B/clk,
 // all the shared-memory bandwidth of an SM, so the weight stream (one-tile groups of the split-bf16 mode: 590 KB per layer)
 // and the epilogue's stores slow the tensor pipe down (tools/micro/mma_shapes.cu, DESIGN.md section 9); a pair MMA reads
-// 4 + 2 KiB per CTA.  Rows are bit-identical to the cta_group::1 form (same K-block order into the same accumulators).
-template <bool X3 = false, bool PAIR = false>
+// 4 + 2 KiB per CTA.
+template <bool X3 = false>
 struct Cfg {
     static constexpr int LOC_TILES = 2;
     static constexpr int MAX_P = 5;
@@ -56,12 +55,12 @@ struct Cfg {
     static constexpr int PANEL_BYTES = AROWS * 16;
     static constexpr int ACT_PANELS = X3 ? 32 : 16;        // channel panels [ci/8][row][8] bf16 (X3: panels 16.. hold the lo parts)
     static constexpr int A_BYTES = (ACT_PANELS + 2) * PANEL_BYTES;      // + the constant panel pair of the bias MMA
-    static constexpr int STAGES = X3 ? 3 : (PAIR ? 8 : 4);
+    static constexpr int STAGES = X3 ? 3 : 8;
     // K-blocks (one K = 16 slice of a layer: 1 MMA per tile, X3: 3) per weight stage.  An issuer thread pays one barrier
     // wait and one commit per stage (200+ cycles each while the tensor pipe saturates shared memory): with 4-block stages
     // a CTA that owns ONE tile (batches of up to 148 positions) was issue-bound at ~93 cycles per MMA
-    static constexpr int STAGE_BLOCKS = X3 ? (PAIR ? 6 : 3) : 8;
-    static constexpr int NCO = PAIR ? 64 : 128;            // output channels of the B operand held by this CTA
+    static constexpr int STAGE_BLOCKS = X3 ? 6 : 8;
+    static constexpr int NCO = 64;                         // output channels of the B operand held by this CTA
     static constexpr int SUB_BYTES = 2 * NCO * 16;         // one [2 k-panels][NCO co][8] bf16 block
     static constexpr int BLOCK_BYTES = (X3 ? 2 : 1) * SUB_BYTES;   // (X3: hi block, then lo block)
     static constexpr int BIAS_BLOCK_BYTES = SUB_BYTES;     // the BN shift as one block: bf16 hi + lo (+ lo2) in k = 0, 1 (, 2)
@@ -98,11 +97,11 @@ __host__ __device__ inline int group_positions(int n_pos, int n_pairs) {
 // the kernel body (a __device__ function: trunk_auto_kernel, net_auto.cu, puts it behind a device-side dispatch together
 // with pp::trunk_pp_body; trunk_x3_kernel, net_tc2.cu, runs it once per group).  The caller has read the batch size and
 // counted it (count_batch).
-// (PAIR: the three weight arrays hold per-CTA halves, stage-major: [stage][2 ranks][STAGE_BLOCKS blocks]([hi, lo])[2][64][8])
-template <bool X3, bool PAIR>
-__device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__ wq,   // [32][72 K-blocks][2][128][8] bf16 (X3: [32][72][hi, lo][2][128][8])
-                 const __nv_bfloat16* __restrict__ wq_in,// conv_input: [16 tap slots (9 used)][2][128][8] bf16 (X3: [9 taps][hi, lo][2][128][8])
-                 const __nv_bfloat16* __restrict__ wq_bias,   // [33][2][128][8] bf16: per layer the BN shift as a K=16 B block
+// The three weight arrays hold per-CTA halves, stage-major: [stage][2 ranks][STAGE_BLOCKS blocks]([hi, lo])[2][64][8].
+template <bool X3>
+__device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__ wq,   // [32 * 72 / STAGE_BLOCKS stages]...: 72 K-blocks per layer
+                 const __nv_bfloat16* __restrict__ wq_in,// conv_input: [IN_STAGES]...: one K-block per tap (9 of IN_STAGES * STAGE_BLOCKS used)
+                 const __nv_bfloat16* __restrict__ wq_bias,   // [33][2 ranks][1 block]...: per layer the BN shift as a K=16 B block
                  const __nv_bfloat16* __restrict__ planes,   // network input [rows][3][81] bf16
                  const float* __restrict__ headw,        // [3][128] policy conv (2) + value conv, BN scale folded; [384..386] shifts
                  float* headfeat,                        // out: [rows][243] = relu(policy conv)[2][81], relu(value conv)[81]
@@ -112,7 +111,7 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                  const int* src_rows,                    // slot mode: position i of this CTA pair reads planes row src_rows[i], else null
                  int pos_base, bool solo) {              // solo: this CTA pair alone evaluates the n_pos positions that start
                                                          // at row pos_base of planes / headfeat (trunk_x3_kernel)
-    using C = Cfg<X3, PAIR>;
+    using C = Cfg<X3>;
     constexpr int LOC_TILES = C::LOC_TILES, PANEL_BYTES = C::PANEL_BYTES, A_BYTES = C::A_BYTES,
                   STAGES = C::STAGES, BAR_OFF = C::BAR_OFF, EPI_WARPS = C::EPI_WARPS, THREADS = C::THREADS,
                   SKIP_ROWS = C::SKIP_ROWS, NQ = C::NQ, STAGE_BLOCKS = C::STAGE_BLOCKS, STAGE_BYTES = C::STAGE_BYTES,
@@ -137,44 +136,37 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
     const uint32_t sA_u = smem_u32(sA);
     const uint32_t sB_u = sA_u + A_BYTES;
     const uint32_t bar_u = sA_u + BAR_OFF;
-    // barriers: full[STAGES], empty[STAGES], accum[LOC_TILES], act[LOC_TILES][NQ], bnd_accum; then the tmem base holder
+    // barriers: full[STAGES], empty[STAGES], accum[LOC_TILES], act[LOC_TILES][NQ]; then the tmem base holder
     const uint32_t bar_full = bar_u, bar_empty = bar_u + 8 * STAGES, bar_accum = bar_u + 16 * STAGES,
-                   bar_act = bar_accum + 8 * LOC_TILES, bar_bnd = bar_act + 8 * LOC_TILES * NQ;
-    static_assert(16 * STAGES + 8 * LOC_TILES * (1 + NQ) + 8 + 4 <= 256, "barrier block");
-    uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(smem + BAR_OFF + 16 * STAGES + 8 * LOC_TILES * (1 + NQ) + 8);
+                   bar_act = bar_accum + 8 * LOC_TILES;
+    constexpr int N_BARS = 2 * STAGES + LOC_TILES * (1 + NQ);
+    static_assert(8 * N_BARS + 4 <= 256, "barrier block");
+    uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(smem + BAR_OFF + 8 * N_BARS);
     // the tile of this CTA that touches the peer's rows, and the quarter-warp that owns the shared rows
     const int bnd_tile = (rank == 0) ? tiles - 1 : 0;
     const int bnd_quarter = (rank == 0) ? 3 : 0;
 
     if (threadIdx.x == 0) {
         for (int i = 0; i < STAGES; i++) {
-            // PAIR: the leader's full barrier also counts the peer's forwarded "my half has landed"; a stage is released in
+            // the leader's full barrier also counts the peer's forwarded "my half has landed"; a stage is released in
             // both CTAs by the multicast commits of the leader's T0 issuers
-            mbar_init(bar_full + 8 * i, (PAIR && rank == 0) ? 2 : 1);
-            mbar_init(bar_empty + 8 * i, PAIR ? T0 : (tiles > 0 ? tiles : 1));
+            mbar_init(bar_full + 8 * i, rank == 0 ? 2 : 1);
+            mbar_init(bar_empty + 8 * i, T0);
         }
         for (int t = 0; t < LOC_TILES; t++) {
             mbar_init(bar_accum + 8 * t, 1);
             int c = 8 + (t > 0 ? 2 : 0) + (t < tiles - 1 ? 2 : 0);      // (the peer's halo rows arrive as transaction bytes)
-            if (PAIR && rank == 0 && t < T1) c += 1;                    // the peer's forwarded "my rows of tile pair t are in place"
+            if (rank == 0 && t < T1) c += 1;                            // the peer's forwarded "my rows of tile pair t are in place"
             for (int q = 0; q < NQ; q++) mbar_init(bar_act + 8 * (t * NQ + q), c);
         }
-        mbar_init(bar_bnd, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == EPI_WARPS + 1) {
-        if constexpr (PAIR) {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_holder)),
-                         "r"(C::TMEM_COLS)
-                         : "memory");
-            if (!solo) asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_holder)),
-                         "r"(C::TMEM_COLS)
-                         : "memory");
-            // (solo: the body runs again in this launch and allocates again -- a CTA that gave up its permit may not)
-            if (!solo) asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_holder)),
+                     "r"(C::TMEM_COLS)
+                     : "memory");
+        // (solo: the body runs again in this launch and allocates again -- a CTA that gave up its permit may not)
+        if (!solo) asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
     }
     for (int i = threadIdx.x; i < A_BYTES / 16; i += THREADS) reinterpret_cast<uint4*>(sA)[i] = make_uint4(0, 0, 0, 0);
     __syncthreads();
@@ -279,12 +271,9 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                 mbar_wait_spin<false>(bar_accum + 8 * lt, lpar);
                 if (nb_lo) mbar_wait_spin<false>(bar_accum + 8 * (lt - 1), lpar);
                 if (nb_hi) mbar_wait_spin<false>(bar_accum + 8 * (lt + 1), lpar);
-                // the peer's boundary-tile MMAs have retired (PAIR: they are the other half of the pair MMAs of index 0 -- rank
-                // 1's first tile -- or T0 - 1 -- rank 0's last tile --, whose multicast commits arrive on this CTA's barrier)
-                if (bnd) {
-                    if constexpr (PAIR) mbar_wait_spin<false>(bar_accum + 8 * ((rank == 0) ? 0 : T0 - 1), lpar);
-                    else mbar_wait_spin<false>(bar_bnd, lpar);
-                }
+                // the peer's boundary-tile MMAs have retired: they are the other half of the pair MMAs of index 0 -- rank
+                // 1's first tile -- or T0 - 1 -- rank 0's last tile --, whose multicast commits arrive on this CTA's barrier
+                if (bnd) mbar_wait_spin<false>(bar_accum + 8 * ((rank == 0) ? 0 : T0 - 1), lpar);
                 if (dbg && blockIdx.x == 0 && iter == 0 && threadIdx.x == 0 && layer >= 0) dbg[layer * 4 + 2] = clock64();
                 const bool detail = dbg && blockIdx.x == 0 && iter == 0 && threadIdx.x == 0 && layer == 20;   // diagnostics: dbg[160..175]
                 if (detail) dbg[160] = clock64();
@@ -381,7 +370,7 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
             tc_fence_before();
         } else if (warp == EPI_WARPS) {
             // ================= weight producer =================
-            if (PAIR ? (T0 == 0) : (tiles == 0)) continue;      // (PAIR: the peer's half of the B operand is needed whatever it owns)
+            // (also in a CTA that owns no tile: the leader's pair MMAs read this CTA's half of every B operand)
             int gn = iter * GROUP_STAGES;
 #pragma unroll 1
             for (int layer = -1; layer < NET_LAYERS; layer++) {
@@ -394,11 +383,10 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                     if (lane == 0) {
                         const __nv_bfloat16* src;
                         uint32_t bytes = STAGE_BYTES;
-                        constexpr int RK = PAIR ? 2 : 1;           // per-CTA halves are stored stage-major: [stage][rank]
-                        const int rk = PAIR ? (int)rank : 0;
-                        if (st == 0) { src = wq_bias + (size_t)((layer + 1) * RK + rk) * (C::BIAS_BLOCK_BYTES / 2); bytes = C::BIAS_BLOCK_BYTES; }   // (sizes in bf16 elements)
-                        else if (layer < 0) src = wq_in + (size_t)((st - 1) * RK + rk) * (STAGE_BYTES / 2);
-                        else src = wq + (size_t)((layer * STAGES_PER_LAYER + st - 1) * RK + rk) * (STAGE_BYTES / 2);
+                        const int rk = (int)rank;          // per-CTA halves are stored stage-major: [stage][rank]
+                        if (st == 0) { src = wq_bias + (size_t)((layer + 1) * 2 + rk) * (C::BIAS_BLOCK_BYTES / 2); bytes = C::BIAS_BLOCK_BYTES; }   // (sizes in bf16 elements)
+                        else if (layer < 0) src = wq_in + (size_t)((st - 1) * 2 + rk) * (STAGE_BYTES / 2);
+                        else src = wq + (size_t)((layer * STAGES_PER_LAYER + st - 1) * 2 + rk) * (STAGE_BYTES / 2);
                         mbar_expect_tx(bar_full + 8 * stage, bytes);
                         bulk_g2s(sB_u + stage * STAGE_BYTES, src, bytes, bar_full + 8 * stage);
                     }
@@ -411,56 +399,48 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
             // MMA before it becomes the bottleneck.  Its loop is therefore unrolled over the 18 weight stages of a layer
             // (all K-block offsets are immediates), keeps stage / parity as running counters and waits without back-off.
             const int lt = warp - (EPI_WARPS + 1);
-            if constexpr (PAIR) {
-                if (rank != 0) {
-                    // rank 1 has no MMAs to issue (the leader issues for the pair): its two issuer warps forward its barriers
-                    // to the leader with CTA-scope remote arrives (see net_pp_kernel.cuh).  Warp 0: "my half of weight stage i
-                    // has landed"; warp 1: "chunk q of my rows of tile pair t is in place".  Neither can be lapped: the
-                    // events they wait for need the leader's next MMAs, which need their arrive.
-                    if (lt == 0) {
-                        int gn = iter * GROUP_STAGES;
+            if (rank != 0) {
+                // rank 1 has no MMAs to issue (the leader issues for the pair): its two issuer warps forward its barriers
+                // to the leader with CTA-scope remote arrives (see net_pp_kernel.cuh).  Warp 0: "my half of weight stage i
+                // has landed"; warp 1: "chunk q of my rows of tile pair t is in place".  Neither can be lapped: the
+                // events they wait for need the leader's next MMAs, which need their arrive.
+                if (lt == 0) {
+                    int gn = iter * GROUP_STAGES;
 #pragma unroll 1
-                        for (int i = 0; i < GROUP_STAGES; i++, gn++) {
-                            const int stage = gn % STAGES;
-                            mbar_wait_spin<false>(bar_full + 8 * stage, (uint32_t)((gn / STAGES) & 1));
-                            if (lane == 0) mbar_arrive_peer(map_to_rank(bar_full + 8 * stage, 0));
-                            __syncwarp();
-                        }
-                    } else if (lt == 1) {
-#pragma unroll 1
-                        for (int layer = -1; layer < NET_LAYERS; layer++) {
-                            const uint32_t apar = (uint32_t)((iter * GROUP_LAYERS + layer + 1) & 1);
-#pragma unroll 1
-                            for (int q = 0; q < NQ; q++)
-#pragma unroll 1
-                                for (int t = 0; t < T1; t++) {
-                                    mbar_wait_spin<false>(bar_act + 8 * (t * NQ + q), apar);
-                                    if (lane == 0) mbar_arrive_peer(map_to_rank(bar_act + 8 * (t * NQ + q), 0));
-                                    __syncwarp();
-                                }
-                        }
+                    for (int i = 0; i < GROUP_STAGES; i++, gn++) {
+                        const int stage = gn % STAGES;
+                        mbar_wait_spin<false>(bar_full + 8 * stage, (uint32_t)((gn / STAGES) & 1));
+                        if (lane == 0) mbar_arrive_peer(map_to_rank(bar_full + 8 * stage, 0));
+                        __syncwarp();
                     }
-                    continue;
+                } else if (lt == 1) {
+#pragma unroll 1
+                    for (int layer = -1; layer < NET_LAYERS; layer++) {
+                        const uint32_t apar = (uint32_t)((iter * GROUP_LAYERS + layer + 1) & 1);
+#pragma unroll 1
+                        for (int q = 0; q < NQ; q++)
+#pragma unroll 1
+                            for (int t = 0; t < T1; t++) {
+                                mbar_wait_spin<false>(bar_act + 8 * (t * NQ + q), apar);
+                                if (lane == 0) mbar_arrive_peer(map_to_rank(bar_act + 8 * (t * NQ + q), 0));
+                                __syncwarp();
+                            }
+                    }
                 }
+                continue;
             }
             if (lt >= tiles) continue;
             const bool leader = elect_one();
             const uint32_t a_tile = sA_u + (uint32_t)(LEAD + lt * 128) * 16u;
-            const bool signal_peer = !PAIR && has_peer && (lt == bnd_tile);
-            constexpr uint32_t idesc = PAIR ? tcx::IDESC_M256_N128_BF16 : IDESC;
             const uint64_t a_desc = make_desc(a_tile, PANEL_BYTES, 128);         // + (row shift + panel offset) / 16: shared
             const uint64_t b_desc = make_desc(sB_u, C::NCO * 16, 128);           //   addresses are < 256 KiB, no carry
             const uint64_t bias_a = a_desc + (uint64_t)((uint32_t)ACT_PANELS * PANEL_BYTES / 16u);
             constexpr uint64_t A_LO = (uint64_t)(16u * PANEL_BYTES / 16u);      // X3: descriptor offset of the lo panels
             constexpr uint64_t B_BLK = (uint64_t)(BLOCK_BYTES / 16), B_LO = (uint64_t)(C::SUB_BYTES / 16); // per K-block / X3: of its lo half
-            // one MMA of this tile (PAIR: of this tile and the peer's tile of the same index)
-            auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t acc) {
-                if constexpr (PAIR) umma_bf16_2sm(d, a, b, idesc, acc);
-                else umma_bf16(d, a, b, idesc, acc);
-            };
+            // one MMA of this tile and the peer's tile of the same index
+            auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t acc) { umma_bf16_2sm(d, a, b, IDESC_M256_N128_BF16, acc); };
             auto commit_accum = [&]() {            // the layer's accumulator is complete when the MMAs issued so far retire
-                if constexpr (PAIR) umma_commit_2sm(bar_accum + 8 * lt, (uint16_t)3);
-                else umma_commit(bar_accum + 8 * lt);
+                umma_commit_2sm(bar_accum + 8 * lt, (uint16_t)3);                            // (in both CTAs)
             };
             int gn = iter * GROUP_STAGES;
             int stage = gn % STAGES;
@@ -477,8 +457,7 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                 b_st = b_desc + (uint64_t)(uint32_t)(stage * (STAGE_BYTES / 16));
             };
             auto release_stage = [&]() {           // leader only: frees the stage when the MMAs issued so far retire
-                if constexpr (PAIR) umma_commit_2sm(bar_empty + 8 * stage, (uint16_t)3);       // (in both CTAs)
-                else umma_commit(bar_empty + 8 * stage);
+                umma_commit_2sm(bar_empty + 8 * stage, (uint16_t)3);                         // (in both CTAs)
             };
             auto advance = [&]() {
                 if (++stage == STAGES) { stage = 0; par ^= 1u; }
@@ -517,10 +496,7 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                                 }
                             }
                             release_stage();
-                            if (s == IN_STAGES - 1) {
-                                commit_accum();
-                                if (signal_peer) umma_commit_mcast(bar_bnd, (uint16_t)(1u << peer));
-                            }
+                            if (s == IN_STAGES - 1) commit_accum();
                         }
                         advance();
                     }
@@ -552,7 +528,6 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                             release_stage();
                             if (s == STAGES_PER_LAYER - 1) {
                                 commit_accum();
-                                if (signal_peer) umma_commit_mcast(bar_bnd, (uint16_t)(1u << peer));
                                 if (dbg && blockIdx.x == 0 && iter == 0 && lt == 0) dbg[layer * 4 + 1] = clock64();
                                 if (dbg && blockIdx.x == 0 && iter == 0 && lt == 0 && layer == 20) dbg[172] = clock64();
                             }
@@ -569,12 +544,11 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
     tc_fence_before();
     __syncthreads();
     cluster_sync_all();                 // nobody exits while the peer may still write its margins / barriers
-    if (warp == EPI_WARPS + 1) {
-        if constexpr (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::TMEM_COLS) : "memory");
-        else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::TMEM_COLS) : "memory");
-    }
+    if (warp == EPI_WARPS + 1)
+        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::TMEM_COLS) : "memory");
     if (solo && threadIdx.x == 0) {     // the body runs again in this launch: leave no valid mbarrier objects behind
-        for (uint32_t b = bar_u; b < bar_bnd + 8; b += 8) asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(b) : "memory");
+#pragma unroll
+        for (int i = 0; i < N_BARS; i++) asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(bar_u + 8 * i) : "memory");
     }
     if (dbg && blockIdx.x == 0 && threadIdx.x == 0) dbg[195] = clock64();
 }

@@ -11,22 +11,12 @@
 namespace uttt {
 namespace tcx {
 
-// instruction descriptor (kind::f16): D=f32 (bit 4), A=B=bf16 (bits 7,10), K-major A and B, N=128, M=128
-constexpr uint32_t IDESC_M128_N128_BF16 = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
-
 // K order of a 3x3 layer: 72 blocks of K = 16 (one MMA each).  Block m = 18*q + 2*tap + h multiplies tap `tap` of
 // the 16 input channels of unit u = q + 4h (channels 16u .. 16u+15).  The order is channel-quarter-major: an epilogue
 // warp writes units 0..3 (column half 0) or 4..7 (column half 1) in that order, so the blocks of quarter q only need
 // the q-th 16-column chunk of every epilogue warp -- the next layer's MMAs start while the epilogue is still running.
 // The pre-packed weights (pack_res_kernel, weights.cu) are stored in the same order, 4 KiB per block.
 __host__ __device__ __forceinline__ int kblock_of(int tap, int unit) { return 18 * (unit & 3) + 2 * tap + (unit >> 2); }
-__device__ __forceinline__ void kblock_decode(int m, int& q, int& tap, int& unit) {
-    q = m / 18;
-    int r = m - 18 * q;
-    tap = r >> 1;
-    unit = q + 4 * (r & 1);
-}
-__device__ __forceinline__ int tap_shift(int tap) { return (tap / 3 - 1) * 10 + (tap % 3 - 1); }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
@@ -39,9 +29,6 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
@@ -49,11 +36,6 @@ __device__ __forceinline__ uint32_t map_to_rank(uint32_t local_addr, uint32_t ra
     uint32_t r;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(rank));
     return r;
-}
-__device__ __forceinline__ void st_cluster_v4(uint32_t cluster_addr, const uint4& v) {
-    asm volatile("st.shared::cluster.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(cluster_addr), "r"(v.x), "r"(v.y), "r"(v.z),
-                 "r"(v.w)
-                 : "memory");
 }
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
@@ -145,28 +127,11 @@ __device__ __forceinline__ void bulk_s2peer(uint32_t dst_cluster, uint32_t src_c
 }
 __device__ __forceinline__ void fence_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_dsmem() { asm volatile("fence.proxy.async.shared::cluster;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// arrive on the barrier at the same shared-memory offset in every CTA of `mask`
-__device__ __forceinline__ void umma_commit_mcast(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(mask)
-                 : "memory");
-}
 // cta_group::2: one MMA of M = 256 over the CTA pair (128 rows from each CTA's shared memory at the same offsets, the B
-// operand split by N between the two CTAs); issued by the leader CTA only
+// operand split by N between the two CTAs); issued by the leader CTA only.  Instruction descriptor (kind::f16): D = f32
+// (bit 4), A = B = bf16 (bits 7, 10), K-major A and B, N = 128, M = 256
 constexpr uint32_t IDESC_M256_N128_BF16 = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((256u >> 4) << 24);
 __device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
     asm volatile(
@@ -205,24 +170,8 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t*>(&h);
 }
-__device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {
-    __half2 h = __floats2half2_rn(fminf(lo, 65504.0f), fminf(hi, 65504.0f));
-    return *reinterpret_cast<uint32_t*>(&h);
-}
-__device__ __forceinline__ void f16x8_add(const uint4& q, float* v) {
-    const __half2* h = reinterpret_cast<const __half2*>(&q);
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-        float2 f = __half22float2(h[i]);
-        v[2 * i] += f.x;
-        v[2 * i + 1] += f.y;
-    }
-}
 __device__ __forceinline__ uint4 pack8_bf16(const float* v) {
     return make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
-}
-__device__ __forceinline__ uint4 pack8_f16(const float* v) {
-    return make_uint4(pack_f16x2(v[0], v[1]), pack_f16x2(v[2], v[3]), pack_f16x2(v[4], v[5]), pack_f16x2(v[6], v[7]));
 }
 // v[0..3] += 4 fp32 values
 __device__ __forceinline__ void f32x4_add(const uint4& q, float* v) {

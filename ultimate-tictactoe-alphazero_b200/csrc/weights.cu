@@ -31,8 +31,8 @@ __host__ __device__ __forceinline__ size_t half_unit(int b, int sub, int pnl, in
 }
 
 // Folding and packing of the 32 residual 3x3 convolutions: raw (32)(co,ci,ky,kx) fp32 + bn (32)(4)(128) ->
-// fp32 [l][tap][ci][co] and shift [l][co], bf16 [l][K-block][ci/8 % 2][co][ci%8] (K-blocks in the order of
-// tcx::kblock_of), and its per-CTA halves in stages of 8 and 18 blocks and, with lo = bf16(w - hi), of 6 blocks.
+// fp32 [l][tap][ci][co] and shift [l][co], and bf16 blocks [l][K-block][ci/8 % 2][co][ci%8] (K-blocks in the order of
+// tcx::kblock_of) as per-CTA halves in stages of 8 and 18 blocks and, with lo = bf16(w - hi), of 6 blocks.
 __global__ void __launch_bounds__(256) pack_res_kernel(NetWeights w) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;      // index into raw
     if (i >= N_RES) return;
@@ -49,7 +49,6 @@ __global__ void __launch_bounds__(256) pack_res_kernel(NetWeights w) {
     w.res_w[(((size_t)l * 9 + tap) * 128 + ci) * 128 + co] = val;
     const int blk = l * 72 + tcx::kblock_of(tap, ci / 16), pnl = (ci / 8) & 1, k = ci % 8;
     const __nv_bfloat16 hi = __float2bfloat16(val);
-    w.res_w_bf16[(((size_t)blk * 2 + pnl) * 128 + co) * 8 + k] = hi;
     w.res_w_2sm[half_unit(blk, 0, pnl, co, 8, 1) * 8 + k] = hi;
     w.res_w_2sm18[half_unit(blk, 0, pnl, co, 18, 1) * 8 + k] = hi;
     w.res_w_x3p[half_unit(blk, 0, pnl, co, 6, 2) * 8 + k] = hi;
@@ -67,16 +66,15 @@ size_t carve(NetWeights& w, uintptr_t base, size_t& host_bytes) {
         off += (n * sizeof(*p) + 255) / 256 * 256;
     };
     at(w.conv_in_w, 9 * 3 * 128); at(w.conv_in_b, 128);
-    at(w.conv_in_w_bf16, 16 * BLK); at(w.conv_in_w_2sm, 16 * BLK); at(w.conv_in_w_2sm18, 18 * BLK);
-    at(w.conv_in_w_x3p, 12 * 2 * BLK);
-    at(w.bias_blk, 33 * BLK); at(w.bias_blk_2sm, 33 * BLK); at(w.bias_blk_x3p, 33 * BLK);
+    at(w.conv_in_w_2sm, 16 * BLK); at(w.conv_in_w_2sm18, 18 * BLK); at(w.conv_in_w_x3p, 12 * 2 * BLK);
+    at(w.bias_blk_2sm, 33 * BLK); at(w.bias_blk_x3p, 33 * BLK);
     at(w.head_w, 387); at(w.heads_pack, HEADS_PACK_FLOATS);
     at(w.pol_fc_w, 162 * 81); at(w.pol_fc_b, 81); at(w.val_fc1_w, 81 * 256); at(w.val_fc1_b, 256);
     at(w.val_fc2_w, 256); at(w.val_fc2_b, 1);
     host_bytes = off;
     at(w.raw_res, N_RES); at(w.raw_res_bn, N_RES_BN);
     at(w.res_w, N_RES); at(w.res_b, NET_LAYERS * 128);
-    at(w.res_w_bf16, N_RES); at(w.res_w_2sm, N_RES); at(w.res_w_2sm18, N_RES); at(w.res_w_x3p, 2 * N_RES);
+    at(w.res_w_2sm, N_RES); at(w.res_w_2sm18, N_RES); at(w.res_w_x3p, 2 * N_RES);
     return off;
 }
 
@@ -149,15 +147,13 @@ int upload_weights(NetWeights& W, const uttt_weights* w, int on_device, const fl
     bn_fold(bni.data(), 128, sc, sh);
     float* ci_w = host(W.conv_in_w);
     memcpy(host(W.conv_in_b), sh.data(), 128 * sizeof(float));
-    __nv_bfloat16 *c16 = host(W.conv_in_w_bf16), *c8 = host(W.conv_in_w_2sm), *c18 = host(W.conv_in_w_2sm18),
-                  *cx3 = host(W.conv_in_w_x3p);
+    __nv_bfloat16 *c8 = host(W.conv_in_w_2sm), *c18 = host(W.conv_in_w_2sm18), *cx3 = host(W.conv_in_w_x3p);
     for (int co = 0; co < 128; co++)
         for (int ci = 0; ci < 3; ci++)
             for (int tap = 0; tap < 9; tap++) {
                 const float v = ciw[(co * 3 + ci) * 9 + tap] * sc[co];
                 ci_w[(tap * 3 + ci) * 128 + co] = v;
                 const __nv_bfloat16 hi = __float2bfloat16(v);
-                c16[((size_t)tap * 2 * 128 + co) * 8 + ci] = hi;
                 c8[half_unit(tap, 0, 0, co, 8, 1) * 8 + ci] = hi;
                 c18[half_unit(tap, 0, 0, co, 18, 1) * 8 + ci] = hi;
                 cx3[half_unit(tap, 0, 0, co, 6, 2) * 8 + ci] = hi;
@@ -197,16 +193,13 @@ int upload_weights(NetWeights& W, const uttt_weights* w, int on_device, const fl
     memcpy(shift.data(), host(W.conv_in_b), 128 * sizeof(float));
     UTTT_CUDA_OK(cudaMemcpyAsync(shift.data() + 128, W.res_b, 32 * 128 * sizeof(float), cudaMemcpyDeviceToHost, s));
     UTTT_CUDA_OK(cudaStreamSynchronize(s));
-    __nv_bfloat16 *bb = host(W.bias_blk), *bb2 = host(W.bias_blk_2sm), *bx3 = host(W.bias_blk_x3p);
+    __nv_bfloat16 *bb2 = host(W.bias_blk_2sm), *bx3 = host(W.bias_blk_x3p);
     for (int l = 0; l < 33; l++)
         for (int co = 0; co < 128; co++) {
             float b = shift[l * 128 + co];
             for (int k = 0; k < 3; k++) {
                 const __nv_bfloat16 t = __float2bfloat16(b);
-                if (k < 2) {
-                    bb[((size_t)l * 2 * 128 + co) * 8 + k] = t;
-                    bb2[half_unit(l, 0, 0, co, 1, 1) * 8 + k] = t;
-                }
+                if (k < 2) bb2[half_unit(l, 0, 0, co, 1, 1) * 8 + k] = t;
                 bx3[half_unit(l, 0, 0, co, 1, 1) * 8 + k] = t;
                 b -= __bfloat162float(t);
             }
