@@ -9,6 +9,8 @@ Tolerance (BASELINE.json north_star): |policy - ref| <= 1e-2, |value - ref| <= 1
     ill-conditioned (SURVEY.md H1: logits reach +-400, fp32 softmax is one-hot) and plain bf16 operands
     cannot meet 1e-2 on every position -- there we assert argmax agreement and the exceed fraction and
     print the statistics instead of silently loosening the bound.
+    The damped copy's policy is close to uniform, so 1e-2 there is a smoke check, not the accuracy test: every forward
+    path is compared row by row, in logit space, with a float64 emulation of its rounding in tests/test_gpu_net_reference.py.
 """
 import os
 
