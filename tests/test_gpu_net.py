@@ -319,7 +319,7 @@ def test_trunk_variant_boundaries_give_identical_rows(setup):
     net_auto.cu): one group per CTA pair up to 370 positions (net_tc2), two groups in flight above (net_pp), both with
     cta_group::2 MMAs on per-CTA weight halves.  All of them accumulate a row in the
     same order: bit-identical rows -- including the one-tile group of the 6/7-positions-per-pair case (371..518
-    positions), whose weight stages are issued by two threads in turn into one accumulator."""
+    positions), whose weight stages are issued by one thread in quarter layers."""
     import copy
     import engine
     e, model, sts = setup
@@ -420,22 +420,31 @@ def test_profile_levels_and_identical_play(setup):
 
 
 def test_network_selfplay_is_reproducible_run_to_run(setup):
-    """Slot mode (net_auto.cu): with up to 518 concurrent games the leaves of a round are ordered by slot, not by their
-    arrival at an atomic counter, and the first games go to the slots in slot order -- so which leaves fall into the
-    split-K group of the large-batch trunk, and therefore every bit of the run, is a function of the seed alone.
-    420 games keep the batches in the 371..518 band where that group exists."""
+    """Every bit of a self-play run is a function of the seed: the leaves of a round claim their evaluator rows in the
+    order the warps arrive at an atomic counter, which differs from run to run, but a row does not depend on its place
+    in the batch and each tree reads back its own row.  420 games on 420 slots keep the batches in the 371..518 band
+    (the one-tile group of trunk_pp_body<1>); 200 games on 160 slots recycle slots (later games are claimed in arrival
+    order too) and run two lanes, each with its own queue."""
     import engine
     e, model, sts = setup
-    eng = engine.Engine(n_slots=420, max_sims=16, max_batch=8, max_games=420)
-    try:
-        eng.upload_model(model)
-        runs = []
-        for _ in range(3):
-            h = eng.selfplay(420, sims=16, batch=8, seed=5, evaluator=engine.EVAL_NET_BF16)
-            runs.append((h.lens.copy(), h.actions.copy(), h.counts.copy()))
-        hist = eng.batch_histogram()
-        assert hist[24:33].sum() > 0, hist             # launches with 384..527 positions did occur
-        for other in runs[1:]:
-            assert all((a == b).all() for a, b in zip(runs[0], other))
-    finally:
-        eng.close()
+    for slots, games, n_runs, lane_threshold in ((420, 420, 3, None), (160, 200, 2, "100")):
+        if lane_threshold:
+            os.environ["UTTT_LANE_THRESHOLD"] = lane_threshold
+        try:
+            eng = engine.Engine(n_slots=slots, max_sims=16, max_batch=8, max_games=games)
+        finally:
+            os.environ.pop("UTTT_LANE_THRESHOLD", None)
+        try:
+            eng.upload_model(model)
+            runs = []
+            for _ in range(n_runs):
+                h = eng.selfplay(games, sims=16, batch=8, seed=5, evaluator=engine.EVAL_NET_BF16)
+                assert (h.lens > 0).all()
+                runs.append((h.lens.copy(), h.actions.copy(), h.counts.copy()))
+            if games == 420:
+                hist = eng.batch_histogram()
+                assert hist[24:33].sum() > 0, hist             # launches with 384..527 positions did occur
+            for other in runs[1:]:
+                assert all((a == b).all() for a, b in zip(runs[0], other)), (slots, games)
+        finally:
+            eng.close()

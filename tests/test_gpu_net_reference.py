@@ -9,8 +9,8 @@ on the calibrated weight set (net_reference.calibrated: logits of standard devia
 gammas, running variances from 1e-3 to 10) and, for bf16 and bf16x3, the seed-0 random init.
 
 uttt_net_forward cuts a batch into calls of at most n_slots rows, and each call picks its path from its row count m
-(engine.cu run_evaluator, net_auto.cu): bf16 m <= 370 trunk_auto_kernel's tc2 body, 371..518 its pp<1> body (one-tile
-split-K group), both with the heads' FC layers fused into the kernel's tail; m > 518 trunk_pp_large_kernel and the
+(engine.cu run_evaluator, net_auto.cu): bf16 m <= 370 trunk_auto_kernel's tc2 body, 371..518 its pp<1> body (two
+groups per CTA pair), both with the heads' FC layers fused into the kernel's tail; m > 518 trunk_pp_large_kernel and the
 separate heads_fc_kernel.  bf16x3: trunk_x3_kernel, one wave of 74 groups of <= 5 positions per 370 rows, then
 heads_fc_kernel.  fp32: conv3x3_fp32_kernel and the fp32 heads.  (On a B200: 148 SMs, 74 CTA pairs.)
 

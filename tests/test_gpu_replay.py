@@ -1,7 +1,7 @@
 """GPU: the reference search fed the ENGINE's OWN network rows (north_star: "MCTS visit counts must be bit-exact against
 the reference C++ MCTS when both are fed identical network outputs").
 
-With the network evaluator the leaves never leave the GPU (slot-mode queue -> trunk_auto_kernel -> fused heads -> tree
+With the network evaluator the leaves never leave the GPU (evaluator queue -> trunk_auto_kernel -> fused heads -> tree
 kernel), so the engine records, per evaluated leaf, the policy / value row its tree is about to consume
 (uttt_debug_trace).  Each root is then searched again by UTTT::pv_mcts_scores (cpp/uttt_mcts.cpp:84-196; the compiled
 reference from oracle/_ref when it was built, else the C restatement) with a callback that returns exactly those rows
@@ -68,10 +68,10 @@ def _search_and_replay(e, roots, sims, batch, evaluator, exact_rows, temperature
 
 
 @pytest.mark.parametrize("n_roots", [60, 148, 300, 370, 450, 518])
-def test_slot_mode_search_replays_bit_exactly_in_every_band(nets, n_roots):
-    """UTTT_EVAL_NET_BF16 with up to 518 trees = slot mode + trunk_auto_kernel + fused heads (the benchmarked path):
+def test_benchmarked_path_search_replays_bit_exactly_in_every_band(nets, n_roots):
+    """UTTT_EVAL_NET_BF16 with up to 518 trees = trunk_auto_kernel + fused heads (the benchmarked path):
     <= 148 (one tile per CTA), 149-370 (two tiles), 371-518 (two groups in flight, cta_group::2 MMAs; the one-tile group's
-    weight stages issued by two threads in turn).  The recorded rows equal a stand-alone forward of the same leaves bit for
+    weight stages issued by one thread in quarter layers).  The recorded rows equal a stand-alone forward of the same leaves bit for
     bit in every band: a row's arithmetic does not depend on the batch it was evaluated in."""
     import engine
     model, damped = nets
@@ -83,7 +83,7 @@ def test_slot_mode_search_replays_bit_exactly_in_every_band(nets, n_roots):
         _search_and_replay(e, roots, 50, 8, engine.EVAL_NET_BF16, exact_rows=True)
         hist = e.batch_histogram()
         assert hist[(n_roots - 1) >> 4] + hist[min(63, n_roots >> 4)] > 0, hist      # the band did occur
-        if n_roots > 370:          # the band whose one-tile group is issued by two threads in turn, on a second network
+        if n_roots > 370:          # the band with the one-tile group of trunk_pp_body<1>, on a second network
             e.upload_model(damped)
             _search_and_replay(e, roots, 50, 8, engine.EVAL_NET_BF16, exact_rows=True)
         # other search shapes of the same path
@@ -96,8 +96,7 @@ def test_slot_mode_search_replays_bit_exactly_in_every_band(nets, n_roots):
 @pytest.mark.parametrize("n_roots,evaluator", [(700, "bf16"), (1200, "bf16"), (100, "bf16x3"), (450, "bf16x3"), (800, "bf16x3"),
                                                (64, "fp32")])
 def test_compacted_queue_search_replays_bit_exactly(nets, n_roots, evaluator):
-    """engines above 518 trees (arrival-order queue, 10-positions-per-pair trunk + separate heads kernel), and the
-    bf16x3 / fp32 evaluators (always the arrival-order queue)"""
+    """engines above 518 trees (10-positions-per-pair trunk + separate heads kernel), and the bf16x3 / fp32 evaluators"""
     import engine
     model, _ = nets
     ev = {"bf16": engine.EVAL_NET_BF16, "bf16x3": engine.EVAL_NET_BF16X3, "fp32": engine.EVAL_NET_FP32}[evaluator]
@@ -141,7 +140,7 @@ def test_gating_search_with_network_replays_bit_exactly(nets, evaluator):
 
 
 def test_full_selfplay_cycle_replays_bit_exactly(nets):
-    """BASELINE config 3 as benchmarked (500 concurrent games, 50 simulations, batch 8, bf16 trunk, slot mode): every move
+    """BASELINE config 3 as benchmarked (500 concurrent games, 50 simulations, batch 8, bf16 trunk, fused heads): every move
     of every game is searched again by the reference MCTS fed the rows the engine's network produced for that move's
     leaves; the visit counts in the history must be identical."""
     import engine

@@ -86,7 +86,7 @@ def full(name):
 launches()
 full("trunk2")     # trunk_auto_kernel -> trunk_tc2_body<2> (CTA pair per group, 2 tiles per CTA; batch of 345 positions)
 full("trunkx3")    # trunk_x3_kernel (split-bf16: 3 MMAs per K-block; batch of 500 positions = groups of 5 + 2 per CTA pair)
-full("trunkpp")    # trunk_auto_kernel, launch 200 of a 500-game cycle (slot mode, ~495 positions): trunk_pp_body<1> (two groups in
+full("trunkpp")    # trunk_auto_kernel, launch 200 of a 500-game cycle (~495 positions): trunk_pp_body<1> (two groups in
                    # flight, cta_group::2) + heads FC tail
 full("heads")      # heads_fc_kernel (standalone form of the heads' FC layers; 500 positions, warm L2)
 full("tree")

@@ -117,8 +117,6 @@ struct TreeParams {
     uint8_t* hist_actions;         // [n_games][81]
     int32_t* hist_len;             // [n_games]
     int8_t* hist_final;            // [n_games]
-    uint8_t* slot_flags;           // slot mode (null = off): a leaf stays in row t of the evaluator buffers, slot_flags[t] = the
-                                   // tree queued one this round (trunk_auto_kernel counts and orders them: reproducible runs)
     unsigned long long* dbg_tree;  // diagnostics (null = off): [16 classes][3] = sum of cycles, warps, max cycles per class of
                                    // a tree's round: class = min(terminal descents, 7) + 8 * (a move was decided)
 };
@@ -213,7 +211,6 @@ cudaError_t launch_trunk_pp_large(const NetWeights& w, const __nv_bfloat16* plan
 // one launch for every batch up to trunk_pp_cap1: device-side choice between the bodies of net_tc2_kernel.cuh and net_pp_kernel.cuh
 // (policy / value non-null: the heads' FC layers run in the kernel's tail; requires max_rows <= trunk_pp_cap1)
 cudaError_t launch_trunk_auto(const NetWeights& w, const __nv_bfloat16* planes, float* headfeat, const int32_t* count, int max_rows,
-                              float* skip, int n_sm, cudaStream_t s, long long* dbg, float* policy, float* value,
-                              const uint8_t* slot_flags = nullptr, int n_slots = 0);
+                              float* skip, int n_sm, cudaStream_t s, long long* dbg, float* policy, float* value);
 
 }  // namespace uttt

@@ -58,7 +58,6 @@ struct uttt_engine {
     float* tc_resid;        // [n_sm][32][512][4] fp32 residual stream of the tensor-core trunk (per CTA)
     int32_t* fwd_count;     // device int for uttt_net_forward
     int64_t* hist_offsets;  // [max_games + 1] exclusive prefix sums of the game lengths (uttt_selfplay_pack)
-    uint8_t* slot_flags;    // [n_slots] slot mode of the evaluator queue (see net_auto.cu)
     long long* tc_dbg;      // [32][4] clock64 timeline of trunk CTA 0, then [64] histogram of batch sizes (diagnostics)
     int prof_level;         // self-play kernel timing: 2 = tree / trunk / heads events every round, 1 = trunk only, 0 = none
     int prof_sample;        // level 1: the trunk is bracketed in every prof_sample-th window of rounds only (see uttt_set_profile_level)
@@ -98,8 +97,6 @@ struct EvalBufs {
     const int32_t* nn_k;
     const __nv_bfloat16* nn_planes;
     float *policy, *value, *act_a, *act_b, *resid, *headfeat;
-    const uint8_t* slot_flags;     // non-null: slot mode (the tree kernel left the leaves in their trees' rows)
-    int n_slots;
 };
 
 EvalBufs bufs_of(uttt_engine* e, size_t first_slot, int lane) {
@@ -114,8 +111,6 @@ EvalBufs bufs_of(uttt_engine* e, size_t first_slot, int lane) {
     b.act_b = e->act_b + first_row * 81 * 128;
     b.headfeat = e->headfeat + first_row * 243;
     b.resid = e->tc_resid + (size_t)lane * e->n_sm * 512 * 64;     // fp16 panels: 128 KiB per CTA
-    b.slot_flags = nullptr;
-    b.n_slots = 0;
     return b;
 }
 
@@ -158,10 +153,8 @@ int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_
         // batches above 7 positions per CTA pair (only possible when max_rows allows them) are left to the
         // 10-positions-per-pair kernel; if no batch can exceed that, the heads' FC layers run in the tail of trunk_auto_kernel
         heads_fused = max_rows <= trunk_pp_cap1(e->n_sm);
-        UTTT_CHECK(heads_fused || !b.slot_flags, "slot mode needs the fused heads");
         UTTT_CUDA_OK(launch_trunk_auto(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg,
-                                       heads_fused ? b.policy : nullptr, heads_fused ? b.value : nullptr, b.slot_flags,
-                                       b.n_slots));
+                                       heads_fused ? b.policy : nullptr, heads_fused ? b.value : nullptr));
         if (!heads_fused)
             UTTT_CUDA_OK(launch_trunk_pp_large(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg));
         e->prof_launches[1] += 1;
@@ -186,21 +179,11 @@ int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_
 // Synchronises the stream (diagnostics only).
 int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const int32_t* count, cudaStream_t s) {
     UTTT_CUDA_OK(cudaStreamSynchronize(s));
-    int n_rows = 0;
-    std::vector<uint8_t> flags;
-    std::vector<int32_t> trees;
-    if (b.slot_flags) {
-        n_rows = b.n_slots;
-        flags.resize((size_t)n_rows);
-        UTTT_CUDA_OK(cudaMemcpy(flags.data(), b.slot_flags, (size_t)n_rows, cudaMemcpyDeviceToHost));
-    } else {
-        int32_t n = 0;
-        UTTT_CUDA_OK(cudaMemcpy(&n, count, sizeof(n), cudaMemcpyDeviceToHost));
-        n_rows = n;
-        trees.resize((size_t)n_rows);
-        if (n_rows) UTTT_CUDA_OK(cudaMemcpy(trees.data(), p.nn_tree, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
-    }
+    int32_t n_rows = 0;
+    UTTT_CUDA_OK(cudaMemcpy(&n_rows, count, sizeof(n_rows), cudaMemcpyDeviceToHost));
     if (n_rows == 0) return 0;
+    std::vector<int32_t> trees((size_t)n_rows);
+    UTTT_CUDA_OK(cudaMemcpy(trees.data(), p.nn_tree, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
     std::vector<uint32_t> st((size_t)n_rows * 8);
     std::vector<float> pol((size_t)n_rows * 81), val((size_t)n_rows);
     std::vector<TreeCtl> ctl((size_t)p.n_trees);
@@ -209,8 +192,7 @@ int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const in
     UTTT_CUDA_OK(cudaMemcpy(val.data(), b.value, val.size() * 4, cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(ctl.data(), p.ctl, ctl.size() * sizeof(TreeCtl), cudaMemcpyDeviceToHost));
     for (int r = 0; r < n_rows; r++) {
-        if (b.slot_flags && !flags[r]) continue;
-        const int t = b.slot_flags ? r : trees[r];
+        const int t = trees[r];
         UTTT_CHECK(t >= 0 && t < p.n_trees && ctl[t].phase == PHASE_PENDING && ctl[t].nn_row == r,
                    "trace: row %d does not belong to a pending tree", r);
         uttt_engine::TraceRec rec;
@@ -223,12 +205,6 @@ int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const in
         e->trace.push_back(rec);
     }
     return 0;
-}
-
-// Slot mode (net_auto.cu: reproducible runs with the split-K group of the large-batch trunk): the reference-exact search
-// with the tensor-core evaluator, when one trunk_auto_kernel launch with fused heads covers every possible batch.
-bool slot_mode_applies(uttt_engine* e, int evaluator, bool throughput, int rows) {
-    return evaluator == UTTT_EVAL_NET_BF16 && !throughput && rows <= trunk_pp_cap1(e->n_sm) && rows <= 544;
 }
 
 int check_search_args(uttt_engine* e, int n_roots, int sims, int batch) {
@@ -288,7 +264,7 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
         ealloc(e, &e->value, S * cfg->max_batch) || ealloc(e, &e->scores, S * 81) ||
         ealloc(e, &e->headfeat, R * 243) || ealloc(e, &e->act_a, R * 81 * 128) || ealloc(e, &e->act_b, R * 81 * 128) ||
         ealloc(e, &e->tc_resid, (size_t)N_LANES * e->n_sm * 512 * 64) || ealloc(e, &e->fwd_count, 1) || ealloc(e, &e->tc_dbg, 128 + 64 + 8 + 16) ||
-        ealloc(e, &e->slot_flags, S) || ealloc(e, &e->hist_offsets, G + 1)) {
+        ealloc(e, &e->hist_offsets, G + 1)) {
         uttt_destroy(e);
         return 1;
     }
@@ -395,7 +371,7 @@ static int mcts_begin_impl(uttt_engine* e, const uint32_t* roots, int32_t n_root
     UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
     TreeParams& t = e->tp;
     t.n_trees = n_roots; t.sims = sims; t.batch = batch; t.mode = MODE_SEARCH; t.flags = flags;
-    t.parity = 0; t.row_stride = 1; t.copy_stride = 0; t.slot_flags = nullptr;
+    t.parity = 0; t.row_stride = 1; t.copy_stride = 0;
     e->s_n_roots = n_roots; e->s_sims = sims; e->s_batch = batch; e->s_round = 0; e->s_pending = 0;
     e->s_per_copy = 0; e->s_have_results = 0;
     if (n_roots == 0) return 0;
@@ -488,13 +464,7 @@ int uttt_mcts_search(uttt_engine* e, const uint32_t* roots, int32_t n_roots, int
     // rounds are enqueued without host synchronisation; the tree kernel ignores finished trees.
     // Upper bound on rounds: every round retires >= 1 simulation of every unfinished tree (+ root evaluation).
     const int rows = tp ? n_roots * batch : n_roots;
-    EvalBufs bufs = bufs_of(e, 0, 0);
-    if (slot_mode_applies(e, evaluator, tp, rows)) {
-        UTTT_CUDA_OK(cudaMemsetAsync(e->slot_flags, 0, (size_t)n_roots, e->stream));
-        t.slot_flags = e->slot_flags;
-        bufs.slot_flags = e->slot_flags;
-        bufs.n_slots = n_roots;
-    }
+    const EvalBufs bufs = bufs_of(e, 0, 0);
     int max_rounds = sims + 3;
     int r = 0;
     while (r < max_rounds) {
@@ -590,15 +560,12 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
     t.sims = sims; t.batch = batch; t.mode = MODE_SELFPLAY; t.flags = flags;
     t.parity = 0; t.row_stride = 1; t.copy_stride = 0;
     t.seed = seed; t.game0 = game0; t.n_games = n_games;
-    const bool slots = slot_mode_applies(e, evaluator, tp, n_trees * rows_per_tree);
-    t.slot_flags = slots ? e->slot_flags : nullptr;
     // Two lanes (halves of the slots) run on two streams: each lane is the sequential chain
     // tree_round -> conv_input -> trunk -> heads, so one lane's tree/heads work runs in the shadow of the
     // other lane's trunk (the tree blocks fit beside a trunk CTA on an SM).  Lanes share only the atomic
     // game/progress counters and the history buffers (disjoint rows).
     // (worth it only when half a batch still fills the machine; small batches are latency-bound)
-    // (slot mode addresses the evaluator rows by global slot: one lane)
-    const int n_lanes = (n_trees >= e->lane_threshold && !slots) ? N_LANES : 1;
+    const int n_lanes = (n_trees >= e->lane_threshold) ? N_LANES : 1;
     TreeParams lane_tp[N_LANES];
     EvalBufs lane_bufs[N_LANES];
     int lane_trees[N_LANES];
@@ -619,9 +586,7 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
         p.value = e->value + first * e->cfg.max_batch;
         lane_tp[l] = p;
         lane_bufs[l] = bufs_of(e, first, l);
-        if (slots) { lane_bufs[l].slot_flags = e->slot_flags; lane_bufs[l].n_slots = n_trees; }
     }
-    if (slots) UTTT_CUDA_OK(cudaMemsetAsync(e->slot_flags, 0, (size_t)n_trees, s));
     UTTT_CUDA_OK(cudaMemsetAsync(t.counters, 0, 8 * sizeof(unsigned long long), s));
     // (counters[0] = next game to hand out: the first n_trees games are assigned by tree_begin; set here, before the lanes
     // fork, so that no lane's begin kernel races with another lane's first recycled slot)

@@ -41,8 +41,7 @@ __host__ __device__ inline HeadsFC heads_fc_of(const NetWeights& w) {
 // EVERY thread of the block must call this (block-uniform arguments): it contains __syncthreads.
 __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* headfeat, int row0, int row_step, int np,
                                                float* __restrict__ policy, float* __restrict__ value, int row_stride,
-                                               float* sm /* HEADS_SMEM_BYTES, 16-byte aligned */, long long* stamps = nullptr,
-                                               const int* dst_rows = nullptr /* position p is written to row dst_rows[p * row_step] */) {
+                                               float* sm /* HEADS_SMEM_BYTES, 16-byte aligned */, long long* stamps = nullptr) {
     const float4* f = reinterpret_cast<const float4*>(sm + HEADS_F_OFF);
     float (*part)[HEADS_P][81] = reinterpret_cast<float (*)[HEADS_P][81]>(sm + HEADS_PART_OFF);
     float (*hid)[256] = reinterpret_cast<float (*)[256]>(sm + HEADS_HID_OFF);
@@ -157,7 +156,7 @@ __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* he
         }
 #pragma unroll
         for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xFFFFFFFFu, s, off);
-        float* prow = policy + (size_t)(dst_rows ? dst_rows[p * row_step] : row0 + p * row_step) * row_stride * 81;
+        float* prow = policy + (size_t)(row0 + p * row_step) * row_stride * 81;
 #pragma unroll
         for (int k = 0; k < 3; k++)
             if (lane + 32 * k < 81) prow[lane + 32 * k] = e[k] / s;
@@ -169,7 +168,7 @@ __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* he
         for (int k = 0; k < 8; k++) a += hid[p][lane + 32 * k];
 #pragma unroll
         for (int off = 16; off > 0; off >>= 1) a += __shfl_xor_sync(0xFFFFFFFFu, a, off);
-        if (lane == 0) value[(size_t)(dst_rows ? dst_rows[p * row_step] : row0 + p * row_step) * row_stride] = tanhf(a + vb);
+        if (lane == 0) value[(size_t)(row0 + p * row_step) * row_stride] = tanhf(a + vb);
     }
 }
 

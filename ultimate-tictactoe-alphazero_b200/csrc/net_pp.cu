@@ -18,7 +18,7 @@ trunk_pp_large_kernel(const __nv_bfloat16* __restrict__ wq,
     const int n_pos = *count;
     if (n_pos <= cap1) return;
     count_batch(dbg, n_pos);
-    trunk_pp_body<2>(wq, wq_in, wq_bias, planes, headw, headfeat, skip, dbg, n_pos, nullptr);
+    trunk_pp_body<2>(wq, wq_in, wq_bias, planes, headw, headfeat, skip, dbg, n_pos);
 }
 
 }  // namespace pp

@@ -116,9 +116,7 @@ __device__ __forceinline__ void trunk_pp_body(const __nv_bfloat16* __restrict__ 
                 float* headfeat,                             // out: [rows][243]
                 uint4* skip,                                 // [gridDim][NG][16 panels][256 rows] fp16x8 skip connection
                 long long* dbg,
-                int n_pos,                                   // the batch size
-                const int* src_rows) {                       // slot mode (net_auto.cu): position i of this pair reads planes row
-                                                             // src_rows[i], else null
+                int n_pos) {                                 // the batch size
     using C = Cfg<LTB>;
     constexpr int STAGES = C::STAGES, BAR_OFF = C::BAR_OFF, HEAD_OFF = C::HEAD_OFF, CONST_OFF = C::CONST_OFF,
                   STAGE_BLOCKS = C::STAGE_BLOCKS, STAGE_BYTES = C::STAGE_BYTES, STAGES_PER_LAYER = C::STAGES_PER_LAYER,
@@ -245,7 +243,7 @@ __device__ __forceinline__ void trunk_pp_body(const __nv_bfloat16* __restrict__ 
                 if (!r.active) continue;
                 uint4 pk = zero4;
                 if (chalf == 0 && r.valid) {
-                    const __nv_bfloat16* px = planes + (size_t)(src_rows ? src_rows[r.gpos - sg * Ptot] : r.gpos) * 243 + (size_t)r.cell;
+                    const __nv_bfloat16* px = planes + (size_t)r.gpos * 243 + (size_t)r.cell;
                     uint32_t x0 = (uint32_t)__bfloat16_as_ushort(px[0]), x1 = (uint32_t)__bfloat16_as_ushort(px[81]),
                              x2 = (uint32_t)__bfloat16_as_ushort(px[162]);
                     pk = make_uint4(x0 | (x1 << 16), x2, 0u, 0u);

@@ -27,7 +27,7 @@ trunk_x3_kernel(const __nv_bfloat16* __restrict__ wq, const __nv_bfloat16* __res
     const int first = pair * per_pair, last = min(n_pos, first + per_pair);
     for (int off = first; off < last; off += Cfg<true>::MAX_P)
         trunk_tc2_body<true>(wq, wq_in, wq_bias, planes, headw, headfeat, skip, off == first ? dbg : nullptr,
-                             min(Cfg<true>::MAX_P, last - off), nullptr, off, true);     // (dbg: timeline of the first pass)
+                             min(Cfg<true>::MAX_P, last - off), off, true);     // (dbg: timeline of the first pass)
 }
 
 }  // namespace tc2

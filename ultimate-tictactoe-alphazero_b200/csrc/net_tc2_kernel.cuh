@@ -108,7 +108,6 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
                  uint4* skip,                            // [gridDim][16 panels][256 rows] fp16x8 skip connection (X3: fp32x8)
                  long long* dbg,
                  int n_pos,                              // the batch size
-                 const int* src_rows,                    // slot mode: position i of this CTA pair reads planes row src_rows[i], else null
                  int pos_base, bool solo) {              // solo: this CTA pair alone evaluates the n_pos positions that start
                                                          // at row pos_base of planes / headfeat (trunk_x3_kernel)
     using C = Cfg<X3>;
@@ -233,7 +232,7 @@ __device__ __forceinline__ void trunk_tc2_body(const __nv_bfloat16* __restrict__
             {
                 uint4 pk = zero4;
                 if (chalf == 0 && valid) {
-                    const __nv_bfloat16* px = planes + (size_t)(src_rows ? src_rows[pos] : pos_base + gpos) * 243 + (size_t)(r * 9 + c);
+                    const __nv_bfloat16* px = planes + (size_t)(pos_base + gpos) * 243 + (size_t)(r * 9 + c);
                     uint32_t x0 = (uint32_t)__bfloat16_as_ushort(px[0]), x1 = (uint32_t)__bfloat16_as_ushort(px[81]),
                              x2 = (uint32_t)__bfloat16_as_ushort(px[162]);
                     pk = make_uint4(x0 | (x1 << 16), x2, 0u, 0u);

@@ -207,9 +207,9 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_begin_kernel(TreePa
     c.ply = 0; c.game = 0; c.game_idx = -1; c.nn_row = 0; c.pad = 0;
     PackedState rs;
     if (P.mode == MODE_SELFPLAY) {
-        // the first games go to the slots in slot order (not in arrival order at an atomic counter: which game a slot
-        // plays decides its row in the evaluator batch, and a run should be reproducible); later games are claimed from
-        // counters[0] as slots finish (the host starts it at the number of slots before the lanes fork)
+        // game g starts in slot g: the first games need no counter (a game's moves do not depend on its slot); later
+        // games are claimed from counters[0] as slots finish (the host starts it at the number of slots before the lanes
+        // fork)
         unsigned long long g = (unsigned long long)(P.slot0 + t);
         if ((int64_t)g >= P.n_games) {
             c.phase = PHASE_DONE;
@@ -254,7 +254,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_round_kernel(TreePa
         if (P.flags & UTTT_SP_PYSEARCH) apply_leaf_py(P, T, c, warp_load_state_finish(leaf_raw), lane);
         else apply_leaf(P, T, c, warp_load_state_finish(leaf_raw), lane);
         if (c.phase == PHASE_DONE) {
-            if (lane == 0) { P.ctl[t] = c; if (P.slot_flags) P.slot_flags[t] = 0; }
+            if (lane == 0) P.ctl[t] = c;
             return;
         }
         c.phase = PHASE_SEARCH;
@@ -389,12 +389,12 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_round_kernel(TreePa
 
         // ---------------- queue the leaf for the evaluator; fused leaf gather (cpp/uttt_game.cpp:244-280)
         int k = min(P.batch, c.sims_left);                            // cpp/uttt_mcts.cpp:127 flush rule
-        int row = t;                                                  // slot mode: the leaf stays in its tree's row
+        int row = 0;
         if (lane == 0) {
-            if (!P.slot_flags) row = atomicAdd(P.nn_count + P.parity, 1);
+            row = atomicAdd(P.nn_count + P.parity, 1);
             atomicAdd(P.counters + 4, 1ull);
         }
-        if (!P.slot_flags) row = __shfl_sync(FULL, row, 0);
+        row = __shfl_sync(FULL, row, 0);
         warp_store_state(P.nn_states + row, st, lane);
         warp_store_state(P.leaf_state + t, st, lane);
         if (lane == 0) { P.nn_tree[row] = t; P.nn_k[row] = k; }
@@ -405,10 +405,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_round_kernel(TreePa
         c.path_len = plen;
         break;
     }
-    if (lane == 0) {
-        P.ctl[t] = c;
-        if (P.slot_flags) P.slot_flags[t] = (c.phase == PHASE_PENDING) ? 1 : 0;
-    }
+    if (lane == 0) P.ctl[t] = c;
     if (P.dbg_tree && lane == 0) {
         unsigned long long dt = (unsigned long long)(clock64() - t_start);
         unsigned long long* d = P.dbg_tree + 3 * (min(n_terminal, 7) + dbg_moved);
