@@ -49,6 +49,20 @@ extern "C" {
                                            of the C++ one's: the root is evaluated like any leaf, a flush's k expansions
                                            of a leaf replace each other (one child list), priors are normalised with
                                            numpy's float32 pairwise sum */
+#define UTTT_SP_RANDOM_SYMMETRY 8       /* uttt_mcts_search and uttt_selfplay_run*, any search mode and device evaluator:
+                                           every leaf is evaluated under a board symmetry g drawn at random (AlphaGo Zero's
+                                           evaluation-time augmentation) and the policy is mapped back.  Symmetry
+                                           g = 4f + r (0..7) of the 9x9 picture (R, C) of uttt_state_encode (action
+                                           9b + c at R = 3(b/3) + c/3, C = 3(b%3) + c%3): transpose (R,C) -> (C,R) if f,
+                                           then numpy.rot90(picture, k=r); stones, main-board flags and the forced board
+                                           move with it (see uttt_state_symmetry).  The evaluator sees g(leaf); the prior
+                                           of legal action a is read from row entry sigma_g(a), everything else is
+                                           unchanged.  g = philox4x32(key=(seed, 2), ctr=(game_lo, game_hi, ply, j)).x >> 29
+                                           with j = 0, 1, ... the evaluations of that move's search in the order its tree
+                                           queues them (reference-exact and _PYSEARCH: a leaf's k queued copies are one
+                                           evaluation; _THROUGHPUT: the root is j = 0).  uttt_mcts_search keys it with
+                                           seed 0, game = root index in the call, ply 0.  g depends on neither slot nor
+                                           batch position, so runs stay reproducible. */
 
 typedef struct uttt_engine uttt_engine;
 
@@ -69,6 +83,9 @@ int uttt_state_legal_actions(const uint32_t *state, int32_t *out81, int *n_out);
 int uttt_state_flags(const uint32_t *state, int *flags_out);
 int uttt_state_encode(const uint32_t *state, float *out243);                      /* cpp/uttt_game.cpp:244-280 */
 int uttt_state_to_string(const uint32_t *state, char *buf, int cap, int *len_out);/* cpp/uttt_game.cpp:194-241 */
+/* out = the image of the position under board symmetry g (0..7, numbering of UTTT_SP_RANDOM_SYMMETRY);
+ * action_map81 (may be NULL): [a] = sigma_g(a), the action at the image of action a's cell */
+int uttt_state_symmetry(const uint32_t *state, int g, uint32_t *out, int32_t *action_map81);
 
 /* ------------------------------------------------------------------------------------------
  * Rules kernels over arrays of packed states in HBM (replace UTTT::State, cpp/uttt_game.cpp)
@@ -255,7 +272,8 @@ int uttt_debug_counters(uttt_engine *e, uint64_t *out8);
  * record every evaluated leaf with the evaluator rows its tree is about to consume -- (tree, game index, ply), packed leaf
  * state, policy[81], value -- in evaluation order; the host synchronises after every round.  `enable` also clears the log.
  * uttt_debug_trace_read: *n_out = records; with cap >= *n_out the arrays meta[n][3], states[n][8], policy[n][81],
- * value[n] (HOST pointers) are filled; cap = 0 only asks for the size.  Feeding these rows to the reference's
+ * value[n] (HOST pointers) are filled; cap = 0 only asks for the size.  With UTTT_SP_RANDOM_SYMMETRY a record holds the
+ * untransformed leaf and its row mapped back into the leaf's own action ids.  Feeding these rows to the reference's
  * UTTT::pv_mcts_scores (cpp/uttt_mcts.cpp:84-196) must reproduce the engine's scores bit for bit. */
 int uttt_debug_trace(uttt_engine *e, int enable);
 int uttt_debug_trace_read(uttt_engine *e, int64_t cap, int64_t *n_out, int32_t *meta, uint32_t *states,

@@ -76,7 +76,7 @@ struct alignas(16) TreeCtl {
     int32_t ply;
     uint64_t game;      // absolute game id (self-play)
     int32_t game_idx;   // index into the history buffers
-    int32_t pad;
+    int32_t n_eval;     // evaluations queued by the current move's search (keys UTTT_SP_RANDOM_SYMMETRY's draw)
 };
 
 struct TreeParams {

@@ -175,8 +175,9 @@ int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_
     return 0;
 }
 
-// uttt_debug_trace: after a round's evaluator, record (tree, game, ply, leaf state, policy row, value) of every queued leaf.
-// Synchronises the stream (diagnostics only).
+// uttt_debug_trace: after a round's evaluator, record (tree, game, ply, leaf state, policy row, value) of every queued leaf:
+// the untransformed leaf and its row in the leaf's own action ids (UTTT_SP_RANDOM_SYMMETRY: entry a = row entry sigma_g(a)),
+// i.e. exactly what the tree consumes.  Synchronises the stream (diagnostics only).
 int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const int32_t* count, cudaStream_t s) {
     UTTT_CUDA_OK(cudaStreamSynchronize(s));
     int32_t n_rows = 0;
@@ -184,10 +185,10 @@ int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const in
     if (n_rows == 0) return 0;
     std::vector<int32_t> trees((size_t)n_rows);
     UTTT_CUDA_OK(cudaMemcpy(trees.data(), p.nn_tree, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
-    std::vector<uint32_t> st((size_t)n_rows * 8);
     std::vector<float> pol((size_t)n_rows * 81), val((size_t)n_rows);
     std::vector<TreeCtl> ctl((size_t)p.n_trees);
-    UTTT_CUDA_OK(cudaMemcpy(st.data(), b.nn_states, st.size() * 4, cudaMemcpyDeviceToHost));
+    std::vector<uint32_t> leaf((size_t)p.n_trees * 8);
+    UTTT_CUDA_OK(cudaMemcpy(leaf.data(), p.leaf_state, leaf.size() * 4, cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(pol.data(), b.policy, pol.size() * 4, cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(val.data(), b.value, val.size() * 4, cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(ctl.data(), p.ctl, ctl.size() * sizeof(TreeCtl), cudaMemcpyDeviceToHost));
@@ -200,8 +201,11 @@ int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const in
         rec.game_idx = (p.mode == MODE_SELFPLAY) ? ctl[t].game_idx : p.slot0 + t;
         rec.ply = (p.mode == MODE_SELFPLAY) ? ctl[t].ply : 0;
         rec.value = val[r];
-        memcpy(rec.state, st.data() + (size_t)r * 8, 32);
-        memcpy(rec.policy, pol.data() + (size_t)r * 81, 81 * 4);
+        memcpy(rec.state, leaf.data() + (size_t)t * 8, 32);
+        const int g = (p.flags & UTTT_SP_RANDOM_SYMMETRY)
+                          ? sym_draw(p.mode == MODE_SELFPLAY ? p.seed : 0u, ctl[t].game, (uint32_t)ctl[t].ply, (uint32_t)(ctl[t].n_eval - 1))
+                          : 0;
+        for (int a = 0; a < 81; a++) rec.policy[a] = pol[(size_t)r * 81 + sym_action(a, g)];
         e->trace.push_back(rec);
     }
     return 0;

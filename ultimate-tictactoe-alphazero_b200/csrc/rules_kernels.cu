@@ -343,6 +343,18 @@ int uttt_state_encode(const uint32_t* state, float* out243) {
     return 0;
 }
 
+int uttt_state_symmetry(const uint32_t* state, int g, uint32_t* out, int32_t* action_map81) {
+    UTTT_CHECK(state && out, "null argument");
+    UTTT_CHECK(g >= 0 && g < 8, "symmetry %d out of range [0,8)", g);
+    PackedState s, o;
+    memcpy(s.w, state, 32);
+    sym_state(s, g, o);
+    memcpy(out, o.w, 32);
+    if (action_map81)
+        for (int a = 0; a < 81; a++) action_map81[a] = sym_action(a, g);
+    return 0;
+}
+
 // Debug rendering, same text as cpp/uttt_game.cpp:194-241.
 int uttt_state_to_string(const uint32_t* state, char* buf, int cap, int* len_out) {
     PackedState s;

@@ -66,6 +66,39 @@ __device__ __forceinline__ void warp_write_planes(__nv_bfloat16* pl, const Packe
     }
 }
 
+// UTTT_SP_RANDOM_SYMMETRY: the symmetry under which evaluation j of the tree's current move is made (0, the identity,
+// without the flag).  Search calls key it with seed 0, the root's index (c.game) and ply 0.
+__device__ __forceinline__ int leaf_symmetry(const TreeParams& P, const TreeCtl& c, int j) {
+    if (!(P.flags & UTTT_SP_RANDOM_SYMMETRY)) return 0;
+    return sym_draw(P.mode == MODE_SELFPLAY ? P.seed : 0u, c.game, (uint32_t)c.ply, (uint32_t)j);
+}
+
+// evaluator row `row` for leaf `st` (legal mask lm) under symmetry g: the row's position and planes are those of g(st)
+__device__ __forceinline__ void warp_write_row(const TreeParams& P, int row, const PackedState& st, const uint32_t lm[3], int g,
+                                               int lane) {
+    if (g == 0) {
+        warp_store_state(P.nn_states + row, st, lane);
+        warp_write_planes(P.nn_planes + (size_t)row * 243, st, lm, lane);
+        return;
+    }
+    PackedState gs;
+    sym_state(st, g, gs);
+    uint32_t glm[3];
+    legal_mask(gs, glm);
+    warp_store_state(P.nn_states + row, gs, lane);
+    warp_write_planes(P.nn_planes + (size_t)row * 243, gs, glm, lane);
+}
+
+// one coalesced read of a policy row for the leaf it was evaluated for under symmetry g: lane l gets the priors of actions
+// l, l + 32, l + 64 (p2: lanes < 17), i.e. row entries sigma_g(a)
+__device__ __forceinline__ void warp_load_priors(const float* pol, int g, int lane, float& p0, float& p1, float& p2) {
+    int e0 = lane, e1 = 32 + lane, e2 = 64 + lane;
+    if (g != 0) { e0 = sym_action(e0, g); e1 = sym_action(e1, g); e2 = (lane < 17) ? sym_action(e2, g) : 0; }
+    p0 = __ldg(pol + e0);
+    p1 = __ldg(pol + e1);
+    p2 = (lane < 17) ? __ldg(pol + e2) : 0.0f;
+}
+
 // Philox temperature-1 sampling over the root visit counts; returns the chosen action.
 // SP_TEMPERATURE != 1 (self_play_cpp.py:27,62 -> cpp/uttt_mcts.cpp:183-216): T == 0 plays the first maximum of the visit
 // counts (the reference's one-hot scores leave np.random.choice no choice); otherwise the move is drawn from

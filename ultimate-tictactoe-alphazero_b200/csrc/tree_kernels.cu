@@ -41,6 +41,7 @@ __device__ void init_root(const TreeParams& P, const TreeView& T, TreeCtl& c, co
         c.sims_left = P.sims;
         c.path_len = 0;
         c.pend_k = 0;
+        c.n_eval = 0;
         return;
     }
     float pu = (L > 0) ? __fdiv_rn(1.0f, (float)L) : 0.0f;
@@ -52,6 +53,7 @@ __device__ void init_root(const TreeParams& P, const TreeView& T, TreeCtl& c, co
     c.sims_left = P.sims;
     c.path_len = 0;
     c.pend_k = 0;
+    c.n_eval = 0;
 }
 
 // cpp/uttt_mcts.cpp:47-54, k sequential backups of the same path (values may differ per copy)
@@ -122,8 +124,8 @@ __device__ void apply_leaf_py(const TreeParams& P, const TreeView& T, TreeCtl& c
         return;
     }
     size_t row = (size_t)c.nn_row * (size_t)P.row_stride;
-    const float* pol = P.policy + row * 81;
-    float p0 = __ldg(pol + lane), p1 = __ldg(pol + 32 + lane), p2 = (lane < 17) ? __ldg(pol + 64 + lane) : 0.0f;
+    float p0, p1, p2;
+    warp_load_priors(P.policy + row * 81, leaf_symmetry(P, c, c.n_eval - 1), lane, p0, p1, p2);
     // legal policies in legal order: rank i sits in lane i % 32, register i / 32
     float lp[3];
 #pragma unroll
@@ -161,11 +163,13 @@ __device__ void apply_leaf(const TreeParams& P, const TreeView& T, TreeCtl& c, c
         return;
     }
     size_t row = (size_t)c.nn_row * (size_t)P.row_stride;
+    const int g = leaf_symmetry(P, c, c.n_eval - 1);
     for (int cp = 0; cp < k; cp++) {
         const float* pol = P.policy + (row + (size_t)cp * P.copy_stride) * 81;
         // one coalesced read of the policy row (lane a holds actions a, a+32, a+64), then the reference's serial
         // fp32 sum over the legal actions in ascending id (:144-152) with the addends fetched by shuffle
-        float p0 = __ldg(pol + lane), p1 = __ldg(pol + 32 + lane), p2 = (lane < 17) ? __ldg(pol + 64 + lane) : 0.0f;
+        float p0, p1, p2;
+        warp_load_priors(pol, g, lane, p0, p1, p2);
         float sum = 0.0f;
 #pragma unroll
         for (int j = 0; j < 3; j++) {
@@ -204,7 +208,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_begin_kernel(TreePa
     if (t >= P.n_trees) return;
     TreeView T = view_of(P, t);
     TreeCtl c = P.ctl[t];
-    c.ply = 0; c.game = 0; c.game_idx = -1; c.nn_row = 0; c.pad = 0;
+    c.ply = 0; c.game = 0; c.game_idx = -1; c.nn_row = 0; c.n_eval = 0;
     PackedState rs;
     if (P.mode == MODE_SELFPLAY) {
         // game g starts in slot g: the first games need no counter (a game's moves do not depend on its slot); later
@@ -221,6 +225,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_begin_kernel(TreePa
         init_state(rs);
         warp_store_state(P.root + t, rs, lane);
     } else {
+        c.game = (uint64_t)t;                 // search mode: the root's index keys UTTT_SP_RANDOM_SYMMETRY's draw
         rs = warp_load_state(P.root + t, lane);
     }
     init_root(P, T, c, rs, lane);
@@ -395,10 +400,10 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_round_kernel(TreePa
             atomicAdd(P.counters + 4, 1ull);
         }
         row = __shfl_sync(FULL, row, 0);
-        warp_store_state(P.nn_states + row, st, lane);
         warp_store_state(P.leaf_state + t, st, lane);
         if (lane == 0) { P.nn_tree[row] = t; P.nn_k[row] = k; }
-        warp_write_planes(P.nn_planes + (size_t)row * 243, st, lm, lane);
+        warp_write_row(P, row, st, lm, leaf_symmetry(P, c, c.n_eval), lane);
+        c.n_eval += 1;
         c.phase = PHASE_PENDING;
         c.pend_k = k;
         c.nn_row = row;

@@ -69,21 +69,24 @@ __device__ __forceinline__ int32_t* tp_path(const TreeParams& P, int t, int j) {
     return P.tp_paths + ((size_t)t * TP_MAX_LEAVES + j) * PATH_CAP;
 }
 
-// expansion of `leaf` from one policy row: masked, serially renormalised priors (same arithmetic as the
-// reference-exact mode, cpp/uttt_mcts.cpp:144-163), optional Dirichlet mix for the root
+// expansion of `leaf` from one policy row, evaluated under symmetry `sym`: masked, serially renormalised priors (same arithmetic
+// as the reference-exact mode, cpp/uttt_mcts.cpp:144-163), optional Dirichlet mix for the root
 __device__ void tp_expand(const TreeParams& P, const TreeView& T, TreeCtl& c, const PackedState& st, int leaf,
-                          const float* pol, bool is_root, int lane) {
+                          const float* pol, int sym, bool is_root, int lane) {
     uint32_t lm[3];
     int L = legal_mask(st, lm);
     int base = c.n_nodes;
+    float p0, p1, p2;
+    warp_load_priors(pol, sym, lane, p0, p1, p2);
     float sum = 0.0f;
 #pragma unroll
     for (int j = 0; j < 3; j++) {
         uint32_t m = lm[j];
         while (m) {
-            int b = __ffs((int)m) - 1;
+            int a = 27 * j + __ffs((int)m) - 1;
             m &= m - 1u;
-            sum = __fadd_rn(sum, __ldg(pol + 27 * j + b));
+            const float src = a < 32 ? p0 : (a < 64 ? p1 : p2);          // `a` is warp-uniform
+            sum = __fadd_rn(sum, __shfl_sync(FULL, src, a & 31));
         }
     }
     float uni = (L > 0) ? __fdiv_rn(1.0f, (float)L) : 0.0f;
@@ -97,7 +100,7 @@ __device__ void tp_expand(const TreeParams& P, const TreeView& T, TreeCtl& c, co
     }
     for (int q = 0, a = lane; a < 81; a += 32, q++) {
         if (legal_bit(lm, a)) {
-            float pr = (sum > 0.0f) ? __fdiv_rn(__ldg(pol + a), sum) : uni;
+            float pr = (sum > 0.0f) ? __fdiv_rn(q == 0 ? p0 : (q == 1 ? p1 : p2), sum) : uni;
             if (noise) pr = (1.0f - P.dir_eps) * pr + P.dir_eps * (gsum > 0.0f ? g[q] / gsum : uni);
             T.node[base + legal_rank(lm, a)] = make_node(a, pr);
         }
@@ -128,7 +131,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_begin_kernel(Tre
     if (blockIdx.x == 0 && threadIdx.x == 0) { P.nn_count[0] = 0; P.nn_count[1] = 0; }
     if (t >= P.n_trees) return;
     TreeCtl c = P.ctl[t];
-    c.ply = 0; c.game = 0; c.game_idx = -1; c.nn_row = 0; c.pad = 0; c.pend_k = 0; c.path_len = 0;
+    c.ply = 0; c.game = 0; c.game_idx = -1; c.nn_row = 0; c.n_eval = 0; c.pend_k = 0; c.path_len = 0;
     c.sims_left = P.sims; c.n_nodes = 1; c.n_root = 0;
     if (P.mode == MODE_SELFPLAY) {
         unsigned long long g = 0;
@@ -151,7 +154,8 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_begin_kernel(Tre
     if (lane == 0) P.ctl[t] = c;
 }
 
-__device__ __forceinline__ int tp_queue_leaf(const TreeParams& P, int t, const PackedState& st, const uint32_t lm[3],
+// queues evaluation j of the tree's current move
+__device__ __forceinline__ int tp_queue_leaf(const TreeParams& P, int t, TreeCtl& c, const PackedState& st, const uint32_t lm[3],
                                              int lane) {
     int row = 0;
     if (lane == 0) {
@@ -159,9 +163,9 @@ __device__ __forceinline__ int tp_queue_leaf(const TreeParams& P, int t, const P
         atomicAdd(P.counters + 4, 1ull);
     }
     row = __shfl_sync(FULL, row, 0);
-    warp_store_state(P.nn_states + row, st, lane);
     if (lane == 0) { P.nn_tree[row] = t; P.nn_k[row] = 1; }
-    warp_write_planes(P.nn_planes + (size_t)row * 243, st, lm, lane);
+    warp_write_row(P, row, st, lm, leaf_symmetry(P, c, c.n_eval), lane);
+    c.n_eval += 1;
     return row;
 }
 
@@ -182,7 +186,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
         if (lane == 0) T.node[0] = make_uint4(0x7Fu << 16, 0u, 0u, 0u);
         __syncwarp();
         c.n_nodes = 1;
-        tp_expand(P, T, c, root, 0, P.policy + (size_t)c.nn_row * 81, true, lane);
+        tp_expand(P, T, c, root, 0, P.policy + (size_t)c.nn_row * 81, leaf_symmetry(P, c, 0), true, lane);
         uint32_t lm[3];
         c.n_root = legal_mask(root, lm);
         c.sims_left = P.sims;
@@ -200,7 +204,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
                 if (lane == 0) P.ctl[t] = c;
                 return;
             }
-            tp_expand(P, T, c, st, leaf, P.policy + (size_t)row * 81, false, lane);
+            tp_expand(P, T, c, st, leaf, P.policy + (size_t)row * 81, leaf_symmetry(P, c, c.n_eval - c.pend_k + j), false, lane);
             tp_backup(T, path, plen, P.value[row], true, lane);
         }
         c.sims_left -= c.pend_k;
@@ -258,7 +262,8 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
                 c.phase = PHASE_DONE;
                 break;
             }
-            c.nn_row = tp_queue_leaf(P, t, root, lm, lane);
+            c.n_eval = 0;                                   // the root is evaluation 0 of the move's search
+            c.nn_row = tp_queue_leaf(P, t, c, root, lm, lane);
             c.phase = PHASE_ROOT_PENDING;
             break;
         }
@@ -332,7 +337,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
             for (int i = lane; i < plen; i += 32) T.node[path[i]].x += (1u << 23);
             if (lane == 0) T.node[node].w = LINK_PENDING;
             __syncwarp();
-            int row = tp_queue_leaf(P, t, st, lm, lane);
+            int row = tp_queue_leaf(P, t, c, st, lm, lane);
             warp_store_state(P.leaf_state + (size_t)t * TP_MAX_LEAVES + got, st, lane);
             if (lane == 0) { aux->path_len[got] = plen; aux->nn_row[got] = row; }
             got++;

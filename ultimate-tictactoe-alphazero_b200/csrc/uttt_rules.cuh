@@ -221,4 +221,55 @@ UTTT_HD uint32_t state_hash(const PackedState& s) {
 
 UTTT_HD uint64_t fnv64(uint64_t h, uint32_t x) { return (h ^ (uint64_t)x) * 0x100000001B3ull; }
 
+// ---- board symmetries (include/uttt_b200.h, UTTT_SP_RANDOM_SYMMETRY) ----
+// Symmetry g = 4f + r of the 9x9 picture (R, C): transpose if f, then numpy.rot90(picture, k=r).  It maps sub-board
+// (R/3, C/3) and cell (R%3, C%3) by the same map of the 3x3 grid, so it acts on a 9-bit mask (bit 3y+x) of boards or
+// cells.  On that grid rot90 is (y,x) -> (2-x,y) = transpose, then flip rows; every g is therefore "transpose, then
+// flip rows (y -> 2-y), then flip columns (x -> 2-x)", each step present or not -- bits 0, 1, 2 of nibble g of
+// SYM_STEPS:  g0 -, g1 T V, g2 V H, g3 T H, g4 T, g5 V, g6 T V H, g7 H.
+constexpr uint32_t SYM_STEPS = 0x47215630u;
+
+UTTT_HD uint32_t sym9(uint32_t m, int g) {
+    const uint32_t steps = (SYM_STEPS >> (4 * g)) & 7u;
+    if (steps & 1u) m = (m & 0x111u) | ((m & 0x022u) << 2) | ((m & 0x088u) >> 2) | ((m & 0x004u) << 4) | ((m & 0x040u) >> 4);
+    if (steps & 2u) m = ((m & 0x007u) << 6) | (m & 0x038u) | ((m >> 6) & 0x007u);
+    if (steps & 4u) m = ((m & 0x049u) << 2) | (m & 0x092u) | ((m >> 2) & 0x049u);
+    return m;
+}
+
+// image of index i (0..8) of the 3x3 grid
+UTTT_HD int sym_index(int i, int g) {
+#if defined(__CUDA_ARCH__)
+    return __ffs((int)sym9(1u << i, g)) - 1;
+#else
+    return __builtin_ctz(sym9(1u << i, g));
+#endif
+}
+
+// sigma_g(a): the action at the image of action a's cell
+UTTT_HD int sym_action(int a, int g) {
+    const int b = a / 9;
+    return 9 * sym_index(b, g) + sym_index(a - 9 * b, g);
+}
+
+// the image of a position: stones, main-board flags and the forced board moved by the map (-1 stays -1)
+UTTT_HD void sym_state(const PackedState& s, int g, PackedState& o) {
+#pragma unroll
+    for (int i = 0; i < 8; i++) o.w[i] = 0u;
+#pragma unroll
+    for (int b = 0; b < 9; b++) {
+        const int nb = sym_index(b, g), j = b / 3, sh = 9 * (b - 3 * j), nj = nb / 3, nsh = 9 * (nb - 3 * nj);
+        const uint32_t me = sym9((s.w[j] >> sh) & 0x1FFu, g), op = sym9((s.w[3 + j] >> sh) & 0x1FFu, g);
+        o.w[0] |= (nj == 0) ? me << nsh : 0u; o.w[1] |= (nj == 1) ? me << nsh : 0u; o.w[2] |= (nj == 2) ? me << nsh : 0u;
+        o.w[3] |= (nj == 0) ? op << nsh : 0u; o.w[4] |= (nj == 1) ? op << nsh : 0u; o.w[5] |= (nj == 2) ? op << nsh : 0u;
+    }
+    const int act = active_board(s);
+    o.w[6] = sym9(main_me(s), g) | (sym9(main_opp(s), g) << 9) | ((uint32_t)(act < 0 ? 0 : sym_index(act, g) + 1) << 18);
+}
+
+// the symmetry a leaf is evaluated under: Philox key (seed, 2), counter (game, ply, j = evaluation of the move's search)
+UTTT_HD int sym_draw(uint32_t seed, uint64_t game, uint32_t ply, uint32_t j) {
+    return (int)(philox4x32(seed, 2u, (uint32_t)game, (uint32_t)(game >> 32), ply, j).x >> 29);
+}
+
 }  // namespace uttt

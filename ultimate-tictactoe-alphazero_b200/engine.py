@@ -29,6 +29,7 @@ DEFAULT_NUMERICS = os.environ.get("UTTT_NUMERICS", "bf16x3")
 SP_CORRECT_TERMINAL_SIGN = 1
 SP_THROUGHPUT = 2
 SP_PYSEARCH = 4
+SP_RANDOM_SYMMETRY = 8     # evaluate every leaf under a random board symmetry (include/uttt_b200.h)
 
 _vp = C.c_void_p
 _u32p = np.ctypeslib.ndpointer(np.uint32, flags="C_CONTIGUOUS")
@@ -65,6 +66,7 @@ ABI = {
     "uttt_state_flags": ([_u32p, C.POINTER(C.c_int)], C.c_int),
     "uttt_state_encode": ([_u32p, _f32p], C.c_int),
     "uttt_state_to_string": ([_u32p, C.c_char_p, C.c_int, C.POINTER(C.c_int)], C.c_int),
+    "uttt_state_symmetry": ([_u32p, C.c_int, _u32p, _vp], C.c_int),
     "uttt_game_step": ([_vp, _vp, _vp, C.c_int64, _vp], C.c_int),
     "uttt_game_legal_mask": ([_vp, _vp, _vp, C.c_int64, _vp], C.c_int),
     "uttt_game_encode": ([_vp, _vp, C.c_int64, _vp], C.c_int),
@@ -143,6 +145,17 @@ def _stream(stream=None):
     import torch
     s = stream if stream is not None else torch.cuda.current_stream()
     return s.cuda_stream
+
+
+# ------------------------------------------------------------------------------------ single-state helpers
+def state_symmetry(state, g):
+    """image of one packed state under board symmetry g (0..7: transpose if g >= 4, then numpy.rot90 by g % 4 of the 9x9
+    picture) -> (packed state (8,) uint32, action map (81,) int32: [a] = the action at the image of action a's cell)"""
+    st = np.ascontiguousarray(state, dtype=np.uint32).reshape(8)
+    out = np.zeros(8, np.uint32)
+    amap = np.zeros(81, np.int32)
+    _check(load_library().uttt_state_symmetry(st, int(g), out, amap.ctypes.data))
+    return out, amap
 
 
 # ------------------------------------------------------------------------------------ rules on device tensors

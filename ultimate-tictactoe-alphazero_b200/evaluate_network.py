@@ -25,6 +25,7 @@ MCTS_BATCH_SIZE = 8       # pv_mcts.py:17
 EN_SEED = None            # None: derived from numpy's global RNG
 EN_SEARCH = "python"      # "python": pv_mcts.py semantics (what the reference's gating match runs); "cpp": uttt_mcts.cpp semantics
 EN_NUMERICS = _eng.DEFAULT_NUMERICS    # "bf16x3" | "bf16" | "fp32" (engine.evaluator_of)
+EN_RANDOM_SYMMETRY = False             # evaluate every leaf under a random board symmetry, policy mapped back (AlphaGo Zero)
 
 
 def first_player_point(ended_state):
@@ -51,12 +52,13 @@ def pv_mcts_scores_batch(engine, roots, temperature, evaluator, search=None, eva
     search = EN_SEARCH if search is None else search
     sims = PV_EVALUATE_COUNT if evaluate_count is None else evaluate_count
     batch = MCTS_BATCH_SIZE if batch_size is None else batch_size
+    sym = _eng.SP_RANDOM_SYMMETRY if EN_RANDOM_SYMMETRY else 0
     if search == "cpp":
-        sc, _, ns = engine.mcts_search(roots, sims, batch, temperature, evaluator)
+        sc, _, ns = engine.mcts_search(roots, sims, batch, temperature, evaluator, flags=sym)
         return sc, ns                  # float32, renormalised in float64 by the caller (pv_mcts_cpp.py:129-133)
     if search != "python":
         raise ValueError("EN_SEARCH must be 'python' or 'cpp', not %r" % (search,))
-    _, counts, ns = engine.mcts_search(roots, sims, batch, 1.0, evaluator, flags=_eng.SP_PYSEARCH)
+    _, counts, ns = engine.mcts_search(roots, sims, batch, 1.0, evaluator, flags=_eng.SP_PYSEARCH | sym)
     sc = np.zeros((len(ns), 81), np.float64)
     for i, n in enumerate(ns):
         if n:

@@ -41,6 +41,7 @@ SP_SEARCH_MODE = "compat"     # "compat": reference-exact search; "throughput": 
                               #   (evaluated root + Dirichlet noise, virtual loss, MCTS_BATCH_SIZE leaves / round)
 SP_DIRICHLET_ALPHA = 0.3      # throughput mode only
 SP_DIRICHLET_EPS = 0.25
+SP_RANDOM_SYMMETRY = False    # evaluate every leaf under a random board symmetry, policy mapped back (AlphaGo Zero)
 SP_WRITE_PACKED = False       # also write ./data/<timestamp>.packed.npz (357 B/sample instead of ~1.7 KB; SURVEY 8f-3)
 
 _engine = None
@@ -126,6 +127,8 @@ def _run(model, n_games, progress=False):
     if SP_SEARCH_MODE == "throughput":
         flags |= _eng.SP_THROUGHPUT
         eng.set_root_noise(SP_DIRICHLET_ALPHA, SP_DIRICHLET_EPS)
+    if SP_RANDOM_SYMMETRY:
+        flags |= _eng.SP_RANDOM_SYMMETRY
     eng.set_selfplay_temperature(SP_TEMPERATURE)
     if SP_PROGRESS and progress:
         shown = [0]
