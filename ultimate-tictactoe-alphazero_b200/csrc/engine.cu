@@ -267,13 +267,13 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
         ealloc(e, &t.hist_final, G) || ealloc(e, &e->policy, S * cfg->max_batch * 81) ||
         ealloc(e, &e->value, S * cfg->max_batch) || ealloc(e, &e->scores, S * 81) ||
         ealloc(e, &e->headfeat, R * 243) || ealloc(e, &e->act_a, R * 81 * 128) || ealloc(e, &e->act_b, R * 81 * 128) ||
-        ealloc(e, &e->tc_resid, (size_t)N_LANES * e->n_sm * 512 * 64) || ealloc(e, &e->fwd_count, 1) || ealloc(e, &e->tc_dbg, 128 + 64 + 8 + 16) ||
+        ealloc(e, &e->tc_resid, (size_t)N_LANES * e->n_sm * 512 * 64) || ealloc(e, &e->fwd_count, 1) || ealloc(e, &e->tc_dbg, 128 + 64) ||
         ealloc(e, &e->hist_offsets, G + 1)) {
         uttt_destroy(e);
         return 1;
     }
     UTTT_CUDA_OK(cudaMemset(t.ctl, 0, S * sizeof(TreeCtl)));
-    UTTT_CUDA_OK(cudaMemset(e->tc_dbg, 0, (128 + 64 + 8 + 16) * sizeof(long long)));
+    UTTT_CUDA_OK(cudaMemset(e->tc_dbg, 0, (128 + 64) * sizeof(long long)));
     UTTT_CUDA_OK(cudaMemset(t.nn_count, 0, 2 * N_LANES * sizeof(int32_t)));
     for (int i = 0; i < N_LANES; i++) {
         UTTT_CUDA_OK(cudaStreamCreateWithFlags(&e->lane_stream[i], cudaStreamNonBlocking));
@@ -767,29 +767,6 @@ int uttt_debug_trunk_timeline(uttt_engine* e, int64_t* out128) {
     UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
     UTTT_CUDA_OK(cudaDeviceSynchronize());
     UTTT_CUDA_OK(cudaMemcpy(out128, e->tc_dbg, 128 * sizeof(long long), cudaMemcpyDeviceToHost));
-    if (getenv("UTTT_DEBUG_PHASES")) {      // experiments: kernel entry / setup done / last epilogue done / exit of CTA 0 (cluster trunk)
-        long long ph[4];
-        UTTT_CUDA_OK(cudaMemcpy(ph, e->tc_dbg + 192, sizeof(ph), cudaMemcpyDeviceToHost));
-        long long d[16];
-        UTTT_CUDA_OK(cudaMemcpy(d, e->tc_dbg + 160, sizeof(d), cudaMemcpyDeviceToHost));
-        fprintf(stderr, "pp detail layer 20 (rel): A: loop %lld act %lld pact %lld fence %lld stage %lld bias-issued %lld last-commit %lld | B: loop %lld act %lld pact %lld fence %lld stage %lld bias-issued %lld last-commit %lld\n",
-                0ll, d[1] - d[0], d[2] - d[0], d[3] - d[0], d[4] - d[0], d[5] - d[0], d[6] - d[0], d[8] - d[0], d[9] - d[0], d[10] - d[0], d[11] - d[0],
-                d[12] - d[0], d[13] - d[0], d[14] - d[0]);
-        // (the tc2 bodies use the same slots: epilogue thread 0 of layer 20 and the tile-0 issuer of layer 21)
-        fprintf(stderr, "tc2 detail, layer 20 -> 21 (cycles rel. accumulator observed by epilogue thread 0): last MMA of layer 20 committed %lld | "
-                "first chunk loaded %lld, stored %lld, fenced %lld, chunks published %lld %lld %lld %lld | issuer of tile 0 passed the "
-                "act barrier of quarter 0..3 at %lld %lld %lld %lld\n", d[12] - d[0], d[1] - d[0], d[2] - d[0], d[3] - d[0], d[4] - d[0],
-                d[5] - d[0], d[6] - d[0], d[7] - d[0], d[8] - d[0], d[9] - d[0], d[10] - d[0], d[11] - d[0]);
-        long long au[10];
-        UTTT_CUDA_OK(cudaMemcpy(au, e->tc_dbg + 200, sizeof(au), cudaMemcpyDeviceToHost));
-        fprintf(stderr, "heads FC tail (cycles rel. body done): barriers ready %lld, features loaded %lld, chunk 0/1/2 landed %lld %lld %lld, "
-                "policy FC done %lld, all FC done %lld, exit %lld\n", au[3] - au[1], au[4] - au[1], au[5] - au[1], au[6] - au[1],
-                au[7] - au[1], au[8] - au[1], au[9] - au[1], au[2] - au[1]);
-        fprintf(stderr, "trunk_auto_kernel CTA 0 (cycles rel. entry): body done %lld, heads FC done %lld (warp 0's exit; heads = %lld)\n",
-                au[1] - au[0], au[2] - au[0], au[2] - au[1]);
-        fprintf(stderr, "trunk phases (cycles rel. entry): setup %lld, first MMA %lld, last epilogue %lld, exit %lld\n", ph[1] - ph[0],
-                (long long)out128[0] - ph[0], ph[2] - ph[0], ph[3] - ph[0]);
-    }
     return 0;
 }
 

@@ -41,7 +41,7 @@ __host__ __device__ inline HeadsFC heads_fc_of(const NetWeights& w) {
 // EVERY thread of the block must call this (block-uniform arguments): it contains __syncthreads.
 __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* headfeat, int row0, int row_step, int np,
                                                float* __restrict__ policy, float* __restrict__ value, int row_stride,
-                                               float* sm /* HEADS_SMEM_BYTES, 16-byte aligned */, long long* stamps = nullptr) {
+                                               float* sm /* HEADS_SMEM_BYTES, 16-byte aligned */) {
     const float4* f = reinterpret_cast<const float4*>(sm + HEADS_F_OFF);
     float (*part)[HEADS_P][81] = reinterpret_cast<float (*)[HEADS_P][81]>(sm + HEADS_PART_OFF);
     float (*hid)[256] = reinterpret_cast<float (*)[256]>(sm + HEADS_HID_OFF);
@@ -71,7 +71,6 @@ __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* he
     }
     tcx::fence_async_smem();            // earlier generic-proxy accesses to this shared memory precede the bulk copies
     __syncthreads();
-    if (stamps && t == 0) stamps[0] = clock64();
     if (t == 0) {
         for (int c = 0; c < HEADS_CHUNKS; c++) {
             tcx::mbar_expect_tx(bar + 8 * c, HEADS_CHUNK_BYTES);
@@ -87,7 +86,6 @@ __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* he
         }
     }
     __syncthreads();
-    if (stamps && t == 0) stamps[1] = clock64();
     if (t < 162) {
         // policy_fc: output o over input half h
         const int h = t / 81, o = t - 81 * h;
@@ -97,7 +95,6 @@ __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* he
 #pragma unroll 1
         for (int c = 0; c < HEADS_CHUNKS; c++) {
             tcx::mbar_wait(bar + 8 * c, 0);
-            if (stamps && t == 0) stamps[2 + c] = clock64();
             const float* wp = sm + c * HEADS_CHUNK_FLOATS + h * HEADS_POL_FLOATS + o;
             const float4* fp4 = f + h * 81 + c * HEADS_CHUNK_ROWS;
 #pragma unroll 9
@@ -110,7 +107,6 @@ __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* he
         }
 #pragma unroll
         for (int p = 0; p < HEADS_P; p++) part[h][p][o] = ap[p];
-        if (stamps && t == 0) stamps[5] = clock64();
     } else if (t >= 256 && t < 512) {
         // value_fc1: hidden unit j (on its own warps, so the two FC layers run side by side)
         const int j = t - 256;
@@ -135,7 +131,6 @@ __device__ __forceinline__ void heads_fc_block(const HeadsFC& W, const float* he
         for (int p = 0; p < HEADS_P; p++) hid[p][j] = fmaxf(av[p], 0.0f) * w2;
     }
     __syncthreads();
-    if (stamps && t == 0) stamps[6] = clock64();
     if (warp < HEADS_P) {
         const int p = warp;
         if (p >= np) return;

@@ -1,10 +1,10 @@
 // net_auto.cu -- trunk_auto_kernel: ONE launch per evaluator round.  The queue length is only known on the device, and a
 // kernel that exits at once still costs a full kernel boundary (3.4 us under ncu, ~6 us between dependent launches), so
 // the bodies sit behind one device-side branch on the batch size: batches of up to one wave of 5-position groups run
-// tc2::trunk_tc2_body (next layer overlaps the epilogue), larger ones pp::trunk_pp_body<1> (two groups in flight).  Both
-// issue cta_group::2 MMAs on per-CTA weight halves and use 19 warps, clusters of two CTAs and the same grid; shared memory
-// is the larger footprint.  Batches above 7 positions per pair are left to a second launch, trunk_pp_large_kernel
-// (net_pp.cu).
+// tc2::trunk_tc2_body (next layer overlaps the epilogue), larger ones pp::trunk_pp_body<1> (two groups in flight).  The
+// two schedules are built from the same CTA-pair pipeline pieces (trunk_pair.cuh): cta_group::2 MMAs on per-CTA weight
+// halves, 19 warps, clusters of two CTAs and the same grid; shared memory is the larger footprint.  Batches above 7
+// positions per pair are left to a second launch, trunk_pp_large_kernel (net_pp.cu).
 #include "heads_fc.cuh"
 #include "net_pp_kernel.cuh"
 #include "net_tc2_kernel.cuh"
@@ -25,8 +25,6 @@ trunk_auto_kernel(const __nv_bfloat16* __restrict__ res_w8, const __nv_bfloat16*
     extern __shared__ __align__(1024) uint8_t smem[];
     pdl_trigger();          // the next round's tree kernel may be scheduled (it waits for this grid's policy / value rows)
     pdl_wait();             // this round's tree kernel has finished: queue length and planes are visible
-    const bool stamp = dbg && blockIdx.x == 0 && threadIdx.x == 0;          // diagnostics: phases of CTA 0
-    if (stamp) dbg[200] = clock64();
     const int n_pairs = (int)gridDim.x >> 1, pair = (int)blockIdx.x >> 1;
     const int n_pos = *count;
     const bool small = n_pos <= small_cap;
@@ -38,7 +36,6 @@ trunk_auto_kernel(const __nv_bfloat16* __restrict__ res_w8, const __nv_bfloat16*
         pp::trunk_pp_body<1>(res_w18, conv_in_w18, bias_2sm, planes, headw, headfeat, skip, dbg, n_pos);
     else
         tc2::trunk_tc2_body<false>(res_w8, conv_in_w8, bias_2sm, planes, headw, headfeat, skip, dbg, n_pos, 0, false);
-    if (stamp) dbg[201] = clock64();
     if (policy == nullptr) return;
     // Fused heads (the host passes policy / value only if no batch can exceed one group per pair): the pair's head
     // features were written to global memory by both CTAs' last epilogues and ordered by the cluster barrier that ends
@@ -51,8 +48,7 @@ trunk_auto_kernel(const __nv_bfloat16* __restrict__ res_w8, const __nv_bfloat16*
     const int np = row0 < last ? (last - row0 + 1) >> 1 : 0;
     static_assert((pp::Cfg<1>::MAX_PA + pp::Cfg<1>::MAX_PB + 1) / 2 <= HEADS_P, "one heads call per CTA");
     if (np == 0) return;
-    heads_fc_block(fc, headfeat, row0, 2, np, policy, value, 1, reinterpret_cast<float*>(smem), stamp ? dbg + 203 : nullptr);
-    if (stamp) dbg[202] = clock64();
+    heads_fc_block(fc, headfeat, row0, 2, np, policy, value, 1, reinterpret_cast<float*>(smem));
 }
 
 cudaError_t trunk_auto_init() {

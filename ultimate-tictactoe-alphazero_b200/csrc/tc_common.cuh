@@ -17,6 +17,13 @@ namespace tcx {
 // the q-th 16-column chunk of every epilogue warp -- the next layer's MMAs start while the epilogue is still running.
 // The pre-packed weights (pack_res_kernel, weights.cu) are stored in the same order, 4 KiB per block.
 __host__ __device__ __forceinline__ int kblock_of(int tap, int unit) { return 18 * (unit & 3) + 2 * tap + (unit >> 2); }
+// The inverse, as offsets of the A descriptor (16-byte units) from a tile's first row in channel panel 0.  Tap t of the
+// 100-row position layout (row = 10 r + c) is the row shift 10 dy + dx:
+__host__ __device__ __forceinline__ constexpr int tap_shift(int tap) { return (tap / 3 - 1) * 10 + (tap % 3 - 1); }
+// K-block m reads that shift in the panel pair of its unit (panel16: bytes per channel panel / 16).
+__host__ __device__ __forceinline__ constexpr int kblock_a_offset(int m, int panel16) {
+    return tap_shift((m % 18) >> 1) + 2 * (m / 18 + 4 * ((m % 18) & 1)) * panel16;
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
@@ -26,6 +33,8 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t lbo_bytes,
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
 }
+// after the mbarrier.init of barriers that the peer CTA or the async proxy will signal
+__device__ __forceinline__ void fence_mbar_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
