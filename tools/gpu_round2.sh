@@ -13,7 +13,7 @@ for n in 16 148 370 500 740; do python tools/fwd_loop.py $n 100 bf16x3; done 2>&
 python tools/pp_timeline.py 500 > "$OUT"/tl_pp_r2.log 2>&1
 python tools/trunk_timeline.py 345 > "$OUT"/tl_r2.log 2>&1
 python tools/trunk_timeline.py 40 > "$OUT"/tl40_r2.log 2>&1
-UTTT_PROFILE=2 UTTT_DEBUG_TREE=1 python tools/prof_selfplay.py --games 500 --reps 3 > "$OUT"/plain_r2.log 2>&1
+UTTT_PROFILE=2 python tools/prof_selfplay.py --games 500 --reps 3 > "$OUT"/plain_r2.log 2>&1
 python tools/determinism_check.py 500 > "$OUT"/determinism_r2.log 2>&1
 echo '`ncu --metrics gpu__time_duration.sum --clock-control none -s 2600 -c 800 python bench.py --steps 2 --warmup 3 --no-extras --no-cpu-baseline --saturated-games 0` (launches 2600..3399 of the bench command: inside its warm-up / timed self-play cycles)' > "$OUT"/launches_r2.cmd
 ncu --metrics gpu__time_duration.sum --clock-control none -s 2600 -c 800 --csv --log-file "$OUT"/launches_r2.csv python bench.py --steps 2 --warmup 3 --no-extras --no-cpu-baseline --saturated-games 0 > "$OUT"/ncu_launch_r2.log 2>&1

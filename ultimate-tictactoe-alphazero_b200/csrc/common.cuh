@@ -84,14 +84,13 @@ struct TreeParams {
     int32_t slot0;            // global index of this lane's first slot (self-play: slot s starts with game game0 + s)
     int32_t max_terminal;     // terminal descents one tree may retire per round (the rest continues next round)
     PackedState* root;        // [n_trees]
-    PackedState* leaf_state;  // [n_trees]
-    // throughput mode (tree_tp_kernels.cu): per tree up to TP_MAX_LEAVES pending leaves
-    int32_t* tp_paths;        // [n_trees][TP_MAX_LEAVES][PATH_CAP]
-    int32_t* tp_aux;          // [n_trees][2][TP_MAX_LEAVES]: path lengths, evaluator rows
+    // per tree up to TP_MAX_LEAVES pending leaves (the reference-exact mode has one, leaf 0): position and node path
+    PackedState* leaf_state;  // [n_trees][TP_MAX_LEAVES]
+    int32_t* paths;           // [n_trees][TP_MAX_LEAVES][PATH_CAP]
+    int32_t* tp_aux;          // [n_trees][2][TP_MAX_LEAVES]: throughput mode's path lengths, evaluator rows
     float dir_alpha, dir_eps; // Dirichlet root noise
     float temperature;        // self-play move sampling (SP_TEMPERATURE, self_play_cpp.py:27); 1 = the reference's setting
     TreeCtl* ctl;             // [n_trees]
-    int32_t* path;            // [n_trees][PATH_CAP]
     // nodes, [n_trees][node_cap], 16 B each: {n:16 | action<<16, w, p, first_child:20 | n_children<<20}
     uint4* nodes;
     // evaluator queue (rows are compacted with an atomic counter, double-buffered by round parity)
@@ -117,17 +116,14 @@ struct TreeParams {
     uint8_t* hist_actions;         // [n_games][81]
     int32_t* hist_len;             // [n_games]
     int8_t* hist_final;            // [n_games]
-    unsigned long long* dbg_tree;  // diagnostics (null = off): [16 classes][3] = sum of cycles, warps, max cycles per class of
-                                   // a tree's round: class = min(terminal descents, 7) + 8 * (a move was decided)
 };
 
 // kernels' host launchers (each returns cudaGetLastError of the launch)
 cudaError_t launch_tree_begin(const TreeParams& p, cudaStream_t s);
 cudaError_t launch_tree_round(const TreeParams& p, cudaStream_t s);
-cudaError_t launch_tree_tp_begin(const TreeParams& p, cudaStream_t s);
 cudaError_t launch_tree_tp_round(const TreeParams& p, cudaStream_t s);
-cudaError_t launch_hash_eval(const PackedState* states, const int32_t* k, const int32_t* count, int max_rows,
-                             float* policy, float* value, int row_stride, int copy_stride, cudaStream_t s);
+cudaError_t launch_hash_eval(const PackedState* states, const int32_t* count, int max_rows, float* policy, float* value,
+                             cudaStream_t s);
 cudaError_t launch_scores(const int32_t* counts, const int32_t* n, int n_trees, float temperature,
                           float* scores, cudaStream_t s);
 cudaError_t launch_dirichlet(uint32_t seed, uint64_t game0, int64_t n, int n_children, float alpha, float* out, cudaStream_t s);

@@ -93,9 +93,8 @@ int ealloc(uttt_engine* e, T** p, size_t n) {
 
 // the buffers one evaluator invocation works on (the whole engine, or one lane's slice of it)
 struct EvalBufs {
-    const PackedState* nn_states;
-    const int32_t* nn_k;
-    const __nv_bfloat16* nn_planes;
+    PackedState* nn_states;
+    __nv_bfloat16* nn_planes;
     float *policy, *value, *act_a, *act_b, *resid, *headfeat;
 };
 
@@ -103,7 +102,6 @@ EvalBufs bufs_of(uttt_engine* e, size_t first_slot, int lane) {
     EvalBufs b;
     size_t first_row = first_slot * (size_t)e->rows_per_slot;
     b.nn_states = e->tp.nn_states + first_row;
-    b.nn_k = e->tp.nn_k + first_row;
     b.nn_planes = e->tp.nn_planes + first_row * 243;
     b.policy = e->policy + first_slot * e->cfg.max_batch * 81;
     b.value = e->value + first_slot * e->cfg.max_batch;
@@ -112,6 +110,23 @@ EvalBufs bufs_of(uttt_engine* e, size_t first_slot, int lane) {
     b.headfeat = e->headfeat + first_row * 243;
     b.resid = e->tc_resid + (size_t)lane * e->n_sm * 512 * 64;     // fp16 panels: 128 KiB per CTA
     return b;
+}
+
+// self-play lane `lane` runs the slots [first, first + n_trees): its slice of the trees and of the evaluator queue (p),
+// and of the evaluator's buffers (b)
+void lane_of(uttt_engine* e, size_t first, int n_trees, int lane, TreeParams& p, EvalBufs& b) {
+    b = bufs_of(e, first, lane);
+    p = e->tp;
+    p.n_trees = n_trees;
+    p.slot0 = (int32_t)first;
+    p.root += first; p.ctl += first;
+    p.nodes += first * (size_t)e->node_cap;
+    p.leaf_state += first * TP_MAX_LEAVES; p.paths += first * TP_MAX_LEAVES * PATH_CAP; p.tp_aux += first * 2 * TP_MAX_LEAVES;
+    const ptrdiff_t first_row = b.nn_states - e->tp.nn_states;
+    p.nn_states = b.nn_states; p.nn_planes = b.nn_planes; p.nn_tree += first_row; p.nn_k += first_row;
+    p.nn_count += 2 * lane;
+    p.policy = b.policy;
+    p.value = b.value;
 }
 
 // work about to be enqueued on `s` touches the evaluator buffers / weights: order it behind an unfinished uttt_net_forward
@@ -127,7 +142,7 @@ int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_
                   cudaEvent_t* ev3 /* optional: [0] before trunk, [1] after trunk, [2] after heads */) {
     if (evaluator == UTTT_EVAL_HASH) {
         if (ev3) cudaEventRecord(ev3[0], s);
-        UTTT_CUDA_OK(launch_hash_eval(b.nn_states, b.nn_k, count, max_rows, b.policy, b.value, 1, 0, s));
+        UTTT_CUDA_OK(launch_hash_eval(b.nn_states, count, max_rows, b.policy, b.value, s));
         if (ev3) { cudaEventRecord(ev3[1], s); cudaEventRecord(ev3[2], s); }
         e->prof_launches[1] += 1;
         return 0;
@@ -187,8 +202,9 @@ int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const in
     UTTT_CUDA_OK(cudaMemcpy(trees.data(), p.nn_tree, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
     std::vector<float> pol((size_t)n_rows * 81), val((size_t)n_rows);
     std::vector<TreeCtl> ctl((size_t)p.n_trees);
-    std::vector<uint32_t> leaf((size_t)p.n_trees * 8);
-    UTTT_CUDA_OK(cudaMemcpy(leaf.data(), p.leaf_state, leaf.size() * 4, cudaMemcpyDeviceToHost));
+    std::vector<PackedState> leaf((size_t)p.n_trees);       // a tree's pending leaf is its leaf 0
+    UTTT_CUDA_OK(cudaMemcpy2D(leaf.data(), sizeof(PackedState), p.leaf_state, TP_MAX_LEAVES * sizeof(PackedState), sizeof(PackedState),
+                              leaf.size(), cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(pol.data(), b.policy, pol.size() * 4, cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(val.data(), b.value, val.size() * 4, cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(ctl.data(), p.ctl, ctl.size() * sizeof(TreeCtl), cudaMemcpyDeviceToHost));
@@ -201,7 +217,7 @@ int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const in
         rec.game_idx = (p.mode == MODE_SELFPLAY) ? ctl[t].game_idx : p.slot0 + t;
         rec.ply = (p.mode == MODE_SELFPLAY) ? ctl[t].ply : 0;
         rec.value = val[r];
-        memcpy(rec.state, leaf.data() + (size_t)t * 8, 32);
+        memcpy(rec.state, &leaf[(size_t)t], 32);
         const int g = (p.flags & UTTT_SP_RANDOM_SYMMETRY)
                           ? sym_draw(p.mode == MODE_SELFPLAY ? p.seed : 0u, ctl[t].game, (uint32_t)ctl[t].ply, (uint32_t)(ctl[t].n_eval - 1))
                           : 0;
@@ -258,8 +274,8 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     TreeParams& t = e->tp;
     t.node_cap = e->node_cap;
     if (ealloc(e, &t.root, S) || ealloc(e, &t.leaf_state, S * TP_MAX_LEAVES) ||
-        ealloc(e, &t.tp_paths, S * TP_MAX_LEAVES * PATH_CAP) || ealloc(e, &t.tp_aux, S * 2 * TP_MAX_LEAVES) || ealloc(e, &t.ctl, S) ||
-        ealloc(e, &t.path, S * PATH_CAP) || ealloc(e, &t.nodes, S * NC) ||
+        ealloc(e, &t.paths, S * TP_MAX_LEAVES * PATH_CAP) || ealloc(e, &t.tp_aux, S * 2 * TP_MAX_LEAVES) || ealloc(e, &t.ctl, S) ||
+        ealloc(e, &t.nodes, S * NC) ||
         ealloc(e, &t.nn_states, R) || ealloc(e, &t.nn_planes, R * 243 + 8) || ealloc(e, &t.nn_tree, R) ||
         ealloc(e, &t.nn_k, R) || ealloc(e, &t.nn_count, 2 * N_LANES) || ealloc(e, &t.out_counts, S * 81) ||
         ealloc(e, &t.out_n, S) || ealloc(e, &t.counters, 8) || ealloc(e, &t.hist_states, G * 81) ||
@@ -289,11 +305,6 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     for (int i = 0; i < EV_POOL; i++) UTTT_CUDA_OK(cudaEventCreate(&e->ev[i]));
     t.policy = e->policy;
     t.value = e->value;
-    t.dbg_tree = nullptr;
-    if (getenv("UTTT_DEBUG_TREE")) {
-        if (ealloc(e, &t.dbg_tree, 48)) { uttt_destroy(e); return 1; }
-        UTTT_CUDA_OK(cudaMemset(t.dbg_tree, 0, 48 * sizeof(unsigned long long)));
-    }
     t.max_terminal = getenv("UTTT_MAX_TERMINAL") ? atoi(getenv("UTTT_MAX_TERMINAL")) : 4;   // measured on the 500-game cycle: 2..4 best, 8: +0.8 %, 50: +8 %
     t.dir_alpha = 0.3f;
     t.dir_eps = 0.25f;
@@ -461,10 +472,9 @@ int uttt_mcts_search(uttt_engine* e, const uint32_t* roots, int32_t n_roots, int
     const bool tp = (flags & UTTT_SP_THROUGHPUT) != 0;
     UTTT_CHECK(!tp || batch <= TP_MAX_LEAVES, "throughput mode: at most %d leaves per tree per round", TP_MAX_LEAVES);
     UTTT_CHECK(!(tp && (flags & UTTT_SP_PYSEARCH)), "UTTT_SP_PYSEARCH and UTTT_SP_THROUGHPUT exclude each other");
-    if (mcts_begin_impl(e, roots, n_roots, sims, batch, flags)) return 1;     // uploads roots, runs the compat begin kernel
+    if (mcts_begin_impl(e, roots, n_roots, sims, batch, flags)) return 1;     // uploads roots, runs the begin kernel
     if (n_roots == 0) return 0;
     TreeParams& t = e->tp;
-    if (tp) UTTT_CUDA_OK(launch_tree_tp_begin(t, e->stream));
     // rounds are enqueued without host synchronisation; the tree kernel ignores finished trees.
     // Upper bound on rounds: every round retires >= 1 simulation of every unfinished tree (+ root evaluation).
     const int rows = tp ? n_roots * batch : n_roots;
@@ -576,32 +586,19 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
     for (int l = 0; l < n_lanes; l++) {
         size_t first = (size_t)l * (size_t)(n_trees / n_lanes);
         lane_trees[l] = (l == n_lanes - 1) ? n_trees - (int)first : n_trees / n_lanes;
-        TreeParams p = t;
-        p.n_trees = lane_trees[l];
-        p.slot0 = (int32_t)first;
-        p.root += first; p.leaf_state += first; p.ctl += first; p.path += first * PATH_CAP;
-        p.nodes += first * (size_t)e->node_cap;
-        size_t first_row = first * (size_t)e->rows_per_slot;
-        p.leaf_state += first * (TP_MAX_LEAVES - 1);      // leaf_state is [slot][TP_MAX_LEAVES]
-        p.tp_paths += first * TP_MAX_LEAVES * PATH_CAP; p.tp_aux += first * 2 * TP_MAX_LEAVES;
-        p.nn_states += first_row; p.nn_planes += first_row * 243; p.nn_tree += first_row; p.nn_k += first_row;
-        p.nn_count += 2 * l;
-        p.policy = e->policy + first * e->cfg.max_batch * 81;
-        p.value = e->value + first * e->cfg.max_batch;
-        lane_tp[l] = p;
-        lane_bufs[l] = bufs_of(e, first, l);
+        lane_of(e, first, lane_trees[l], l, lane_tp[l], lane_bufs[l]);
     }
     UTTT_CUDA_OK(cudaMemsetAsync(t.counters, 0, 8 * sizeof(unsigned long long), s));
     // (counters[0] = next game to hand out: the first n_trees games are assigned by tree_begin; set here, before the lanes
     // fork, so that no lane's begin kernel races with another lane's first recycled slot)
-    if (!tp) set_u64_kernel<<<1, 1, 0, s>>>(t.counters, (unsigned long long)n_trees);
+    set_u64_kernel<<<1, 1, 0, s>>>(t.counters, (unsigned long long)n_trees);
     UTTT_CUDA_OK(cudaMemsetAsync(t.hist_len, 0, (size_t)n_games * sizeof(int32_t), s));
     UTTT_CUDA_OK(cudaEventRecord(e->ev_fork, s));
     cudaStream_t ls[N_LANES];
     for (int l = 0; l < n_lanes; l++) {
         ls[l] = (n_lanes == 1) ? s : e->lane_stream[l];
         if (n_lanes > 1) UTTT_CUDA_OK(cudaStreamWaitEvent(ls[l], e->ev_fork, 0));
-        UTTT_CUDA_OK(tp ? launch_tree_tp_begin(lane_tp[l], ls[l]) : launch_tree_begin(lane_tp[l], ls[l]));
+        UTTT_CUDA_OK(launch_tree_begin(lane_tp[l], ls[l]));
         e->prof_launches[0] += 1;
     }
     // every round retires >= 1 simulation of every live slot: hard upper bound on rounds
@@ -694,15 +691,6 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
         }
     }
     UTTT_CUDA_OK(cudaMemcpy(e->h_counters, t.counters, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    if (t.dbg_tree) {              // UTTT_DEBUG_TREE: cycles of one tree's round by class (terminal descents, move decided)
-        unsigned long long d[48];
-        UTTT_CUDA_OK(cudaMemcpy(d, t.dbg_tree, sizeof(d), cudaMemcpyDeviceToHost));
-        UTTT_CUDA_OK(cudaMemset(t.dbg_tree, 0, sizeof(d)));
-        for (int c = 0; c < 16; c++)
-            if (d[3 * c + 1])
-                fprintf(stderr, "tree round class terminal=%d moved=%d: %llu warps, mean %llu cycles, max %llu\n", c & 7, c >> 3,
-                        d[3 * c + 1], d[3 * c] / d[3 * c + 1], d[3 * c + 2]);
-    }
     UTTT_CHECK(done, "self-play did not finish within %lld rounds", (long long)max_rounds);
     e->prof_launches[3] = e->prof_launches[0] + e->prof_launches[1] + e->prof_launches[2];
     if (stats) {

@@ -1,5 +1,7 @@
-// tree_common.cuh -- helpers shared by the reference-exact (tree_kernels.cu) and throughput (tree_tp_kernels.cu)
-// search kernels: node word accessors, warp-wide state load/store, Philox move sampling.
+// tree_common.cuh -- the warp pieces both search kernels are built from, the reference-exact (tree_kernels.cu) and the
+// throughput (tree_tp_kernels.cu) round: node word accessors, warp-wide state load/store, the evaluator row, the prior
+// normalisation, the PUCT descent, the leaf queue and the move decision with its Philox sampling.  None of them
+// depends on which kernel calls it; each kernel keeps its own schedule (phases, apply step, backup, round loop).
 #pragma once
 #include "common.cuh"
 
@@ -7,15 +9,23 @@ namespace uttt {
 
 constexpr unsigned FULL = 0xFFFFFFFFu;
 constexpr int WARPS_PER_BLOCK = 4;
+constexpr uint32_t LINK_PENDING = 0xFFFFFu;      // first_child marker: leaf queued, expansion outstanding (throughput mode)
 
 struct TreeView {
     uint4* node;     // [node_cap]
-    int32_t* path;   // [PATH_CAP]
 };
 
 __device__ __forceinline__ TreeView view_of(const TreeParams& P, int t) {
-    TreeView v = {P.nodes + (size_t)t * (size_t)P.node_cap, P.path + (size_t)t * PATH_CAP};
+    TreeView v = {P.nodes + (size_t)t * (size_t)P.node_cap};
     return v;
+}
+
+// the recorded path of pending leaf j of tree t (the reference-exact mode has one pending leaf, j = 0)
+__device__ __forceinline__ int32_t* leaf_path(const TreeParams& P, int t, int j) {
+    return P.paths + ((size_t)t * TP_MAX_LEAVES + j) * PATH_CAP;
+}
+__device__ __forceinline__ PackedState* leaf_state(const TreeParams& P, int t, int j) {
+    return P.leaf_state + (size_t)t * TP_MAX_LEAVES + j;
 }
 
 __device__ __forceinline__ uint4 make_node(int action, float p) {
@@ -99,6 +109,126 @@ __device__ __forceinline__ void warp_load_priors(const float* pol, int g, int la
     p2 = (lane < 17) ? __ldg(pol + e2) : 0.0f;
 }
 
+// priors of a leaf with legal mask lm (L legal actions) from its policy row: policy[legal] / sum in fp32, the sum taken
+// serially over the legal actions in ascending id (cpp/uttt_mcts.cpp:144-163), uniform if it is not positive.  One
+// coalesced read of the row, then one shuffle per addend (`a` is warp-uniform).  pr[q] is the prior of action
+// lane + 32 q (meaningful where that action is legal).
+__device__ __forceinline__ void legal_priors(const float* pol, int g, const uint32_t lm[3], int L, int lane, float pr[3]) {
+    float p0, p1, p2;
+    warp_load_priors(pol, g, lane, p0, p1, p2);
+    float sum = 0.0f;
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+        uint32_t m = lm[j];
+        while (m) {
+            int a = 27 * j + __ffs((int)m) - 1;
+            m &= m - 1u;
+            const float src = a < 32 ? p0 : (a < 64 ? p1 : p2);
+            sum = __fadd_rn(sum, __shfl_sync(FULL, src, a & 31));
+        }
+    }
+    const float uni = (L > 0) ? __fdiv_rn(1.0f, (float)L) : 0.0f;
+    pr[0] = (sum > 0.0f) ? __fdiv_rn(p0, sum) : uni;
+    pr[1] = (sum > 0.0f) ? __fdiv_rn(p1, sum) : uni;
+    pr[2] = (sum > 0.0f) ? __fdiv_rn(p2, sum) : uni;
+}
+
+// queues leaf `st` (legal mask lm) for the evaluator as evaluation c.n_eval of the tree's current move, standing for k
+// simulations; returns its row
+__device__ __forceinline__ int queue_leaf(const TreeParams& P, int t, TreeCtl& c, const PackedState& st, const uint32_t lm[3],
+                                          int k, int lane) {
+    int row = 0;
+    if (lane == 0) {
+        row = atomicAdd(P.nn_count + P.parity, 1);
+        atomicAdd(P.counters + 4, 1ull);
+    }
+    row = __shfl_sync(FULL, row, 0);
+    if (lane == 0) { P.nn_tree[row] = t; P.nn_k[row] = k; }
+    warp_write_row(P, row, st, lm, leaf_symmetry(P, c, c.n_eval), lane);
+    c.n_eval += 1;
+    return row;
+}
+
+enum : int { LEAF_UNEXPANDED = 0, LEAF_LOST = 1, LEAF_DRAWN = 2, LEAF_BLOCKED = 3 };
+
+struct Descent {
+    PackedState st;      // the position the descent ended on
+    uint32_t lm[3];      // its legal mask
+    int node, plen;      // its node, and the length of the path root..node
+    int end;             // LEAF_UNEXPANDED, LEAF_LOST / LEAF_DRAWN (terminal), LEAF_BLOCKED (a child already queued)
+};
+
+// descend from the root by PUCT (cpp/uttt_mcts.cpp:15-32,57-81), recording the node path into `path`.  Children are
+// read once (one 128-bit load each); lanes keep their first three in registers, longer lists (the reference-exact mode's
+// k-fold duplicated lists, Q-M3) are re-read through L1.  A child with vl units of virtual loss counts as n + vl
+// visits and w + vl lost value (the reference-exact mode sets none).
+__device__ __forceinline__ Descent descend(const TreeView& T, const PackedState& root, int32_t* path, int lane) {
+    Descent d;
+    d.st = root;
+    d.node = 0;
+    d.plen = 1;
+    d.end = LEAF_UNEXPANDED;
+    if (lane == 0) path[0] = 0;
+    uint32_t link = T.node[0].w;               // first_child | n_children<<20 of the current node
+    for (;;) {
+        const int L = legal_mask(d.st, d.lm);
+        if (is_lose(d.st)) { d.end = LEAF_LOST; break; }
+        if (L == 0) { d.end = LEAF_DRAWN; break; }
+        const uint32_t cbase = link & 0xFFFFFu;
+        if (cbase == 0u) break;
+        if (cbase == LINK_PENDING) { d.end = LEAF_BLOCKED; break; }
+        const int cnt = (int)(link >> 20);
+        const uint4* ch = T.node + cbase;
+        uint4 c0 = make_uint4(0, 0, 0, 0), c1 = c0, c2 = c0;
+        int tot = 0;
+        if (lane < cnt) { c0 = ch[lane]; tot += node_n(c0) + node_vloss(c0); }
+        if (lane + 32 < cnt) { c1 = ch[lane + 32]; tot += node_n(c1) + node_vloss(c1); }
+        if (lane + 64 < cnt) { c2 = ch[lane + 64]; tot += node_n(c2) + node_vloss(c2); }
+        for (int i = lane + 96; i < cnt; i += 32) { const uint4 q = ch[i]; tot += node_n(q) + node_vloss(q); }
+        tot = __reduce_add_sync(FULL, tot);
+        const float sq = __fsqrt_rn((float)tot);
+        float best = -1e9f;
+        int besti = 0x7FFFFFFF;
+        uint32_t bestx = 0u, bestlink = 0u;
+        auto consider = [&](const uint4& q, int i) {
+            const int vl = node_vloss(q), n = node_n(q) + vl;
+            // unvisited child (most of a k-fold duplicated list): q = 0 and u = (p*sq)/1, so pucb = p*sq exactly --
+            // the two IEEE divisions are only executed for visited children
+            float s = __fmul_rn(__uint_as_float(q.z), sq);
+            if (n > 0) {
+                const float qv = __fdiv_rn(-__fadd_rn(__uint_as_float(q.y), (float)vl), (float)n);
+                s = __fadd_rn(qv, __fdiv_rn(s, (float)(1 + n)));
+            }
+            if (s > best) { best = s; besti = i; bestx = q.x; bestlink = q.w; }
+        };
+        if (lane < cnt) consider(c0, lane);
+        if (lane + 32 < cnt) consider(c1, lane + 32);
+        if (lane + 64 < cnt) consider(c2, lane + 64);
+        for (int i = lane + 96; i < cnt; i += 32) consider(ch[i], i);
+        // first maximum wins (Q-M6): the largest score by one warp reduction on an order-preserving integer image of
+        // the float (scores are never -0.0 or NaN: q + u with u >= +0), then the smallest child index among the lanes
+        // that hold it, then that lane's node word -- 2 reductions + 2 shuffles instead of a 20-shuffle butterfly
+        {
+            const uint32_t fb = __float_as_uint(best);
+            const uint32_t key = (fb & 0x80000000u) ? ~fb : (fb | 0x80000000u);
+            const uint32_t kmax = __reduce_max_sync(FULL, key);
+            besti = (int)__reduce_min_sync(FULL, key == kmax ? (uint32_t)besti : 0x7FFFFFFFu);
+            const int src = besti & 31;                          // child i is held by lane i % 32
+            // (a lane's own candidate is its FIRST maximum, so the winning lane's registers hold child besti)
+            bestx = __shfl_sync(FULL, bestx, src);
+            bestlink = __shfl_sync(FULL, bestlink, src);
+        }
+        d.node = (int)cbase + besti;
+        link = bestlink;
+        PackedState nx;
+        next_state(d.st, (int)((bestx >> 16) & 0x7Fu), nx);
+        d.st = nx;
+        if (lane == 0) path[d.plen] = d.node;
+        d.plen++;
+    }
+    return d;
+}
+
 // Philox temperature-1 sampling over the root visit counts; returns the chosen action.
 // SP_TEMPERATURE != 1 (self_play_cpp.py:27,62 -> cpp/uttt_mcts.cpp:183-216): T == 0 plays the first maximum of the visit
 // counts (the reference's one-hot scores leave np.random.choice no choice); otherwise the move is drawn from
@@ -177,6 +307,49 @@ __device__ __forceinline__ int sample_move(const TreeParams& P, const TreeView& 
     }
     if (chosen < 0) chosen = 0;
     return nth_legal(lm, chosen);
+}
+
+// the move is decided (the simulation budget is spent).  Search: the root visit counts are the tree's output
+// (cpp/uttt_mcts.cpp:177-180) and the tree is done.  Self-play: record the history row, sample the move, play it; when
+// the game is over (lost or drawn, self_play_cpp.py:50-51,95) record it and claim the next game from counters[0].
+// Returns whether the tree goes on; if so `root` is the position of its next search, already stored in P.root[t].
+__device__ __forceinline__ bool decide_move(const TreeParams& P, const TreeView& T, int t, TreeCtl& c, PackedState& root, int lane) {
+    if (P.mode == MODE_SEARCH) {
+        for (int i = lane; i < 81; i += 32) P.out_counts[(size_t)t * 81 + i] = (i < c.n_root) ? node_n(T.node[1 + i]) : 0;
+        if (lane == 0) { P.out_n[t] = c.n_root; atomicAdd(P.counters + 6, 1ull); }
+        c.phase = PHASE_DONE;
+        return false;
+    }
+    uint32_t lm[3];
+    legal_mask(root, lm);
+    const size_t hrow = (size_t)c.game_idx * 81 + (size_t)c.ply;
+    warp_store_state(P.hist_states + hrow, root, lane);
+    for (int a = lane; a < 81; a += 32)
+        P.hist_counts[hrow * 81 + a] = legal_bit(lm, a) ? (uint16_t)node_n(T.node[1 + legal_rank(lm, a)]) : (uint16_t)0;
+    const int action = sample_move(P, T, c, lm, lane);
+    if (lane == 0) P.hist_actions[hrow] = (uint8_t)action;
+    PackedState nx;
+    next_state(root, action, nx);
+    root = nx;
+    c.ply += 1;
+    if (legal_mask(root, lm) == 0) {
+        if (lane == 0) {
+            P.hist_len[c.game_idx] = c.ply;
+            P.hist_final[c.game_idx] = is_lose(root) ? 1 : 0;
+            atomicAdd(P.counters + 1, 1ull);
+            atomicAdd(P.counters + 2, (unsigned long long)c.ply);
+        }
+        unsigned long long g = 0;
+        if (lane == 0) g = atomicAdd(P.counters + 0, 1ull);
+        g = __shfl_sync(FULL, g, 0);
+        if ((int64_t)g >= P.n_games) { c.phase = PHASE_DONE; return false; }
+        c.game = P.game0 + g;
+        c.game_idx = (int32_t)g;
+        c.ply = 0;
+        init_state(root);
+    }
+    warp_store_state(P.root + t, root, lane);
+    return true;
 }
 
 

@@ -25,6 +25,10 @@
 //
 // All float arithmetic on n/w/p uses explicit round-to-nearest intrinsics in the reference's
 // operation order (no FMA contraction, no reassociation): cpp/setup.py:10 builds with -O3 only.
+//
+// The round is built from the warp pieces of tree_common.cuh (prior normalisation, descent, leaf queue, move decision),
+// which the throughput round (tree_tp_kernels.cu) shares; its apply step, backup and round loop are its own.  This file
+// also holds the begin kernel of both modes, the device hash evaluator and the scores / boltzman kernels.
 #include "tree_common.cuh"
 
 namespace uttt {
@@ -57,10 +61,11 @@ __device__ void init_root(const TreeParams& P, const TreeView& T, TreeCtl& c, co
 }
 
 // cpp/uttt_mcts.cpp:47-54, k sequential backups of the same path (values may differ per copy)
-__device__ void backup(const TreeView& T, int plen, int k, const float* vals, int vstride, float v_single, int lane) {
+__device__ void backup(const TreeView& T, const int32_t* path, int plen, int k, const float* vals, int vstride, float v_single,
+                       int lane) {
     __syncwarp();
     for (int i = lane; i < plen; i += 32) {
-        int node = T.path[i];
+        int node = path[i];
         bool flip = ((plen - 1 - i) & 1) != 0;
         uint2* nw = reinterpret_cast<uint2*>(T.node + node);     // {n|action, w}
         uint2 q = *nw;
@@ -112,11 +117,12 @@ __device__ float numpy_sum_f32(float lp0, float lp1, float lp2, int L, int lane)
 
 // pv_mcts.py:105-109,157-160 for the k queued copies of one leaf: every copy REPLACES the child list (one list survives),
 // priors = policy[legal] / np.sum(policy[legal]) in float32 (pv_mcts.py:45-49), k sequential backups
-__device__ void apply_leaf_py(const TreeParams& P, const TreeView& T, TreeCtl& c, const PackedState& st, int lane) {
+__device__ void apply_leaf_py(const TreeParams& P, const TreeView& T, TreeCtl& c, const PackedState& st, const int32_t* path,
+                              int lane) {
     uint32_t lm[3];
     int L = legal_mask(st, lm);
     int k = c.pend_k, plen = c.path_len;
-    int leaf = T.path[plen - 1];
+    int leaf = path[plen - 1];
     int base = c.n_nodes;
     if (base + L > P.node_cap) {
         if (lane == 0) atomicExch(P.counters + 5, 1ull);
@@ -144,18 +150,19 @@ __device__ void apply_leaf_py(const TreeParams& P, const TreeView& T, TreeCtl& c
     }
     if (lane == 0) T.node[leaf].w = (uint32_t)base | ((uint32_t)L << 20);
     c.n_nodes = base + L;
-    backup(T, plen, k, P.value + row, 0, 0.0f, lane);
+    backup(T, path, plen, k, P.value + row, 0, 0.0f, lane);
     c.sims_left -= k;
     c.pend_k = 0;
     if (lane == 0) atomicAdd(P.counters + 3, (unsigned long long)k);
 }
 
 // cpp/uttt_mcts.cpp:138-167 for the k queued copies of one leaf
-__device__ void apply_leaf(const TreeParams& P, const TreeView& T, TreeCtl& c, const PackedState& st, int lane) {
+__device__ void apply_leaf(const TreeParams& P, const TreeView& T, TreeCtl& c, const PackedState& st, const int32_t* path,
+                           int lane) {
     uint32_t lm[3];
     int L = legal_mask(st, lm);
     int k = c.pend_k, plen = c.path_len;
-    int leaf = T.path[plen - 1];
+    int leaf = path[plen - 1];
     int base = c.n_nodes;
     if (base + k * L > P.node_cap) {          // cannot happen with node_cap = 1 + 81 + 81*max_sims
         if (lane == 0) atomicExch(P.counters + 5, 1ull);
@@ -165,42 +172,31 @@ __device__ void apply_leaf(const TreeParams& P, const TreeView& T, TreeCtl& c, c
     size_t row = (size_t)c.nn_row * (size_t)P.row_stride;
     const int g = leaf_symmetry(P, c, c.n_eval - 1);
     for (int cp = 0; cp < k; cp++) {
-        const float* pol = P.policy + (row + (size_t)cp * P.copy_stride) * 81;
-        // one coalesced read of the policy row (lane a holds actions a, a+32, a+64), then the reference's serial
-        // fp32 sum over the legal actions in ascending id (:144-152) with the addends fetched by shuffle
-        float p0, p1, p2;
-        warp_load_priors(pol, g, lane, p0, p1, p2);
-        float sum = 0.0f;
-#pragma unroll
-        for (int j = 0; j < 3; j++) {
-            uint32_t m = lm[j];
-            while (m) {
-                int a = 27 * j + __ffs((int)m) - 1;
-                m &= m - 1u;
-                const float src = a < 32 ? p0 : (a < 64 ? p1 : p2);          // `a` is warp-uniform: one shuffle per addend
-                sum = __fadd_rn(sum, __shfl_sync(FULL, src, a & 31));
-            }
-        }
-        float uni = (L > 0) ? __fdiv_rn(1.0f, (float)L) : 0.0f;
+        float pr[3];
+        legal_priors(P.policy + (row + (size_t)cp * P.copy_stride) * 81, g, lm, L, lane, pr);
         int reps = (P.copy_stride == 0) ? k : 1;       // identical rows: write all k copies at once
-        for (int q = 0, a = lane; a < 81; a += 32, q++) {
-            if (legal_bit(lm, a)) {
-                float pa = (q == 0) ? p0 : (q == 1 ? p1 : p2);
-                float pr = (sum > 0.0f) ? __fdiv_rn(pa, sum) : uni;                 // :155-163
+#pragma unroll
+        for (int q = 0; q < 3; q++) {
+            const int a = lane + 32 * q;
+            if (a < 81 && legal_bit(lm, a)) {
                 int r = legal_rank(lm, a);
-                for (int c2 = 0; c2 < reps; c2++) T.node[base + (cp + c2) * L + r] = make_node(a, pr);
+                for (int c2 = 0; c2 < reps; c2++) T.node[base + (cp + c2) * L + r] = make_node(a, pr[q]);
             }
         }
         if (P.copy_stride == 0) break;
     }
     if (lane == 0) T.node[leaf].w = (uint32_t)base | ((uint32_t)(k * L) << 20);
     c.n_nodes = base + k * L;
-    backup(T, plen, k, P.value + row, P.copy_stride, 0.0f, lane);
+    backup(T, path, plen, k, P.value + row, P.copy_stride, 0.0f, lane);
     c.sims_left -= k;
     c.pend_k = 0;
     if (lane == 0) atomicAdd(P.counters + 3, (unsigned long long)k);
 }
 
+// both search modes: reset the evaluator queue and give every tree its root.  Self-play slot t starts game slot0 + t
+// (a game's moves do not depend on its slot); later games are claimed from counters[0] as slots finish, which the
+// host starts at the number of slots before the lanes fork.  Search mode keys UTTT_SP_RANDOM_SYMMETRY's draw and the
+// root noise by the root's index.
 __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_begin_kernel(TreeParams P) {
     int t = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
     int lane = threadIdx.x & 31;
@@ -211,9 +207,6 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_begin_kernel(TreePa
     c.ply = 0; c.game = 0; c.game_idx = -1; c.nn_row = 0; c.n_eval = 0;
     PackedState rs;
     if (P.mode == MODE_SELFPLAY) {
-        // game g starts in slot g: the first games need no counter (a game's moves do not depend on its slot); later
-        // games are claimed from counters[0] as slots finish (the host starts it at the number of slots before the lanes
-        // fork)
         unsigned long long g = (unsigned long long)(P.slot0 + t);
         if ((int64_t)g >= P.n_games) {
             c.phase = PHASE_DONE;
@@ -225,20 +218,25 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_begin_kernel(TreePa
         init_state(rs);
         warp_store_state(P.root + t, rs, lane);
     } else {
-        c.game = (uint64_t)t;                 // search mode: the root's index keys UTTT_SP_RANDOM_SYMMETRY's draw
+        c.game = (uint64_t)t;
         rs = warp_load_state(P.root + t, lane);
     }
-    init_root(P, T, c, rs, lane);
-    if (c.n_root == 0) {                     // cpp/uttt_mcts.cpp:96-98: no legal move -> empty result
-        c.phase = PHASE_DONE;
-        if (lane == 0) { P.out_n[t] = 0; atomicAdd(P.counters + 6, 1ull); }
+    if (P.flags & UTTT_SP_THROUGHPUT) {
+        c.phase = PHASE_ROOT;                // the first round queues the root for evaluation
     } else {
-        c.phase = PHASE_SEARCH;
+        init_root(P, T, c, rs, lane);
+        if (c.n_root == 0) {                 // cpp/uttt_mcts.cpp:96-98: no legal move -> empty result
+            c.phase = PHASE_DONE;
+            if (lane == 0) { P.out_n[t] = 0; atomicAdd(P.counters + 6, 1ull); }
+        } else {
+            c.phase = PHASE_SEARCH;
+        }
     }
     if (lane == 0) P.ctl[t] = c;
 }
 
-__global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_round_kernel(TreeParams P) {
+// 7 blocks per SM (at most 73 registers): left to itself ptxas gives the inlined pieces more registers, and spills
+__global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 7) tree_round_kernel(TreeParams P) {
     pdl_trigger();          // the evaluator kernel behind this one may be scheduled now (it waits for this grid's results)
     pdl_wait();             // the previous round's evaluator has finished: policy / value rows are visible
     int t = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
@@ -246,18 +244,17 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_round_kernel(TreePa
     // the other parity's counter was consumed by the previous round's evaluator: reset it
     if (blockIdx.x == 0 && threadIdx.x == 0) P.nn_count[P.parity ^ 1] = 0;
     if (t >= P.n_trees) return;
-    const long long t_start = P.dbg_tree ? clock64() : 0;
-    int dbg_moved = 0;
     // the control block, the pending leaf and the root position have nothing to wait for: one L2 round trip for the three
-    const uint32_t leaf_raw = warp_load_state_issue(P.leaf_state + t, lane);
+    const uint32_t leaf_raw = warp_load_state_issue(leaf_state(P, t, 0), lane);
     const uint32_t root_raw = warp_load_state_issue(P.root + t, lane);
     TreeCtl c = P.ctl[t];
     if (c.phase == PHASE_DONE) return;
     TreeView T = view_of(P, t);
+    int32_t* path = leaf_path(P, t, 0);
 
     if (c.phase == PHASE_PENDING) {
-        if (P.flags & UTTT_SP_PYSEARCH) apply_leaf_py(P, T, c, warp_load_state_finish(leaf_raw), lane);
-        else apply_leaf(P, T, c, warp_load_state_finish(leaf_raw), lane);
+        if (P.flags & UTTT_SP_PYSEARCH) apply_leaf_py(P, T, c, warp_load_state_finish(leaf_raw), path, lane);
+        else apply_leaf(P, T, c, warp_load_state_finish(leaf_raw), path, lane);
         if (c.phase == PHASE_DONE) {
             if (lane == 0) P.ctl[t] = c;
             return;
@@ -269,121 +266,20 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_round_kernel(TreePa
     int n_terminal = 0;
     for (;;) {
         if (c.sims_left <= 0) {
-            // ---------------- the move is decided: root visit counts (cpp/uttt_mcts.cpp:177-180)
-            if (P.mode == MODE_SEARCH) {
-                for (int i = lane; i < 81; i += 32) P.out_counts[(size_t)t * 81 + i] = (i < c.n_root) ? node_n(T.node[1 + i]) : 0;
-                if (lane == 0) { P.out_n[t] = c.n_root; atomicAdd(P.counters + 6, 1ull); }
-                c.phase = PHASE_DONE;
-                break;
-            }
-            uint32_t lm[3];
-            legal_mask(root, lm);
-            size_t hrow = (size_t)c.game_idx * 81 + (size_t)c.ply;
-            warp_store_state(P.hist_states + hrow, root, lane);
-            for (int a = lane; a < 81; a += 32)
-                P.hist_counts[hrow * 81 + a] = legal_bit(lm, a) ? (uint16_t)node_n(T.node[1 + legal_rank(lm, a)]) : (uint16_t)0;
-            dbg_moved = 8;
-            int action = sample_move(P, T, c, lm, lane);
-            if (lane == 0) P.hist_actions[hrow] = (uint8_t)action;
-            PackedState nx;
-            next_state(root, action, nx);
-            root = nx;
-            c.ply += 1;
-            uint32_t lm2[3];
-            int L2 = legal_mask(root, lm2);
-            if (L2 == 0) {                     // game over (lost or drawn): self_play_cpp.py:50-51,95
-                if (lane == 0) {
-                    P.hist_len[c.game_idx] = c.ply;
-                    P.hist_final[c.game_idx] = is_lose(root) ? 1 : 0;
-                    atomicAdd(P.counters + 1, 1ull);
-                    atomicAdd(P.counters + 2, (unsigned long long)c.ply);
-                }
-                unsigned long long g = 0;
-                if (lane == 0) g = atomicAdd(P.counters + 0, 1ull);
-                g = __shfl_sync(FULL, g, 0);
-                if ((int64_t)g >= P.n_games) { c.phase = PHASE_DONE; break; }
-                c.game = P.game0 + g;
-                c.game_idx = (int32_t)g;
-                c.ply = 0;
-                init_state(root);
-            }
-            warp_store_state(P.root + t, root, lane);
+            if (!decide_move(P, T, t, c, root, lane)) break;
             __syncwarp();
             init_root(P, T, c, root, lane);
             __syncwarp();
         }
 
-        // ---------------- descend (cpp/uttt_mcts.cpp:15-32)
-        PackedState st = root;
-        int node = 0, plen = 1;
-        if (lane == 0) T.path[0] = 0;
-        uint32_t link = T.node[0].w;               // first_child | n_children<<20 of the current node
-        bool terminal = false, lost = false;
-        uint32_t lm[3];
-        for (;;) {
-            int L = legal_mask(st, lm);
-            lost = is_lose(st);
-            if (lost || L == 0) { terminal = true; break; }
-            const uint32_t cbase = link & 0xFFFFFu;
-            if (cbase == 0u) break;                                  // unexpanded leaf
-            const int cnt = (int)(link >> 20);
-            const uint4* ch = T.node + cbase;
-            // PUCT, cpp/uttt_mcts.cpp:57-81.  Children are read once (one 128-bit load each); lanes keep their
-            // first three children in registers, longer lists (k-fold duplicated, Q-M3) re-read through L1.
-            uint4 c0 = make_uint4(0, 0, 0, 0), c1 = c0, c2 = c0;
-            int tot = 0;
-            if (lane < cnt) { c0 = ch[lane]; tot += node_n(c0); }
-            if (lane + 32 < cnt) { c1 = ch[lane + 32]; tot += node_n(c1); }
-            if (lane + 64 < cnt) { c2 = ch[lane + 64]; tot += node_n(c2); }
-            for (int i = lane + 96; i < cnt; i += 32) tot += node_n(ch[i]);
-            tot = __reduce_add_sync(FULL, tot);
-            const float sq = __fsqrt_rn((float)tot);
-            float best = -1e9f;
-            int besti = 0x7FFFFFFF;
-            uint32_t bestx = 0u, bestlink = 0u;
-            auto consider = [&](const uint4& q, int i) {
-                int n = node_n(q);
-                // unvisited child (most of a k-fold duplicated list): q = 0 and u = (p*sq)/1, so pucb = p*sq exactly --
-                // the two IEEE divisions are only executed for visited children
-                float s = __fmul_rn(__uint_as_float(q.z), sq);
-                if (n > 0) {
-                    float qv = __fdiv_rn(-__uint_as_float(q.y), (float)n);
-                    s = __fadd_rn(qv, __fdiv_rn(s, (float)(1 + n)));
-                }
-                if (s > best) { best = s; besti = i; bestx = q.x; bestlink = q.w; }
-            };
-            if (lane < cnt) consider(c0, lane);
-            if (lane + 32 < cnt) consider(c1, lane + 32);
-            if (lane + 64 < cnt) consider(c2, lane + 64);
-            for (int i = lane + 96; i < cnt; i += 32) consider(ch[i], i);
-            // first maximum wins (Q-M6): the largest score by one warp reduction on an order-preserving integer image of
-            // the float (scores are never -0.0: q + u with u >= +0), then the smallest child index among the lanes that
-            // hold it, then that lane's node word -- 2 reductions + 2 shuffles instead of a 20-shuffle butterfly
-            {
-                const uint32_t fb = __float_as_uint(best);
-                const uint32_t key = (fb & 0x80000000u) ? ~fb : (fb | 0x80000000u);
-                const uint32_t kmax = __reduce_max_sync(FULL, key);
-                besti = (int)__reduce_min_sync(FULL, key == kmax ? (uint32_t)besti : 0x7FFFFFFFu);
-                const int src = besti & 31;                          // child i is held by lane i % 32
-                // (a lane's own candidate is its FIRST maximum, so the winning lane's registers hold child besti)
-                bestx = __shfl_sync(FULL, bestx, src);
-                bestlink = __shfl_sync(FULL, bestlink, src);
-            }
-            node = (int)cbase + besti;
-            link = bestlink;
-            PackedState nx;
-            next_state(st, (int)((bestx >> 16) & 0x7Fu), nx);
-            st = nx;
-            if (lane == 0) T.path[plen] = node;
-            plen++;
-        }
-
-        if (terminal) {
+        const Descent d = descend(T, root, path, lane);
+        if (d.end != LEAF_UNEXPANDED) {
             // cpp/uttt_mcts.cpp:19-21,115-118: the reference backs up -value with value = -1 for a lost
             // mover, i.e. +1 lands on the lost node itself (inverted sign, Q-M2); draws back up -0.0f.
+            const bool lost = d.end == LEAF_LOST;
             float v = lost ? 1.0f : -0.0f;
             if (P.flags & UTTT_SP_CORRECT_TERMINAL_SIGN) v = lost ? -1.0f : 0.0f;
-            backup(T, plen, 1, nullptr, 0, v, lane);
+            backup(T, path, d.plen, 1, nullptr, 0, v, lane);
             c.sims_left -= 1;
             if (lane == 0) atomicAdd(P.counters + 3, 1ull);
             // Every tree of the batch waits for the slowest warp of the round: bound the work of one round.  The
@@ -393,52 +289,31 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_round_kernel(TreePa
         }
 
         // ---------------- queue the leaf for the evaluator; fused leaf gather (cpp/uttt_game.cpp:244-280)
-        int k = min(P.batch, c.sims_left);                            // cpp/uttt_mcts.cpp:127 flush rule
-        int row = 0;
-        if (lane == 0) {
-            row = atomicAdd(P.nn_count + P.parity, 1);
-            atomicAdd(P.counters + 4, 1ull);
-        }
-        row = __shfl_sync(FULL, row, 0);
-        warp_store_state(P.leaf_state + t, st, lane);
-        if (lane == 0) { P.nn_tree[row] = t; P.nn_k[row] = k; }
-        warp_write_row(P, row, st, lm, leaf_symmetry(P, c, c.n_eval), lane);
-        c.n_eval += 1;
+        const int k = min(P.batch, c.sims_left);                      // cpp/uttt_mcts.cpp:127 flush rule
+        warp_store_state(leaf_state(P, t, 0), d.st, lane);
+        c.nn_row = queue_leaf(P, t, c, d.st, d.lm, k, lane);
         c.phase = PHASE_PENDING;
         c.pend_k = k;
-        c.nn_row = row;
-        c.path_len = plen;
+        c.path_len = d.plen;
         break;
     }
     if (lane == 0) P.ctl[t] = c;
-    if (P.dbg_tree && lane == 0) {
-        unsigned long long dt = (unsigned long long)(clock64() - t_start);
-        unsigned long long* d = P.dbg_tree + 3 * (min(n_terminal, 7) + dbg_moved);
-        atomicAdd(d, dt); atomicAdd(d + 1, 1ull); atomicMax(d + 2, dt);
-    }
 }
 
 // Deterministic integer-hash evaluator on the device (the "oracle evaluator" of the parity tests):
 // identical arithmetic to orc_hash_eval in oracle/uttt_oracle.c.
-__global__ void __launch_bounds__(128) hash_eval_kernel(const PackedState* __restrict__ states,
-                                                        const int32_t* __restrict__ kk,
-                                                        const int32_t* __restrict__ count, float* __restrict__ policy,
-                                                        float* __restrict__ value, int row_stride, int copy_stride) {
+__global__ void __launch_bounds__(128) hash_eval_kernel(const PackedState* __restrict__ states, const int32_t* __restrict__ count,
+                                                        float* __restrict__ policy, float* __restrict__ value) {
     int row = blockIdx.x * 4 + (threadIdx.x >> 5);
     int lane = threadIdx.x & 31;
     if (row >= *count) return;
     PackedState st = warp_load_state(states + row, lane);
     uint32_t h = state_hash(st);
-    int copies = (copy_stride == 0) ? 1 : kk[row];
-    for (int c = 0; c < copies; c++) {
-        size_t r = (size_t)row * row_stride + (size_t)c * copy_stride;
-        for (int a = lane; a < 81; a += 32) {
-            float num = (float)((mix32(h + (uint32_t)a) & 0xFFFFu) + 1u);
-            policy[r * 81 + a] = __fdiv_rn(__fdiv_rn(num, 65536.0f), 81.0f);
-        }
-        if (lane == 0)
-            value[r] = __fdiv_rn(__fsub_rn((float)(int)(mix32(h ^ 0xABCDu) & 0xFFFFu), 32768.0f), 32768.0f);
+    for (int a = lane; a < 81; a += 32) {
+        float num = (float)((mix32(h + (uint32_t)a) & 0xFFFFu) + 1u);
+        policy[(size_t)row * 81 + a] = __fdiv_rn(__fdiv_rn(num, 65536.0f), 81.0f);
     }
+    if (lane == 0) value[row] = __fdiv_rn(__fsub_rn((float)(int)(mix32(h ^ 0xABCDu) & 0xFFFFu), 32768.0f), 32768.0f);
 }
 
 // cpp/uttt_mcts.cpp:177-193: counts -> scores (one-hot at the first maximum for T==0, boltzman otherwise)
@@ -488,9 +363,9 @@ cudaError_t launch_tree_begin(const TreeParams& p, cudaStream_t s) {
 cudaError_t launch_tree_round(const TreeParams& p, cudaStream_t s) {
     return launch_pdl(tree_round_kernel, dim3(ceil_div(p.n_trees, WARPS_PER_BLOCK)), dim3(32 * WARPS_PER_BLOCK), 0, s, p);
 }
-cudaError_t launch_hash_eval(const PackedState* states, const int32_t* k, const int32_t* count, int max_rows,
-                             float* policy, float* value, int row_stride, int copy_stride, cudaStream_t s) {
-    hash_eval_kernel<<<ceil_div(max_rows, 4), 128, 0, s>>>(states, k, count, policy, value, row_stride, copy_stride);
+cudaError_t launch_hash_eval(const PackedState* states, const int32_t* count, int max_rows, float* policy, float* value,
+                             cudaStream_t s) {
+    hash_eval_kernel<<<ceil_div(max_rows, 4), 128, 0, s>>>(states, count, policy, value);
     return cudaGetLastError();
 }
 cudaError_t launch_scores(const int32_t* counts, const int32_t* n, int n_trees, float temperature, float* scores,

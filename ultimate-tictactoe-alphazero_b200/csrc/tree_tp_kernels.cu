@@ -11,11 +11,12 @@
 //     (seed, m), never on scheduling.
 // With m = 1 and eps = 0 it is plain sequential PUCT with an evaluated root; oracle/uttt_oracle.c carries a
 // CPU cross-check of exactly that configuration (orc_az_search_hash) for the bit-exact GPU test.
+// The round takes its descent, prior normalisation, leaf queue and move decision from tree_common.cuh, like the
+// reference-exact round; its phases, expansion (tp_expand, with the root noise), backup (tp_backup, removing virtual
+// loss) and round loop are its own.  tree_begin_kernel (tree_kernels.cu) starts its trees in PHASE_ROOT.
 #include "tree_common.cuh"
 
 namespace uttt {
-
-constexpr uint32_t LINK_PENDING = 0xFFFFFu;      // first_child marker: leaf queued, expansion outstanding
 
 // uniform in (0,1) from 24 random bits
 __device__ __forceinline__ float u01(uint32_t x) { return ((float)(x >> 8) + 0.5f) * (1.0f / 16777216.0f); }
@@ -65,31 +66,15 @@ struct TpAux {                 // per tree, per pending leaf
     int32_t nn_row[TP_MAX_LEAVES];
 };
 
-__device__ __forceinline__ int32_t* tp_path(const TreeParams& P, int t, int j) {
-    return P.tp_paths + ((size_t)t * TP_MAX_LEAVES + j) * PATH_CAP;
-}
-
-// expansion of `leaf` from one policy row, evaluated under symmetry `sym`: masked, serially renormalised priors (same arithmetic
-// as the reference-exact mode, cpp/uttt_mcts.cpp:144-163), optional Dirichlet mix for the root
+// expansion of `leaf` from one policy row, evaluated under symmetry `sym`: masked, serially renormalised priors (the
+// reference-exact mode's arithmetic), optional Dirichlet mix for the root
 __device__ void tp_expand(const TreeParams& P, const TreeView& T, TreeCtl& c, const PackedState& st, int leaf,
                           const float* pol, int sym, bool is_root, int lane) {
     uint32_t lm[3];
     int L = legal_mask(st, lm);
     int base = c.n_nodes;
-    float p0, p1, p2;
-    warp_load_priors(pol, sym, lane, p0, p1, p2);
-    float sum = 0.0f;
-#pragma unroll
-    for (int j = 0; j < 3; j++) {
-        uint32_t m = lm[j];
-        while (m) {
-            int a = 27 * j + __ffs((int)m) - 1;
-            m &= m - 1u;
-            const float src = a < 32 ? p0 : (a < 64 ? p1 : p2);          // `a` is warp-uniform
-            sum = __fadd_rn(sum, __shfl_sync(FULL, src, a & 31));
-        }
-    }
-    float uni = (L > 0) ? __fdiv_rn(1.0f, (float)L) : 0.0f;
+    float pr[3];
+    legal_priors(pol, sym, lm, L, lane, pr);
     const bool noise = is_root && P.dir_eps > 0.0f;
     float gsum = 0.0f, g[3] = {0.f, 0.f, 0.f};
     if (noise) {
@@ -98,11 +83,14 @@ __device__ void tp_expand(const TreeParams& P, const TreeView& T, TreeCtl& c, co
 #pragma unroll
         for (int off = 16; off > 0; off >>= 1) gsum += __shfl_xor_sync(FULL, gsum, off);
     }
-    for (int q = 0, a = lane; a < 81; a += 32, q++) {
-        if (legal_bit(lm, a)) {
-            float pr = (sum > 0.0f) ? __fdiv_rn(q == 0 ? p0 : (q == 1 ? p1 : p2), sum) : uni;
-            if (noise) pr = (1.0f - P.dir_eps) * pr + P.dir_eps * (gsum > 0.0f ? g[q] / gsum : uni);
-            T.node[base + legal_rank(lm, a)] = make_node(a, pr);
+    const float uni = (L > 0) ? __fdiv_rn(1.0f, (float)L) : 0.0f;
+#pragma unroll
+    for (int q = 0; q < 3; q++) {
+        const int a = lane + 32 * q;
+        if (a < 81 && legal_bit(lm, a)) {
+            float p = pr[q];
+            if (noise) p = (1.0f - P.dir_eps) * p + P.dir_eps * (gsum > 0.0f ? g[q] / gsum : uni);
+            T.node[base + legal_rank(lm, a)] = make_node(a, p);
         }
     }
     if (lane == 0) T.node[leaf].w = (uint32_t)base | ((uint32_t)L << 20);
@@ -125,51 +113,9 @@ __device__ void tp_backup(const TreeView& T, const int32_t* path, int plen, floa
     __syncwarp();
 }
 
-__global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_begin_kernel(TreeParams P) {
-    int t = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (blockIdx.x == 0 && threadIdx.x == 0) { P.nn_count[0] = 0; P.nn_count[1] = 0; }
-    if (t >= P.n_trees) return;
-    TreeCtl c = P.ctl[t];
-    c.ply = 0; c.game = 0; c.game_idx = -1; c.nn_row = 0; c.n_eval = 0; c.pend_k = 0; c.path_len = 0;
-    c.sims_left = P.sims; c.n_nodes = 1; c.n_root = 0;
-    if (P.mode == MODE_SELFPLAY) {
-        unsigned long long g = 0;
-        if (lane == 0) g = atomicAdd(P.counters + 0, 1ull);
-        g = __shfl_sync(FULL, g, 0);
-        if ((int64_t)g >= P.n_games) {
-            c.phase = PHASE_DONE;
-            if (lane == 0) P.ctl[t] = c;
-            return;
-        }
-        c.game = P.game0 + g;
-        c.game_idx = (int32_t)g;
-        PackedState rs;
-        init_state(rs);
-        warp_store_state(P.root + t, rs, lane);
-    } else {
-        c.game = (uint64_t)t;                 // search mode: the tree index keys the noise stream
-    }
-    c.phase = PHASE_ROOT;                     // the first round queues the root for evaluation
-    if (lane == 0) P.ctl[t] = c;
-}
-
-// queues evaluation j of the tree's current move
-__device__ __forceinline__ int tp_queue_leaf(const TreeParams& P, int t, TreeCtl& c, const PackedState& st, const uint32_t lm[3],
-                                             int lane) {
-    int row = 0;
-    if (lane == 0) {
-        row = atomicAdd(P.nn_count + P.parity, 1);
-        atomicAdd(P.counters + 4, 1ull);
-    }
-    row = __shfl_sync(FULL, row, 0);
-    if (lane == 0) { P.nn_tree[row] = t; P.nn_k[row] = 1; }
-    warp_write_row(P, row, st, lm, leaf_symmetry(P, c, c.n_eval), lane);
-    c.n_eval += 1;
-    return row;
-}
-
-__global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(TreeParams P) {
+// 5 blocks per SM (at most 102 registers): left to itself ptxas gives the inlined descent more registers, and fewer trees
+// would be resident
+__global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 5) tree_tp_round_kernel(TreeParams P) {
     int t = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
     int lane = threadIdx.x & 31;
     if (blockIdx.x == 0 && threadIdx.x == 0) P.nn_count[P.parity ^ 1] = 0;
@@ -195,9 +141,9 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
     } else if (c.phase == PHASE_PENDING) {
         for (int j = 0; j < c.pend_k; j++) {
             int plen = aux->path_len[j], row = aux->nn_row[j];
-            const int32_t* path = tp_path(P, t, j);
+            const int32_t* path = leaf_path(P, t, j);
             int leaf = path[plen - 1];
-            PackedState st = warp_load_state(P.leaf_state + (size_t)t * TP_MAX_LEAVES + j, lane);
+            PackedState st = warp_load_state(leaf_state(P, t, j), lane);
             if (c.n_nodes + 81 > P.node_cap) {
                 if (lane == 0) atomicExch(P.counters + 5, 1ull);
                 c.phase = PHASE_DONE;
@@ -215,43 +161,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
 
     for (int guard = 0; guard < 4; guard++) {
         if (c.phase == PHASE_SEARCH && c.sims_left <= 0) {
-            // ---------------- the move is decided
-            if (P.mode == MODE_SEARCH) {
-                for (int i = lane; i < 81; i += 32) P.out_counts[(size_t)t * 81 + i] = (i < c.n_root) ? node_n(T.node[1 + i]) : 0;
-                if (lane == 0) { P.out_n[t] = c.n_root; atomicAdd(P.counters + 6, 1ull); }
-                c.phase = PHASE_DONE;
-                break;
-            }
-            uint32_t lm[3];
-            legal_mask(root, lm);
-            size_t hrow = (size_t)c.game_idx * 81 + (size_t)c.ply;
-            warp_store_state(P.hist_states + hrow, root, lane);
-            for (int a = lane; a < 81; a += 32)
-                P.hist_counts[hrow * 81 + a] = legal_bit(lm, a) ? (uint16_t)node_n(T.node[1 + legal_rank(lm, a)]) : (uint16_t)0;
-            int action = sample_move(P, T, c, lm, lane);
-            if (lane == 0) P.hist_actions[hrow] = (uint8_t)action;
-            PackedState nx;
-            next_state(root, action, nx);
-            root = nx;
-            c.ply += 1;
-            uint32_t lm2[3];
-            if (legal_mask(root, lm2) == 0) {
-                if (lane == 0) {
-                    P.hist_len[c.game_idx] = c.ply;
-                    P.hist_final[c.game_idx] = is_lose(root) ? 1 : 0;
-                    atomicAdd(P.counters + 1, 1ull);
-                    atomicAdd(P.counters + 2, (unsigned long long)c.ply);
-                }
-                unsigned long long g = 0;
-                if (lane == 0) g = atomicAdd(P.counters + 0, 1ull);
-                g = __shfl_sync(FULL, g, 0);
-                if ((int64_t)g >= P.n_games) { c.phase = PHASE_DONE; break; }
-                c.game = P.game0 + g;
-                c.game_idx = (int32_t)g;
-                c.ply = 0;
-                init_state(root);
-            }
-            warp_store_state(P.root + t, root, lane);
+            if (!decide_move(P, T, t, c, root, lane)) break;
             c.phase = PHASE_ROOT;
         }
         if (c.phase == PHASE_ROOT) {
@@ -263,7 +173,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
                 break;
             }
             c.n_eval = 0;                                   // the root is evaluation 0 of the move's search
-            c.nn_row = tp_queue_leaf(P, t, c, root, lm, lane);
+            c.nn_row = queue_leaf(P, t, c, root, lm, 1, lane);
             c.phase = PHASE_ROOT_PENDING;
             break;
         }
@@ -272,74 +182,23 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
         int want = c.sims_left < m ? c.sims_left : m;
         int got = 0, terminals = 0;
         while (got < want && got + terminals < c.sims_left && terminals < 2 * m) {
-            int32_t* path = tp_path(P, t, got);
-            PackedState st = root;
-            int node = 0, plen = 1;
-            if (lane == 0) path[0] = 0;
-            uint32_t link = T.node[0].w;
-            bool terminal = false, lost = false, blocked = false;
-            uint32_t lm[3];
-            for (;;) {
-                int L = legal_mask(st, lm);
-                lost = is_lose(st);
-                if (lost || L == 0) { terminal = true; break; }
-                const uint32_t cbase = link & 0xFFFFFu;
-                if (cbase == 0u) break;
-                if (cbase == LINK_PENDING) { blocked = true; break; }
-                const int cnt = (int)(link >> 20);
-                const uint4* ch = T.node + cbase;
-                uint4 c0 = make_uint4(0, 0, 0, 0), c1 = c0, c2 = c0;
-                int tot = 0;
-                if (lane < cnt) { c0 = ch[lane]; tot += node_n(c0) + node_vloss(c0); }
-                if (lane + 32 < cnt) { c1 = ch[lane + 32]; tot += node_n(c1) + node_vloss(c1); }
-                if (lane + 64 < cnt) { c2 = ch[lane + 64]; tot += node_n(c2) + node_vloss(c2); }
-                tot = __reduce_add_sync(FULL, tot);
-                const float sq = __fsqrt_rn((float)tot);
-                float best = -1e9f;
-                int besti = 0x7FFFFFFF;
-                uint32_t bestx = 0u, bestlink = 0u;
-                auto consider = [&](const uint4& q, int i) {
-                    int vl = node_vloss(q), n = node_n(q) + vl;
-                    float w = __fadd_rn(__uint_as_float(q.y), (float)vl), p = __uint_as_float(q.z);
-                    float qv = (n > 0) ? __fdiv_rn(-w, (float)n) : 0.0f;
-                    float u = __fdiv_rn(__fmul_rn(p, sq), (float)(1 + n));
-                    float s = __fadd_rn(qv, u);
-                    if (s > best) { best = s; besti = i; bestx = q.x; bestlink = q.w; }
-                };
-                if (lane < cnt) consider(c0, lane);
-                if (lane + 32 < cnt) consider(c1, lane + 32);
-                if (lane + 64 < cnt) consider(c2, lane + 64);
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) {
-                    float ob = __shfl_xor_sync(FULL, best, off);
-                    int oi = __shfl_xor_sync(FULL, besti, off);
-                    uint32_t ox = __shfl_xor_sync(FULL, bestx, off);
-                    uint32_t ol = __shfl_xor_sync(FULL, bestlink, off);
-                    if (ob > best || (ob == best && oi < besti)) { best = ob; besti = oi; bestx = ox; bestlink = ol; }
-                }
-                node = (int)cbase + besti;
-                link = bestlink;
-                PackedState nx;
-                next_state(st, (int)((bestx >> 16) & 0x7Fu), nx);
-                st = nx;
-                if (lane == 0) path[plen] = node;
-                plen++;
-            }
-            if (blocked) break;                 // the best line ends in a leaf already queued this round
-            if (terminal) {
+            int32_t* path = leaf_path(P, t, got);
+            const Descent d = descend(T, root, path, lane);
+            if (d.end == LEAF_BLOCKED) break;       // the best line ends in a leaf already queued this round
+            if (d.end != LEAF_UNEXPANDED) {
                 // value for the mover of the terminal node: -1 lost, 0 draw (correct sign, unlike cpp/uttt_mcts.cpp:19-21)
-                tp_backup(T, path, plen, lost ? -1.0f : 0.0f, false, lane);
+                tp_backup(T, path, d.plen, d.end == LEAF_LOST ? -1.0f : 0.0f, false, lane);
                 terminals++;
                 continue;
             }
             // unexpanded leaf: mark it, add virtual loss along the path, queue it
             __syncwarp();
-            for (int i = lane; i < plen; i += 32) T.node[path[i]].x += (1u << 23);
-            if (lane == 0) T.node[node].w = LINK_PENDING;
+            for (int i = lane; i < d.plen; i += 32) T.node[path[i]].x += (1u << 23);
+            if (lane == 0) T.node[d.node].w = LINK_PENDING;
             __syncwarp();
-            int row = tp_queue_leaf(P, t, c, st, lm, lane);
-            warp_store_state(P.leaf_state + (size_t)t * TP_MAX_LEAVES + got, st, lane);
-            if (lane == 0) { aux->path_len[got] = plen; aux->nn_row[got] = row; }
+            int row = queue_leaf(P, t, c, d.st, d.lm, 1, lane);
+            warp_store_state(leaf_state(P, t, got), d.st, lane);
+            if (lane == 0) { aux->path_len[got] = d.plen; aux->nn_row[got] = row; }
             got++;
         }
         if (terminals) {
@@ -356,10 +215,6 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_tp_round_kernel(Tre
     if (lane == 0) P.ctl[t] = c;
 }
 
-cudaError_t launch_tree_tp_begin(const TreeParams& p, cudaStream_t s) {
-    tree_tp_begin_kernel<<<ceil_div(p.n_trees, WARPS_PER_BLOCK), 32 * WARPS_PER_BLOCK, 0, s>>>(p);
-    return cudaGetLastError();
-}
 cudaError_t launch_tree_tp_round(const TreeParams& p, cudaStream_t s) {
     tree_tp_round_kernel<<<ceil_div(p.n_trees, WARPS_PER_BLOCK), 32 * WARPS_PER_BLOCK, 0, s>>>(p);
     return cudaGetLastError();
