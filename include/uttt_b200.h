@@ -44,11 +44,12 @@ extern "C" {
                                            with Dirichlet noise, virtual loss, `batch_size` = leaves per tree per round
                                            (<= 16), single expansion per leaf, correct terminal sign (not in the reference) */
 
-#define UTTT_SP_PYSEARCH 4              /* uttt_mcts_search only: the semantics of the reference's pure-Python search
-                                           (pv_mcts.py:74-180, used by its gating match evaluate_network.py:73-75) instead
-                                           of the C++ one's: the root is evaluated like any leaf, a flush's k expansions
-                                           of a leaf replace each other (one child list), priors are normalised with
-                                           numpy's float32 pairwise sum */
+#define UTTT_SP_PYSEARCH 4              /* uttt_mcts_search, and uttt_selfplay_run* together with UTTT_SP_MATCH: the
+                                           semantics of the reference's pure-Python search (pv_mcts.py:74-180, used by its
+                                           gating match evaluate_network.py:73-75) instead of the C++ one's: the root is
+                                           evaluated like any leaf, a flush's k expansions of a leaf replace each other (one
+                                           child list), priors are normalised with numpy's float32 pairwise sum.  Excludes
+                                           UTTT_SP_THROUGHPUT. */
 #define UTTT_SP_RANDOM_SYMMETRY 8       /* uttt_mcts_search and uttt_selfplay_run*, any search mode and device evaluator:
                                            every leaf is evaluated under a board symmetry g drawn at random (AlphaGo Zero's
                                            evaluation-time augmentation) and the policy is mapped back.  Symmetry
@@ -63,6 +64,17 @@ extern "C" {
                                            evaluation; _THROUGHPUT: the root is j = 0).  uttt_mcts_search keys it with
                                            seed 0, game = root index in the call, ply 0.  g depends on neither slot nor
                                            batch position, so runs stay reproducible. */
+#define UTTT_SP_MATCH 16                /* uttt_selfplay_run* only: a match between the networks of weight slots 0 and 1
+                                           (uttt_upload_weights_slot).  Colour rule: in game g (the absolute id, game0 +
+                                           index) the position at ply p is searched with the network of slot (g + p) & 1,
+                                           i.e. slot 0 moves first in even games and slot 1 in odd ones (the reference's
+                                           evaluate_network.py:80-85); the rule keys on g, so a match split over calls by
+                                           game0 is the same match.  Everything else is self-play as without the flag
+                                           (search flags, temperature, Philox move draw, history).  The history is the
+                                           result: the point of slot 0 in game g is 0.5 if hist_final[g] == 0 (a draw),
+                                           else 1 if the last mover, slot (g + hist_len[g] - 1) & 1, is slot 0 and 0 if
+                                           not.  Fails if a network evaluator is asked for and slot 1 was never uploaded
+                                           (the hash evaluator reads no weights). */
 
 typedef struct uttt_engine uttt_engine;
 
@@ -159,6 +171,12 @@ typedef struct {
 } uttt_weights_scattered;
 int uttt_upload_weights_scattered(uttt_engine *e, const uttt_weights_scattered *w, int on_device);
 
+/* Weight slots: slot 0 is what uttt_upload_weights / _scattered write and what every evaluator reads; slot 1 is a second
+ * network, read only by the moves UTTT_SP_MATCH gives it.  slot must be 0 or 1.  The first upload to slot 1 allocates its
+ * weights and a second evaluator queue (about 1.8 KB per evaluator row); uttt_destroy frees them. */
+int uttt_upload_weights_slot(uttt_engine *e, int slot, const uttt_weights *w, int on_device);
+int uttt_upload_weights_scattered_slot(uttt_engine *e, int slot, const uttt_weights_scattered *w, int on_device);
+
 /* DualNetwork.forward on n packed states (dual_network.py:89-121 behind pv_mcts_cpp.py:37-78):
  * policy[n][81] (softmax over all 81 actions), value[n].  mode = UTTT_EVAL_NET_BF16 / _BF16X3 / _FP32. */
 int uttt_net_forward(uttt_engine *e, const uint32_t *states_dev, int64_t n, int mode,
@@ -246,7 +264,8 @@ int uttt_samples_unpack(const void *samples_dev, int64_t n, float *x_dev, float 
 /* timing of the engine's own kernels during the last uttt_selfplay_run*: CUDA-event ms on the
  * launching stream and launch counts; kind: 0 tree kernels, 1 trunk, 2 heads, 3 everything (ms: of the launches that were
  * bracketed by events, see uttt_set_profile_level; counts: of all launches); 4: the bracketed trunk launches (their ms,
- * their number), 5: the same ms and the number of positions those launches evaluated */
+ * their number), 5: the same ms and the number of positions those launches evaluated.  A match (UTTT_SP_MATCH) runs two
+ * evaluator passes per round: both are counted and bracketed. */
 int uttt_last_run_profile(uttt_engine *e, int kind, double *ms_out, int64_t *launches_out);
 
 /* which of those kernels are bracketed by CUDA events during self-play (an event between two dependent kernels costs
@@ -268,8 +287,8 @@ int uttt_debug_batch_histogram(uttt_engine *e, int64_t *out64, int32_t reset);
  * [5] node-arena overflow flag, [6] finished trees (search), [1] finished games (self-play) */
 int uttt_debug_counters(uttt_engine *e, uint64_t *out8);
 
-/* diagnostics for the parity tests: while enabled, uttt_mcts_search and uttt_selfplay_run* (reference-exact search only)
- * record every evaluated leaf with the evaluator rows its tree is about to consume -- (tree, game index, ply), packed leaf
+/* diagnostics for the parity tests: while enabled, uttt_mcts_search and uttt_selfplay_run* (reference-exact and
+ * UTTT_SP_PYSEARCH searches; a match records the rows of both networks' evaluator passes) record every evaluated leaf with the evaluator rows its tree is about to consume -- (tree, game index, ply), packed leaf
  * state, policy[81], value -- in evaluation order; the host synchronises after every round.  `enable` also clears the log.
  * uttt_debug_trace_read: *n_out = records; with cap >= *n_out the arrays meta[n][3], states[n][8], policy[n][81],
  * value[n] (HOST pointers) are filled; cap = 0 only asks for the size.  With UTTT_SP_RANDOM_SYMMETRY a record holds the

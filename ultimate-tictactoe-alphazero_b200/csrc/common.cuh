@@ -103,6 +103,15 @@ struct TreeParams {
     const float* policy;      // [(row*row_stride + copy*copy_stride)][81]
     const float* value;
     int32_t row_stride, copy_stride;
+    // UTTT_SP_MATCH: the queue of weight slot 1 (same layout as the one above, which is slot 0's), for the leaves of the
+    // moves that slot 1's network plays; nn1_count is always valid (the tree kernels reset it), the rest only in a match
+    PackedState* nn1_states;
+    __nv_bfloat16* nn1_planes;
+    int32_t* nn1_tree;
+    int32_t* nn1_k;
+    int32_t* nn1_count;       // [2]
+    const float* policy1;
+    const float* value1;
     // search outputs
     int32_t* out_counts;      // [n_trees][81]
     int32_t* out_n;           // [n_trees]

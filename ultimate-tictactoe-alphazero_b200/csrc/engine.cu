@@ -8,6 +8,7 @@
 // Here every game of a self-play cycle is a slot on the device; one "round" is
 //   tree_round kernel (apply previous evaluation, select next leaf, gather planes)
 //   -> evaluator (trunk_auto_kernel: tensor-core trunk + heads in one launch; or the fp32 kernels / hash evaluator)
+// (a match between two networks, UTTT_SP_MATCH, runs a second evaluator pass per round: slot 1's weights on slot 1's queue)
 // enqueued back to back on one stream; the host keeps two windows of CHECK_EVERY rounds in flight and reads the
 // progress counters of a window while the next one runs.
 #include <math.h>
@@ -25,7 +26,8 @@ namespace {
 constexpr int CHECK_EVERY = 8;             // rounds per host progress check (self-play: per window)
 constexpr int N_LANES = 2;
 constexpr int N_WINDOWS = 2;           // self-play keeps two windows of CHECK_EVERY rounds in flight
-constexpr int EV_POOL = N_WINDOWS * CHECK_EVERY * 4 * N_LANES;
+constexpr int EV_PER_ROUND = 8;        // events of one lane's round: before the tree round, then 3 per evaluator pass (2 passes)
+constexpr int EV_POOL = N_WINDOWS * CHECK_EVERY * EV_PER_ROUND * N_LANES;
 
 __global__ void set_int_kernel(int32_t* p, int32_t v) { *p = v; }
 __global__ void set_u64_kernel(unsigned long long* p, unsigned long long v) { *p = v; }
@@ -63,7 +65,14 @@ struct uttt_engine {
     int prof_sample;        // level 1: the trunk is bracketed in every prof_sample-th window of rounds only (see uttt_set_profile_level)
     int64_t prof_sampled_launches, prof_sampled_evals;      // trunk launches with events in the last run, positions they evaluated
     int lane_threshold;     // slots from which self-play splits into two overlapped lanes
-    NetWeights w;
+    NetWeights w;           // weight slot 0
+    NetWeights w1;          // weight slot 1 (UTTT_SP_MATCH), allocated by its first upload
+    // slot 1's evaluator queue, the same per-row arrays as slot 0's (e->tp.nn_*, policy, value, headfeat); allocated by the
+    // first slot-1 upload or match run, so that an engine that never plays a match keeps its footprint.  act_a / act_b /
+    // tc_resid are scratch that both passes of a round share (they run one after the other on a lane's stream).
+    struct {
+        PackedState* states; __nv_bfloat16* planes; int32_t *tree, *k; float *policy, *value, *headfeat;
+    } q1;
     unsigned long long* h_counters;   // pinned [8 * (1 + N_WINDOWS)]: [0..7] general use, then one copy per self-play window
     int32_t* h_count;                 // pinned [2]
     // step-wise search state
@@ -91,42 +100,69 @@ int ealloc(uttt_engine* e, T** p, size_t n) {
     return 0;
 }
 
-// the buffers one evaluator invocation works on (the whole engine, or one lane's slice of it)
+// the buffers one evaluator invocation works on (the whole engine, or one lane's slice of it) and the queue it reads
 struct EvalBufs {
     PackedState* nn_states;
     __nv_bfloat16* nn_planes;
+    int32_t *nn_tree, *nn_k;
     float *policy, *value, *act_a, *act_b, *resid, *headfeat;
 };
 
-EvalBufs bufs_of(uttt_engine* e, size_t first_slot, int lane) {
+// net 0: slot 0's queue; net 1: slot 1's (q1, allocated)
+EvalBufs bufs_of(uttt_engine* e, size_t first_slot, int lane, int net = 0) {
     EvalBufs b;
     size_t first_row = first_slot * (size_t)e->rows_per_slot;
-    b.nn_states = e->tp.nn_states + first_row;
-    b.nn_planes = e->tp.nn_planes + first_row * 243;
-    b.policy = e->policy + first_slot * e->cfg.max_batch * 81;
-    b.value = e->value + first_slot * e->cfg.max_batch;
+    b.nn_states = (net ? e->q1.states : e->tp.nn_states) + first_row;
+    b.nn_planes = (net ? e->q1.planes : e->tp.nn_planes) + first_row * 243;
+    b.nn_tree = (net ? e->q1.tree : e->tp.nn_tree) + first_row;
+    b.nn_k = (net ? e->q1.k : e->tp.nn_k) + first_row;
+    b.policy = (net ? e->q1.policy : e->policy) + first_slot * e->cfg.max_batch * 81;
+    b.value = (net ? e->q1.value : e->value) + first_slot * e->cfg.max_batch;
     b.act_a = e->act_a + first_row * 81 * 128;
     b.act_b = e->act_b + first_row * 81 * 128;
-    b.headfeat = e->headfeat + first_row * 243;
+    b.headfeat = (net ? e->q1.headfeat : e->headfeat) + first_row * 243;
     b.resid = e->tc_resid + (size_t)lane * e->n_sm * 512 * 64;     // fp16 panels: 128 KiB per CTA
     return b;
 }
 
-// self-play lane `lane` runs the slots [first, first + n_trees): its slice of the trees and of the evaluator queue (p),
-// and of the evaluator's buffers (b)
-void lane_of(uttt_engine* e, size_t first, int n_trees, int lane, TreeParams& p, EvalBufs& b) {
-    b = bufs_of(e, first, lane);
+// self-play lane `lane` runs the slots [first, first + n_trees): its slice of the trees and of the evaluator queues (p),
+// and of the evaluator's buffers of each network (b[net]; net 1 only with `match`)
+void lane_of(uttt_engine* e, size_t first, int n_trees, int lane, bool match, TreeParams& p, EvalBufs b[2]) {
+    b[0] = bufs_of(e, first, lane, 0);
     p = e->tp;
     p.n_trees = n_trees;
     p.slot0 = (int32_t)first;
     p.root += first; p.ctl += first;
     p.nodes += first * (size_t)e->node_cap;
     p.leaf_state += first * TP_MAX_LEAVES; p.paths += first * TP_MAX_LEAVES * PATH_CAP; p.tp_aux += first * 2 * TP_MAX_LEAVES;
-    const ptrdiff_t first_row = b.nn_states - e->tp.nn_states;
-    p.nn_states = b.nn_states; p.nn_planes = b.nn_planes; p.nn_tree += first_row; p.nn_k += first_row;
+    p.nn_states = b[0].nn_states; p.nn_planes = b[0].nn_planes; p.nn_tree = b[0].nn_tree; p.nn_k = b[0].nn_k;
     p.nn_count += 2 * lane;
-    p.policy = b.policy;
-    p.value = b.value;
+    p.nn1_count += 2 * lane;
+    p.policy = b[0].policy;
+    p.value = b[0].value;
+    if (match) {
+        b[1] = bufs_of(e, first, lane, 1);
+        p.nn1_states = b[1].nn_states; p.nn1_planes = b[1].nn_planes; p.nn1_tree = b[1].nn_tree; p.nn1_k = b[1].nn_k;
+        p.policy1 = b[1].policy;
+        p.value1 = b[1].value;
+    }
+}
+
+// slot 1's evaluator queue (q1), on first use
+int alloc_queue1(uttt_engine* e) {
+    if (e->q1.states) return 0;
+    const size_t S = (size_t)e->cfg.n_slots, R = S * (size_t)e->rows_per_slot;
+    auto al = [&](auto** p, size_t n) -> int {
+        UTTT_CUDA_OK(cudaMalloc((void**)p, (n ? n : 1) * sizeof(**p)));
+        e->allocs.push_back((void*)*p);
+        return 0;
+    };
+    decltype(e->q1) q;
+    if (al(&q.planes, R * 243 + 8) || al(&q.tree, R) || al(&q.k, R) || al(&q.policy, S * e->cfg.max_batch * 81) ||
+        al(&q.value, S * e->cfg.max_batch) || al(&q.headfeat, R * 243) || al(&q.states, R))
+        return 1;
+    e->q1 = q;
+    return 0;
 }
 
 // work about to be enqueued on `s` touches the evaluator buffers / weights: order it behind an unfinished uttt_net_forward
@@ -138,8 +174,9 @@ int wait_for_forward(uttt_engine* e, cudaStream_t s) {
     return 0;
 }
 
-int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_t* count, int max_rows, cudaStream_t s,
-                  cudaEvent_t* ev3 /* optional: [0] before trunk, [1] after trunk, [2] after heads */) {
+// one evaluator pass: the network `w` over the queue whose rows are b's and whose length is *count
+int run_evaluator(uttt_engine* e, const NetWeights& w, const EvalBufs& b, int evaluator, const int32_t* count, int max_rows,
+                  cudaStream_t s, cudaEvent_t* ev3 /* optional: [0] before trunk, [1] after trunk, [2] after heads */) {
     if (evaluator == UTTT_EVAL_HASH) {
         if (ev3) cudaEventRecord(ev3[0], s);
         UTTT_CUDA_OK(launch_hash_eval(b.nn_states, count, max_rows, b.policy, b.value, s));
@@ -147,17 +184,17 @@ int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_
         e->prof_launches[1] += 1;
         return 0;
     }
-    UTTT_CHECK(e->w.loaded, "network weights not uploaded (uttt_upload_weights)");
+    UTTT_CHECK(w.loaded, "network weights not uploaded (uttt_upload_weights)");
     bool heads_fused = false;
     if (evaluator == UTTT_EVAL_NET_FP32) {
         if (ev3) cudaEventRecord(ev3[0], s);
-        UTTT_CUDA_OK(launch_trunk_fp32(e->w, b.nn_planes, count, max_rows, b.act_a, b.act_b, s));
+        UTTT_CUDA_OK(launch_trunk_fp32(w, b.nn_planes, count, max_rows, b.act_a, b.act_b, s));
         e->prof_launches[1] += 1 + 2 * NET_BLOCKS;
     } else if (evaluator == UTTT_EVAL_NET_BF16X3) {
         // split-bf16 numerics: one launch for any batch (groups of <= 5 positions per CTA pair, several waves if needed);
         // the heads' FC layers follow as their own kernel (1 % of a round here: the trunk issues 3x the MMAs)
         if (ev3) cudaEventRecord(ev3[0], s);
-        UTTT_CUDA_OK(launch_trunk_x3(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg));
+        UTTT_CUDA_OK(launch_trunk_x3(w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg));
         e->prof_launches[1] += 1;
     } else if (evaluator == UTTT_EVAL_NET_BF16) {
         // conv_input runs inside the trunk kernels (tensor pipe, "layer -1").  The queue length is only known on the
@@ -168,10 +205,10 @@ int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_
         // batches above 7 positions per CTA pair (only possible when max_rows allows them) are left to the
         // 10-positions-per-pair kernel; if no batch can exceed that, the heads' FC layers run in the tail of trunk_auto_kernel
         heads_fused = max_rows <= trunk_pp_cap1(e->n_sm);
-        UTTT_CUDA_OK(launch_trunk_auto(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg,
+        UTTT_CUDA_OK(launch_trunk_auto(w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg,
                                        heads_fused ? b.policy : nullptr, heads_fused ? b.value : nullptr));
         if (!heads_fused)
-            UTTT_CUDA_OK(launch_trunk_pp_large(e->w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg));
+            UTTT_CUDA_OK(launch_trunk_pp_large(w, b.nn_planes, b.headfeat, count, max_rows, b.resid, e->n_sm, s, e->tc_dbg));
         e->prof_launches[1] += 1;
     } else {
         UTTT_CHECK(false, "evaluator %d cannot run on the device", evaluator);
@@ -182,24 +219,24 @@ int run_evaluator(uttt_engine* e, const EvalBufs& b, int evaluator, const int32_
         return 0;
     }
     if (evaluator == UTTT_EVAL_NET_BF16 || evaluator == UTTT_EVAL_NET_BF16X3)
-        UTTT_CUDA_OK(launch_heads_fc(e->w, b.headfeat, count, max_rows, b.policy, b.value, 1, s));
+        UTTT_CUDA_OK(launch_heads_fc(w, b.headfeat, count, max_rows, b.policy, b.value, 1, s));
     else
-        UTTT_CUDA_OK(launch_heads(e->w, b.act_a, nullptr, count, max_rows, b.policy, b.value, 1, s));
+        UTTT_CUDA_OK(launch_heads(w, b.act_a, nullptr, count, max_rows, b.policy, b.value, 1, s));
     e->prof_launches[2] += 1;
     if (ev3 && e->prof_level >= 2) cudaEventRecord(ev3[2], s);
     return 0;
 }
 
-// uttt_debug_trace: after a round's evaluator, record (tree, game, ply, leaf state, policy row, value) of every queued leaf:
-// the untransformed leaf and its row in the leaf's own action ids (UTTT_SP_RANDOM_SYMMETRY: entry a = row entry sigma_g(a)),
-// i.e. exactly what the tree consumes.  Synchronises the stream (diagnostics only).
+// uttt_debug_trace: after a round's evaluator pass over queue b, record (tree, game, ply, leaf state, policy row, value) of
+// every leaf queued there: the untransformed leaf and its row in the leaf's own action ids (UTTT_SP_RANDOM_SYMMETRY: entry
+// a = row entry sigma_g(a)), i.e. exactly what the tree consumes.  Synchronises the stream (diagnostics only).
 int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const int32_t* count, cudaStream_t s) {
     UTTT_CUDA_OK(cudaStreamSynchronize(s));
     int32_t n_rows = 0;
     UTTT_CUDA_OK(cudaMemcpy(&n_rows, count, sizeof(n_rows), cudaMemcpyDeviceToHost));
     if (n_rows == 0) return 0;
     std::vector<int32_t> trees((size_t)n_rows);
-    UTTT_CUDA_OK(cudaMemcpy(trees.data(), p.nn_tree, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
+    UTTT_CUDA_OK(cudaMemcpy(trees.data(), b.nn_tree, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
     std::vector<float> pol((size_t)n_rows * 81), val((size_t)n_rows);
     std::vector<TreeCtl> ctl((size_t)p.n_trees);
     std::vector<PackedState> leaf((size_t)p.n_trees);       // a tree's pending leaf is its leaf 0
@@ -250,6 +287,8 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     uttt_engine* e = new uttt_engine();
     memset(&e->tp, 0, sizeof(e->tp));
     memset(&e->w, 0, sizeof(e->w));
+    memset(&e->w1, 0, sizeof(e->w1));
+    memset(&e->q1, 0, sizeof(e->q1));
     e->cfg = *cfg;
     e->trace_on = false;
     e->progress_cb = nullptr;
@@ -277,7 +316,7 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
         ealloc(e, &t.paths, S * TP_MAX_LEAVES * PATH_CAP) || ealloc(e, &t.tp_aux, S * 2 * TP_MAX_LEAVES) || ealloc(e, &t.ctl, S) ||
         ealloc(e, &t.nodes, S * NC) ||
         ealloc(e, &t.nn_states, R) || ealloc(e, &t.nn_planes, R * 243 + 8) || ealloc(e, &t.nn_tree, R) ||
-        ealloc(e, &t.nn_k, R) || ealloc(e, &t.nn_count, 2 * N_LANES) || ealloc(e, &t.out_counts, S * 81) ||
+        ealloc(e, &t.nn_k, R) || ealloc(e, &t.nn_count, 4 * N_LANES) || ealloc(e, &t.out_counts, S * 81) ||
         ealloc(e, &t.out_n, S) || ealloc(e, &t.counters, 8) || ealloc(e, &t.hist_states, G * 81) ||
         ealloc(e, &t.hist_counts, G * 81 * 81) || ealloc(e, &t.hist_actions, G * 81) || ealloc(e, &t.hist_len, G) ||
         ealloc(e, &t.hist_final, G) || ealloc(e, &e->policy, S * cfg->max_batch * 81) ||
@@ -290,7 +329,8 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     }
     UTTT_CUDA_OK(cudaMemset(t.ctl, 0, S * sizeof(TreeCtl)));
     UTTT_CUDA_OK(cudaMemset(e->tc_dbg, 0, (128 + 64) * sizeof(long long)));
-    UTTT_CUDA_OK(cudaMemset(t.nn_count, 0, 2 * N_LANES * sizeof(int32_t)));
+    UTTT_CUDA_OK(cudaMemset(t.nn_count, 0, 4 * N_LANES * sizeof(int32_t)));
+    t.nn1_count = t.nn_count + 2 * N_LANES;         // slot 1's queue lengths: [lane][parity] behind slot 0's
     for (int i = 0; i < N_LANES; i++) {
         UTTT_CUDA_OK(cudaStreamCreateWithFlags(&e->lane_stream[i], cudaStreamNonBlocking));
         UTTT_CUDA_OK(cudaEventCreateWithFlags(&e->ev_join[i], cudaEventDisableTiming));
@@ -319,6 +359,7 @@ int uttt_destroy(uttt_engine* e) {
     cudaDeviceSynchronize();
     for (void* p : e->allocs) cudaFree(p);
     release_weights(e->w);
+    release_weights(e->w1);
     if (e->h_counters) cudaFreeHost(e->h_counters);
     if (e->h_count) cudaFreeHost(e->h_count);
     for (int i = 0; i < EV_POOL; i++) if (e->ev[i]) cudaEventDestroy(e->ev[i]);
@@ -336,24 +377,35 @@ int uttt_destroy(uttt_engine* e) {
 }
 
 // ---------------------------------------------------------------------------- weights
-static int upload_impl(uttt_engine* e, const uttt_weights* w, int on_device, const float* const* res_tab,
+static int upload_impl(uttt_engine* e, int slot, const uttt_weights* w, int on_device, const float* const* res_tab,
                        const float* const (*res_bn_tab)[4]) {
+    UTTT_CHECK(slot == 0 || slot == 1, "weight slot %d: must be 0 or 1", slot);
     UTTT_CHECK(e && w, "null argument");
     UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
     if (e->fwd_pending) {          // (the upload is synchronous and partly uses blocking copies: wait on the host)
         UTTT_CUDA_OK(cudaEventSynchronize(e->ev_fwd));
         e->fwd_pending = false;
     }
-    return upload_weights(e->w, w, on_device, res_tab, res_bn_tab, e->stream);
+    if (slot == 1 && alloc_queue1(e)) return 1;
+    return upload_weights(slot ? e->w1 : e->w, w, on_device, res_tab, res_bn_tab, e->stream);
+}
+
+int uttt_upload_weights_slot(uttt_engine* e, int slot, const uttt_weights* w, int on_device) {
+    return upload_impl(e, slot, w, on_device, nullptr, nullptr);
+}
+
+int uttt_upload_weights_scattered_slot(uttt_engine* e, int slot, const uttt_weights_scattered* w, int on_device) {
+    UTTT_CHECK(slot == 0 || slot == 1, "weight slot %d: must be 0 or 1", slot);
+    UTTT_CHECK(e && w, "null argument");
+    return upload_impl(e, slot, &w->small, on_device, w->res_conv_w, w->res_bn);
 }
 
 int uttt_upload_weights(uttt_engine* e, const uttt_weights* w, int on_device) {
-    return upload_impl(e, w, on_device, nullptr, nullptr);
+    return uttt_upload_weights_slot(e, 0, w, on_device);
 }
 
 int uttt_upload_weights_scattered(uttt_engine* e, const uttt_weights_scattered* w, int on_device) {
-    UTTT_CHECK(e && w, "null argument");
-    return upload_impl(e, &w->small, on_device, w->res_conv_w, w->res_bn);
+    return uttt_upload_weights_scattered_slot(e, 0, w, on_device);
 }
 
 int uttt_net_forward(uttt_engine* e, const uint32_t* states_dev, int64_t n, int mode, float* policy_dev,
@@ -370,7 +422,7 @@ int uttt_net_forward(uttt_engine* e, const uint32_t* states_dev, int64_t n, int 
         int m = (int)((n - off < e->cfg.n_slots) ? (n - off) : e->cfg.n_slots);
         if (uttt_game_gather_planes(states_dev + off * 8, e->tp.nn_planes, m, s)) return 1;
         set_int_kernel<<<1, 1, 0, s>>>(e->fwd_count, m);
-        if (run_evaluator(e, bufs_of(e, 0, 0), mode, e->fwd_count, m, s, nullptr)) return 1;
+        if (run_evaluator(e, e->w, bufs_of(e, 0, 0), mode, e->fwd_count, m, s, nullptr)) return 1;
         UTTT_CUDA_OK(cudaMemcpyAsync(policy_dev + off * 81, e->policy, (size_t)m * 81 * sizeof(float),
                                      cudaMemcpyDeviceToDevice, s));
         UTTT_CUDA_OK(cudaMemcpyAsync(value_dev + off, e->value, (size_t)m * sizeof(float), cudaMemcpyDeviceToDevice, s));
@@ -472,6 +524,7 @@ int uttt_mcts_search(uttt_engine* e, const uint32_t* roots, int32_t n_roots, int
     const bool tp = (flags & UTTT_SP_THROUGHPUT) != 0;
     UTTT_CHECK(!tp || batch <= TP_MAX_LEAVES, "throughput mode: at most %d leaves per tree per round", TP_MAX_LEAVES);
     UTTT_CHECK(!(tp && (flags & UTTT_SP_PYSEARCH)), "UTTT_SP_PYSEARCH and UTTT_SP_THROUGHPUT exclude each other");
+    UTTT_CHECK(!(flags & UTTT_SP_MATCH), "UTTT_SP_MATCH is a self-play mode (uttt_selfplay_run*), not a search option");
     if (mcts_begin_impl(e, roots, n_roots, sims, batch, flags)) return 1;     // uploads roots, runs the begin kernel
     if (n_roots == 0) return 0;
     TreeParams& t = e->tp;
@@ -486,7 +539,7 @@ int uttt_mcts_search(uttt_engine* e, const uint32_t* roots, int32_t n_roots, int
         for (; r < stop; r++) {
             t.parity = r & 1;
             UTTT_CUDA_OK(tp ? launch_tree_tp_round(t, e->stream) : launch_tree_round(t, e->stream));
-            if (run_evaluator(e, bufs, evaluator, t.nn_count + t.parity, rows, e->stream, nullptr)) return 1;
+            if (run_evaluator(e, e->w, bufs, evaluator, t.nn_count + t.parity, rows, e->stream, nullptr)) return 1;
             if (e->trace_on && !tp && trace_round(e, t, bufs, t.nn_count + t.parity, e->stream)) return 1;
         }
         UTTT_CUDA_OK(cudaMemcpyAsync(e->h_count, t.nn_count + ((r - 1) & 1), sizeof(int32_t), cudaMemcpyDeviceToHost,
@@ -559,11 +612,17 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
                "self-play needs a device evaluator");
     int n_trees = (int)((n_games < e->cfg.n_slots) ? n_games : e->cfg.n_slots);
     if (check_search_args(e, n_trees, sims, batch)) return 1;
-    UTTT_CHECK(!(flags & UTTT_SP_PYSEARCH), "UTTT_SP_PYSEARCH is a search option (uttt_mcts_search), not a self-play mode");
+    const bool match = (flags & UTTT_SP_MATCH) != 0;
+    UTTT_CHECK(match || !(flags & UTTT_SP_PYSEARCH),
+               "UTTT_SP_PYSEARCH is a search option (uttt_mcts_search) and a match option (UTTT_SP_MATCH), not a self-play mode");
     const bool tp = (flags & UTTT_SP_THROUGHPUT) != 0;
+    UTTT_CHECK(!(tp && (flags & UTTT_SP_PYSEARCH)), "UTTT_SP_PYSEARCH and UTTT_SP_THROUGHPUT exclude each other");
     UTTT_CHECK(!tp || batch <= TP_MAX_LEAVES, "throughput mode: at most %d leaves per tree per round", TP_MAX_LEAVES);
+    UTTT_CHECK(!match || evaluator == UTTT_EVAL_HASH || e->w1.loaded,
+               "UTTT_SP_MATCH: weight slot 1 was never uploaded (uttt_upload_weights_slot(e, 1, ...))");
     const int rows_per_tree = tp ? batch : 1;
     UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
+    if (match && alloc_queue1(e)) return 1;
     cudaStream_t s = stream ? (cudaStream_t)stream : e->stream;
     for (int i = 0; i < 4; i++) { e->prof_ms[i] = 0.0; e->prof_launches[i] = 0; }
     e->prof_sampled_launches = e->prof_sampled_evals = 0;
@@ -580,13 +639,18 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
     // game/progress counters and the history buffers (disjoint rows).
     // (worth it only when half a batch still fills the machine; small batches are latency-bound)
     const int n_lanes = (n_trees >= e->lane_threshold) ? N_LANES : 1;
+    // A match runs two evaluator passes per round and lane, slot 0's network on slot 0's queue, then slot 1's on slot 1's:
+    // each is the usual chain of programmatic dependent launches, so the second trunk launch follows the first pass's
+    // last kernel (which, like every kernel of the chain, waits for its predecessor before it touches memory) and reuses
+    // its scratch.  A pass whose queue is empty costs its launches only: the kernels read the count and exit.
+    const int n_nets = match ? 2 : 1;
     TreeParams lane_tp[N_LANES];
-    EvalBufs lane_bufs[N_LANES];
+    EvalBufs lane_bufs[N_LANES][2];
     int lane_trees[N_LANES];
     for (int l = 0; l < n_lanes; l++) {
         size_t first = (size_t)l * (size_t)(n_trees / n_lanes);
         lane_trees[l] = (l == n_lanes - 1) ? n_trees - (int)first : n_trees / n_lanes;
-        lane_of(e, first, lane_trees[l], l, lane_tp[l], lane_bufs[l]);
+        lane_of(e, first, lane_trees[l], l, match, lane_tp[l], lane_bufs[l]);
     }
     UTTT_CUDA_OK(cudaMemsetAsync(t.counters, 0, 8 * sizeof(unsigned long long), s));
     // (counters[0] = next game to hand out: the first n_trees games are assigned by tree_begin; set here, before the lanes
@@ -622,17 +686,21 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
         n_enqueued++;
         for (int i = 0; i < CHECK_EVERY; i++, r++) {
             for (int l = 0; l < n_lanes; l++) {
-                cudaEvent_t* ev = e->ev + 4 * ((slot * CHECK_EVERY + i) * N_LANES + l);
+                cudaEvent_t* ev = e->ev + EV_PER_ROUND * ((slot * CHECK_EVERY + i) * N_LANES + l);
                 lane_tp[l].parity = (int)(r & 1);
                 if (e->prof_level >= 2) cudaEventRecord(ev[0], ls[l]);
                 UTTT_CUDA_OK(tp ? launch_tree_tp_round(lane_tp[l], ls[l]) : launch_tree_round(lane_tp[l], ls[l]));
                 e->prof_launches[0] += 1;
-                if (run_evaluator(e, lane_bufs[l], evaluator, lane_tp[l].nn_count + lane_tp[l].parity,
-                                  lane_trees[l] * rows_per_tree,
-                                  ls[l], sampled ? ev + 1 : nullptr))
-                    return 1;
-                if (e->trace_on && !tp && trace_round(e, lane_tp[l], lane_bufs[l], lane_tp[l].nn_count + lane_tp[l].parity, ls[l]))
-                    return 1;
+                for (int net = 0; net < n_nets; net++) {
+                    const int32_t* count = (net ? lane_tp[l].nn1_count : lane_tp[l].nn_count) + lane_tp[l].parity;
+                    if (run_evaluator(e, net ? e->w1 : e->w, lane_bufs[l][net], evaluator, count, lane_trees[l] * rows_per_tree,
+                                      ls[l], sampled ? ev + 1 + 3 * net : nullptr))
+                        return 1;
+                }
+                for (int net = 0; net < n_nets && e->trace_on && !tp; net++)
+                    if (trace_round(e, lane_tp[l], lane_bufs[l][net],
+                                    (net ? lane_tp[l].nn1_count : lane_tp[l].nn_count) + lane_tp[l].parity, ls[l]))
+                        return 1;
             }
         }
         UTTT_CUDA_OK(cudaMemcpyAsync(e->h_counters + 8 * (1 + slot), t.counters, 8 * sizeof(unsigned long long),
@@ -645,12 +713,15 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
         for (int i = 0; i < CHECK_EVERY; i++) {
             for (int l = 0; l < n_lanes; l++) {
                 float ms = 0.f;
-                cudaEvent_t* ev = e->ev + 4 * ((slot * CHECK_EVERY + i) * N_LANES + l);
-                if (win_sampled[slot]) { cudaEventElapsedTime(&ms, ev[1], ev[2]); e->prof_ms[1] += ms; e->prof_sampled_launches += 1; }
+                cudaEvent_t* ev = e->ev + EV_PER_ROUND * ((slot * CHECK_EVERY + i) * N_LANES + l);
+                for (int net = 0; net < n_nets; net++) {       // pass `net`: [1 + 3 net] trunk [2 + 3 net] heads [3 + 3 net]
+                    cudaEvent_t* p = ev + 3 * net;
+                    if (win_sampled[slot]) { cudaEventElapsedTime(&ms, p[1], p[2]); e->prof_ms[1] += ms; e->prof_sampled_launches += 1; }
+                    if (e->prof_level >= 2) { cudaEventElapsedTime(&ms, p[2], p[3]); e->prof_ms[2] += ms; }
+                }
                 if (e->prof_level >= 2) {
                     cudaEventElapsedTime(&ms, ev[0], ev[1]); e->prof_ms[0] += ms;
-                    cudaEventElapsedTime(&ms, ev[2], ev[3]); e->prof_ms[2] += ms;
-                    cudaEventElapsedTime(&ms, ev[0], ev[3]); e->prof_ms[3] += ms;
+                    cudaEventElapsedTime(&ms, ev[0], ev[3 * n_nets]); e->prof_ms[3] += ms;
                 }
             }
         }

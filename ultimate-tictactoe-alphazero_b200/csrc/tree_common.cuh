@@ -83,20 +83,33 @@ __device__ __forceinline__ int leaf_symmetry(const TreeParams& P, const TreeCtl&
     return sym_draw(P.mode == MODE_SELFPLAY ? P.seed : 0u, c.game, (uint32_t)c.ply, (uint32_t)j);
 }
 
-// evaluator row `row` for leaf `st` (legal mask lm) under symmetry g: the row's position and planes are those of g(st)
-__device__ __forceinline__ void warp_write_row(const TreeParams& P, int row, const PackedState& st, const uint32_t lm[3], int g,
-                                               int lane) {
+// UTTT_SP_MATCH: the network that evaluates the leaves of the tree's current move -- weight slot (game + ply) & 1, so slot 0
+// moves first in even games and slot 1 in odd ones; 0 without the flag.  The ply does not change between queueing a leaf
+// and applying its row, so the apply step finds the row in the queue it was written to.
+__device__ __forceinline__ int leaf_net(const TreeParams& P, const TreeCtl& c) {
+    return (P.flags & UTTT_SP_MATCH) ? (int)(((uint32_t)c.game + (uint32_t)c.ply) & 1u) : 0;
+}
+// the evaluator rows of that network
+__device__ __forceinline__ const float* net_policy(const TreeParams& P, int net) { return net ? P.policy1 : P.policy; }
+__device__ __forceinline__ const float* net_value(const TreeParams& P, int net) { return net ? P.value1 : P.value; }
+
+// evaluator row `row` of network `net`'s queue for leaf `st` (legal mask lm) under symmetry g: the row's position and planes
+// are those of g(st)
+__device__ __forceinline__ void warp_write_row(const TreeParams& P, int net, int row, const PackedState& st, const uint32_t lm[3],
+                                               int g, int lane) {
+    PackedState* states = (net ? P.nn1_states : P.nn_states) + row;
+    __nv_bfloat16* planes = (net ? P.nn1_planes : P.nn_planes) + (size_t)row * 243;
     if (g == 0) {
-        warp_store_state(P.nn_states + row, st, lane);
-        warp_write_planes(P.nn_planes + (size_t)row * 243, st, lm, lane);
+        warp_store_state(states, st, lane);
+        warp_write_planes(planes, st, lm, lane);
         return;
     }
     PackedState gs;
     sym_state(st, g, gs);
     uint32_t glm[3];
     legal_mask(gs, glm);
-    warp_store_state(P.nn_states + row, gs, lane);
-    warp_write_planes(P.nn_planes + (size_t)row * 243, gs, glm, lane);
+    warp_store_state(states, gs, lane);
+    warp_write_planes(planes, gs, glm, lane);
 }
 
 // one coalesced read of a policy row for the leaf it was evaluated for under symmetry g: lane l gets the priors of actions
@@ -134,17 +147,19 @@ __device__ __forceinline__ void legal_priors(const float* pol, int g, const uint
 }
 
 // queues leaf `st` (legal mask lm) for the evaluator as evaluation c.n_eval of the tree's current move, standing for k
-// simulations; returns its row
+// simulations, in the queue of the network to move (leaf_net); returns its row there
 __device__ __forceinline__ int queue_leaf(const TreeParams& P, int t, TreeCtl& c, const PackedState& st, const uint32_t lm[3],
                                           int k, int lane) {
+    const int net = leaf_net(P, c);
     int row = 0;
     if (lane == 0) {
-        row = atomicAdd(P.nn_count + P.parity, 1);
+        row = atomicAdd((net ? P.nn1_count : P.nn_count) + P.parity, 1);
         atomicAdd(P.counters + 4, 1ull);
+        (net ? P.nn1_tree : P.nn_tree)[row] = t;
+        (net ? P.nn1_k : P.nn_k)[row] = k;
     }
     row = __shfl_sync(FULL, row, 0);
-    if (lane == 0) { P.nn_tree[row] = t; P.nn_k[row] = k; }
-    warp_write_row(P, row, st, lm, leaf_symmetry(P, c, c.n_eval), lane);
+    warp_write_row(P, net, row, st, lm, leaf_symmetry(P, c, c.n_eval), lane);
     c.n_eval += 1;
     return row;
 }

@@ -131,7 +131,7 @@ __device__ void apply_leaf_py(const TreeParams& P, const TreeView& T, TreeCtl& c
     }
     size_t row = (size_t)c.nn_row * (size_t)P.row_stride;
     float p0, p1, p2;
-    warp_load_priors(P.policy + row * 81, leaf_symmetry(P, c, c.n_eval - 1), lane, p0, p1, p2);
+    warp_load_priors(net_policy(P, leaf_net(P, c)) + row * 81, leaf_symmetry(P, c, c.n_eval - 1), lane, p0, p1, p2);
     // legal policies in legal order: rank i sits in lane i % 32, register i / 32
     float lp[3];
 #pragma unroll
@@ -150,7 +150,7 @@ __device__ void apply_leaf_py(const TreeParams& P, const TreeView& T, TreeCtl& c
     }
     if (lane == 0) T.node[leaf].w = (uint32_t)base | ((uint32_t)L << 20);
     c.n_nodes = base + L;
-    backup(T, path, plen, k, P.value + row, 0, 0.0f, lane);
+    backup(T, path, plen, k, net_value(P, leaf_net(P, c)) + row, 0, 0.0f, lane);
     c.sims_left -= k;
     c.pend_k = 0;
     if (lane == 0) atomicAdd(P.counters + 3, (unsigned long long)k);
@@ -173,7 +173,7 @@ __device__ void apply_leaf(const TreeParams& P, const TreeView& T, TreeCtl& c, c
     const int g = leaf_symmetry(P, c, c.n_eval - 1);
     for (int cp = 0; cp < k; cp++) {
         float pr[3];
-        legal_priors(P.policy + (row + (size_t)cp * P.copy_stride) * 81, g, lm, L, lane, pr);
+        legal_priors(net_policy(P, leaf_net(P, c)) + (row + (size_t)cp * P.copy_stride) * 81, g, lm, L, lane, pr);
         int reps = (P.copy_stride == 0) ? k : 1;       // identical rows: write all k copies at once
 #pragma unroll
         for (int q = 0; q < 3; q++) {
@@ -187,7 +187,7 @@ __device__ void apply_leaf(const TreeParams& P, const TreeView& T, TreeCtl& c, c
     }
     if (lane == 0) T.node[leaf].w = (uint32_t)base | ((uint32_t)(k * L) << 20);
     c.n_nodes = base + k * L;
-    backup(T, path, plen, k, P.value + row, P.copy_stride, 0.0f, lane);
+    backup(T, path, plen, k, net_value(P, leaf_net(P, c)) + row, P.copy_stride, 0.0f, lane);
     c.sims_left -= k;
     c.pend_k = 0;
     if (lane == 0) atomicAdd(P.counters + 3, (unsigned long long)k);
@@ -200,7 +200,7 @@ __device__ void apply_leaf(const TreeParams& P, const TreeView& T, TreeCtl& c, c
 __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) tree_begin_kernel(TreeParams P) {
     int t = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
     int lane = threadIdx.x & 31;
-    if (blockIdx.x == 0 && threadIdx.x == 0) { P.nn_count[0] = 0; P.nn_count[1] = 0; }
+    if (blockIdx.x == 0 && threadIdx.x == 0) { P.nn_count[0] = 0; P.nn_count[1] = 0; P.nn1_count[0] = 0; P.nn1_count[1] = 0; }
     if (t >= P.n_trees) return;
     TreeView T = view_of(P, t);
     TreeCtl c = P.ctl[t];
@@ -241,8 +241,8 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 7) tree_round_kernel(Tre
     pdl_wait();             // the previous round's evaluator has finished: policy / value rows are visible
     int t = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
     int lane = threadIdx.x & 31;
-    // the other parity's counter was consumed by the previous round's evaluator: reset it
-    if (blockIdx.x == 0 && threadIdx.x == 0) P.nn_count[P.parity ^ 1] = 0;
+    // the other parity's counters were consumed by the previous round's evaluator passes: reset them
+    if (blockIdx.x == 0 && threadIdx.x == 0) { P.nn_count[P.parity ^ 1] = 0; P.nn1_count[P.parity ^ 1] = 0; }
     if (t >= P.n_trees) return;
     // the control block, the pending leaf and the root position have nothing to wait for: one L2 round trip for the three
     const uint32_t leaf_raw = warp_load_state_issue(leaf_state(P, t, 0), lane);

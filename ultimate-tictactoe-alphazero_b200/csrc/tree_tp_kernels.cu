@@ -118,7 +118,7 @@ __device__ void tp_backup(const TreeView& T, const int32_t* path, int plen, floa
 __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 5) tree_tp_round_kernel(TreeParams P) {
     int t = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
     int lane = threadIdx.x & 31;
-    if (blockIdx.x == 0 && threadIdx.x == 0) P.nn_count[P.parity ^ 1] = 0;
+    if (blockIdx.x == 0 && threadIdx.x == 0) { P.nn_count[P.parity ^ 1] = 0; P.nn1_count[P.parity ^ 1] = 0; }
     if (t >= P.n_trees) return;
     TreeCtl c = P.ctl[t];
     if (c.phase == PHASE_DONE) return;
@@ -132,7 +132,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 5) tree_tp_round_kernel(
         if (lane == 0) T.node[0] = make_uint4(0x7Fu << 16, 0u, 0u, 0u);
         __syncwarp();
         c.n_nodes = 1;
-        tp_expand(P, T, c, root, 0, P.policy + (size_t)c.nn_row * 81, leaf_symmetry(P, c, 0), true, lane);
+        tp_expand(P, T, c, root, 0, net_policy(P, leaf_net(P, c)) + (size_t)c.nn_row * 81, leaf_symmetry(P, c, 0), true, lane);
         uint32_t lm[3];
         c.n_root = legal_mask(root, lm);
         c.sims_left = P.sims;
@@ -150,8 +150,9 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 5) tree_tp_round_kernel(
                 if (lane == 0) P.ctl[t] = c;
                 return;
             }
-            tp_expand(P, T, c, st, leaf, P.policy + (size_t)row * 81, leaf_symmetry(P, c, c.n_eval - c.pend_k + j), false, lane);
-            tp_backup(T, path, plen, P.value[row], true, lane);
+            tp_expand(P, T, c, st, leaf, net_policy(P, leaf_net(P, c)) + (size_t)row * 81, leaf_symmetry(P, c, c.n_eval - c.pend_k + j), false,
+                      lane);
+            tp_backup(T, path, plen, net_value(P, leaf_net(P, c))[row], true, lane);
         }
         c.sims_left -= c.pend_k;
         if (lane == 0) atomicAdd(P.counters + 3, (unsigned long long)c.pend_k);

@@ -30,6 +30,7 @@ SP_CORRECT_TERMINAL_SIGN = 1
 SP_THROUGHPUT = 2
 SP_PYSEARCH = 4
 SP_RANDOM_SYMMETRY = 8     # evaluate every leaf under a random board symmetry (include/uttt_b200.h)
+SP_MATCH = 16              # self-play as a match: weight slot (game + ply) & 1 moves (include/uttt_b200.h)
 
 _vp = C.c_void_p
 _u32p = np.ctypeslib.ndpointer(np.uint32, flags="C_CONTIGUOUS")
@@ -76,6 +77,8 @@ ABI = {
     "uttt_destroy": ([_vp], C.c_int),
     "uttt_upload_weights": ([_vp, C.POINTER(UtttWeights), C.c_int], C.c_int),
     "uttt_upload_weights_scattered": ([_vp, C.POINTER(UtttWeightsScattered), C.c_int], C.c_int),
+    "uttt_upload_weights_slot": ([_vp, C.c_int, C.POINTER(UtttWeights), C.c_int], C.c_int),
+    "uttt_upload_weights_scattered_slot": ([_vp, C.c_int, C.POINTER(UtttWeightsScattered), C.c_int], C.c_int),
     "uttt_net_forward": ([_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp], C.c_int),
     "uttt_mcts_search": ([_vp, _vp, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_int32, C.c_int32, _vp, _vp, _vp],
                          C.c_int),
@@ -303,6 +306,17 @@ def samples_to_numpy(samples):
     return st, cn, raw[:, 194].copy().view(np.int8), raw[:, 195].copy()
 
 
+def match_points(history, game0=0):
+    """points of the network in weight slot 0 in the games of an SP_MATCH run (include/uttt_b200.h): 0.5 for a draw
+    (final == 0), else 1 if the last mover -- slot (game + len - 1) & 1, game = game0 + i -- is slot 0 and 0 if not.
+    `history`: a History or any object with `lens` and `final` arrays -> float64 array of n_games points"""
+    lens = np.asarray(history.lens, np.int64)
+    final = np.asarray(history.final)
+    games = int(game0) + np.arange(len(lens), dtype=np.int64)
+    last_mover = (games + lens - 1) & 1
+    return np.where(final == 0, 0.5, np.where(last_mover == 0, 1.0, 0.0))
+
+
 class History:
     """Packed self-play history of n_games games (host numpy arrays; rows = game*81 + ply)."""
 
@@ -374,14 +388,17 @@ class Engine:
             pass
 
     # ---- weights
-    def upload_state_dict(self, sd):
-        """best.pth state_dict -> device (BN folded, tensor-core layouts).  Contiguous fp32 tensors (host, pinned or not, or
-        CUDA memory) are copied from where they lie; anything else goes through one packed host copy first."""
+    def upload_state_dict(self, sd, slot=0):
+        """best.pth state_dict -> device (BN folded, tensor-core layouts) into weight slot `slot`: 0 is what every evaluator
+        reads, 1 the second network of match().  Contiguous fp32 tensors (host, pinned or not, or CUDA memory) are copied
+        from where they lie; anything else goes through one packed host copy first."""
+        if slot not in (0, 1):
+            raise ValueError("weight slot must be 0 or 1, not %r" % (slot,))
         res = scattered_residual_tensors(sd)
         if res is None:
             packed = pack_state_dict(sd)
             w = UtttWeights(*[packed[k].ctypes.data for k in _WEIGHT_FIELDS])
-            _check(self.lib.uttt_upload_weights(self.h, C.byref(w), 0))
+            _check(self.lib.uttt_upload_weights_slot(self.h, slot, C.byref(w), 0))
             return
         small = pack_small(sd)
         w = UtttWeightsScattered()
@@ -393,10 +410,10 @@ class Engine:
             w.res_conv_w[l] = convs[l].data_ptr()
             for j in range(4):
                 w.res_bn[l][j] = bns[l][j].data_ptr()
-        _check(self.lib.uttt_upload_weights_scattered(self.h, C.byref(w), 0))      # synchronous: sd may go away after
+        _check(self.lib.uttt_upload_weights_scattered_slot(self.h, slot, C.byref(w), 0))   # synchronous: sd may go away after
 
-    def upload_model(self, model):
-        self.upload_state_dict(model.state_dict())
+    def upload_model(self, model, slot=0):
+        self.upload_state_dict(model.state_dict(), slot)
 
     # ---- network forward on packed states (cuda tensor (n,8) int32)
     def net_forward(self, states, mode=EVAL_NET_BF16, stream=None):
@@ -469,6 +486,15 @@ class Engine:
                                           _ptr(hist.states), _ptr(hist.counts), _ptr(hist.actions), _ptr(hist.lens),
                                           _ptr(hist.final), _ptr(hist.stats)))
         return hist
+
+    def match(self, n_games, sims=50, batch=8, seed=0, evaluator=EVAL_NET_BF16, flags=0, game0=0, history=None):
+        """A match between the networks of weight slots 0 and 1, all games on the device: selfplay() with SP_MATCH, so in
+        game game0 + i slot (game0 + i + ply) & 1 moves (slot 0 first in even games).  `flags` may add SP_PYSEARCH (the
+        reference gating match's search), SP_THROUGHPUT, SP_RANDOM_SYMMETRY, SP_CORRECT_TERMINAL_SIGN; the move draw is
+        self-play's (set_selfplay_temperature).  -> (points, history): points[i] = match_points of slot 0 in game game0 + i."""
+        hist = self.selfplay(n_games, sims=sims, batch=batch, seed=seed, evaluator=evaluator, flags=int(flags) | SP_MATCH,
+                             game0=game0, history=history)
+        return match_points(hist, game0)[:n_games], hist
 
     def selfplay_device(self, n_games, sims=50, batch=8, seed=0, evaluator=EVAL_NET_BF16, flags=0, game0=0,
                         stream=None):

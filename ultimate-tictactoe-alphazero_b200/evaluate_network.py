@@ -8,7 +8,11 @@ whose search differs from the C++ one used for self-play (evaluated root, replac
 float64 scores; pv_mcts.py:74-180).  EN_SEARCH = "python" (default) runs exactly that search on the engine
 (UTTT_SP_PYSEARCH; pinned bit-exactly against the unmodified pv_mcts.py by tests/golden/pymcts.npz); EN_SEARCH = "cpp"
 selects the C++ semantics (cpp/uttt_mcts.cpp:84-196) instead.
+
+EN_DEVICE_MATCH (environment UTTT_DEVICE_MATCH=1; off by default) plays the whole match inside one engine instead
+(device_match): both networks' games live on the device as in self-play, see evaluate_network().
 """
+import os
 from shutil import copy
 
 import numpy as np
@@ -26,6 +30,7 @@ EN_SEED = None            # None: derived from numpy's global RNG
 EN_SEARCH = "python"      # "python": pv_mcts.py semantics (what the reference's gating match runs); "cpp": uttt_mcts.cpp semantics
 EN_NUMERICS = _eng.DEFAULT_NUMERICS    # "bf16x3" | "bf16" | "fp32" (engine.evaluator_of)
 EN_RANDOM_SYMMETRY = False             # evaluate every leaf under a random board symmetry, policy mapped back (AlphaGo Zero)
+EN_DEVICE_MATCH = os.environ.get("UTTT_DEVICE_MATCH") == "1"    # play the match on the device (device_match)
 
 
 def first_player_point(ended_state):
@@ -144,6 +149,34 @@ def play_matches(actors, n_games, seed):
     return points
 
 
+def device_match(model0, model1, n_games, seed, temperature=None, numerics=None, search=None):
+    """The match of play_matches (model0 first in even games, model1 in odd ones) played by ONE engine, all games
+    device-resident like self-play (Engine.match, UTTT_SP_MATCH): model0 in weight slot 0, model1 in slot 1, every leaf
+    evaluated by the network whose side is to move, no host work between plies.  Same searches (EN_SEARCH, EN_NUMERICS,
+    EN_RANDOM_SYMMETRY) and the same temperature rule; the one difference: moves are drawn by the engine's Philox sampler
+    from the same distribution (the visit counts, or n^(1/T), the first maximum at T = 0) instead of by
+    RandomState(seed, i).choice, so both paths play the same kind of match but not identical games.
+    Returns the points of model0 per game (a list, as play_matches)."""
+    temperature = EN_TEMPERATURE if temperature is None else temperature
+    search = EN_SEARCH if search is None else search
+    if search not in ("python", "cpp"):
+        raise ValueError("EN_SEARCH must be 'python' or 'cpp', not %r" % (search,))
+    flags = (_eng.SP_PYSEARCH if search == "python" else 0) | (_eng.SP_RANDOM_SYMMETRY if EN_RANDOM_SYMMETRY else 0)
+    evaluator = _eng.evaluator_of(EN_NUMERICS if numerics is None else numerics)
+    e = _eng.Engine(n_slots=n_games, max_sims=PV_EVALUATE_COUNT, max_batch=MCTS_BATCH_SIZE, max_games=n_games)
+    try:
+        model0.eval()
+        model1.eval()
+        e.upload_model(model0, slot=0)
+        e.upload_model(model1, slot=1)
+        e.set_selfplay_temperature(temperature)
+        points, _ = e.match(n_games, sims=PV_EVALUATE_COUNT, batch=MCTS_BATCH_SIZE, seed=seed & 0xFFFFFFFF,
+                            evaluator=evaluator, flags=flags)
+    finally:
+        e.close()
+    return points.tolist()
+
+
 def update_best_player():
     """evaluate_network.py:57-59"""
     copy('./model/latest.pth', './model/best.pth')
@@ -151,18 +184,22 @@ def update_best_player():
 
 
 def evaluate_network():
-    """evaluate_network.py:62-104"""
+    """evaluate_network.py:62-104.  With EN_DEVICE_MATCH the games are played by device_match (one engine, latest.pth in
+    weight slot 0, best.pth in slot 1, same seed); the printed lines and the promotion rule do not change."""
     model0 = DualNetwork().to(device)
     model0.load_state_dict(torch.load('./model/latest.pth', map_location=device, weights_only=True))
     model1 = DualNetwork().to(device)
     model1.load_state_dict(torch.load('./model/best.pth', map_location=device, weights_only=True))
-    actors = (NetworkActor(model0, EN_TEMPERATURE, EN_GAME_COUNT), NetworkActor(model1, EN_TEMPERATURE, EN_GAME_COUNT))
     seed = int(np.random.randint(0, 2 ** 31 - 1)) if EN_SEED is None else int(EN_SEED)
-    try:
-        points = play_matches(actors, EN_GAME_COUNT, seed)
-    finally:
-        for a in actors:
-            a.close()
+    if EN_DEVICE_MATCH:
+        points = device_match(model0, model1, EN_GAME_COUNT, seed)
+    else:
+        actors = (NetworkActor(model0, EN_TEMPERATURE, EN_GAME_COUNT), NetworkActor(model1, EN_TEMPERATURE, EN_GAME_COUNT))
+        try:
+            points = play_matches(actors, EN_GAME_COUNT, seed)
+        finally:
+            for a in actors:
+                a.close()
     print('\rEvaluate {}/{}'.format(EN_GAME_COUNT, EN_GAME_COUNT), end='')
     print('')
     average_point = sum(points) / EN_GAME_COUNT
