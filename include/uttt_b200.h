@@ -75,6 +75,20 @@ extern "C" {
                                            else 1 if the last mover, slot (g + hist_len[g] - 1) & 1, is slot 0 and 0 if
                                            not.  Fails if a network evaluator is asked for and slot 1 was never uploaded
                                            (the hash evaluator reads no weights). */
+#define UTTT_SP_RESIGN 32               /* uttt_selfplay_run* only, alone or with UTTT_SP_MATCH: resignation (AlphaGo Zero).
+                                           Every decided move records v, its mover's root value: -w/n of the root child
+                                           with the most visits (the first maximum in legal order), 0 if that child is
+                                           unvisited -- with or without the flag (uttt_selfplay_fetch_values).  Game g
+                                           (absolute id) is a check game iff u < check_fraction, u = (philox4x32(
+                                           key=(seed, 4), ctr=(g_lo, g_hi, 0, 0)).x >> 8) * 2^-24; a check game is never
+                                           resigned.  In any other game the mover at ply p >= 1 resigns when v < threshold
+                                           (uttt_set_resign): v goes to hist_value row p, rows p of hist_states / _counts
+                                           / _actions are not written, hist_len = p, hist_final = 1 (the final position is
+                                           lost for its mover, the resigner), hist_resigned = 1, and the slot goes on to
+                                           the next game as after a natural end.  A resigned game is therefore the first
+                                           p plies of the same game played out, and its labels, packed samples and match
+                                           points give the resigner's opponent the win.  Needs terminal values of the
+                                           correct sign: UTTT_SP_THROUGHPUT or UTTT_SP_CORRECT_TERMINAL_SIGN. */
 
 typedef struct uttt_engine uttt_engine;
 
@@ -247,6 +261,14 @@ int uttt_selfplay_run_device(uttt_engine *e, int64_t n_games, uint64_t game0, in
                              int64_t *stats, void *stream);
 int uttt_selfplay_fetch(uttt_engine *e, int64_t n_games, uint32_t *hist_states, uint16_t *hist_counts,
                         uint8_t *hist_actions, int32_t *hist_len, int8_t *hist_final);
+
+/* UTTT_SP_RESIGN's threshold (a number in [-1, 1]; default -0.95) and the fraction of check games (in [0, 1]; default
+ * 0.1).  Fails on a NaN or out-of-range value. */
+int uttt_set_resign(uttt_engine *e, float threshold, float check_fraction);
+/* the root values of the last uttt_selfplay_run*, like uttt_selfplay_fetch: hist_value[g*81 + ply] = v of every decided
+ * move (rows 0..hist_len-1, and row hist_len of a resigned game; later rows are unspecified), hist_resigned[g] = 1 if
+ * game g resigned.  HOST pointers, either may be NULL.  Synchronous. */
+int uttt_selfplay_fetch_values(uttt_engine *e, int64_t n_games, float *hist_value /* n*81 */, int8_t *hist_resigned /* n */);
 
 /* The history of the last uttt_selfplay_run_device as ONE contiguous device buffer of fixed-size samples (one per played
  * ply, game-major order): bytes 0..31 packed position, 32..193 root visit counts u16[81], 194 z (int8, the label of

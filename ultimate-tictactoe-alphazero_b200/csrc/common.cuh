@@ -125,6 +125,10 @@ struct TreeParams {
     uint8_t* hist_actions;         // [n_games][81]
     int32_t* hist_len;             // [n_games]
     int8_t* hist_final;            // [n_games]
+    float* hist_value;             // [n_games][81]: the mover's root value of every decided move
+    int8_t* hist_resigned;         // [n_games]
+    float resign_threshold;        // UTTT_SP_RESIGN (uttt_set_resign)
+    float resign_check_fraction;
 };
 
 // kernels' host launchers (each returns cudaGetLastError of the launch)

@@ -319,7 +319,8 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
         ealloc(e, &t.nn_k, R) || ealloc(e, &t.nn_count, 4 * N_LANES) || ealloc(e, &t.out_counts, S * 81) ||
         ealloc(e, &t.out_n, S) || ealloc(e, &t.counters, 8) || ealloc(e, &t.hist_states, G * 81) ||
         ealloc(e, &t.hist_counts, G * 81 * 81) || ealloc(e, &t.hist_actions, G * 81) || ealloc(e, &t.hist_len, G) ||
-        ealloc(e, &t.hist_final, G) || ealloc(e, &e->policy, S * cfg->max_batch * 81) ||
+        ealloc(e, &t.hist_final, G) || ealloc(e, &t.hist_value, G * 81) || ealloc(e, &t.hist_resigned, G) ||
+        ealloc(e, &e->policy, S * cfg->max_batch * 81) ||
         ealloc(e, &e->value, S * cfg->max_batch) || ealloc(e, &e->scores, S * 81) ||
         ealloc(e, &e->headfeat, R * 243) || ealloc(e, &e->act_a, R * 81 * 128) || ealloc(e, &e->act_b, R * 81 * 128) ||
         ealloc(e, &e->tc_resid, (size_t)N_LANES * e->n_sm * 512 * 64) || ealloc(e, &e->fwd_count, 1) || ealloc(e, &e->tc_dbg, 128 + 64) ||
@@ -349,6 +350,8 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     t.dir_alpha = 0.3f;
     t.dir_eps = 0.25f;
     t.temperature = 1.0f;
+    t.resign_threshold = -0.95f;
+    t.resign_check_fraction = 0.1f;
     *out = e;
     return 0;
 }
@@ -525,6 +528,7 @@ int uttt_mcts_search(uttt_engine* e, const uint32_t* roots, int32_t n_roots, int
     UTTT_CHECK(!tp || batch <= TP_MAX_LEAVES, "throughput mode: at most %d leaves per tree per round", TP_MAX_LEAVES);
     UTTT_CHECK(!(tp && (flags & UTTT_SP_PYSEARCH)), "UTTT_SP_PYSEARCH and UTTT_SP_THROUGHPUT exclude each other");
     UTTT_CHECK(!(flags & UTTT_SP_MATCH), "UTTT_SP_MATCH is a self-play mode (uttt_selfplay_run*), not a search option");
+    UTTT_CHECK(!(flags & UTTT_SP_RESIGN), "UTTT_SP_RESIGN is a self-play mode (uttt_selfplay_run*), not a search option");
     if (mcts_begin_impl(e, roots, n_roots, sims, batch, flags)) return 1;     // uploads roots, runs the begin kernel
     if (n_roots == 0) return 0;
     TreeParams& t = e->tp;
@@ -618,6 +622,10 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
     const bool tp = (flags & UTTT_SP_THROUGHPUT) != 0;
     UTTT_CHECK(!(tp && (flags & UTTT_SP_PYSEARCH)), "UTTT_SP_PYSEARCH and UTTT_SP_THROUGHPUT exclude each other");
     UTTT_CHECK(!tp || batch <= TP_MAX_LEAVES, "throughput mode: at most %d leaves per tree per round", TP_MAX_LEAVES);
+    // under the reference's inverted terminal sign (tree_kernels.cu, round kernel) a move that wins at once backs up as
+    // a loss, so a root value says nothing a resignation could rest on
+    UTTT_CHECK(!(flags & UTTT_SP_RESIGN) || tp || (flags & UTTT_SP_CORRECT_TERMINAL_SIGN),
+               "UTTT_SP_RESIGN needs terminal values of the correct sign: add UTTT_SP_CORRECT_TERMINAL_SIGN or use UTTT_SP_THROUGHPUT");
     UTTT_CHECK(!match || evaluator == UTTT_EVAL_HASH || e->w1.loaded,
                "UTTT_SP_MATCH: weight slot 1 was never uploaded (uttt_upload_weights_slot(e, 1, ...))");
     const int rows_per_tree = tp ? batch : 1;
@@ -657,6 +665,7 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
     // fork, so that no lane's begin kernel races with another lane's first recycled slot)
     set_u64_kernel<<<1, 1, 0, s>>>(t.counters, (unsigned long long)n_trees);
     UTTT_CUDA_OK(cudaMemsetAsync(t.hist_len, 0, (size_t)n_games * sizeof(int32_t), s));
+    UTTT_CUDA_OK(cudaMemsetAsync(t.hist_resigned, 0, (size_t)n_games, s));
     UTTT_CUDA_OK(cudaEventRecord(e->ev_fork, s));
     cudaStream_t ls[N_LANES];
     for (int l = 0; l < n_lanes; l++) {
@@ -786,6 +795,28 @@ int uttt_selfplay_fetch(uttt_engine* e, int64_t n_games, uint32_t* hist_states, 
     if (hist_actions) UTTT_CUDA_OK(cudaMemcpyAsync(hist_actions, t.hist_actions, G * 81, cudaMemcpyDeviceToHost, s));
     if (hist_len) UTTT_CUDA_OK(cudaMemcpyAsync(hist_len, t.hist_len, G * 4, cudaMemcpyDeviceToHost, s));
     if (hist_final) UTTT_CUDA_OK(cudaMemcpyAsync(hist_final, t.hist_final, G, cudaMemcpyDeviceToHost, s));
+    UTTT_CUDA_OK(cudaStreamSynchronize(s));
+    return 0;
+}
+
+int uttt_set_resign(uttt_engine* e, float threshold, float check_fraction) {
+    UTTT_CHECK(threshold >= -1.0f && threshold <= 1.0f, "resign threshold %g: must be a number in [-1, 1]", (double)threshold);
+    UTTT_CHECK(check_fraction >= 0.0f && check_fraction <= 1.0f, "resign check fraction %g: must be in [0, 1]",
+               (double)check_fraction);
+    UTTT_CHECK(e != nullptr, "null engine");
+    e->tp.resign_threshold = threshold;
+    e->tp.resign_check_fraction = check_fraction;
+    return 0;
+}
+
+int uttt_selfplay_fetch_values(uttt_engine* e, int64_t n_games, float* hist_value, int8_t* hist_resigned) {
+    UTTT_CHECK(e && n_games <= e->cfg.max_games, "bad argument");
+    if (n_games <= 0) return 0;
+    UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
+    const size_t G = (size_t)n_games;
+    cudaStream_t s = e->stream;
+    if (hist_value) UTTT_CUDA_OK(cudaMemcpyAsync(hist_value, e->tp.hist_value, G * 81 * sizeof(float), cudaMemcpyDeviceToHost, s));
+    if (hist_resigned) UTTT_CUDA_OK(cudaMemcpyAsync(hist_resigned, e->tp.hist_resigned, G, cudaMemcpyDeviceToHost, s));
     UTTT_CUDA_OK(cudaStreamSynchronize(s));
     return 0;
 }

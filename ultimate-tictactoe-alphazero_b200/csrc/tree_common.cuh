@@ -244,6 +244,39 @@ __device__ __forceinline__ Descent descend(const TreeView& T, const PackedState&
     return d;
 }
 
+// the legal-order index of the root child with the most visits, the first maximum (the same on every lane)
+__device__ __forceinline__ int most_visited(const TreeView& T, int L, int lane) {
+    int best = -1, besti = 0x7FFFFFFF;
+    for (int i = lane; i < L; i += 32) {
+        int n = node_n(T.node[1 + i]);
+        if (n > best) { best = n; besti = i; }
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        int ob = __shfl_xor_sync(FULL, best, off), oi = __shfl_xor_sync(FULL, besti, off);
+        if (ob > best || (ob == best && oi < besti)) { best = ob; besti = oi; }
+    }
+    return besti;
+}
+
+// The mover's value of the searched position: Q = -w / n of the most visited root child (the child sample_move plays
+// at T = 0), exactly as descend computes it without virtual loss, and 0 for an unvisited child (descend's Q).  No
+// virtual loss is outstanding when a move is decided: the reference-exact mode sets none, and the throughput round
+// decides only in PHASE_SEARCH, which it enters after the tp_backup of every leaf it queued has removed that leaf's unit
+// (terminal descents add none).
+__device__ __forceinline__ float root_value(const TreeView& T, const TreeCtl& c, int lane) {
+    const uint4 q = T.node[1 + most_visited(T, c.n_root, lane)];
+    const int n = node_n(q);
+    return n > 0 ? __fdiv_rn(-__uint_as_float(q.y), (float)n) : 0.0f;
+}
+
+// UTTT_SP_RESIGN: game g is a check game, never resigned, iff u < check fraction, u = (philox(key=(seed, 4),
+// ctr=(g_lo, g_hi, 0, 0)).x >> 8) * 2^-24
+__device__ __forceinline__ bool check_game(const TreeParams& P, uint64_t game) {
+    const Philox4 r = philox4x32(P.seed, 4u, (uint32_t)game, (uint32_t)(game >> 32), 0u, 0u);
+    return (float)(r.x >> 8) * (1.0f / 16777216.0f) < P.resign_check_fraction;
+}
+
 // Philox temperature-1 sampling over the root visit counts; returns the chosen action.
 // SP_TEMPERATURE != 1 (self_play_cpp.py:27,62 -> cpp/uttt_mcts.cpp:183-216): T == 0 plays the first maximum of the visit
 // counts (the reference's one-hot scores leave np.random.choice no choice); otherwise the move is drawn from
@@ -251,19 +284,7 @@ __device__ __forceinline__ Descent descend(const TreeView& T, const PackedState&
 __device__ __forceinline__ int sample_move_temperature(const TreeParams& P, const TreeView& T, const TreeCtl& c, const uint32_t lm[3],
                                                        int lane) {
     const int L = c.n_root;
-    if (P.temperature == 0.0f) {
-        int best = -1, besti = 0x7FFFFFFF;
-        for (int i = lane; i < L; i += 32) {
-            int n = node_n(T.node[1 + i]);
-            if (n > best) { best = n; besti = i; }
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            int ob = __shfl_xor_sync(FULL, best, off), oi = __shfl_xor_sync(FULL, besti, off);
-            if (ob > best || (ob == best && oi < besti)) { best = ob; besti = oi; }
-        }
-        return nth_legal(lm, besti);
-    }
+    if (P.temperature == 0.0f) return nth_legal(lm, most_visited(T, L, lane));
     const float inv = __fdiv_rn(1.0f, P.temperature);
     Philox4 r = philox4x32(P.seed, 1u, (uint32_t)c.game, (uint32_t)(c.game >> 32), (uint32_t)c.ply, 0u);
     const float u = (float)(r.x >> 8) * (1.0f / 16777216.0f);          // [0, 1)
@@ -325,9 +346,12 @@ __device__ __forceinline__ int sample_move(const TreeParams& P, const TreeView& 
 }
 
 // the move is decided (the simulation budget is spent).  Search: the root visit counts are the tree's output
-// (cpp/uttt_mcts.cpp:177-180) and the tree is done.  Self-play: record the history row, sample the move, play it; when
-// the game is over (lost or drawn, self_play_cpp.py:50-51,95) record it and claim the next game from counters[0].
-// Returns whether the tree goes on; if so `root` is the position of its next search, already stored in P.root[t].
+// (cpp/uttt_mcts.cpp:177-180) and the tree is done.  Self-play: record the root value and the history row, sample the
+// move, play it; when the game is over (lost or drawn, self_play_cpp.py:50-51,95) record it and claim the next game from
+// counters[0].  With UTTT_SP_RESIGN, a mover at ply p >= 1 of a game that is not a check game resigns instead when its
+// root value is below the threshold: only the value of ply p is recorded, and the game ends with p plies as one whose
+// final position is lost for its mover.  Returns whether the tree goes on; if so `root` is the position of its next
+// search, already stored in P.root[t].
 __device__ __forceinline__ bool decide_move(const TreeParams& P, const TreeView& T, int t, TreeCtl& c, PackedState& root, int lane) {
     if (P.mode == MODE_SEARCH) {
         for (int i = lane; i < 81; i += 32) P.out_counts[(size_t)t * 81 + i] = (i < c.n_root) ? node_n(T.node[1 + i]) : 0;
@@ -338,19 +362,27 @@ __device__ __forceinline__ bool decide_move(const TreeParams& P, const TreeView&
     uint32_t lm[3];
     legal_mask(root, lm);
     const size_t hrow = (size_t)c.game_idx * 81 + (size_t)c.ply;
-    warp_store_state(P.hist_states + hrow, root, lane);
-    for (int a = lane; a < 81; a += 32)
-        P.hist_counts[hrow * 81 + a] = legal_bit(lm, a) ? (uint16_t)node_n(T.node[1 + legal_rank(lm, a)]) : (uint16_t)0;
-    const int action = sample_move(P, T, c, lm, lane);
-    if (lane == 0) P.hist_actions[hrow] = (uint8_t)action;
-    PackedState nx;
-    next_state(root, action, nx);
-    root = nx;
-    c.ply += 1;
-    if (legal_mask(root, lm) == 0) {
+    const float v = root_value(T, c, lane);
+    if (lane == 0) P.hist_value[hrow] = v;
+    const bool resign = (P.flags & UTTT_SP_RESIGN) && c.ply >= 1 && v < P.resign_threshold && !check_game(P, c.game);
+    bool over = resign;
+    if (!resign) {
+        warp_store_state(P.hist_states + hrow, root, lane);
+        for (int a = lane; a < 81; a += 32)
+            P.hist_counts[hrow * 81 + a] = legal_bit(lm, a) ? (uint16_t)node_n(T.node[1 + legal_rank(lm, a)]) : (uint16_t)0;
+        const int action = sample_move(P, T, c, lm, lane);
+        if (lane == 0) P.hist_actions[hrow] = (uint8_t)action;
+        PackedState nx;
+        next_state(root, action, nx);
+        root = nx;
+        c.ply += 1;
+        over = legal_mask(root, lm) == 0;
+    }
+    if (over) {
         if (lane == 0) {
             P.hist_len[c.game_idx] = c.ply;
-            P.hist_final[c.game_idx] = is_lose(root) ? 1 : 0;
+            P.hist_final[c.game_idx] = (resign || is_lose(root)) ? 1 : 0;
+            if (resign) P.hist_resigned[c.game_idx] = 1;
             atomicAdd(P.counters + 1, 1ull);
             atomicAdd(P.counters + 2, (unsigned long long)c.ply);
         }

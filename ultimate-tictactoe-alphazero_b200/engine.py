@@ -31,11 +31,13 @@ SP_THROUGHPUT = 2
 SP_PYSEARCH = 4
 SP_RANDOM_SYMMETRY = 8     # evaluate every leaf under a random board symmetry (include/uttt_b200.h)
 SP_MATCH = 16              # self-play as a match: weight slot (game + ply) & 1 moves (include/uttt_b200.h)
+SP_RESIGN = 32             # a mover whose root value falls below the threshold resigns (include/uttt_b200.h)
 
 _vp = C.c_void_p
 _u32p = np.ctypeslib.ndpointer(np.uint32, flags="C_CONTIGUOUS")
 _i32p = np.ctypeslib.ndpointer(np.int32, flags="C_CONTIGUOUS")
 _f32p = np.ctypeslib.ndpointer(np.float32, flags="C_CONTIGUOUS")
+_F32 = np.float32
 
 
 class UtttConfig(C.Structure):
@@ -97,6 +99,8 @@ ABI = {
     "uttt_selfplay_run_device": ([_vp, C.c_int64, C.c_uint64, C.c_int32, C.c_int32, C.c_uint32, C.c_int32,
                                   C.c_int32, _vp, _vp], C.c_int),
     "uttt_selfplay_fetch": ([_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp], C.c_int),
+    "uttt_set_resign": ([_vp, C.c_float, C.c_float], C.c_int),
+    "uttt_selfplay_fetch_values": ([_vp, C.c_int64, _vp, _vp], C.c_int),
     "uttt_selfplay_pack": ([_vp, C.c_int64, _vp, C.c_int64, C.POINTER(C.c_int64), _vp], C.c_int),
     "uttt_samples_unpack": ([_vp, C.c_int64, _vp, _vp, _vp, _vp], C.c_int),
     "uttt_debug_trunk_timeline": ([_vp, _vp], C.c_int),
@@ -317,6 +321,112 @@ def match_points(history, game0=0):
     return np.where(final == 0, 0.5, np.where(last_mover == 0, 1.0, 0.0))
 
 
+# ------------------------------------------------------------------------------------ resignation (host side)
+def _philox4x32_x(k0, k1, c0, c1, c2, c3):
+    """word x of Philox4x32-10 (the engine's counter-based generator, csrc/uttt_rules.cuh), vectorised over numpy
+    uint64 arrays holding 32-bit values"""
+    M = np.uint64(0xFFFFFFFF)
+    k0, k1, c0, c1, c2, c3 = (np.asarray(a, np.uint64) & M for a in (k0, k1, c0, c1, c2, c3))
+    for _ in range(10):
+        p0 = np.uint64(0xD2511F53) * c0
+        p1 = np.uint64(0xCD9E8D57) * c2
+        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ k0, p1 & M, (p0 >> np.uint64(32)) ^ c3 ^ k1, p0 & M
+        k0 = (k0 + np.uint64(0x9E3779B9)) & M
+        k1 = (k1 + np.uint64(0xBB67AE85)) & M
+    return c0
+
+
+def check_games(seed, game0, n, check_fraction):
+    """SP_RESIGN's check games among games game0 .. game0 + n - 1 -> bool array (n,): game g is a check game (never
+    resigned) iff (philox4x32(key=(seed, 4), ctr=(g_lo, g_hi, 0, 0)).x >> 8) * 2^-24 < check_fraction (compared in fp32)"""
+    g = np.uint64(int(game0)) + np.arange(int(n), dtype=np.uint64)
+    x = _philox4x32_x(int(seed), 4, g & np.uint64(0xFFFFFFFF), g >> np.uint64(32), 0, 0)
+    u = (x >> np.uint64(8)).astype(_F32) * _F32(1.0 / 16777216.0)
+    return u < _F32(check_fraction)
+
+
+def _recorded_values(history):
+    """(values (n,81) f32, mask of the recorded rows): rows 0..len-1, plus row len of a resigned game"""
+    lens = np.asarray(history.lens, np.int64)
+    resigned = np.asarray(history.resigned) != 0
+    last = lens + resigned - 1
+    return np.asarray(history.values, _F32), np.arange(81)[None, :] <= last[:, None]
+
+
+def would_resign_ply(history, threshold):
+    """per game, the first ply p >= 1 whose recorded root value is below `threshold` (strictly, in fp32), over the rows
+    `history` recorded (0..len-1, and row len of a game that resigned); -1 where there is none -> int64 array (n,).
+    For a game played out with resignation off, p is where SP_RESIGN with that threshold would have ended it."""
+    values, rec = _recorded_values(history)
+    hit = rec & (values < _F32(threshold))
+    hit[:, 0] = False
+    return np.where(hit.any(axis=1), hit.argmax(axis=1), -1).astype(np.int64)
+
+
+def _games(history, games):
+    n = len(history.lens)
+    idx = np.arange(n) if games is None else np.asarray(games)
+    return np.nonzero(idx)[0] if idx.dtype == bool else idx.astype(np.int64)
+
+
+def resign_calibration(history, threshold, games=None):
+    """over the played-out games `games` (indices or a bool mask; None: all) of `history`: how many would resign with
+    `threshold` (would_resign_ply >= 1) and how many of those are false positives -- the would-be resigner, the mover
+    at that ply, did not lose the game (it won or drew) -> dict(games, would_resign, false_positives)"""
+    g = _games(history, games)
+    p = would_resign_ply(history, threshold)[g]
+    w = p >= 1
+    # the mover at ply p lost iff the final position is lost for its mover and (len - p) is even
+    lost = (np.asarray(history.final)[g] == 1) & ((np.asarray(history.lens, np.int64)[g] - p) % 2 == 0)
+    return {"games": int(len(g)), "would_resign": int(w.sum()), "false_positives": int((w & ~lost).sum())}
+
+
+class _Rows:
+    """the lens / final / values / resigned rows `g` of a history"""
+
+    def __init__(self, history, g):
+        self.lens = np.asarray(history.lens)[g]
+        self.final = np.asarray(history.final)[g]
+        self.values = np.asarray(history.values)[g]
+        self.resigned = np.asarray(history.resigned)[g]
+
+
+def resign_threshold(history, target_fp, games=None):
+    """AlphaGo Zero's calibration: the largest threshold whose false-positive rate over the played-out games `games`
+    (false positives / would-resign games, see resign_calibration) is at most `target_fp`.  Candidates are the distinct
+    recorded root values of those games; a candidate that resigns no game does not qualify.  -> float, or -1.0 (never
+    resigns: values are >= -1 and the rule is strict) if no candidate qualifies.  Calibrate on the check games of a run
+    with resignation on and on all games of a run without it: resigned games have no known outcome."""
+    h = _Rows(history, _games(history, games))
+    values, rec = _recorded_values(h)
+    cand = np.unique(values[rec])
+    if len(cand) == 0:
+        return -1.0
+    # for a game, "resign if v < c" fires at the first ply p >= 1 whose value is below c: as c rises past each new low of
+    # the running minimum over plies 1.., that ply moves to the ply of the low.  Candidate i (sorted) fires at the last
+    # low l_k < cand[i], i.e. at the low's ply for every candidate above it up to and including the previous low.
+    wr = np.zeros(len(cand) + 1, np.int64)
+    fp = np.zeros(len(cand) + 1, np.int64)
+    lens = np.asarray(h.lens, np.int64)
+    for gi in range(len(lens)):
+        prev = np.inf
+        for p in np.nonzero(rec[gi])[0]:
+            v = values[gi, p]
+            if p == 0 or not v < prev:
+                continue
+            lo = np.searchsorted(cand, v, side="right")          # candidates c > v ...
+            hi = np.searchsorted(cand, prev, side="right")       # ... and c <= the previous low
+            lost = bool(h.final[gi] == 1 and (lens[gi] - p) % 2 == 0)
+            wr[lo] += 1; wr[hi] -= 1
+            if not lost:
+                fp[lo] += 1; fp[hi] -= 1
+            prev = v
+    wr = np.cumsum(wr)[:-1]
+    fp = np.cumsum(fp)[:-1]
+    ok = (wr > 0) & (fp <= np.float64(target_fp) * wr)
+    return float(cand[np.nonzero(ok)[0][-1]]) if ok.any() else -1.0
+
+
 class History:
     """Packed self-play history of n_games games (host numpy arrays; rows = game*81 + ply)."""
 
@@ -338,11 +448,14 @@ class History:
         self.actions = alloc((n_games, 81), torch.uint8)
         self.lens = alloc((n_games,), torch.int32)
         self.final = alloc((n_games,), torch.int8)
+        self.values = alloc((n_games, 81), torch.float32)     # the mover's root value of every decided move
+        self.resigned = alloc((n_games,), torch.int8)         # 1: the game ended by resignation (SP_RESIGN)
         self.stats = np.zeros(4, np.int64)
 
     @property
     def nbytes(self):
-        return self.states.nbytes + self.counts.nbytes + self.actions.nbytes + self.lens.nbytes + self.final.nbytes
+        return (self.states.nbytes + self.counts.nbytes + self.actions.nbytes + self.lens.nbytes + self.final.nbytes
+                + self.values.nbytes + self.resigned.nbytes)
 
     def samples(self):
         """-> (states (N,8) uint32, counts (N,81) uint16, z (N,) int8) over all plies, game-major order.
@@ -438,6 +551,11 @@ class Engine:
         """SP_TEMPERATURE of the self-play loop (1: the reference's setting; 0: always the most visited move)"""
         _check(self.lib.uttt_set_selfplay_temperature(self.h, float(temperature)))
 
+    def set_resign(self, threshold=-0.95, check_fraction=0.1):
+        """SP_RESIGN's threshold (a mover at ply >= 1 resigns when its root value is below it; in [-1, 1]) and the fraction
+        of check games that are never resigned (in [0, 1]); see include/uttt_b200.h"""
+        _check(self.lib.uttt_set_resign(self.h, float(threshold), float(check_fraction)))
+
     def mcts_search(self, roots, sims, batch, temperature, evaluator, flags=0):
         roots = np.ascontiguousarray(roots, dtype=np.uint32).reshape(-1, 8)
         n = roots.shape[0]
@@ -485,6 +603,7 @@ class Engine:
         _check(self.lib.uttt_selfplay_run(self.h, n_games, game0, sims, batch, seed, evaluator, flags,
                                           _ptr(hist.states), _ptr(hist.counts), _ptr(hist.actions), _ptr(hist.lens),
                                           _ptr(hist.final), _ptr(hist.stats)))
+        _check(self.lib.uttt_selfplay_fetch_values(self.h, n_games, _ptr(hist.values), _ptr(hist.resigned)))
         return hist
 
     def match(self, n_games, sims=50, batch=8, seed=0, evaluator=EVAL_NET_BF16, flags=0, game0=0, history=None):
@@ -509,6 +628,7 @@ class Engine:
         hist = history if history is not None else History(n_games)
         _check(self.lib.uttt_selfplay_fetch(self.h, n_games, _ptr(hist.states), _ptr(hist.counts), _ptr(hist.actions),
                                             _ptr(hist.lens), _ptr(hist.final)))
+        _check(self.lib.uttt_selfplay_fetch_values(self.h, n_games, _ptr(hist.values), _ptr(hist.resigned)))
         return hist
 
     def selfplay_pack(self, n_games, out=None, stream=None):

@@ -43,6 +43,12 @@ SP_DIRICHLET_ALPHA = 0.3      # throughput mode only
 SP_DIRICHLET_EPS = 0.25
 SP_RANDOM_SYMMETRY = False    # evaluate every leaf under a random board symmetry, policy mapped back (AlphaGo Zero)
 SP_WRITE_PACKED = False       # also write ./data/<timestamp>.packed.npz (357 B/sample instead of ~1.7 KB; SURVEY 8f-3)
+SP_RESIGN_THRESHOLD = None    # a float: a mover resigns when its root value is below it (AlphaGo Zero; engine.SP_RESIGN).
+                              # Needs CORRECTED_TERMINAL_SIGN = True or SP_SEARCH_MODE = "throughput"
+SP_RESIGN_CHECK_FRACTION = 0.1    # fraction of games never resigned, to measure the false positives
+SP_RESIGN_TARGET_FP = None    # a float: after each cycle SP_RESIGN_THRESHOLD becomes the largest threshold whose false-positive
+                              # rate on that cycle's played-out games (the check games; all games while resignation is off)
+                              # is at most this (engine.resign_threshold)
 
 _engine = None
 last_stats = {}
@@ -117,7 +123,35 @@ def _to_reference_format(xs, pis, zs):
     return [[xs[i], pis[i], int(zs[i])] for i in range(len(zs))]
 
 
+def _resign_flags():
+    """engine.SP_RESIGN if SP_RESIGN_THRESHOLD is set, else 0; ValueError if resignation is asked for (a threshold or a
+    calibration target) under the reference's terminal sign, where a move that wins at once backs up as a loss"""
+    if SP_RESIGN_THRESHOLD is None and SP_RESIGN_TARGET_FP is None:
+        return 0
+    if not (CORRECTED_TERMINAL_SIGN or SP_SEARCH_MODE == "throughput"):
+        raise ValueError("resignation needs root values with the correct terminal sign: set CORRECTED_TERMINAL_SIGN = True "
+                         "or SP_SEARCH_MODE = \"throughput\"")
+    return _eng.SP_RESIGN if SP_RESIGN_THRESHOLD is not None else 0
+
+
+def _resign_stats(hist, n_games, seed, resign):
+    """resigned games and the false positives of the played-out calibration games (the check games while resigning, all
+    games otherwise); with SP_RESIGN_TARGET_FP, the threshold calibrated on them becomes SP_RESIGN_THRESHOLD"""
+    global SP_RESIGN_THRESHOLD
+    calib = (_eng.check_games(seed, 0, n_games, SP_RESIGN_CHECK_FRACTION) if resign
+             else np.ones(n_games, bool))
+    out = {"resigned": int((hist.resigned[:n_games] != 0).sum()), "check_games": int(calib.sum()) if resign else 0}
+    if resign:
+        cal = _eng.resign_calibration(hist, SP_RESIGN_THRESHOLD, calib)
+        out.update(check_would_resign=cal["would_resign"], check_false_positives=cal["false_positives"])
+    if SP_RESIGN_TARGET_FP is not None:
+        SP_RESIGN_THRESHOLD = _eng.resign_threshold(hist, SP_RESIGN_TARGET_FP, calib)
+        out["calibrated_threshold"] = SP_RESIGN_THRESHOLD
+    return out
+
+
 def _run(model, n_games, progress=False):
+    resign = _resign_flags()
     eng = _get_engine(n_games)
     model.eval()
     eng.upload_model(model)
@@ -129,6 +163,9 @@ def _run(model, n_games, progress=False):
         eng.set_root_noise(SP_DIRICHLET_ALPHA, SP_DIRICHLET_EPS)
     if SP_RANDOM_SYMMETRY:
         flags |= _eng.SP_RANDOM_SYMMETRY
+    if resign:
+        flags |= resign
+        eng.set_resign(SP_RESIGN_THRESHOLD, SP_RESIGN_CHECK_FRACTION)
     eng.set_selfplay_temperature(SP_TEMPERATURE)
     if SP_PROGRESS and progress:
         shown = [0]
@@ -145,6 +182,9 @@ def _run(model, n_games, progress=False):
         eng.set_selfplay_temperature(1.0)
     last_stats.update(plies=int(hist.stats[0]), sims=int(hist.stats[1]), evals=int(hist.stats[2]),
                       rounds=int(hist.stats[3]), seed=seed)
+    for k in ("check_would_resign", "check_false_positives", "calibrated_threshold"):     # only what this cycle reports
+        last_stats.pop(k, None)
+    last_stats.update(_resign_stats(hist, n_games, seed, bool(resign)))
     return eng, hist
 
 
