@@ -89,6 +89,21 @@ extern "C" {
                                            p plies of the same game played out, and its labels, packed samples and match
                                            points give the resigner's opponent the win.  Needs terminal values of the
                                            correct sign: UTTT_SP_THROUGHPUT or UTTT_SP_CORRECT_TERMINAL_SIGN. */
+#define UTTT_SP_PLAYOUT_CAP 64          /* uttt_selfplay_run* only, any search mode, alone or with UTTT_SP_RANDOM_SYMMETRY,
+                                           UTTT_SP_RESIGN or UTTT_SP_CORRECT_TERMINAL_SIGN: playout cap randomization
+                                           (KataGo, Wu 2019, section 3.1).  The move at ply p of game g (absolute id) is a
+                                           full search iff u < full_fraction, u = (philox4x32(key=(seed, 5), ctr=(g_lo,
+                                           g_hi, p, 0)).x >> 8) * 2^-24 compared in fp32; a full search spends
+                                           evaluate_count simulations, a fast search fast_sims (uttt_set_playout_cap).  In
+                                           the throughput mode a fast search mixes no Dirichlet noise into its root
+                                           priors; a full search keeps it.  Everything else about a move is the same for
+                                           both kinds: temperature and Philox move draw, symmetry draws, root value and the
+                                           resignation rule, and rows of hist_states / _counts / _actions.  hist_full[g*81
+                                           + p] (uttt_selfplay_fetch_full) is 1 for a full search and 0 for a fast one,
+                                           written for every decided move that is not a resignation, and 1 for every move
+                                           without the flag.  Only full-search plies become packed samples
+                                           (uttt_selfplay_pack).  Fails with fast_sims > evaluate_count and with
+                                           UTTT_SP_MATCH (a match records no training targets). */
 
 typedef struct uttt_engine uttt_engine;
 
@@ -270,8 +285,16 @@ int uttt_set_resign(uttt_engine *e, float threshold, float check_fraction);
  * game g resigned.  HOST pointers, either may be NULL.  Synchronous. */
 int uttt_selfplay_fetch_values(uttt_engine *e, int64_t n_games, float *hist_value /* n*81 */, int8_t *hist_resigned /* n */);
 
+/* UTTT_SP_PLAYOUT_CAP's fast-search budget (1 <= fast_sims <= the engine's max_sims; default 8) and the probability of a
+ * full search (in [0, 1]; default 0.25): KataGo's ratio at the reference's 50 simulations, and its p.  Fails on a NaN or
+ * out-of-range value. */
+int uttt_set_playout_cap(uttt_engine *e, int32_t fast_sims, float full_fraction);
+/* the search kinds of the last uttt_selfplay_run*, like uttt_selfplay_fetch: hist_full[g*81 + ply] = 1 for a full search,
+ * 0 for a fast one (rows 0..hist_len-1; later rows are unspecified).  HOST pointer.  Synchronous. */
+int uttt_selfplay_fetch_full(uttt_engine *e, int64_t n_games, uint8_t *hist_full /* n*81 */);
+
 /* The history of the last uttt_selfplay_run_device as ONE contiguous device buffer of fixed-size samples (one per played
- * ply, game-major order): bytes 0..31 packed position, 32..193 root visit counts u16[81], 194 z (int8, the label of
+ * ply with hist_full = 1, i.e. every played ply without UTTT_SP_PLAYOUT_CAP; game-major, ply order): bytes 0..31 packed position, 32..193 root visit counts u16[81], 194 z (int8, the label of
  * self_play_cpp.py:95-99), 195 ply.  This is what a rank sends to the trainer rank in the multi-GPU cycle (one
  * exact-length transfer instead of the ~1.7 KB/sample pickle of self_play_cpp.py:125-130).
  * uttt_selfplay_pack: out_dev must hold cap_samples samples; *n_samples_out (HOST) = samples written; synchronises `stream`.

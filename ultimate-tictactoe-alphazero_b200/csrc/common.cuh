@@ -129,6 +129,9 @@ struct TreeParams {
     int8_t* hist_resigned;         // [n_games]
     float resign_threshold;        // UTTT_SP_RESIGN (uttt_set_resign)
     float resign_check_fraction;
+    uint8_t* hist_full;            // [n_games][81]: 1 if the move was a full search, 0 if a fast one
+    int32_t fast_sims;             // UTTT_SP_PLAYOUT_CAP (uttt_set_playout_cap)
+    float full_fraction;
 };
 
 // kernels' host launchers (each returns cudaGetLastError of the launch)
@@ -143,9 +146,10 @@ cudaError_t launch_dirichlet(uint32_t seed, uint64_t game0, int64_t n, int n_chi
 cudaError_t launch_boltzman(const float* xs, int n, float temperature, float* out, cudaStream_t s);
 
 // history as fixed-size samples (history_kernels.cu)
-cudaError_t launch_scan_lens(const int32_t* lens, int64_t n, int64_t* offsets, cudaStream_t s);
-cudaError_t launch_pack_samples(const PackedState* states, const uint16_t* counts, const int32_t* lens, const int8_t* final_lose,
-                                const int64_t* offsets, int64_t n_games, void* out, int64_t cap_samples, cudaStream_t s);
+cudaError_t launch_scan_samples(const int32_t* lens, const uint8_t* full, int64_t n, int64_t* offsets, cudaStream_t s);
+cudaError_t launch_pack_samples(const PackedState* states, const uint16_t* counts, const int32_t* lens, const uint8_t* full,
+                                const int8_t* final_lose, const int64_t* offsets, int64_t n_games, void* out, int64_t cap_samples,
+                                cudaStream_t s);
 cudaError_t launch_unpack_samples(const void* samples, int64_t n, float* x, float* policy, float* value, cudaStream_t s);
 
 // ---------------------------------------------------------------- network

@@ -59,7 +59,7 @@ struct uttt_engine {
     float* headfeat;        // [rows][243] head 1x1-conv outputs written by the tensor-core trunk
     float* tc_resid;        // [n_sm][32][512][4] fp32 residual stream of the tensor-core trunk (per CTA)
     int32_t* fwd_count;     // device int for uttt_net_forward
-    int64_t* hist_offsets;  // [max_games + 1] exclusive prefix sums of the game lengths (uttt_selfplay_pack)
+    int64_t* hist_offsets;  // [max_games + 1] exclusive prefix sums of the games' sample counts (uttt_selfplay_pack)
     long long* tc_dbg;      // [32][4] clock64 timeline of trunk CTA 0, then [64] histogram of batch sizes (diagnostics)
     int prof_level;         // self-play kernel timing: 2 = tree / trunk / heads events every round, 1 = trunk only, 0 = none
     int prof_sample;        // level 1: the trunk is bracketed in every prof_sample-th window of rounds only (see uttt_set_profile_level)
@@ -320,6 +320,7 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
         ealloc(e, &t.out_n, S) || ealloc(e, &t.counters, 8) || ealloc(e, &t.hist_states, G * 81) ||
         ealloc(e, &t.hist_counts, G * 81 * 81) || ealloc(e, &t.hist_actions, G * 81) || ealloc(e, &t.hist_len, G) ||
         ealloc(e, &t.hist_final, G) || ealloc(e, &t.hist_value, G * 81) || ealloc(e, &t.hist_resigned, G) ||
+        ealloc(e, &t.hist_full, G * 81) ||
         ealloc(e, &e->policy, S * cfg->max_batch * 81) ||
         ealloc(e, &e->value, S * cfg->max_batch) || ealloc(e, &e->scores, S * 81) ||
         ealloc(e, &e->headfeat, R * 243) || ealloc(e, &e->act_a, R * 81 * 128) || ealloc(e, &e->act_b, R * 81 * 128) ||
@@ -352,6 +353,8 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     t.temperature = 1.0f;
     t.resign_threshold = -0.95f;
     t.resign_check_fraction = 0.1f;
+    t.fast_sims = 8;
+    t.full_fraction = 0.25f;
     *out = e;
     return 0;
 }
@@ -529,6 +532,7 @@ int uttt_mcts_search(uttt_engine* e, const uint32_t* roots, int32_t n_roots, int
     UTTT_CHECK(!(tp && (flags & UTTT_SP_PYSEARCH)), "UTTT_SP_PYSEARCH and UTTT_SP_THROUGHPUT exclude each other");
     UTTT_CHECK(!(flags & UTTT_SP_MATCH), "UTTT_SP_MATCH is a self-play mode (uttt_selfplay_run*), not a search option");
     UTTT_CHECK(!(flags & UTTT_SP_RESIGN), "UTTT_SP_RESIGN is a self-play mode (uttt_selfplay_run*), not a search option");
+    UTTT_CHECK(!(flags & UTTT_SP_PLAYOUT_CAP), "UTTT_SP_PLAYOUT_CAP is a self-play mode (uttt_selfplay_run*), not a search option");
     if (mcts_begin_impl(e, roots, n_roots, sims, batch, flags)) return 1;     // uploads roots, runs the begin kernel
     if (n_roots == 0) return 0;
     TreeParams& t = e->tp;
@@ -626,6 +630,10 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
     // a loss, so a root value says nothing a resignation could rest on
     UTTT_CHECK(!(flags & UTTT_SP_RESIGN) || tp || (flags & UTTT_SP_CORRECT_TERMINAL_SIGN),
                "UTTT_SP_RESIGN needs terminal values of the correct sign: add UTTT_SP_CORRECT_TERMINAL_SIGN or use UTTT_SP_THROUGHPUT");
+    if (flags & UTTT_SP_PLAYOUT_CAP) {
+        UTTT_CHECK(!match, "UTTT_SP_PLAYOUT_CAP and UTTT_SP_MATCH exclude each other (a match records no training targets)");
+        UTTT_CHECK(e->tp.fast_sims <= sims, "UTTT_SP_PLAYOUT_CAP: fast_sims %d exceeds evaluate_count %d", e->tp.fast_sims, sims);
+    }
     UTTT_CHECK(!match || evaluator == UTTT_EVAL_HASH || e->w1.loaded,
                "UTTT_SP_MATCH: weight slot 1 was never uploaded (uttt_upload_weights_slot(e, 1, ...))");
     const int rows_per_tree = tp ? batch : 1;
@@ -821,6 +829,25 @@ int uttt_selfplay_fetch_values(uttt_engine* e, int64_t n_games, float* hist_valu
     return 0;
 }
 
+int uttt_set_playout_cap(uttt_engine* e, int32_t fast_sims, float full_fraction) {
+    UTTT_CHECK(full_fraction >= 0.0f && full_fraction <= 1.0f, "playout cap full fraction %g: must be in [0, 1]", (double)full_fraction);
+    UTTT_CHECK(fast_sims >= 1, "playout cap fast_sims %d: must be at least 1", fast_sims);
+    UTTT_CHECK(e != nullptr, "null engine");
+    UTTT_CHECK(fast_sims <= e->cfg.max_sims, "playout cap fast_sims %d exceeds the engine's max_sims %d", fast_sims, e->cfg.max_sims);
+    e->tp.fast_sims = fast_sims;
+    e->tp.full_fraction = full_fraction;
+    return 0;
+}
+
+int uttt_selfplay_fetch_full(uttt_engine* e, int64_t n_games, uint8_t* hist_full) {
+    UTTT_CHECK(e && n_games <= e->cfg.max_games && (hist_full || n_games <= 0), "bad argument");
+    if (n_games <= 0) return 0;
+    UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
+    UTTT_CUDA_OK(cudaMemcpyAsync(hist_full, e->tp.hist_full, (size_t)n_games * 81, cudaMemcpyDeviceToHost, e->stream));
+    UTTT_CUDA_OK(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
 int uttt_selfplay_pack(uttt_engine* e, int64_t n_games, void* out_dev, int64_t cap_samples, int64_t* n_samples_out, void* stream) {
     UTTT_CHECK(e && n_samples_out && n_games >= 0 && n_games <= e->cfg.max_games && (out_dev || cap_samples == 0), "bad argument");
     UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
@@ -828,13 +855,13 @@ int uttt_selfplay_pack(uttt_engine* e, int64_t n_games, void* out_dev, int64_t c
     const TreeParams& t = e->tp;
     *n_samples_out = 0;
     if (n_games == 0) return 0;
-    UTTT_CUDA_OK(launch_scan_lens(t.hist_len, n_games, e->hist_offsets, s));
+    UTTT_CUDA_OK(launch_scan_samples(t.hist_len, t.hist_full, n_games, e->hist_offsets, s));
     long long total = 0;
     UTTT_CUDA_OK(cudaMemcpyAsync(&total, e->hist_offsets + n_games, sizeof(total), cudaMemcpyDeviceToHost, s));
     UTTT_CUDA_OK(cudaStreamSynchronize(s));
     UTTT_CHECK(total <= cap_samples, "sample buffer too small: %lld samples, room for %lld", total, (long long)cap_samples);
-    UTTT_CUDA_OK(launch_pack_samples(t.hist_states, t.hist_counts, t.hist_len, t.hist_final, e->hist_offsets, n_games, out_dev,
-                                     cap_samples, s));
+    UTTT_CUDA_OK(launch_pack_samples(t.hist_states, t.hist_counts, t.hist_len, t.hist_full, t.hist_final, e->hist_offsets, n_games,
+                                     out_dev, cap_samples, s));
     *n_samples_out = total;
     return 0;
 }

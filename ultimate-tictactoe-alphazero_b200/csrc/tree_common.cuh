@@ -89,6 +89,17 @@ __device__ __forceinline__ int leaf_symmetry(const TreeParams& P, const TreeCtl&
 __device__ __forceinline__ int leaf_net(const TreeParams& P, const TreeCtl& c) {
     return (P.flags & UTTT_SP_MATCH) ? (int)(((uint32_t)c.game + (uint32_t)c.ply) & 1u) : 0;
 }
+// UTTT_SP_PLAYOUT_CAP: the tree's current move (game c.game, ply c.ply) is a full search iff u < full fraction,
+// u = (philox(key=(seed, 5), ctr=(g_lo, g_hi, ply, 0)).x >> 8) * 2^-24; without the flag every move is one.  Recomputed
+// wherever it is needed, like leaf_net: the ply does not change while the move is searched.
+__device__ __forceinline__ bool full_search(const TreeParams& P, const TreeCtl& c) {
+    if (!(P.flags & UTTT_SP_PLAYOUT_CAP)) return true;
+    const Philox4 r = philox4x32(P.seed, 5u, (uint32_t)c.game, (uint32_t)(c.game >> 32), (uint32_t)c.ply, 0u);
+    return (float)(r.x >> 8) * (1.0f / 16777216.0f) < P.full_fraction;
+}
+// the simulation budget of that move: evaluate_count for a full search, fast_sims for a fast one
+__device__ __forceinline__ int move_sims(const TreeParams& P, const TreeCtl& c) { return full_search(P, c) ? P.sims : P.fast_sims; }
+
 // the evaluator rows of that network
 __device__ __forceinline__ const float* net_policy(const TreeParams& P, int net) { return net ? P.policy1 : P.policy; }
 __device__ __forceinline__ const float* net_value(const TreeParams& P, int net) { return net ? P.value1 : P.value; }
@@ -346,9 +357,9 @@ __device__ __forceinline__ int sample_move(const TreeParams& P, const TreeView& 
 }
 
 // the move is decided (the simulation budget is spent).  Search: the root visit counts are the tree's output
-// (cpp/uttt_mcts.cpp:177-180) and the tree is done.  Self-play: record the root value and the history row, sample the
-// move, play it; when the game is over (lost or drawn, self_play_cpp.py:50-51,95) record it and claim the next game from
-// counters[0].  With UTTT_SP_RESIGN, a mover at ply p >= 1 of a game that is not a check game resigns instead when its
+// (cpp/uttt_mcts.cpp:177-180) and the tree is done.  Self-play: record the root value and the history row (with whether
+// the move was a full search), sample the move, play it; when the game is over (lost or drawn,
+// self_play_cpp.py:50-51,95) record it and claim the next game from counters[0].  With UTTT_SP_RESIGN, a mover at ply p >= 1 of a game that is not a check game resigns instead when its
 // root value is below the threshold: only the value of ply p is recorded, and the game ends with p plies as one whose
 // final position is lost for its mover.  Returns whether the tree goes on; if so `root` is the position of its next
 // search, already stored in P.root[t].
@@ -371,7 +382,10 @@ __device__ __forceinline__ bool decide_move(const TreeParams& P, const TreeView&
         for (int a = lane; a < 81; a += 32)
             P.hist_counts[hrow * 81 + a] = legal_bit(lm, a) ? (uint16_t)node_n(T.node[1 + legal_rank(lm, a)]) : (uint16_t)0;
         const int action = sample_move(P, T, c, lm, lane);
-        if (lane == 0) P.hist_actions[hrow] = (uint8_t)action;
+        if (lane == 0) {
+            P.hist_actions[hrow] = (uint8_t)action;
+            P.hist_full[hrow] = full_search(P, c) ? 1 : 0;
+        }
         PackedState nx;
         next_state(root, action, nx);
         root = nx;

@@ -42,7 +42,7 @@ __device__ void init_root(const TreeParams& P, const TreeView& T, TreeCtl& c, co
         if (lane == 0) T.node[0] = make_uint4(0x7Fu << 16, 0u, 0u, 0u);
         c.n_nodes = 1;
         c.n_root = L;
-        c.sims_left = P.sims;
+        c.sims_left = move_sims(P, c);
         c.path_len = 0;
         c.pend_k = 0;
         c.n_eval = 0;
@@ -54,7 +54,7 @@ __device__ void init_root(const TreeParams& P, const TreeView& T, TreeCtl& c, co
         if (legal_bit(lm, a)) T.node[1 + legal_rank(lm, a)] = make_node(a, pu);
     c.n_nodes = 1 + L;
     c.n_root = L;
-    c.sims_left = P.sims;
+    c.sims_left = move_sims(P, c);
     c.path_len = 0;
     c.pend_k = 0;
     c.n_eval = 0;

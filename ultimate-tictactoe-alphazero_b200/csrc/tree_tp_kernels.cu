@@ -67,7 +67,7 @@ struct TpAux {                 // per tree, per pending leaf
 };
 
 // expansion of `leaf` from one policy row, evaluated under symmetry `sym`: masked, serially renormalised priors (the
-// reference-exact mode's arithmetic), optional Dirichlet mix for the root
+// reference-exact mode's arithmetic), optional Dirichlet mix for the root of a full search
 __device__ void tp_expand(const TreeParams& P, const TreeView& T, TreeCtl& c, const PackedState& st, int leaf,
                           const float* pol, int sym, bool is_root, int lane) {
     uint32_t lm[3];
@@ -75,7 +75,7 @@ __device__ void tp_expand(const TreeParams& P, const TreeView& T, TreeCtl& c, co
     int base = c.n_nodes;
     float pr[3];
     legal_priors(pol, sym, lm, L, lane, pr);
-    const bool noise = is_root && P.dir_eps > 0.0f;
+    const bool noise = is_root && P.dir_eps > 0.0f && full_search(P, c);      // a fast search gets none (KataGo)
     float gsum = 0.0f, g[3] = {0.f, 0.f, 0.f};
     if (noise) {
         for (int q = 0, a = lane; a < 81; a += 32, q++)
@@ -135,7 +135,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 5) tree_tp_round_kernel(
         tp_expand(P, T, c, root, 0, net_policy(P, leaf_net(P, c)) + (size_t)c.nn_row * 81, leaf_symmetry(P, c, 0), true, lane);
         uint32_t lm[3];
         c.n_root = legal_mask(root, lm);
-        c.sims_left = P.sims;
+        c.sims_left = move_sims(P, c);
         c.phase = PHASE_SEARCH;
         __syncwarp();
     } else if (c.phase == PHASE_PENDING) {

@@ -32,6 +32,7 @@ SP_PYSEARCH = 4
 SP_RANDOM_SYMMETRY = 8     # evaluate every leaf under a random board symmetry (include/uttt_b200.h)
 SP_MATCH = 16              # self-play as a match: weight slot (game + ply) & 1 moves (include/uttt_b200.h)
 SP_RESIGN = 32             # a mover whose root value falls below the threshold resigns (include/uttt_b200.h)
+SP_PLAYOUT_CAP = 64        # a random share of moves gets a fast search and makes no training sample (include/uttt_b200.h)
 
 _vp = C.c_void_p
 _u32p = np.ctypeslib.ndpointer(np.uint32, flags="C_CONTIGUOUS")
@@ -101,6 +102,8 @@ ABI = {
     "uttt_selfplay_fetch": ([_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp], C.c_int),
     "uttt_set_resign": ([_vp, C.c_float, C.c_float], C.c_int),
     "uttt_selfplay_fetch_values": ([_vp, C.c_int64, _vp, _vp], C.c_int),
+    "uttt_set_playout_cap": ([_vp, C.c_int32, C.c_float], C.c_int),
+    "uttt_selfplay_fetch_full": ([_vp, C.c_int64, _vp], C.c_int),
     "uttt_selfplay_pack": ([_vp, C.c_int64, _vp, C.c_int64, C.POINTER(C.c_int64), _vp], C.c_int),
     "uttt_samples_unpack": ([_vp, C.c_int64, _vp, _vp, _vp, _vp], C.c_int),
     "uttt_debug_trunk_timeline": ([_vp, _vp], C.c_int),
@@ -345,6 +348,17 @@ def check_games(seed, game0, n, check_fraction):
     return u < _F32(check_fraction)
 
 
+def full_moves(seed, game0, n, full_fraction):
+    """SP_PLAYOUT_CAP's search kinds of games game0 .. game0 + n - 1 -> bool array (n, 81): the move at ply p of game g is
+    a full search iff (philox4x32(key=(seed, 5), ctr=(g_lo, g_hi, p, 0)).x >> 8) * 2^-24 < full_fraction (compared in
+    fp32), a fast one otherwise"""
+    g = (np.uint64(int(game0)) + np.arange(int(n), dtype=np.uint64))[:, None]
+    p = np.arange(81, dtype=np.uint64)[None, :]
+    x = _philox4x32_x(int(seed), 5, g & np.uint64(0xFFFFFFFF), g >> np.uint64(32), p, 0)
+    u = (x >> np.uint64(8)).astype(_F32) * _F32(1.0 / 16777216.0)
+    return u < _F32(full_fraction)
+
+
 def _recorded_values(history):
     """(values (n,81) f32, mask of the recorded rows): rows 0..len-1, plus row len of a resigned game"""
     lens = np.asarray(history.lens, np.int64)
@@ -450,19 +464,26 @@ class History:
         self.final = alloc((n_games,), torch.int8)
         self.values = alloc((n_games, 81), torch.float32)     # the mover's root value of every decided move
         self.resigned = alloc((n_games,), torch.int8)         # 1: the game ended by resignation (SP_RESIGN)
+        self.full = alloc((n_games, 81), torch.uint8)         # 1: the move was a full search (0: a fast one, SP_PLAYOUT_CAP)
+        self.full[:] = 1
         self.stats = np.zeros(4, np.int64)
 
     @property
     def nbytes(self):
         return (self.states.nbytes + self.counts.nbytes + self.actions.nbytes + self.lens.nbytes + self.final.nbytes
-                + self.values.nbytes + self.resigned.nbytes)
+                + self.values.nbytes + self.resigned.nbytes + self.full.nbytes)
+
+    def sample_mask(self, n=None):
+        """-> bool (n, 81) over the first n games (None: all): the plies that are training samples, those played
+        (ply < len) with a full search (every played ply without SP_PLAYOUT_CAP)"""
+        n = len(self.lens) if n is None else int(n)
+        return (np.arange(81)[None, :] < self.lens[:n, None].astype(np.int64)) & (self.full[:n] != 0)
 
     def samples(self):
-        """-> (states (N,8) uint32, counts (N,81) uint16, z (N,) int8) over all plies, game-major order.
+        """-> (states (N,8) uint32, counts (N,81) uint16, z (N,) int8) over the sample plies (sample_mask), game-major order.
         z follows self_play_cpp.py:95-99 verbatim (value of the FINAL position from its mover's view,
         assigned to ply 0 and alternating), i.e. the reference's labelling including its sign quirk."""
-        lens = self.lens.astype(np.int64)
-        mask = np.arange(81)[None, :] < lens[:, None]
+        mask = self.sample_mask()
         st = self.states[mask]
         cn = self.counts[mask]
         z0 = np.where(self.final != 0, -1, 0).astype(np.int8)
@@ -556,6 +577,11 @@ class Engine:
         of check games that are never resigned (in [0, 1]); see include/uttt_b200.h"""
         _check(self.lib.uttt_set_resign(self.h, float(threshold), float(check_fraction)))
 
+    def set_playout_cap(self, fast_sims=8, full_fraction=0.25):
+        """SP_PLAYOUT_CAP's fast-search budget (1 .. max_sims simulations, at most the run's sims) and the probability of a
+        full search (in [0, 1]); see include/uttt_b200.h"""
+        _check(self.lib.uttt_set_playout_cap(self.h, int(fast_sims), float(full_fraction)))
+
     def mcts_search(self, roots, sims, batch, temperature, evaluator, flags=0):
         roots = np.ascontiguousarray(roots, dtype=np.uint32).reshape(-1, 8)
         n = roots.shape[0]
@@ -604,6 +630,7 @@ class Engine:
                                           _ptr(hist.states), _ptr(hist.counts), _ptr(hist.actions), _ptr(hist.lens),
                                           _ptr(hist.final), _ptr(hist.stats)))
         _check(self.lib.uttt_selfplay_fetch_values(self.h, n_games, _ptr(hist.values), _ptr(hist.resigned)))
+        _check(self.lib.uttt_selfplay_fetch_full(self.h, n_games, _ptr(hist.full)))
         return hist
 
     def match(self, n_games, sims=50, batch=8, seed=0, evaluator=EVAL_NET_BF16, flags=0, game0=0, history=None):
@@ -629,11 +656,12 @@ class Engine:
         _check(self.lib.uttt_selfplay_fetch(self.h, n_games, _ptr(hist.states), _ptr(hist.counts), _ptr(hist.actions),
                                             _ptr(hist.lens), _ptr(hist.final)))
         _check(self.lib.uttt_selfplay_fetch_values(self.h, n_games, _ptr(hist.values), _ptr(hist.resigned)))
+        _check(self.lib.uttt_selfplay_fetch_full(self.h, n_games, _ptr(hist.full)))
         return hist
 
     def selfplay_pack(self, n_games, out=None, stream=None):
-        """history of the last selfplay_device() as one device buffer of SAMPLE_BYTES-byte samples -> (uint8 CUDA tensor
-        sliced to the exact length, n_samples).  `out`: optional uint8 CUDA tensor to pack into (81 * n_games samples fit)"""
+        """history of the last selfplay_device() as one device buffer of SAMPLE_BYTES-byte samples, one per ply of
+        History.sample_mask -> (uint8 CUDA tensor sliced to the exact length, n_samples).  `out`: optional uint8 CUDA tensor to pack into (81 * n_games samples fit)"""
         import torch
         cap = 81 * int(n_games)
         if out is None:

@@ -78,12 +78,12 @@ def gather_samples(samples, dst=0, out=None):
 
 
 def pack_history_host(hist, n_local):
-    """engine.History (host arrays) -> uint8 tensor of packed samples, the layout of uttt_selfplay_pack (csrc/history_kernels.cu)"""
-    lens = hist.lens[:n_local].astype(np.int64)
-    n = int(lens.sum())
+    """engine.History (host arrays) -> uint8 tensor of packed samples, the layout of uttt_selfplay_pack (csrc/history_kernels.cu):
+    one per ply of hist.sample_mask"""
+    mask = hist.sample_mask(n_local)
+    n = int(mask.sum())
     raw = np.zeros((n, _eng.SAMPLE_BYTES), np.uint8)
     if n:
-        mask = np.arange(81)[None, :] < lens[:, None]
         raw[:, :32] = hist.states[:n_local][mask].view(np.uint8).reshape(n, 32)
         raw[:, 32:194] = np.ascontiguousarray(hist.counts[:n_local][mask]).view(np.uint8).reshape(n, 162)
         ply = np.broadcast_to(np.arange(81)[None, :], mask.shape)[mask]
@@ -110,15 +110,21 @@ class SelfPlayCycle:
     """BASELINE config 5, the self-play stage of a multi-GPU train_cycle iteration, repeated: rank `src` broadcasts the
     weights (new best.pth), every rank plays its block of games on its own GPU (no collective on the search path), the
     packed histories go to rank `dst` in one transfer per rank and are expanded there into the trainer's tensors.
-    The engine, the pack buffer and the gather buffer live as long as the object."""
+    The engine, the pack buffer and the gather buffer live as long as the object.  fast_sims (None: every move is a full
+    search) turns on playout cap randomization (engine.SP_PLAYOUT_CAP): a move gets a full search of `sims` simulations with
+    probability full_fraction and a fast one of fast_sims otherwise, and only the full searches become samples."""
 
-    def __init__(self, n_games, sims=50, batch=8, numerics=None, device=None, max_slots=4096):
+    def __init__(self, n_games, sims=50, batch=8, numerics=None, device=None, max_slots=4096, fast_sims=None, full_fraction=0.25):
         self.world, self.rank = dist.get_world_size(), dist.get_rank()
         self.n_games, self.sims, self.batch = n_games, sims, batch
         self.game0, self.count = shard_games(n_games, self.world, self.rank)
         self.evaluator = _eng.evaluator_of(_eng.DEFAULT_NUMERICS if numerics is None else numerics)
         cnt = max(self.count, 1)
         self.engine = _eng.Engine(n_slots=min(cnt, max_slots), max_sims=sims, max_batch=batch, max_games=cnt, device=device)
+        self.flags = 0
+        if fast_sims is not None:
+            self.engine.set_playout_cap(fast_sims, full_fraction)
+            self.flags = _eng.SP_PLAYOUT_CAP
         self.dev = torch.device("cuda", self.engine.device)
         self.pack_buf = torch.empty(81 * cnt * _eng.SAMPLE_BYTES, dtype=torch.uint8, device=self.dev)
         self.gather_buf = None
@@ -139,7 +145,7 @@ class SelfPlayCycle:
         self.engine.upload_model(model)
         t1 = tick()
         stats = self.engine.selfplay_device(self.count, sims=self.sims, batch=self.batch, seed=seed, evaluator=self.evaluator,
-                                            game0=cycle * self.n_games + self.game0)
+                                            flags=self.flags, game0=cycle * self.n_games + self.game0)
         t2 = tick()
         samples, n_local = self.engine.selfplay_pack(self.count, out=self.pack_buf)
         t3 = tick()

@@ -49,6 +49,11 @@ SP_RESIGN_CHECK_FRACTION = 0.1    # fraction of games never resigned, to measure
 SP_RESIGN_TARGET_FP = None    # a float: after each cycle SP_RESIGN_THRESHOLD becomes the largest threshold whose false-positive
                               # rate on that cycle's played-out games (the check games; all games while resignation is off)
                               # is at most this (engine.resign_threshold)
+SP_FAST_SIMS = None           # an int in [1, PV_EVALUATE_COUNT]: playout cap randomization (KataGo; engine.SP_PLAYOUT_CAP).
+                              # A move gets the full PV_EVALUATE_COUNT simulations with probability SP_FULL_FRACTION and
+                              # SP_FAST_SIMS otherwise; only the full searches become training samples.  None: every move
+                              # is a full search (the reference's games)
+SP_FULL_FRACTION = 0.25
 
 _engine = None
 last_stats = {}
@@ -111,7 +116,7 @@ def _scores_from_counts(cn):
 def _corrected_labels(hist):
     """value from each mover's own perspective (the labelling of the reference's self_play.py:21-25,96)"""
     lens = hist.lens.astype(np.int64)
-    mask = np.arange(81)[None, :] < lens[:, None]
+    mask = hist.sample_mask()
     # the final position's mover lost iff final != 0; ply t has the same mover as the final position
     # iff (len - t) is even
     par = ((lens[:, None] - np.arange(81)[None, :]) % 2) == 0
@@ -134,6 +139,19 @@ def _resign_flags():
     return _eng.SP_RESIGN if SP_RESIGN_THRESHOLD is not None else 0
 
 
+def _playout_cap_flags():
+    """engine.SP_PLAYOUT_CAP if SP_FAST_SIMS is set, else 0; ValueError if SP_FAST_SIMS is not an integer in
+    [1, PV_EVALUATE_COUNT] or SP_FULL_FRACTION is not in [0, 1]"""
+    if SP_FAST_SIMS is None:
+        return 0
+    if isinstance(SP_FAST_SIMS, bool) or int(SP_FAST_SIMS) != SP_FAST_SIMS or not 1 <= SP_FAST_SIMS <= PV_EVALUATE_COUNT:
+        raise ValueError("SP_FAST_SIMS = %r: must be None or an integer in [1, PV_EVALUATE_COUNT = %d]"
+                         % (SP_FAST_SIMS, PV_EVALUATE_COUNT))
+    if not 0.0 <= SP_FULL_FRACTION <= 1.0:
+        raise ValueError("SP_FULL_FRACTION = %r: must be in [0, 1]" % (SP_FULL_FRACTION,))
+    return _eng.SP_PLAYOUT_CAP
+
+
 def _resign_stats(hist, n_games, seed, resign):
     """resigned games and the false positives of the played-out calibration games (the check games while resigning, all
     games otherwise); with SP_RESIGN_TARGET_FP, the threshold calibrated on them becomes SP_RESIGN_THRESHOLD"""
@@ -152,6 +170,7 @@ def _resign_stats(hist, n_games, seed, resign):
 
 def _run(model, n_games, progress=False):
     resign = _resign_flags()
+    cap = _playout_cap_flags()
     eng = _get_engine(n_games)
     model.eval()
     eng.upload_model(model)
@@ -166,6 +185,9 @@ def _run(model, n_games, progress=False):
     if resign:
         flags |= resign
         eng.set_resign(SP_RESIGN_THRESHOLD, SP_RESIGN_CHECK_FRACTION)
+    if cap:
+        flags |= cap
+        eng.set_playout_cap(int(SP_FAST_SIMS), SP_FULL_FRACTION)
     eng.set_selfplay_temperature(SP_TEMPERATURE)
     if SP_PROGRESS and progress:
         shown = [0]
@@ -182,6 +204,8 @@ def _run(model, n_games, progress=False):
         eng.set_selfplay_temperature(1.0)
     last_stats.update(plies=int(hist.stats[0]), sims=int(hist.stats[1]), evals=int(hist.stats[2]),
                       rounds=int(hist.stats[3]), seed=seed)
+    full = int(hist.sample_mask(n_games).sum())
+    last_stats.update(full_plies=full, fast_plies=int(hist.stats[0]) - full)
     for k in ("check_would_resign", "check_false_positives", "calibrated_threshold"):     # only what this cycle reports
         last_stats.pop(k, None)
     last_stats.update(_resign_stats(hist, n_games, seed, bool(resign)))
