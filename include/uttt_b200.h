@@ -104,6 +104,33 @@ extern "C" {
                                            without the flag.  Only full-search plies become packed samples
                                            (uttt_selfplay_pack).  Fails with fast_sims > evaluate_count and with
                                            UTTT_SP_MATCH (a match records no training targets). */
+#define UTTT_SP_FORCED_PLAYOUTS 128     /* uttt_selfplay_run* only, with UTTT_SP_THROUGHPUT, alone or with
+                                           UTTT_SP_RANDOM_SYMMETRY, UTTT_SP_RESIGN or UTTT_SP_PLAYOUT_CAP: forced playouts
+                                           and policy target pruning (KataGo, Wu 2019, section 3.2).  It applies to every
+                                           full search of the run (every move without UTTT_SP_PLAYOUT_CAP, the full ones
+                                           with it); a fast search neither forces nor prunes.  It does not depend on the
+                                           root noise's eps.  k = forced_k (uttt_set_forced_playouts, default 2).  All
+                                           arithmetic is IEEE fp32, correctly rounded, in the order written, without FMA.
+                                           Forcing (the PUCT step at the root only): N = sum of (n + vl) over the root's
+                                           children, virtual loss included; a root child with m = n + vl and stored prior
+                                           p (the noised one where noise is mixed in) is forced iff m >= 1 and (float)m <
+                                           F, F = sqrt((k * p) * (float)N); a forced child scores 1e20f, so the first
+                                           maximum picks the forced child with the smallest index.  Pruning (when the move
+                                           is decided; no virtual loss is outstanding): N = sum of n, sq = sqrt((float)N),
+                                           c* = the first child with the most visits, S* = q* + (p* * sq) / (float)(1 +
+                                           n*) with q* = -w* / n*.  Every other child c with n >= 1: q = -w / n, F as
+                                           above with this N, R = min(n, (int)F); r is the largest value in [0, R] with
+                                           score(n - j) < S* for every j in 1..r, score(m) = q + (p * sq) / (float)(1 +
+                                           m); the child's target is t = n - r, and 0 if r >= 1 and n - r == 1 (a child
+                                           reduced to a single playout is pruned outright).  c* keeps t = n*, an
+                                           unvisited child 0.  hist_counts keeps the raw visit counts; hist_target[g*81 +
+                                           p][a] (uttt_selfplay_fetch_target) holds t, and equals the counts on a fast
+                                           ply.  The move is drawn from t (the same Philox draw, temperature rule and
+                                           legal order as from the counts; T = 0 still plays c*); the root value and
+                                           resignation use the raw (n, w) of c*, which pruning never changes.  Packed
+                                           samples carry t as their policy counts.  Fails without UTTT_SP_THROUGHPUT (the
+                                           reference-exact root is uniform and never noised) and with UTTT_SP_MATCH (a
+                                           match records no training targets). */
 
 typedef struct uttt_engine uttt_engine;
 
@@ -293,8 +320,16 @@ int uttt_set_playout_cap(uttt_engine *e, int32_t fast_sims, float full_fraction)
  * 0 for a fast one (rows 0..hist_len-1; later rows are unspecified).  HOST pointer.  Synchronous. */
 int uttt_selfplay_fetch_full(uttt_engine *e, int64_t n_games, uint8_t *hist_full /* n*81 */);
 
+/* UTTT_SP_FORCED_PLAYOUTS's k (finite, in (0, 100]; default 2, KataGo's).  Fails on any other value. */
+int uttt_set_forced_playouts(uttt_engine *e, float k);
+/* the policy target counts of the last uttt_selfplay_run*, like uttt_selfplay_fetch's hist_counts: hist_target[(g*81 +
+ * ply)*81 + a] = t of UTTT_SP_FORCED_PLAYOUTS, or a copy of the visit counts if that run had no such flag.  HOST pointer.
+ * Synchronous. */
+int uttt_selfplay_fetch_target(uttt_engine *e, int64_t n_games, uint16_t *hist_target /* n*81*81 */);
+
 /* The history of the last uttt_selfplay_run_device as ONE contiguous device buffer of fixed-size samples (one per played
- * ply with hist_full = 1, i.e. every played ply without UTTT_SP_PLAYOUT_CAP; game-major, ply order): bytes 0..31 packed position, 32..193 root visit counts u16[81], 194 z (int8, the label of
+ * ply with hist_full = 1, i.e. every played ply without UTTT_SP_PLAYOUT_CAP; game-major, ply order): bytes 0..31 packed
+ * position, 32..193 policy target counts u16[81] (the visit counts without UTTT_SP_FORCED_PLAYOUTS), 194 z (int8, the label of
  * self_play_cpp.py:95-99), 195 ply.  This is what a rank sends to the trainer rank in the multi-GPU cycle (one
  * exact-length transfer instead of the ~1.7 KB/sample pickle of self_play_cpp.py:125-130).
  * uttt_selfplay_pack: out_dev must hold cap_samples samples; *n_samples_out (HOST) = samples written; synchronises `stream`.

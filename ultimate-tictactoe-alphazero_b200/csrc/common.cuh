@@ -132,6 +132,8 @@ struct TreeParams {
     uint8_t* hist_full;            // [n_games][81]: 1 if the move was a full search, 0 if a fast one
     int32_t fast_sims;             // UTTT_SP_PLAYOUT_CAP (uttt_set_playout_cap)
     float full_fraction;
+    float forced_k;                // UTTT_SP_FORCED_PLAYOUTS (uttt_set_forced_playouts)
+    uint16_t* hist_target;         // [n_games][81][81]: policy target counts, allocated by the first run with that flag
 };
 
 // kernels' host launchers (each returns cudaGetLastError of the launch)

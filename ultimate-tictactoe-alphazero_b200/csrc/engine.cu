@@ -65,6 +65,7 @@ struct uttt_engine {
     int prof_sample;        // level 1: the trunk is bracketed in every prof_sample-th window of rounds only (see uttt_set_profile_level)
     int64_t prof_sampled_launches, prof_sampled_evals;      // trunk launches with events in the last run, positions they evaluated
     int lane_threshold;     // slots from which self-play splits into two overlapped lanes
+    bool last_forced;       // the last self-play run had UTTT_SP_FORCED_PLAYOUTS: its policy targets are in tp.hist_target
     NetWeights w;           // weight slot 0
     NetWeights w1;          // weight slot 1 (UTTT_SP_MATCH), allocated by its first upload
     // slot 1's evaluator queue, the same per-row arrays as slot 0's (e->tp.nn_*, policy, value, headfeat); allocated by the
@@ -355,6 +356,8 @@ int uttt_create(const uttt_config* cfg, uttt_engine** out) {
     t.resign_check_fraction = 0.1f;
     t.fast_sims = 8;
     t.full_fraction = 0.25f;
+    t.forced_k = 2.0f;
+    e->last_forced = false;
     *out = e;
     return 0;
 }
@@ -533,6 +536,8 @@ int uttt_mcts_search(uttt_engine* e, const uint32_t* roots, int32_t n_roots, int
     UTTT_CHECK(!(flags & UTTT_SP_MATCH), "UTTT_SP_MATCH is a self-play mode (uttt_selfplay_run*), not a search option");
     UTTT_CHECK(!(flags & UTTT_SP_RESIGN), "UTTT_SP_RESIGN is a self-play mode (uttt_selfplay_run*), not a search option");
     UTTT_CHECK(!(flags & UTTT_SP_PLAYOUT_CAP), "UTTT_SP_PLAYOUT_CAP is a self-play mode (uttt_selfplay_run*), not a search option");
+    UTTT_CHECK(!(flags & UTTT_SP_FORCED_PLAYOUTS),
+               "UTTT_SP_FORCED_PLAYOUTS is a self-play mode (uttt_selfplay_run*), not a search option");
     if (mcts_begin_impl(e, roots, n_roots, sims, batch, flags)) return 1;     // uploads roots, runs the begin kernel
     if (n_roots == 0) return 0;
     TreeParams& t = e->tp;
@@ -634,11 +639,20 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
         UTTT_CHECK(!match, "UTTT_SP_PLAYOUT_CAP and UTTT_SP_MATCH exclude each other (a match records no training targets)");
         UTTT_CHECK(e->tp.fast_sims <= sims, "UTTT_SP_PLAYOUT_CAP: fast_sims %d exceeds evaluate_count %d", e->tp.fast_sims, sims);
     }
+    const bool forced = (flags & UTTT_SP_FORCED_PLAYOUTS) != 0;
+    if (forced) {
+        // the reference-exact root is uniform and never noised: forcing its children is not what the rule is for
+        UTTT_CHECK(tp, "UTTT_SP_FORCED_PLAYOUTS needs UTTT_SP_THROUGHPUT");
+        UTTT_CHECK(!match, "UTTT_SP_FORCED_PLAYOUTS and UTTT_SP_MATCH exclude each other (a match records no training targets)");
+    }
     UTTT_CHECK(!match || evaluator == UTTT_EVAL_HASH || e->w1.loaded,
                "UTTT_SP_MATCH: weight slot 1 was never uploaded (uttt_upload_weights_slot(e, 1, ...))");
     const int rows_per_tree = tp ? batch : 1;
     UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
     if (match && alloc_queue1(e)) return 1;
+    // the policy targets on first use, so that an engine that never uses the flag keeps its footprint
+    if (forced && !e->tp.hist_target && ealloc(e, &e->tp.hist_target, (size_t)e->cfg.max_games * 81 * 81)) return 1;
+    e->last_forced = forced;
     cudaStream_t s = stream ? (cudaStream_t)stream : e->stream;
     for (int i = 0; i < 4; i++) { e->prof_ms[i] = 0.0; e->prof_launches[i] = 0; }
     e->prof_sampled_launches = e->prof_sampled_evals = 0;
@@ -848,6 +862,23 @@ int uttt_selfplay_fetch_full(uttt_engine* e, int64_t n_games, uint8_t* hist_full
     return 0;
 }
 
+int uttt_set_forced_playouts(uttt_engine* e, float k) {
+    UTTT_CHECK(k > 0.0f && k <= 100.0f, "forced playouts k %g: must be in (0, 100]", (double)k);
+    UTTT_CHECK(e != nullptr, "null engine");
+    e->tp.forced_k = k;
+    return 0;
+}
+
+int uttt_selfplay_fetch_target(uttt_engine* e, int64_t n_games, uint16_t* hist_target) {
+    UTTT_CHECK(e && n_games <= e->cfg.max_games && (hist_target || n_games <= 0), "bad argument");
+    if (n_games <= 0) return 0;
+    UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
+    const uint16_t* src = e->last_forced ? e->tp.hist_target : e->tp.hist_counts;
+    UTTT_CUDA_OK(cudaMemcpyAsync(hist_target, src, (size_t)n_games * 81 * 81 * 2, cudaMemcpyDeviceToHost, e->stream));
+    UTTT_CUDA_OK(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
 int uttt_selfplay_pack(uttt_engine* e, int64_t n_games, void* out_dev, int64_t cap_samples, int64_t* n_samples_out, void* stream) {
     UTTT_CHECK(e && n_samples_out && n_games >= 0 && n_games <= e->cfg.max_games && (out_dev || cap_samples == 0), "bad argument");
     UTTT_CUDA_OK(cudaSetDevice(e->cfg.device));
@@ -860,7 +891,9 @@ int uttt_selfplay_pack(uttt_engine* e, int64_t n_games, void* out_dev, int64_t c
     UTTT_CUDA_OK(cudaMemcpyAsync(&total, e->hist_offsets + n_games, sizeof(total), cudaMemcpyDeviceToHost, s));
     UTTT_CUDA_OK(cudaStreamSynchronize(s));
     UTTT_CHECK(total <= cap_samples, "sample buffer too small: %lld samples, room for %lld", total, (long long)cap_samples);
-    UTTT_CUDA_OK(launch_pack_samples(t.hist_states, t.hist_counts, t.hist_len, t.hist_full, t.hist_final, e->hist_offsets, n_games,
+    // policy target counts: the pruned ones of a run with UTTT_SP_FORCED_PLAYOUTS, the visit counts otherwise
+    const uint16_t* counts = e->last_forced ? t.hist_target : t.hist_counts;
+    UTTT_CUDA_OK(launch_pack_samples(t.hist_states, counts, t.hist_len, t.hist_full, t.hist_final, e->hist_offsets, n_games,
                                      out_dev, cap_samples, s));
     *n_samples_out = total;
     return 0;

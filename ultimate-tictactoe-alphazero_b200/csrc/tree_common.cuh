@@ -187,8 +187,10 @@ struct Descent {
 // descend from the root by PUCT (cpp/uttt_mcts.cpp:15-32,57-81), recording the node path into `path`.  Children are
 // read once (one 128-bit load each); lanes keep their first three in registers, longer lists (the reference-exact mode's
 // k-fold duplicated lists, Q-M3) are re-read through L1.  A child with vl units of virtual loss counts as n + vl
-// visits and w + vl lost value (the reference-exact mode sets none).
-__device__ __forceinline__ Descent descend(const TreeView& T, const PackedState& root, int32_t* path, int lane) {
+// visits and w + vl lost value (the reference-exact mode sets none).  forced_k > 0 (UTTT_SP_FORCED_PLAYOUTS on a full
+// search; callers without it pass a literal 0, which compiles the test out): at the root, a child with m = n + vl >= 1
+// and (float)m < sqrt((k * p) * (float)N), N the visits summed as below, scores 1e20f (KataGo's forced playouts).
+__device__ __forceinline__ Descent descend(const TreeView& T, const PackedState& root, int32_t* path, float forced_k, int lane) {
     Descent d;
     d.st = root;
     d.node = 0;
@@ -213,6 +215,7 @@ __device__ __forceinline__ Descent descend(const TreeView& T, const PackedState&
         for (int i = lane + 96; i < cnt; i += 32) { const uint4 q = ch[i]; tot += node_n(q) + node_vloss(q); }
         tot = __reduce_add_sync(FULL, tot);
         const float sq = __fsqrt_rn((float)tot);
+        const bool force = forced_k > 0.0f && d.plen == 1;     // the root's children
         float best = -1e9f;
         int besti = 0x7FFFFFFF;
         uint32_t bestx = 0u, bestlink = 0u;
@@ -224,6 +227,7 @@ __device__ __forceinline__ Descent descend(const TreeView& T, const PackedState&
             if (n > 0) {
                 const float qv = __fdiv_rn(-__fadd_rn(__uint_as_float(q.y), (float)vl), (float)n);
                 s = __fadd_rn(qv, __fdiv_rn(s, (float)(1 + n)));
+                if (force && (float)n < __fsqrt_rn(__fmul_rn(__fmul_rn(forced_k, __uint_as_float(q.z)), (float)tot))) s = 1e20f;
             }
             if (s > best) { best = s; besti = i; bestx = q.x; bestlink = q.w; }
         };
@@ -356,14 +360,48 @@ __device__ __forceinline__ int sample_move(const TreeParams& P, const TreeView& 
     return nth_legal(lm, chosen);
 }
 
+// UTTT_SP_FORCED_PLAYOUTS' policy target pruning (include/uttt_b200.h), in place: the n field of every root child
+// becomes its target t, which the move is then drawn from (the tree is discarded after the move).  c* = the first most
+// visited child keeps n*; a visited child c loses the r <= min(n, (int)F) playouts whose removal keeps its PUCT score below
+// c*'s, S*; one left with a single playout is pruned to 0.  score(n - j) grows with j (correctly rounded division and
+// addition are monotone), so r is found by stepping j up.  No virtual loss is outstanding (see root_value).
+__device__ __forceinline__ void prune_root(const TreeView& T, int L, float k, int lane) {
+    int tot = 0;
+    for (int i = lane; i < L; i += 32) tot += node_n(T.node[1 + i]);
+    tot = __reduce_add_sync(FULL, tot);
+    const int cs = most_visited(T, L, lane);
+    const uint4 qs = T.node[1 + cs];
+    const int ns = node_n(qs);
+    const float sq = __fsqrt_rn((float)tot);
+    const float best = __fadd_rn(__fdiv_rn(-__uint_as_float(qs.y), (float)ns),
+                                 __fdiv_rn(__fmul_rn(__uint_as_float(qs.z), sq), (float)(1 + ns)));
+    __syncwarp();                                            // every lane has read the counts it wrote to the history
+    for (int i = lane; i < L; i += 32) {
+        uint4 q = T.node[1 + i];
+        const int n = node_n(q);
+        if (i == cs || n == 0) continue;
+        const float p = __uint_as_float(q.z);
+        const float qv = __fdiv_rn(-__uint_as_float(q.y), (float)n), u = __fmul_rn(p, sq);
+        const int cap = min(n, (int)__fsqrt_rn(__fmul_rn(__fmul_rn(k, p), (float)tot)));
+        int r = 0;
+        while (r < cap && __fadd_rn(qv, __fdiv_rn(u, (float)(n - r))) < best) r++;      // score(n - (r + 1))
+        const int t = (r >= 1 && n - r == 1) ? 0 : n - r;
+        T.node[1 + i].x = (q.x & ~0xFFFFu) | (uint32_t)t;
+    }
+    __syncwarp();
+}
+
 // the move is decided (the simulation budget is spent).  Search: the root visit counts are the tree's output
 // (cpp/uttt_mcts.cpp:177-180) and the tree is done.  Self-play: record the root value and the history row (with whether
 // the move was a full search), sample the move, play it; when the game is over (lost or drawn,
 // self_play_cpp.py:50-51,95) record it and claim the next game from counters[0].  With UTTT_SP_RESIGN, a mover at ply p >= 1 of a game that is not a check game resigns instead when its
 // root value is below the threshold: only the value of ply p is recorded, and the game ends with p plies as one whose
-// final position is lost for its mover.  Returns whether the tree goes on; if so `root` is the position of its next
+// final position is lost for its mover.  With UTTT_SP_FORCED_PLAYOUTS, forced_k > 0 on a full search prunes the root's
+// counts to the policy targets (prune_root) after the counts are recorded, and the targets are recorded and drawn from;
+// callers without that flag pass a literal 0.  Returns whether the tree goes on; if so `root` is the position of its next
 // search, already stored in P.root[t].
-__device__ __forceinline__ bool decide_move(const TreeParams& P, const TreeView& T, int t, TreeCtl& c, PackedState& root, int lane) {
+__device__ __forceinline__ bool decide_move(const TreeParams& P, const TreeView& T, int t, TreeCtl& c, PackedState& root,
+                                            float forced_k, int lane) {
     if (P.mode == MODE_SEARCH) {
         for (int i = lane; i < 81; i += 32) P.out_counts[(size_t)t * 81 + i] = (i < c.n_root) ? node_n(T.node[1 + i]) : 0;
         if (lane == 0) { P.out_n[t] = c.n_root; atomicAdd(P.counters + 6, 1ull); }
@@ -381,6 +419,11 @@ __device__ __forceinline__ bool decide_move(const TreeParams& P, const TreeView&
         warp_store_state(P.hist_states + hrow, root, lane);
         for (int a = lane; a < 81; a += 32)
             P.hist_counts[hrow * 81 + a] = legal_bit(lm, a) ? (uint16_t)node_n(T.node[1 + legal_rank(lm, a)]) : (uint16_t)0;
+        if (P.flags & UTTT_SP_FORCED_PLAYOUTS) {
+            if (forced_k > 0.0f) prune_root(T, c.n_root, forced_k, lane);
+            for (int a = lane; a < 81; a += 32)
+                P.hist_target[hrow * 81 + a] = legal_bit(lm, a) ? (uint16_t)node_n(T.node[1 + legal_rank(lm, a)]) : (uint16_t)0;
+        }
         const int action = sample_move(P, T, c, lm, lane);
         if (lane == 0) {
             P.hist_actions[hrow] = (uint8_t)action;

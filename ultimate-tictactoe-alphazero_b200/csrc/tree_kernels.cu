@@ -266,13 +266,13 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 7) tree_round_kernel(Tre
     int n_terminal = 0;
     for (;;) {
         if (c.sims_left <= 0) {
-            if (!decide_move(P, T, t, c, root, lane)) break;
+            if (!decide_move(P, T, t, c, root, 0.0f, lane)) break;
             __syncwarp();
             init_root(P, T, c, root, lane);
             __syncwarp();
         }
 
-        const Descent d = descend(T, root, path, lane);
+        const Descent d = descend(T, root, path, 0.0f, lane);
         if (d.end != LEAF_UNEXPANDED) {
             // cpp/uttt_mcts.cpp:19-21,115-118: the reference backs up -value with value = -1 for a lost
             // mover, i.e. +1 lands on the lost node itself (inverted sign, Q-M2); draws back up -0.0f.

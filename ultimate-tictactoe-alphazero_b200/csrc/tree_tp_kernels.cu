@@ -160,9 +160,12 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 5) tree_tp_round_kernel(
         c.phase = PHASE_SEARCH;
     }
 
+    // UTTT_SP_FORCED_PLAYOUTS' k for this round's descents and its move decision, which all belong to the move at c.ply
+    // (a decided move ends the round's search: the next move starts by queueing its root)
+    const float forced_k = ((P.flags & UTTT_SP_FORCED_PLAYOUTS) && full_search(P, c)) ? P.forced_k : 0.0f;
     for (int guard = 0; guard < 4; guard++) {
         if (c.phase == PHASE_SEARCH && c.sims_left <= 0) {
-            if (!decide_move(P, T, t, c, root, lane)) break;
+            if (!decide_move(P, T, t, c, root, forced_k, lane)) break;
             c.phase = PHASE_ROOT;
         }
         if (c.phase == PHASE_ROOT) {
@@ -184,7 +187,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, 5) tree_tp_round_kernel(
         int got = 0, terminals = 0;
         while (got < want && got + terminals < c.sims_left && terminals < 2 * m) {
             int32_t* path = leaf_path(P, t, got);
-            const Descent d = descend(T, root, path, lane);
+            const Descent d = descend(T, root, path, forced_k, lane);
             if (d.end == LEAF_BLOCKED) break;       // the best line ends in a leaf already queued this round
             if (d.end != LEAF_UNEXPANDED) {
                 // value for the mover of the terminal node: -1 lost, 0 draw (correct sign, unlike cpp/uttt_mcts.cpp:19-21)

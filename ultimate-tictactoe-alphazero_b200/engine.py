@@ -33,6 +33,7 @@ SP_RANDOM_SYMMETRY = 8     # evaluate every leaf under a random board symmetry (
 SP_MATCH = 16              # self-play as a match: weight slot (game + ply) & 1 moves (include/uttt_b200.h)
 SP_RESIGN = 32             # a mover whose root value falls below the threshold resigns (include/uttt_b200.h)
 SP_PLAYOUT_CAP = 64        # a random share of moves gets a fast search and makes no training sample (include/uttt_b200.h)
+SP_FORCED_PLAYOUTS = 128   # forced root playouts, pruned again from the policy targets (throughput mode; include/uttt_b200.h)
 
 _vp = C.c_void_p
 _u32p = np.ctypeslib.ndpointer(np.uint32, flags="C_CONTIGUOUS")
@@ -104,6 +105,8 @@ ABI = {
     "uttt_selfplay_fetch_values": ([_vp, C.c_int64, _vp, _vp], C.c_int),
     "uttt_set_playout_cap": ([_vp, C.c_int32, C.c_float], C.c_int),
     "uttt_selfplay_fetch_full": ([_vp, C.c_int64, _vp], C.c_int),
+    "uttt_set_forced_playouts": ([_vp, C.c_float], C.c_int),
+    "uttt_selfplay_fetch_target": ([_vp, C.c_int64, _vp], C.c_int),
     "uttt_selfplay_pack": ([_vp, C.c_int64, _vp, C.c_int64, C.POINTER(C.c_int64), _vp], C.c_int),
     "uttt_samples_unpack": ([_vp, C.c_int64, _vp, _vp, _vp, _vp], C.c_int),
     "uttt_debug_trunk_timeline": ([_vp, _vp], C.c_int),
@@ -466,12 +469,19 @@ class History:
         self.resigned = alloc((n_games,), torch.int8)         # 1: the game ended by resignation (SP_RESIGN)
         self.full = alloc((n_games, 81), torch.uint8)         # 1: the move was a full search (0: a fast one, SP_PLAYOUT_CAP)
         self.full[:] = 1
+        self.target = None      # (n_games, 81, 81) uint16 policy target counts of a run with SP_FORCED_PLAYOUTS, else None
         self.stats = np.zeros(4, np.int64)
 
     @property
     def nbytes(self):
         return (self.states.nbytes + self.counts.nbytes + self.actions.nbytes + self.lens.nbytes + self.final.nbytes
-                + self.values.nbytes + self.resigned.nbytes + self.full.nbytes)
+                + self.values.nbytes + self.resigned.nbytes + self.full.nbytes
+                + (self.target.nbytes if self.target is not None else 0))
+
+    def targets(self):
+        """-> (n_games, 81, 81) uint16: the policy target counts of every ply -- the pruned ones (target) of a run with
+        SP_FORCED_PLAYOUTS, the visit counts otherwise"""
+        return self.target if self.target is not None else self.counts
 
     def sample_mask(self, n=None):
         """-> bool (n, 81) over the first n games (None: all): the plies that are training samples, those played
@@ -480,12 +490,12 @@ class History:
         return (np.arange(81)[None, :] < self.lens[:n, None].astype(np.int64)) & (self.full[:n] != 0)
 
     def samples(self):
-        """-> (states (N,8) uint32, counts (N,81) uint16, z (N,) int8) over the sample plies (sample_mask), game-major order.
-        z follows self_play_cpp.py:95-99 verbatim (value of the FINAL position from its mover's view,
+        """-> (states (N,8) uint32, counts (N,81) uint16, z (N,) int8) over the sample plies (sample_mask), game-major order;
+        counts are the policy target counts (targets()).  z follows self_play_cpp.py:95-99 verbatim (value of the FINAL position from its mover's view,
         assigned to ply 0 and alternating), i.e. the reference's labelling including its sign quirk."""
         mask = self.sample_mask()
         st = self.states[mask]
-        cn = self.counts[mask]
+        cn = self.targets()[mask]
         z0 = np.where(self.final != 0, -1, 0).astype(np.int8)
         sign = np.where((np.arange(81) % 2) == 0, 1, -1).astype(np.int8)
         z = (z0[:, None] * sign[None, :])[mask]
@@ -509,6 +519,7 @@ class Engine:
         self.device = int(device)
         self.n_slots, self.max_sims, self.max_batch, self.max_games = n_slots, max_sims, max_batch, max_games
         self.weights_version = None
+        self.last_flags = 0         # the flags of the last self-play run: whether selfplay_fetch has targets to fetch
 
     def close(self):
         if getattr(self, "h", None):
@@ -582,6 +593,20 @@ class Engine:
         full search (in [0, 1]); see include/uttt_b200.h"""
         _check(self.lib.uttt_set_playout_cap(self.h, int(fast_sims), float(full_fraction)))
 
+    def set_forced_playouts(self, k=2.0):
+        """SP_FORCED_PLAYOUTS' k (finite, in (0, 100]): a root child with n >= 1 visits is forced while n < sqrt(k * p * N);
+        see include/uttt_b200.h"""
+        _check(self.lib.uttt_set_forced_playouts(self.h, float(k)))
+
+    def _fetch_target(self, n_games, hist):
+        """hist.target <- the policy targets of the last run if it had SP_FORCED_PLAYOUTS, else None"""
+        if not self.last_flags & SP_FORCED_PLAYOUTS:
+            hist.target = None
+            return
+        if hist.target is None:
+            hist.target = np.zeros(hist.counts.shape, np.uint16)
+        _check(self.lib.uttt_selfplay_fetch_target(self.h, n_games, _ptr(hist.target)))
+
     def mcts_search(self, roots, sims, batch, temperature, evaluator, flags=0):
         roots = np.ascontiguousarray(roots, dtype=np.uint32).reshape(-1, 8)
         n = roots.shape[0]
@@ -629,8 +654,10 @@ class Engine:
         _check(self.lib.uttt_selfplay_run(self.h, n_games, game0, sims, batch, seed, evaluator, flags,
                                           _ptr(hist.states), _ptr(hist.counts), _ptr(hist.actions), _ptr(hist.lens),
                                           _ptr(hist.final), _ptr(hist.stats)))
+        self.last_flags = int(flags)
         _check(self.lib.uttt_selfplay_fetch_values(self.h, n_games, _ptr(hist.values), _ptr(hist.resigned)))
         _check(self.lib.uttt_selfplay_fetch_full(self.h, n_games, _ptr(hist.full)))
+        self._fetch_target(n_games, hist)
         return hist
 
     def match(self, n_games, sims=50, batch=8, seed=0, evaluator=EVAL_NET_BF16, flags=0, game0=0, history=None):
@@ -649,6 +676,7 @@ class Engine:
         s = _stream(stream) if stream is not None else None
         _check(self.lib.uttt_selfplay_run_device(self.h, n_games, game0, sims, batch, seed, evaluator, flags,
                                                  _ptr(stats), s))
+        self.last_flags = int(flags)
         return stats
 
     def selfplay_fetch(self, n_games, history=None):
@@ -657,11 +685,12 @@ class Engine:
                                             _ptr(hist.lens), _ptr(hist.final)))
         _check(self.lib.uttt_selfplay_fetch_values(self.h, n_games, _ptr(hist.values), _ptr(hist.resigned)))
         _check(self.lib.uttt_selfplay_fetch_full(self.h, n_games, _ptr(hist.full)))
+        self._fetch_target(n_games, hist)
         return hist
 
     def selfplay_pack(self, n_games, out=None, stream=None):
         """history of the last selfplay_device() as one device buffer of SAMPLE_BYTES-byte samples, one per ply of
-        History.sample_mask -> (uint8 CUDA tensor sliced to the exact length, n_samples).  `out`: optional uint8 CUDA tensor to pack into (81 * n_games samples fit)"""
+        History.sample_mask, with the policy target counts of History.targets -> (uint8 CUDA tensor sliced to the exact length, n_samples).  `out`: optional uint8 CUDA tensor to pack into (81 * n_games samples fit)"""
         import torch
         cap = 81 * int(n_games)
         if out is None:

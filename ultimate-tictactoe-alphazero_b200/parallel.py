@@ -85,7 +85,7 @@ def pack_history_host(hist, n_local):
     raw = np.zeros((n, _eng.SAMPLE_BYTES), np.uint8)
     if n:
         raw[:, :32] = hist.states[:n_local][mask].view(np.uint8).reshape(n, 32)
-        raw[:, 32:194] = np.ascontiguousarray(hist.counts[:n_local][mask]).view(np.uint8).reshape(n, 162)
+        raw[:, 32:194] = np.ascontiguousarray(hist.targets()[:n_local][mask]).view(np.uint8).reshape(n, 162)
         ply = np.broadcast_to(np.arange(81)[None, :], mask.shape)[mask]
         z0 = np.where(hist.final[:n_local] != 0, -1, 0).astype(np.int8)
         z = np.broadcast_to(z0[:, None], mask.shape)[mask] * np.where(ply % 2 == 0, 1, -1).astype(np.int8)

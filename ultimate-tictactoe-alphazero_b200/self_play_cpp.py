@@ -9,6 +9,7 @@ stream (seeded from numpy's global RNG, so np.random.seed still makes a run repr
 of np.random.choice (self_play_cpp.py:86).  Labelling follows self_play_cpp.py:95-99 verbatim
 unless CORRECTED_LABELS is set (SURVEY.md B3).
 """
+import numbers
 import os
 import pickle
 from datetime import datetime
@@ -54,6 +55,9 @@ SP_FAST_SIMS = None           # an int in [1, PV_EVALUATE_COUNT]: playout cap ra
                               # SP_FAST_SIMS otherwise; only the full searches become training samples.  None: every move
                               # is a full search (the reference's games)
 SP_FULL_FRACTION = 0.25
+SP_FORCED_PLAYOUTS = None     # a float k in (0, 100] (KataGo uses 2): forced root playouts and policy target pruning
+                              # (KataGo; engine.SP_FORCED_PLAYOUTS) on every full search.  Needs SP_SEARCH_MODE =
+                              # "throughput".  The training policies are the pruned visit counts.  None: off
 
 _engine = None
 last_stats = {}
@@ -152,6 +156,20 @@ def _playout_cap_flags():
     return _eng.SP_PLAYOUT_CAP
 
 
+def _forced_playouts_flags():
+    """engine.SP_FORCED_PLAYOUTS if SP_FORCED_PLAYOUTS is set, else 0; ValueError if it is not a number in (0, 100] or
+    SP_SEARCH_MODE is not the throughput mode"""
+    if SP_FORCED_PLAYOUTS is None:
+        return 0
+    k = SP_FORCED_PLAYOUTS
+    if isinstance(k, bool) or not isinstance(k, numbers.Real) or not 0.0 < k <= 100.0:
+        raise ValueError("SP_FORCED_PLAYOUTS = %r: must be None or a number in (0, 100]" % (SP_FORCED_PLAYOUTS,))
+    if SP_SEARCH_MODE != "throughput":
+        raise ValueError("SP_FORCED_PLAYOUTS needs SP_SEARCH_MODE = \"throughput\" (the reference-exact root is uniform "
+                         "and never noised)")
+    return _eng.SP_FORCED_PLAYOUTS
+
+
 def _resign_stats(hist, n_games, seed, resign):
     """resigned games and the false positives of the played-out calibration games (the check games while resigning, all
     games otherwise); with SP_RESIGN_TARGET_FP, the threshold calibrated on them becomes SP_RESIGN_THRESHOLD"""
@@ -171,6 +189,7 @@ def _resign_stats(hist, n_games, seed, resign):
 def _run(model, n_games, progress=False):
     resign = _resign_flags()
     cap = _playout_cap_flags()
+    forced = _forced_playouts_flags()
     eng = _get_engine(n_games)
     model.eval()
     eng.upload_model(model)
@@ -188,6 +207,9 @@ def _run(model, n_games, progress=False):
     if cap:
         flags |= cap
         eng.set_playout_cap(int(SP_FAST_SIMS), SP_FULL_FRACTION)
+    if forced:
+        flags |= forced
+        eng.set_forced_playouts(float(SP_FORCED_PLAYOUTS))
     eng.set_selfplay_temperature(SP_TEMPERATURE)
     if SP_PROGRESS and progress:
         shown = [0]
@@ -206,6 +228,9 @@ def _run(model, n_games, progress=False):
                       rounds=int(hist.stats[3]), seed=seed)
     full = int(hist.sample_mask(n_games).sum())
     last_stats.update(full_plies=full, fast_plies=int(hist.stats[0]) - full)
+    mask = hist.sample_mask(n_games)
+    last_stats["pruned_visits"] = int(hist.counts[:n_games][mask].astype(np.int64).sum()
+                                      - hist.targets()[:n_games][mask].astype(np.int64).sum())
     for k in ("check_would_resign", "check_false_positives", "calibrated_threshold"):     # only what this cycle reports
         last_stats.pop(k, None)
     last_stats.update(_resign_stats(hist, n_games, seed, bool(resign)))
