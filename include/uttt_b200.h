@@ -245,7 +245,12 @@ int uttt_mcts_search(uttt_engine *e, const uint32_t *roots, int32_t n_roots, int
                      int32_t batch_size, float temperature, int32_t evaluator, int32_t flags,
                      float *scores /* n*81 */, int32_t *counts /* n*81 */, int32_t *n_scores /* n */);
 /* Dirichlet root noise of the throughput mode: p = (1-eps) p + eps * Dir(alpha); defaults alpha 0.3, eps 0.25
- * (AlphaZero's settings; the reference has no noise).  eps = 0 disables it. */
+ * (AlphaZero's settings; the reference has no noise).  eps = 0 disables it.  It is mixed into the evaluated root of every
+ * full search (every move without UTTT_SP_PLAYOUT_CAP) as p' = fma(1 - eps, p, eps * eta) in IEEE fp32: 1 - eps and
+ * eps * eta correctly rounded, then one fused multiply-add (one rounding); p is the root's renormalised prior, eta the draw
+ * of uttt_debug_root_noise for the root position under key (seed, game, ply): uttt_selfplay_run* keys it with its seed,
+ * the game and the ply, uttt_mcts_search with seed 0, game = root index in the call and ply 0 (like
+ * UTTT_SP_RANDOM_SYMMETRY), so a search's result does not depend on what the engine ran before. */
 int uttt_set_root_noise(uttt_engine *e, float alpha, float eps);
 
 /* SP_TEMPERATURE of the self-play loop (self_play_cpp.py:27,62 -> cpp/uttt_mcts.cpp:183-216); default 1 (the reference's
@@ -253,10 +258,18 @@ int uttt_set_root_noise(uttt_engine *e, float alpha, float eps);
  * moves are drawn from n^(1/T) / sum.  The history always holds the raw visit counts. */
 int uttt_set_selfplay_temperature(uttt_engine *e, float temperature);
 
-/* diagnostics: the root-noise sampler alone -- out[g][0..n_children) = the Dirichlet(alpha) draw that the throughput mode
- * mixes into the root priors of game game0 + g at ply 0 (Philox key (seed, 3), counter (game, ply, child, attempt)) */
+/* diagnostics: the root-noise sampler alone -- out[g][0..n_children) = the Dirichlet(alpha) draw of game game0 + g at ply 0
+ * for a root whose legal actions are 0 .. n_children - 1 (Philox key (seed, 3), counter (game, ply, child, attempt));
+ * the draw the throughput mode mixes into a game's first root when n_children = 81 */
 int uttt_debug_dirichlet(uint32_t seed, uint64_t game0, int64_t n, int32_t n_children, float alpha, float *out_dev,
                          void *stream);
+/* diagnostics: the root noise the throughput mode mixes into the root priors of position states_dev[i] under key (seed,
+ * games_dev[i], plies_dev[i]) -- eta_dev[i][a] (DEVICE pointers, n rows of 81): for each legal action id a a Gamma(alpha)
+ * sample g_a (Marsaglia-Tsang on the Philox stream above), eta_a = g_a / sum of the g (summed in the device's fixed
+ * order), or 1 / (number of legal actions) if that sum is not positive; 0 for an illegal action.  Exactly the draw of
+ * uttt_set_root_noise, from the same device function. */
+int uttt_debug_root_noise(uint32_t seed, float alpha, const uint32_t *states_dev, const uint64_t *games_dev,
+                          const int32_t *plies_dev, int64_t n, float *eta_dev, void *stream);
 
 /* step-wise form for a caller-side evaluator (python_bindings.cpp:11-47 `wrap_python_inference`) */
 int uttt_mcts_begin(uttt_engine *e, const uint32_t *roots, int32_t n_roots, int32_t evaluate_count,
@@ -367,10 +380,12 @@ int uttt_debug_batch_histogram(uttt_engine *e, int64_t *out64, int32_t reset);
  * [5] node-arena overflow flag, [6] finished trees (search), [1] finished games (self-play) */
 int uttt_debug_counters(uttt_engine *e, uint64_t *out8);
 
-/* diagnostics for the parity tests: while enabled, uttt_mcts_search and uttt_selfplay_run* (reference-exact and
- * UTTT_SP_PYSEARCH searches; a match records the rows of both networks' evaluator passes) record every evaluated leaf with the evaluator rows its tree is about to consume -- (tree, game index, ply), packed leaf
- * state, policy[81], value -- in evaluation order; the host synchronises after every round.  `enable` also clears the log.
- * uttt_debug_trace_read: *n_out = records; with cap >= *n_out the arrays meta[n][3], states[n][8], policy[n][81],
+/* diagnostics for the parity tests: while enabled, uttt_mcts_search and uttt_selfplay_run* (every search mode; a match
+ * records the rows of both networks' evaluator passes) record every evaluated leaf with the evaluator rows its tree is
+ * about to consume -- (tree, game index, ply, round), packed leaf state, policy[81], value -- in evaluation order (the
+ * throughput mode: a move's root, then its leaves in the order they were queued); `round` numbers the rounds of the call
+ * from 0.  The host synchronises after every round.  `enable` also clears the log.
+ * uttt_debug_trace_read: *n_out = records; with cap >= *n_out the arrays meta[n][4], states[n][8], policy[n][81],
  * value[n] (HOST pointers) are filled; cap = 0 only asks for the size.  With UTTT_SP_RANDOM_SYMMETRY a record holds the
  * untransformed leaf and its row mapped back into the leaf's own action ids.  Feeding these rows to the reference's
  * UTTT::pv_mcts_scores (cpp/uttt_mcts.cpp:84-196) must reproduce the engine's scores bit for bit. */

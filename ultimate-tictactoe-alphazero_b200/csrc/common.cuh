@@ -145,6 +145,8 @@ cudaError_t launch_hash_eval(const PackedState* states, const int32_t* count, in
 cudaError_t launch_scores(const int32_t* counts, const int32_t* n, int n_trees, float temperature,
                           float* scores, cudaStream_t s);
 cudaError_t launch_dirichlet(uint32_t seed, uint64_t game0, int64_t n, int n_children, float alpha, float* out, cudaStream_t s);
+cudaError_t launch_root_noise(uint32_t seed, float alpha, const PackedState* states, const uint64_t* games, const int32_t* plies,
+                              int64_t n, float* eta_out, cudaStream_t s);
 cudaError_t launch_boltzman(const float* xs, int n, float temperature, float* out, cudaStream_t s);
 
 // history as fixed-size samples (history_kernels.cu)

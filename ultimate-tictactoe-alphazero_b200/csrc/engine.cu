@@ -83,12 +83,12 @@ struct uttt_engine {
     double prof_ms[4];
     int64_t prof_launches[4];
     std::vector<void*> allocs;
-    // diagnostics (uttt_debug_trace): every evaluated leaf of the reference-exact search with the rows its tree is about to
-    // consume -- what tests/test_gpu_replay.py feeds to the CPU reference search
+    // diagnostics (uttt_debug_trace): every evaluated leaf with the rows its tree is about to consume -- what
+    // tests/test_gpu_replay.py and tests/test_gpu_throughput_oracle.py feed to the CPU searches
     uttt_progress_fn progress_cb;     // self-play: called when the number of finished games changed (per window of rounds)
     void* progress_user;
     bool trace_on;
-    struct TraceRec { int32_t tree, game_idx, ply; float value; uint32_t state[8]; float policy[81]; };
+    struct TraceRec { int32_t tree, game_idx, ply, round; float value; uint32_t state[8]; float policy[81]; };
     std::vector<TraceRec> trace;
 };
 
@@ -228,36 +228,61 @@ int run_evaluator(uttt_engine* e, const NetWeights& w, const EvalBufs& b, int ev
     return 0;
 }
 
-// uttt_debug_trace: after a round's evaluator pass over queue b, record (tree, game, ply, leaf state, policy row, value) of
-// every leaf queued there: the untransformed leaf and its row in the leaf's own action ids (UTTT_SP_RANDOM_SYMMETRY: entry
-// a = row entry sigma_g(a)), i.e. exactly what the tree consumes.  Synchronises the stream (diagnostics only).
-int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const int32_t* count, cudaStream_t s) {
+// uttt_debug_trace: after the evaluator pass of round `round` over queue b, record (tree, game, ply, round, leaf state,
+// policy row, value) of every leaf queued there: the untransformed leaf and its row in the leaf's own action ids
+// (UTTT_SP_RANDOM_SYMMETRY: entry a = row entry sigma_g(a)), i.e. exactly what the tree consumes.  The row's owner:
+// reference-exact mode, a PHASE_PENDING tree's row nn_row with leaf 0, evaluation n_eval - 1; throughput mode, a
+// PHASE_ROOT_PENDING tree's row nn_row with its root, evaluation 0, or a PHASE_PENDING tree's rows tp_aux[t][1][j] (j <
+// pend_k) with leaf j, evaluation n_eval - pend_k + j.  Synchronises the stream (diagnostics only).
+int trace_round(uttt_engine* e, const TreeParams& p, const EvalBufs& b, const int32_t* count, int64_t round, cudaStream_t s) {
     UTTT_CUDA_OK(cudaStreamSynchronize(s));
     int32_t n_rows = 0;
     UTTT_CUDA_OK(cudaMemcpy(&n_rows, count, sizeof(n_rows), cudaMemcpyDeviceToHost));
     if (n_rows == 0) return 0;
+    const bool tp = (p.flags & UTTT_SP_THROUGHPUT) != 0;
+    const size_t T = (size_t)p.n_trees;
     std::vector<int32_t> trees((size_t)n_rows);
     UTTT_CUDA_OK(cudaMemcpy(trees.data(), b.nn_tree, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
     std::vector<float> pol((size_t)n_rows * 81), val((size_t)n_rows);
-    std::vector<TreeCtl> ctl((size_t)p.n_trees);
-    std::vector<PackedState> leaf((size_t)p.n_trees);       // a tree's pending leaf is its leaf 0
-    UTTT_CUDA_OK(cudaMemcpy2D(leaf.data(), sizeof(PackedState), p.leaf_state, TP_MAX_LEAVES * sizeof(PackedState), sizeof(PackedState),
-                              leaf.size(), cudaMemcpyDeviceToHost));
+    std::vector<TreeCtl> ctl(T);
+    std::vector<PackedState> leaf(T * TP_MAX_LEAVES), root(T);
+    std::vector<int32_t> aux(T * 2 * TP_MAX_LEAVES);       // [t][0][j] path length, [t][1][j] row of pending leaf j
+    UTTT_CUDA_OK(cudaMemcpy(leaf.data(), p.leaf_state, leaf.size() * sizeof(PackedState), cudaMemcpyDeviceToHost));
+    UTTT_CUDA_OK(cudaMemcpy(root.data(), p.root, root.size() * sizeof(PackedState), cudaMemcpyDeviceToHost));
+    UTTT_CUDA_OK(cudaMemcpy(aux.data(), p.tp_aux, aux.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(pol.data(), b.policy, pol.size() * 4, cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(val.data(), b.value, val.size() * 4, cudaMemcpyDeviceToHost));
     UTTT_CUDA_OK(cudaMemcpy(ctl.data(), p.ctl, ctl.size() * sizeof(TreeCtl), cudaMemcpyDeviceToHost));
     for (int r = 0; r < n_rows; r++) {
         const int t = trees[r];
-        UTTT_CHECK(t >= 0 && t < p.n_trees && ctl[t].phase == PHASE_PENDING && ctl[t].nn_row == r,
-                   "trace: row %d does not belong to a pending tree", r);
+        UTTT_CHECK(t >= 0 && t < p.n_trees, "trace: row %d does not belong to a pending tree", r);
+        const TreeCtl& c = ctl[(size_t)t];
+        const PackedState* st = nullptr;
+        int j_eval = 0;
+        if (!tp && c.phase == PHASE_PENDING && c.nn_row == r) {
+            st = &leaf[(size_t)t * TP_MAX_LEAVES];
+            j_eval = c.n_eval - 1;
+        } else if (tp && c.phase == PHASE_ROOT_PENDING && c.nn_row == r) {
+            st = &root[(size_t)t];
+            j_eval = 0;
+        } else if (tp && c.phase == PHASE_PENDING) {
+            for (int j = 0; j < c.pend_k && j < TP_MAX_LEAVES; j++)
+                if (aux[((size_t)t * 2 + 1) * TP_MAX_LEAVES + j] == r) {
+                    st = &leaf[(size_t)t * TP_MAX_LEAVES + j];
+                    j_eval = c.n_eval - c.pend_k + j;
+                    break;
+                }
+        }
+        UTTT_CHECK(st != nullptr, "trace: row %d does not belong to a pending tree", r);
         uttt_engine::TraceRec rec;
         rec.tree = p.slot0 + t;
-        rec.game_idx = (p.mode == MODE_SELFPLAY) ? ctl[t].game_idx : p.slot0 + t;
-        rec.ply = (p.mode == MODE_SELFPLAY) ? ctl[t].ply : 0;
+        rec.game_idx = (p.mode == MODE_SELFPLAY) ? c.game_idx : p.slot0 + t;
+        rec.ply = (p.mode == MODE_SELFPLAY) ? c.ply : 0;
+        rec.round = (int32_t)round;
         rec.value = val[r];
-        memcpy(rec.state, &leaf[(size_t)t], 32);
+        memcpy(rec.state, st, 32);
         const int g = (p.flags & UTTT_SP_RANDOM_SYMMETRY)
-                          ? sym_draw(p.mode == MODE_SELFPLAY ? p.seed : 0u, ctl[t].game, (uint32_t)ctl[t].ply, (uint32_t)(ctl[t].n_eval - 1))
+                          ? sym_draw(p.mode == MODE_SELFPLAY ? p.seed : 0u, c.game, (uint32_t)c.ply, (uint32_t)j_eval)
                           : 0;
         for (int a = 0; a < 81; a++) rec.policy[a] = pol[(size_t)r * 81 + sym_action(a, g)];
         e->trace.push_back(rec);
@@ -553,7 +578,7 @@ int uttt_mcts_search(uttt_engine* e, const uint32_t* roots, int32_t n_roots, int
             t.parity = r & 1;
             UTTT_CUDA_OK(tp ? launch_tree_tp_round(t, e->stream) : launch_tree_round(t, e->stream));
             if (run_evaluator(e, e->w, bufs, evaluator, t.nn_count + t.parity, rows, e->stream, nullptr)) return 1;
-            if (e->trace_on && !tp && trace_round(e, t, bufs, t.nn_count + t.parity, e->stream)) return 1;
+            if (e->trace_on && trace_round(e, t, bufs, t.nn_count + t.parity, r, e->stream)) return 1;
         }
         UTTT_CUDA_OK(cudaMemcpyAsync(e->h_count, t.nn_count + ((r - 1) & 1), sizeof(int32_t), cudaMemcpyDeviceToHost,
                                      e->stream));
@@ -583,6 +608,14 @@ int uttt_set_root_noise(uttt_engine* e, float alpha, float eps) {
 int uttt_debug_dirichlet(uint32_t seed, uint64_t game0, int64_t n, int32_t n_children, float alpha, float* out_dev, void* stream) {
     UTTT_CHECK(n >= 0 && n_children >= 1 && n_children <= 81 && alpha > 0.0f && (n == 0 || out_dev), "bad argument");
     UTTT_CUDA_OK(launch_dirichlet(seed, game0, n, n_children, alpha, out_dev, (cudaStream_t)stream));
+    return 0;
+}
+
+int uttt_debug_root_noise(uint32_t seed, float alpha, const uint32_t* states_dev, const uint64_t* games_dev,
+                          const int32_t* plies_dev, int64_t n, float* eta_dev, void* stream) {
+    UTTT_CHECK(n >= 0 && alpha > 0.0f && (n == 0 || (states_dev && games_dev && plies_dev && eta_dev)), "bad argument");
+    UTTT_CUDA_OK(launch_root_noise(seed, alpha, reinterpret_cast<const PackedState*>(states_dev), games_dev, plies_dev, n, eta_dev,
+                                   (cudaStream_t)stream));
     return 0;
 }
 
@@ -728,9 +761,9 @@ int uttt_selfplay_run_device(uttt_engine* e, int64_t n_games, uint64_t game0, in
                                       ls[l], sampled ? ev + 1 + 3 * net : nullptr))
                         return 1;
                 }
-                for (int net = 0; net < n_nets && e->trace_on && !tp; net++)
+                for (int net = 0; net < n_nets && e->trace_on; net++)
                     if (trace_round(e, lane_tp[l], lane_bufs[l][net],
-                                    (net ? lane_tp[l].nn1_count : lane_tp[l].nn_count) + lane_tp[l].parity, ls[l]))
+                                    (net ? lane_tp[l].nn1_count : lane_tp[l].nn_count) + lane_tp[l].parity, r, ls[l]))
                         return 1;
             }
         }
@@ -945,7 +978,7 @@ int uttt_debug_trace_read(uttt_engine* e, int64_t cap, int64_t* n_out, int32_t* 
     UTTT_CHECK(cap >= n && meta && states && policy && value, "trace buffers too small (%lld records)", (long long)n);
     for (int64_t i = 0; i < n; i++) {
         const uttt_engine::TraceRec& r = e->trace[(size_t)i];
-        meta[3 * i] = r.tree; meta[3 * i + 1] = r.game_idx; meta[3 * i + 2] = r.ply;
+        meta[4 * i] = r.tree; meta[4 * i + 1] = r.game_idx; meta[4 * i + 2] = r.ply; meta[4 * i + 3] = r.round;
         memcpy(states + 8 * i, r.state, 32);
         memcpy(policy + 81 * i, r.policy, 81 * 4);
         value[i] = r.value;

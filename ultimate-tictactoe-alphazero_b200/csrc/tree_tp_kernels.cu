@@ -3,14 +3,15 @@
 // Not in the reference (SURVEY.md N1): the reference has no virtual loss, no root noise and never evaluates
 // the root.  This mode is what BASELINE.json's north_star asks for beyond the reference-exact mode:
 //   * the root is evaluated by the network; Dirichlet(alpha) noise from the counter-based Philox stream
-//     keyed by (seed, game, ply, child) is mixed into its priors:  p = (1-eps) p + eps * eta
+//     keyed by (seed, game, ply, child) -- (0, root index, 0, child) in a search call -- is mixed into its priors:
+//     p = (1-eps) p + eps * eta (root_noise, tp_expand)
 //   * up to m leaves per tree per round are collected with VIRTUAL LOSS (a per-node counter in the node word:
 //     selection sees n+vl visits and w+vl lost value, so nothing has to be undone in floating point)
 //   * every leaf is expanded once (no duplicated child lists), terminal values use the correct sign
 //   * one warp still owns one tree, so there are no atomics on tree data and the result depends only on
 //     (seed, m), never on scheduling.
-// With m = 1 and eps = 0 it is plain sequential PUCT with an evaluated root; oracle/uttt_oracle.c carries a
-// CPU cross-check of exactly that configuration (orc_az_search_hash) for the bit-exact GPU test.
+// With m = 1 and eps = 0 it is plain sequential PUCT with an evaluated root (oracle/uttt_oracle.c: orc_az_search_hash);
+// tests/tp_oracle.c restates the round for any m, with the noise taken from uttt_debug_root_noise.
 // The round takes its descent, prior normalisation, leaf queue and move decision from tree_common.cuh, like the
 // reference-exact round; its phases, expansion (tp_expand, with the root noise), backup (tp_backup, removing virtual
 // loss) and round loop are its own.  tree_begin_kernel (tree_kernels.cu) starts its trees in PHASE_ROOT.
@@ -42,22 +43,70 @@ __device__ float gamma_sample(float alpha, uint32_t seed, uint64_t game, uint32_
     return g;
 }
 
-// diagnostics (uttt_debug_dirichlet): the root-noise sampler on its own -- out[g][a] = Dirichlet(alpha) over n_children
-// children for game game0 + g at ply 0, exactly the draw tp_expand mixes into the root priors
+// The root noise eta of a position with legal mask lm (L legal actions) under key (seed, game, ply): a Gamma(alpha) sample
+// g_a = gamma_sample(alpha, seed, game, ply, a) for every legal action id a, their sum taken per lane (actions lane,
+// lane + 32, lane + 64 in that order) and then by a shuffle-xor butterfly (offsets 16, 8, 4, 2, 1), and eta_a = g_a / sum,
+// or 1 / L if the sum is not positive.  eta[q] is that of action lane + 32 q (0 where it is not legal).  tp_expand mixes it
+// into an evaluated root; uttt_debug_root_noise and uttt_debug_dirichlet export it, so that a CPU check can take the
+// draw from the device (it cannot restate logf / cosf / powf / rsqrtf bit for bit).
+__device__ void root_noise(float alpha, uint32_t seed, uint64_t game, uint32_t ply, const uint32_t lm[3], int L, int lane,
+                           float eta[3]) {
+    float gsum = 0.0f, g[3] = {0.f, 0.f, 0.f};
+    for (int q = 0, a = lane; a < 81; a += 32, q++)
+        if (legal_bit(lm, a)) { g[q] = gamma_sample(alpha, seed, game, ply, (uint32_t)a); gsum += g[q]; }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) gsum += __shfl_xor_sync(FULL, gsum, off);
+    const float uni = (L > 0) ? __fdiv_rn(1.0f, (float)L) : 0.0f;
+#pragma unroll
+    for (int q = 0; q < 3; q++) {
+        const int a = lane + 32 * q;
+        eta[q] = (a < 81 && legal_bit(lm, a)) ? (gsum > 0.0f ? __fdiv_rn(g[q], gsum) : uni) : 0.0f;
+    }
+}
+
+// diagnostics (uttt_debug_dirichlet): out[g][a] = eta_a of root_noise for game game0 + g at ply 0 of a root whose legal
+// actions are 0 .. n_children - 1 (a game's first root has all 81; tp_expand keys its draw by action id, so a root with
+// other legal actions gets other draws -- uttt_debug_root_noise gives those)
 __global__ void __launch_bounds__(128) dirichlet_kernel(uint32_t seed, uint64_t game0, int64_t n, int n_children, float alpha,
                                                         float* __restrict__ out) {
     const int64_t g = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (g >= n) return;
-    float v[3] = {0.f, 0.f, 0.f}, sum = 0.0f;
-    for (int q = 0, a = lane; a < n_children; a += 32, q++) { v[q] = gamma_sample(alpha, seed, game0 + (uint64_t)g, 0u, (uint32_t)a); sum += v[q]; }
+    uint32_t lm[3];
 #pragma unroll
-    for (int off = 16; off > 0; off >>= 1) sum += __shfl_xor_sync(FULL, sum, off);
-    for (int q = 0, a = lane; a < n_children; a += 32, q++) out[g * n_children + a] = sum > 0.0f ? v[q] / sum : 1.0f / (float)n_children;
+    for (int j = 0; j < 3; j++) {
+        const int k = n_children - 27 * j;
+        lm[j] = k >= 27 ? 0x7FFFFFFu : (k > 0 ? (1u << k) - 1u : 0u);
+    }
+    float eta[3];
+    root_noise(alpha, seed, game0 + (uint64_t)g, 0u, lm, n_children, lane, eta);
+    for (int q = 0, a = lane; a < n_children; a += 32, q++) out[g * n_children + a] = eta[q];
 }
 cudaError_t launch_dirichlet(uint32_t seed, uint64_t game0, int64_t n, int n_children, float alpha, float* out, cudaStream_t s) {
     if (n == 0) return cudaSuccess;
     dirichlet_kernel<<<(unsigned)((n + 3) / 4), 128, 0, s>>>(seed, game0, n, n_children, alpha, out);
+    return cudaGetLastError();
+}
+
+// diagnostics (uttt_debug_root_noise): eta[i][a] = root_noise of position states[i] under key (seed, games[i], plies[i]),
+// 0 for an illegal action
+__global__ void __launch_bounds__(128) root_noise_kernel(uint32_t seed, float alpha, const PackedState* __restrict__ states,
+                                                         const uint64_t* __restrict__ games, const int32_t* __restrict__ plies,
+                                                         int64_t n, float* __restrict__ eta_out) {
+    const int64_t i = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (i >= n) return;
+    const PackedState st = warp_load_state(states + i, lane);
+    uint32_t lm[3];
+    const int L = legal_mask(st, lm);
+    float eta[3];
+    root_noise(alpha, seed, games[i], (uint32_t)plies[i], lm, L, lane, eta);
+    for (int q = 0, a = lane; a < 81; a += 32, q++) eta_out[i * 81 + a] = eta[q];
+}
+cudaError_t launch_root_noise(uint32_t seed, float alpha, const PackedState* states, const uint64_t* games, const int32_t* plies,
+                              int64_t n, float* eta_out, cudaStream_t s) {
+    if (n == 0) return cudaSuccess;
+    root_noise_kernel<<<(unsigned)((n + 3) / 4), 128, 0, s>>>(seed, alpha, states, games, plies, n, eta_out);
     return cudaGetLastError();
 }
 
@@ -67,7 +116,9 @@ struct TpAux {                 // per tree, per pending leaf
 };
 
 // expansion of `leaf` from one policy row, evaluated under symmetry `sym`: masked, serially renormalised priors (the
-// reference-exact mode's arithmetic), optional Dirichlet mix for the root of a full search
+// reference-exact mode's arithmetic), and for the root of a full search with eps > 0 the root noise mixed in as
+// p = fma(1 - eps, p, eps * eta): eps * eta rounded, then one fused multiply-add (the form nvcc gave the plain expression).  The noise is keyed by
+// (seed, game, ply) in self-play and by (0, root index, 0) in a search call, like leaf_symmetry.
 __device__ void tp_expand(const TreeParams& P, const TreeView& T, TreeCtl& c, const PackedState& st, int leaf,
                           const float* pol, int sym, bool is_root, int lane) {
     uint32_t lm[3];
@@ -76,20 +127,15 @@ __device__ void tp_expand(const TreeParams& P, const TreeView& T, TreeCtl& c, co
     float pr[3];
     legal_priors(pol, sym, lm, L, lane, pr);
     const bool noise = is_root && P.dir_eps > 0.0f && full_search(P, c);      // a fast search gets none (KataGo)
-    float gsum = 0.0f, g[3] = {0.f, 0.f, 0.f};
-    if (noise) {
-        for (int q = 0, a = lane; a < 81; a += 32, q++)
-            if (legal_bit(lm, a)) { g[q] = gamma_sample(P.dir_alpha, P.seed, c.game, (uint32_t)c.ply, (uint32_t)a); gsum += g[q]; }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) gsum += __shfl_xor_sync(FULL, gsum, off);
-    }
-    const float uni = (L > 0) ? __fdiv_rn(1.0f, (float)L) : 0.0f;
+    float eta[3] = {0.f, 0.f, 0.f};
+    if (noise) root_noise(P.dir_alpha, P.mode == MODE_SELFPLAY ? P.seed : 0u, c.game, (uint32_t)c.ply, lm, L, lane, eta);
+    const float keep = 1.0f - P.dir_eps;
 #pragma unroll
     for (int q = 0; q < 3; q++) {
         const int a = lane + 32 * q;
         if (a < 81 && legal_bit(lm, a)) {
             float p = pr[q];
-            if (noise) p = (1.0f - P.dir_eps) * p + P.dir_eps * (gsum > 0.0f ? g[q] / gsum : uni);
+            if (noise) p = __fmaf_rn(keep, p, __fmul_rn(P.dir_eps, eta[q]));
             T.node[base + legal_rank(lm, a)] = make_node(a, p);
         }
     }

@@ -90,6 +90,7 @@ ABI = {
     "uttt_set_selfplay_temperature": ([_vp, C.c_float], C.c_int),
     "uttt_set_progress_callback": ([_vp, _vp, _vp], C.c_int),
     "uttt_debug_dirichlet": ([C.c_uint32, C.c_uint64, C.c_int64, C.c_int32, C.c_float, _vp, _vp], C.c_int),
+    "uttt_debug_root_noise": ([C.c_uint32, C.c_float, _vp, _vp, _vp, C.c_int64, _vp, _vp], C.c_int),
     "uttt_mcts_begin": ([_vp, _vp, C.c_int32, C.c_int32, C.c_int32], C.c_int),
     "uttt_mcts_advance": ([_vp, C.POINTER(C.c_int32)], C.c_int),
     "uttt_mcts_get_leaves": ([_vp, _vp, _vp, _vp], C.c_int),
@@ -225,6 +226,19 @@ def dirichlet_samples(seed, game0, n, n_children, alpha, device="cuda", stream=N
     import torch
     out = torch.empty((n, n_children), dtype=torch.float32, device=device)
     _check(load_library().uttt_debug_dirichlet(seed, game0, n, n_children, float(alpha), _ptr(out), _stream(stream)))
+    return out
+
+
+def root_noise(seed, alpha, states, games, plies, stream=None):
+    """(n, 81) float32 CUDA tensor: the root noise eta the throughput mode mixes into the root priors of packed states
+    (n, 8) under keys (seed, games[i], plies[i]), 0 for illegal actions (diagnostics; see uttt_debug_root_noise)"""
+    import torch
+    st = torch.as_tensor(np.ascontiguousarray(states, dtype=np.uint32).reshape(-1, 8).view(np.int32)).cuda()
+    n = st.shape[0]
+    g = torch.as_tensor(np.ascontiguousarray(games, dtype=np.int64).reshape(n)).cuda()
+    p = torch.as_tensor(np.ascontiguousarray(plies, dtype=np.int32).reshape(n)).cuda()
+    out = torch.empty((n, 81), dtype=torch.float32, device=st.device)
+    _check(load_library().uttt_debug_root_noise(seed, float(alpha), _ptr(st), _ptr(g), _ptr(p), n, _ptr(out), _stream(stream)))
     return out
 
 
@@ -721,15 +735,15 @@ class Engine:
                 "overflow": int(out[5]), "finished_trees": int(out[6])}
 
     def trace(self, enable=True):
-        """start (and clear) / stop recording every evaluated leaf of the reference-exact search (diagnostics, slow)"""
+        """start (and clear) / stop recording every evaluated leaf of the searches (diagnostics, slow)"""
         _check(self.lib.uttt_debug_trace(self.h, 1 if enable else 0))
 
     def trace_read(self):
-        """-> (meta (n,3) int32 [tree, game index, ply], states (n,8) uint32, policy (n,81) f32, value (n,) f32)"""
+        """-> (meta (n,4) int32 [tree, game index, ply, round], states (n,8) uint32, policy (n,81) f32, value (n,) f32)"""
         n = C.c_int64(0)
         _check(self.lib.uttt_debug_trace_read(self.h, 0, C.byref(n), None, None, None, None))
         n = n.value
-        meta = np.zeros((n, 3), np.int32)
+        meta = np.zeros((n, 4), np.int32)
         st = np.zeros((n, 8), np.uint32)
         pol = np.zeros((n, 81), np.float32)
         val = np.zeros((n,), np.float32)
